@@ -6,6 +6,7 @@ stages: interaction CSR + LightGCN normalisation -> L propagation layers -> per-
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload E|B|A|C|D] [--precision fp32|tc]
     python bench.py --impl reference ...        # the reference's CPU path on the host cores
+    python bench.py ... --dump-outputs DIR      # also write the last timed step's outputs as DIR/<name>.npy
 
 The default workload is config E (BASELINE.json configs[4], ogbn-products-shaped: the shape the target is quoted
 on; it fits one GPU) for EVERY N, so the N = 1, 2, 4, 8 lines are one strong-scaling experiment.
@@ -175,6 +176,54 @@ def spmm_bytes(nnz, rows, xrows, F, fused=True, model="min"):
     else:
         b = nnz * (8 + 4 * F) + (rows + 1) * 4 + rows * F * 4
     return b + (2 * rows * F * 4 if fused else 0)
+
+
+# ----------------------------------------------------------------------------------------
+# --dump-outputs DIR: what the last timed step computed, so that two builds can be compared output for output.
+# Outputs larger than the budget are written as a fixed sample of their rows (seed 0: the same rows every run).
+DUMP_ROWS = 16384          # rows written of a per-node feature matrix
+DUMP_GRAPH_ROWS = 128      # rows of a coarsened graph written as dense rows
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_rows(n, cap):
+    """Sorted indices of the rows written of an n-row output: all of them, or a seeded sample of cap rows."""
+    if n <= cap:
+        return np.arange(n)
+    return np.sort(np.random.RandomState(0).choice(n, cap, replace=False))
+
+
+def csr_rows_dense(A, rows):
+    """Rows `rows` of a device CSR as a dense float32 host array."""
+    import torch
+    rp = A.rowptr.cpu().numpy().astype(np.int64)
+    lo, hi = rp[rows], rp[rows + 1]
+    pos = torch.from_numpy(np.concatenate([np.arange(a, b) for a, b in zip(lo, hi)] + [np.zeros(0, np.int64)])).to(A.device)
+    out = np.zeros((len(rows), A.shape[1]), np.float32)
+    out[np.repeat(np.arange(len(rows)), hi - lo), A.colidx[pos].cpu().numpy()] = A.vals[pos].cpu().numpy()
+    return out
+
+
+def graph_outputs(name, A):
+    """A coarsened graph as <name> (DUMP_GRAPH_ROWS dense rows), <name>_rows (their indices) and <name>_row_nnz
+    (the non-zero count of every row)."""
+    rows = dump_rows(A.shape[0], DUMP_GRAPH_ROWS)
+    return {name: csr_rows_dense(A, rows), name + "_rows": rows, name + "_row_nnz": np.diff(A.rowptr.cpu().numpy())}
+
+
+def write_outputs(out_dir, arrays):
+    """<out_dir>/<name>.npy for every entry: float32 stays float32, everything else (labels, indices, scalars)
+    is written as float64."""
+    host = {}
+    for name, a in arrays.items():
+        a = np.asarray(a.cpu().numpy() if hasattr(a, "cpu") else a)
+        host[name] = a if a.dtype == np.float32 else a.astype(np.float64)
+    total = sum(a.nbytes for a in host.values())
+    if total > DUMP_MAX_BYTES:
+        raise RuntimeError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte budget")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 _THREAD_LIMIT = None
@@ -572,7 +621,7 @@ def run_ours(args, rank, world):
     nnz = A0.nnz
     del A0, tgt0
 
-    def step():
+    def step(keep=False):
         e = [ev() for _ in range(5)]
         e[0].record()
         An = build()
@@ -585,8 +634,11 @@ def run_ours(args, rank, world):
         _, adj_syn = gdr.graph_compress(km.labels_, An, [])
         e[4].record()
         # keep only scalars: holding km / adj_syn of every step alive fragments the caching allocator
-        # and forces cudaMalloc (a device-wide sync) inside later timed steps
-        return e, types.SimpleNamespace(n_iter_=km.n_iter_, inertia_=km.inertia_), int(adj_syn._nnz())
+        # and forces cudaMalloc (a device-wide sync) inside later timed steps; `keep` (the last timed step
+        # under --dump-outputs) also returns the outputs themselves
+        out = dict(prop=prop, target=target, labels=km.labels_, centers=km.cluster_centers_, inertia=km.inertia_,
+                   n_iter=km.n_iter_, adj_syn=gdr.CSR.from_torch_coo(adj_syn)) if keep else None
+        return e, types.SimpleNamespace(n_iter_=km.n_iter_, inertia_=km.inertia_), int(adj_syn._nnz()), out
 
     # W warm-up steps, continued until the GPU has been busy for >= 2 s: a fresh process starts
     # with the GPU in its idle power state and the first ~0.5 s of work runs at about half speed
@@ -602,15 +654,24 @@ def run_ours(args, rank, world):
     launches0 = gdr.launch_count()
     recs = []
     t_wall0 = time.perf_counter()
-    for _ in range(args.steps):
+    for s in range(args.steps):
         flush.fill_(1)          # L2 flush between timed iterations (untimed)
         torch.cuda.synchronize()
-        recs.append(step())
+        recs.append(step(keep=args.dump_outputs is not None and s == args.steps - 1))
         sampler.sample_now()    # clocks / throttle reasons while the GPU is still under load
     torch.cuda.synchronize()
     t_wall = time.perf_counter() - t_wall0
     launches = gdr.launch_count() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs is not None:
+        o = recs[-1][3]
+        rows = dump_rows(n, DUMP_ROWS)
+        rows_d = torch.from_numpy(rows).to(dev)
+        o.update(prop=o["prop"][rows_d], target=o["target"][rows_d], feature_rows=rows)
+        o.update(graph_outputs("adj_syn", o.pop("adj_syn")))
+        write_outputs(args.dump_outputs, o)
+        del o, rows_d
+        recs[-1] = recs[-1][:3]
 
     st = np.array([[r[0][i].elapsed_time(r[0][i + 1]) for i in range(4)] for r in recs])  # ms per stage
     step_ms = st.sum(axis=1)
@@ -830,25 +891,32 @@ def run_ours_bipartite(args, dev, w):
     def ev():
         return torch.cuda.Event(enable_timing=True)
 
-    def step():
+    def step(keep=False):
         e = [ev() for _ in range(5)]
         e[0].record()
         R = gdr.coo_to_csr(u_d, i_d, None, (nu, ni))                 # build_interaction_matrix: duplicates summed
         graph = gdr.BipartiteGraph(R.coo_indices(), R.vals, nu, ni)  # degrees + LightGCN edge norm, R and R^T
         e[1].record()
-        gdr.lightgcn_propagate(graph, u0, i0, L)
+        emb_out = gdr.lightgcn_propagate(graph, u0, i0, L)
         e[2].record()
         its, maps, inertia = 0, [], 0.0
-        for emb, K, c0 in ((u0, ku, C0[0]), (i0, ki, C0[1])):
+        out = dict(u_emb=emb_out[0], i_emb=emb_out[1]) if keep else None   # keep: the last timed step under --dump-outputs
+        del emb_out
+        for side, emb, K, c0 in (("u", u0, ku, C0[0]), ("i", i0, ki, C0[1])):
             km = gdr.KMeans(n_clusters=K, init=c0, n_init=1, max_iter=LLOYD_ITERS, tol=0, precision=args.precision)
             km.fit(gdr.standard_scale(emb))
             its += km.n_iter_
             inertia += km.inertia_
             maps.append(km.labels_)
+            if keep:
+                out.update({f"labels_{side}": km.labels_, f"centers_{side}": km.cluster_centers_,
+                            f"inertia_{side}": km.inertia_, f"n_iter_{side}": km.n_iter_})
         e[3].record()
         C = gdr.build_condensed_bipartite(u_d, i_d, maps[0], maps[1], ku, ki, device=dev, return_device=True)
         e[4].record()
-        return e, types.SimpleNamespace(n_iter_=its / 2.0, inertia_=inertia), int(C.nnz)
+        if keep:
+            out["condensed"] = C
+        return e, types.SimpleNamespace(n_iter_=its / 2.0, inertia_=inertia), int(C.nnz), out
 
     t_warm, n_warm = time.perf_counter(), 0
     while n_warm < args.warmup or (not args.profile and time.perf_counter() - t_warm < 2.0):
@@ -861,15 +929,25 @@ def run_ours_bipartite(args, dev, w):
     launches0 = gdr.launch_count()
     recs = []
     t_wall0 = time.perf_counter()
-    for _ in range(args.steps):
+    for s in range(args.steps):
         flush.fill_(1)
         torch.cuda.synchronize()
-        recs.append(step())
+        recs.append(step(keep=args.dump_outputs is not None and s == args.steps - 1))
         sampler.sample_now()
     torch.cuda.synchronize()
     t_wall = time.perf_counter() - t_wall0
     launches = gdr.launch_count() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs is not None:
+        o = recs[-1][3]
+        for side, n_side in (("u", nu), ("i", ni)):
+            rows = dump_rows(n_side, DUMP_ROWS)
+            o[f"{side}_emb"] = o[f"{side}_emb"][torch.from_numpy(rows).to(dev)]
+            o[f"{side}_emb_rows"] = rows
+        o.update(graph_outputs("condensed", o.pop("condensed")))
+        write_outputs(args.dump_outputs, o)
+        del o
+        recs[-1] = recs[-1][:3]
     st = np.array([[r[0][i].elapsed_time(r[0][i + 1]) for i in range(4)] for r in recs])
     n_iter = [r[1].n_iter_ for r in recs]
     iters_per_s = float(np.sum(n_iter) / (st[:, 2].sum() / 1e3))
@@ -1371,9 +1449,16 @@ def main():
     ap.add_argument("--no-extra-legs", action="store_true", help="skip the logit-space and skewed-graph legs")
     ap.add_argument("--no-parity", action="store_true", help="N > 1: skip the parity record")
     ap.add_argument("--profile", action="store_true", help="short run for ncu: no CPU baseline, minimal e2e leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="one GPU: write the outputs of the last timed step as DIR/<name>.npy (float32 / float64, "
+                         "large outputs as a fixed sample of rows, at most 64 MB in all)")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", 0))
     world = int(os.environ.get("WORLD_SIZE", 1))
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and (args.impl != "ours" or world > 1):
+        ap.error("--dump-outputs writes the outputs of the one-GPU path (--impl ours, one process)")
     if args.workload is None:
         # ONE workload for every N, so that the per-N lines are one strong-scaling experiment: config E
         # (configs[4], ogbn-products-shaped), the shape BASELINE.json's target is quoted on; it fits one GPU
