@@ -6,6 +6,7 @@ Four stages behind the reference's own call signatures (see SURVEY.md §8):
   3. k-means / WCSS         kmeans.py       (sklearn KMeans call sites)
   4. coarsened graph        coarsen.py      (graph_compress, build_condensed_bipartite)
   +  edge scoring / top-k   sparsify.py     (ER_estimator, attaw_ER_estimator, graph_sparse; SURVEY §8f item 1)
+  +  top-K evaluation       recsys.py       (recommend_topk, ranking_metrics: recall_at_k, distill_recsys.py:446-497)
 All arithmetic runs in libgdr_b200.so (hand-written sm_100a CUDA, C ABI in include/gdr.h).
 Importing this package loads that library and fails if it has not been built.
 """
@@ -32,6 +33,7 @@ from .sparsify import (  # noqa: E402
 )
 from .recsys import (  # noqa: E402
     BipartiteGraph, lightgcn_propagate, BipartitePropagate, RankformerGCNGraph, rankformer_gcn_forward,
+    recommend_topk, ranking_metrics,
 )
 from .io import (  # noqa: E402
     induced_subgraph, load_graphsaint, load_rankformer_dataset, read_ui_txt, save_condensed, load_condensed,
@@ -48,7 +50,7 @@ __all__ = [
     "build_condensed_bipartite", "condensed_csr_to_edge_index", "coarsen_edges", "label_counts",
     "ER_estimator", "attaw_ER_estimator", "graph_sparse", "er_lower", "cosine_reweight", "softmax_rows",
     "class_edge_weight", "topk_filter", "row_degree", "BipartiteGraph", "lightgcn_propagate", "BipartitePropagate", "RankformerGCNGraph",
-    "rankformer_gcn_forward", "induced_subgraph", "load_graphsaint", "load_rankformer_dataset", "read_ui_txt",
+    "rankformer_gcn_forward", "recommend_topk", "ranking_metrics", "induced_subgraph", "load_graphsaint", "load_rankformer_dataset", "read_ui_txt",
     "save_condensed", "load_condensed", "RecDataset", "GraphSaintData", "compute_svd_embeddings", "truncated_svd",
     "parallel",
 ]

@@ -135,6 +135,10 @@ _SIGNATURES = {
     "gdr_coarsen_ws_bytes": (i64, [i64, i64, i64]),
     "gdr_coarsen": (i32, [i64, vp, vp, i64, vp, vp, vp, vp, vp, i64, i64, i32, vp, vp, vp, vp, vp, vp, i64, vp]),
     "gdr_coarsen_scale": (i32, [i64, vp, vp, vp, vp, vp, vp, vp]),
+    "gdr_topk_scores_ws_bytes": (i64, [i64, i64, i64, i64]),
+    "gdr_topk_scores": (i32, [i64, i64, i64, i64, i64, vp, i64, vp, vp, i64, vp, vp, vp, i64, vp, i64, vp, vp, i64, vp]),
+    "gdr_ranking_metrics_ws_bytes": (i64, [i64, i32]),
+    "gdr_ranking_metrics": (i32, [i64, i64, i64, vp, i64, vp, vp, vp, i32, vp, vp, vp, vp, vp, i64, vp]),
 }
 
 ERROR_NAMES = {-1: "GDR_EINVAL", -2: "GDR_EWORKSPACE", -3: "GDR_ECUDA", -4: "GDR_ERANGE",

@@ -47,6 +47,7 @@ extern int g_coarsen_dense;       // graph.cu
 extern int g_rs_match;            // primitives.cu
 extern int g_rs_max_bits;         // primitives.cu
 extern int g_tc_ablate;
+extern int g_topk_path;           // topk.cu
 }  // namespace gdr
 extern "C" int g_sparsify_batch_cap;   // sparsify.cu
 namespace gdr {
@@ -442,6 +443,7 @@ int gdr_debug_set(const char* key, int value) {
   else if (!strcmp(key, "spmm_split")) gdr::g_spmm_split = value;
   else if (!strcmp(key, "lloyd_graph")) gdr::g_lloyd_graph = value;
   else if (!strcmp(key, "tc_screen")) gdr::g_tc_screen = value;
+  else if (!strcmp(key, "topk_path")) gdr::g_topk_path = value;
   else if (!strcmp(key, "coarsen_dense")) gdr::g_coarsen_dense = value;
   else if (!strcmp(key, "tc_ablate")) gdr::g_tc_ablate = value;
   else if (!strcmp(key, "tc_gate")) gdr::g_tc_gate = value;

@@ -72,11 +72,13 @@ int gdr_profile_collect(double* total_ms_host, int64_t* launches_host);
  * first-level kernel for tools/estep_probe.py / tools/mma_rate_probe.py; results are garbage while it is set);
  * "tc_gate" (first-level epilogue gate of the two-level screen: 0 off, 1 [default] on the running best, 2 also seeded
  * with the previous label's score; every setting produces the same labels);
- * "rs_match" (radix-sort ranking: 0 [default] per-bit warp ballots, 1 MATCH.ANY);
+ * "rs_match" (radix-sort ranking: 0 [default] per-bit warp ballots, 1 MATCH.ANY); "topk_path" (gdr_topk_scores: 1 exact
+ * SIMT path, 2 tensor-core screen);
  * value 0 / -1 = automatic. */
 int gdr_debug_set(const char* key, int value);
 /* Debug read-back (synchronises the device).  keys: "tc_level2_rows" = rows the last two-level
- * tensor-core screen (gdr_kmeans_assign_tc) handed to its 3xTF32 second level; -1 if none ran. */
+ * tensor-core screen (gdr_kmeans_assign_tc) handed to its 3xTF32 second level; -1 if none ran.
+ * "topk_overflow_rows" = rows the last tensor-core gdr_topk_scores finished on the exact path; -1 if none ran. */
 int gdr_debug_get(const char* key, int64_t* value_host);
 /* Tensor-pipe micro-probe: SM cycles for `iters` back-to-back tcgen05.mma of shape 128 x N x (32 bytes of K)
  * issued by one CTA (variant bit 0: kind::f16 instead of kind::tf32, bit 1: two accumulators, bit 2: no K advance). */
@@ -616,6 +618,45 @@ int64_t gdr_topk_filter_ws_bytes(int64_t n, int64_t nnz);
 int     gdr_topk_filter_csr(int64_t n, int64_t nnz, const int32_t* rowptr, const int32_t* colidx,
                             const float* vals, const float* weight, int64_t k, int32_t* rowptr_out,
                             int32_t* colidx_out, float* vals_out, int64_t* nnz_out_dev,
+                            void* ws, int64_t ws_bytes, gdr_stream_t stream);
+
+/* ---- evaluation: full-ranking top-K recommendation and Recall / Precision / NDCG@K -------------------------
+ * The protocol of the reference's recall_at_k (distill_recsys.py:446-497, called at :680 and :733) and of
+ * Rankformer's metrics (Rankformer/code/model.py:27-53): score every item for a user, drop the user's training
+ * items, keep the K best, count hits against the held-out items.  The definitions below are this library's.
+ *
+ * gdr_topk_scores: row r of the output is user u = rows[r] (rows == NULL: u = r, n_rows <= n_users).
+ *   s(u, j) = fp32 chain  acc = 0; for t < d: acc = fmaf(U[u, t], I[j, t], acc)   (-0 reported as +0)
+ *   items_out[r][0..k) = the k items j not in exclusion row u, by (score desc, j asc); a row with fewer eligible
+ *   items is padded with item -1 / score -inf.  scores_out holds the exact scores.  Every stored entry of the
+ *   exclusion CSR (n_users x n_items, both pointers NULL = none) excludes its item, whatever its value.
+ *   The score matrix is never held: either an exact SIMT product one row slab at a time (scratch of a few hundred MB)
+ *   or, for d <= 128 and k <= 256 on large products, a 3xTF32 tensor-core screen that keeps per user only the
+ *   candidates within twice a proven error band of a running top-k threshold and re-scores them exactly (rows whose
+ *   candidate list overflows finish on the exact path).  The choice is automatic (debug key "topk_path": 1 exact,
+ *   2 tensor core); the tensor-core path SYNCHRONISES the stream once (to size the exact finish of overflowed rows).
+ *   status_dev (device int32, zeroed by the caller): bit 0 = a non-finite value in a used row of U or in I,
+ *   bit 1 = a user id outside [0, n_users).  Outputs are deterministic, identical on both paths, and bit-identical to
+ *   the fmaf chain of a correctly rounding CPU fmaf (the test reference tests/topk_ref.c).
+ * gdr_ranking_metrics: items [n_rows][ldit] (from gdr_topk_scores), test CSR n_users x n_items with sorted
+ *   columns.  For every row with |test_u| > 0 and every K = ks_host[q] <= k:
+ *     hits = |{i < K : items[r][i] in test_u}|, recall = hits / |test_u|, precision = hits / K,
+ *     ndcg = sum_{i < K, hit} 1/log2(i+2) / sum_{i < min(K, |test_u|)} 1/log2(i+2).
+ *   sums_out_dev[q*3 + {0,1,2}] = fp64 sums of (recall, precision, ndcg) over the evaluated rows in ascending
+ *   row order; *n_eval_dev = rows with |test_u| > 0.  per_row_out (nullable) [n_ks][3][n_rows] f32, NaN for rows
+ *   without test items.  n_ks <= 32. */
+int64_t gdr_topk_scores_ws_bytes(int64_t n_rows, int64_t n_items, int64_t d, int64_t k);
+int     gdr_topk_scores(int64_t n_rows, int64_t n_users, int64_t n_items, int64_t d, int64_t k,
+                        const float* U, int64_t ldu, const int64_t* rows /*nullable*/,
+                        const float* I, int64_t ldi,
+                        const int32_t* ex_rowptr, const int32_t* ex_colidx /*both nullable*/,
+                        float* scores_out, int64_t lds, int32_t* items_out, int64_t ldit,
+                        int32_t* status_dev, void* ws, int64_t ws_bytes, gdr_stream_t stream);
+int64_t gdr_ranking_metrics_ws_bytes(int64_t n_rows, int n_ks);
+int     gdr_ranking_metrics(int64_t n_rows, int64_t n_users, int64_t k, const int32_t* items, int64_t ldit,
+                            const int64_t* rows /*nullable*/, const int32_t* test_rowptr,
+                            const int32_t* test_colidx, int n_ks, const int32_t* ks_host,
+                            double* sums_out_dev, int64_t* n_eval_dev, float* per_row_out /*nullable*/,
                             void* ws, int64_t ws_bytes, gdr_stream_t stream);
 
 #if defined(__GNUC__)
