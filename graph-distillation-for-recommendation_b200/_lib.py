@@ -38,6 +38,11 @@ _SIGNATURES = {
     "gdr_sym_normalize_dense_ws_bytes": (i64, [i64]),
     "gdr_sym_normalize_dense": (i32, [i64, vp, i64, vp, i64, vp, i64, vp]),
     "gdr_bipartite_normalize": (i32, [i64, i64, i64, vp, vp, vp, vp, vp, f32, vp, vp, vp, vp, vp]),
+    "gdr_csr_locate": (i32, [i64, i64, i64, vp, vp, i64, vp, vp, vp, vp, vp]),
+    "gdr_lightgcn_edge_grad": (i32, [i64, i64, i64, vp, vp, vp, i32, i64, vp, vp, vp, vp, i64, f32, vp, vp, vp]),
+    "gdr_bipartite_normalize_backward_ws_bytes": (i64, [i64, i64]),
+    "gdr_bipartite_normalize_backward": (i32, [i64, i64, i64, vp, vp, vp, vp, vp, vp, vp, f32, vp, vp, i64, vp, vp, vp,
+                                               i64, vp]),
     "gdr_bipartite_pow_normalize": (i32, [i64, i64, i64, vp, vp, vp, vp, vp, f32, f32, vp, vp, vp, vp, vp, vp]),
     "gdr_csr_transpose_ws_bytes": (i64, [i64, i64, i64]),
     "gdr_csr_transpose": (i32, [i64, i64, i64, vp, vp, vp, vp, vp, vp, i64, vp]),

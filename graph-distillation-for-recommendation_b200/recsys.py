@@ -5,8 +5,9 @@ Forward semantics of ``LightGCNCondensed.propagate`` (distill_recsys.py:319-353)
     norm  = w / (sqrt(deg_u[cu] + 1e-8) * sqrt(deg_i[ci] + 1e-8))
     L layers of  u <- sum norm * i ,  i <- sum norm * u  (simultaneous), output = layer mean.
 The two scatter-adds per layer become two CSR SpMMs (the cu x ci matrix and its
-transpose); autograd stays with torch (``BipartitePropagate`` implements the backward
-with the transposed SpMMs for the embedding inputs).
+transpose).  ``BipartitePropagate`` is differentiable w.r.t. the embeddings;
+``LightGCNPropagate`` also w.r.t. the edge weights (the condensed model's trained weights),
+on a graph that is built once and reweighted in place every step.
 """
 from __future__ import annotations
 
@@ -15,15 +16,19 @@ from typing import Dict, Sequence, Tuple
 import numpy as np
 import scipy.sparse as sp
 import torch
+from torch.autograd.function import once_differentiable
 
 from . import _lib
-from ._dev import need_cuda, new_padded, padded_rows, ptr, stream, to_device_i64, workspace
+from ._dev import need_cuda, new_padded, pad4, padded_rows, ptr, stream, to_device_i64, workspace
 from .graph import CSR, coo_to_csr
 from .propagation import spmm
 
 
 class BipartiteGraph:
-    """Device CSR of the cu x ci weight matrix, its transpose, and the normalised values."""
+    """Device CSR of the cu x ci weight matrix, its transpose, and the normalised values.
+
+    ``set_edge_weight`` replaces the weights (in the order of ``edge_index``) and renormalises in place, keeping the
+    sparsity pattern: the refinement loop builds the graph once and reweights it every step."""
 
     def __init__(self, edge_index: torch.Tensor, edge_weight: torch.Tensor, num_u: int, num_i: int,
                  eps: float = 1e-8):
@@ -37,34 +42,108 @@ class BipartiteGraph:
         self.deg_i = torch.empty(self.num_i, dtype=torch.float32, device=dev)
         norm = torch.empty(W.nnz, dtype=torch.float32, device=dev)
         t_norm = torch.empty(W.nnz, dtype=torch.float32, device=dev)
-        _lib.call("gdr_bipartite_normalize", self.num_u, self.num_i, W.nnz, ptr(W.rowptr), ptr(W.colidx),
-                  ptr(W.vals), ptr(WT.rowptr), ptr(t_perm), float(eps), ptr(norm), ptr(t_norm),
-                  ptr(self.deg_u), ptr(self.deg_i), stream())
         self.A = CSR(W.rowptr, W.colidx, norm, W.shape)        # users <- items
         self.AT = CSR(WT.rowptr, WT.colidx, t_norm, WT.shape)  # items <- users
         self.W = W
+        self.eps = float(eps)
+        self.t_perm = t_perm                # position in W of every entry of the transpose
+        self._edge_index = edge_index
+        self._edge_pos = None               # int32 [E]: CSR position of every input edge (first set_edge_weight)
+        self._edge_pos_i64 = None
+        self._normalize()
+
+    def _normalize(self) -> None:
+        """deg_u, deg_i, A.vals and AT.vals from W.vals (gdr_bipartite_normalize), into the existing buffers."""
+        W = self.W
+        _lib.call("gdr_bipartite_normalize", self.num_u, self.num_i, W.nnz, ptr(W.rowptr), ptr(W.colidx),
+                  ptr(W.vals), ptr(self.AT.rowptr), ptr(self.t_perm), self.eps, ptr(self.A.vals), ptr(self.AT.vals),
+                  ptr(self.deg_u), ptr(self.deg_i), stream())
+
+    @property
+    def num_edges(self) -> int:
+        return int(self._edge_index.shape[1])
+
+    def edge_positions(self) -> torch.Tensor:
+        """int32 [E]: position in the CSR of every edge of ``edge_index`` (computed once, on first use).
+        Raises ValueError when ``edge_index`` repeats a (u, i) pair: the CSR then holds their sum, and a weight per
+        input edge has no entry of its own."""
+        if self._edge_pos is None:
+            E, W = self.num_edges, self.W
+            if W.nnz != E:
+                raise ValueError(f"edge_index repeats a (u, i) pair ({E} edges, {W.nnz} distinct pairs): per-edge "
+                                 "weights need unique pairs")
+            dev = W.device
+            pos = torch.empty(E, dtype=torch.int32, device=dev)
+            status = torch.zeros(1, dtype=torch.int32, device=dev)
+            row = to_device_i64(self._edge_index[0], dev)
+            col = to_device_i64(self._edge_index[1], dev)
+            _lib.call("gdr_csr_locate", self.num_u, self.num_i, W.nnz, ptr(W.rowptr), ptr(W.colidx), E, ptr(row),
+                      ptr(col), ptr(pos), ptr(status), stream())
+            if int(status.item()):
+                raise RuntimeError("edge_index holds a pair the graph does not store (was it modified in place?)")
+            self._edge_pos, self._edge_pos_i64 = pos, pos.long()
+        return self._edge_pos
+
+    def set_edge_weight(self, edge_weight: torch.Tensor) -> None:
+        """New edge weights, f32 [E] in the order of the ``edge_index`` the graph was built from: scattered to CSR
+        order, then deg_u, deg_i, A.vals and AT.vals are recomputed in place (no sort, no transpose).  The result is
+        bit-identical to a new ``BipartiteGraph(edge_index, edge_weight, ...)``.  No autograd (see
+        ``LightGCNPropagate``)."""
+        need_cuda(edge_weight, "edge_weight")
+        w = edge_weight.detach().to(torch.float32).reshape(-1)
+        if w.shape[0] != self.num_edges:
+            raise ValueError(f"edge_weight has {w.shape[0]} entries, the graph {self.num_edges} edges")
+        self.edge_positions()
+        if self.num_edges:
+            self.W.vals.index_copy_(0, self._edge_pos_i64, w)
+        self._normalize()
+
+
+def _layer_loop(A: CSR, AT: CSR, u0: torch.Tensor, i0: torch.Tensor, num_layers: int, keep: bool = False):
+    """Layer loop of distill_recsys.py:337-353 on the normalised matrices A (users <- items) and AT.
+
+    Returns (u_out, i_out, Xu, Xi).  With ``keep`` (and L > 0), Xu / Xi are the layers X_0 .. X_{L-1} stacked as
+    [L, n, pad4(d)] f32 (zero padding columns), written by the SpMMs themselves; else None.  Keeping them changes
+    no SpMM call: the outputs are the same bits either way."""
+    u = padded_rows(u0.detach().to(torch.float32))
+    it = padded_rows(i0.detach().to(torch.float32))
+    n_u, n_i = A.shape
+    d = u.shape[1]
+    dev = u.device
+    L = int(num_layers)
+    Xu = Xi = None
+    if keep and L > 0:
+        alloc = torch.empty if pad4(d) == d else torch.zeros
+        Xu = alloc((L, n_u, pad4(d)), dtype=torch.float32, device=dev)
+        Xi = alloc((L, n_i, pad4(d)), dtype=torch.float32, device=dev)
+        Xu[0, :, :d].copy_(u)
+        Xi[0, :, :d].copy_(it)
+        u, it = Xu[0, :, :d], Xi[0, :, :d]
+    u_acc = new_padded(n_u, d, dev)
+    i_acc = new_padded(n_i, d, dev)
+    u_acc.copy_(u)
+    i_acc.copy_(it)
+    for l in range(L):
+        keep_next = Xu is not None and l + 1 < L
+        if A.nnz == 0:   # no edges: every propagated layer is zero (the SpMM entry point takes no empty CSR)
+            u_next = Xu[l + 1, :, :d].zero_() if keep_next else new_padded(n_u, d, dev, zero=True)
+            i_next = Xi[l + 1, :, :d].zero_() if keep_next else new_padded(n_i, d, dev, zero=True)
+        else:
+            u_next = spmm(A, it, out=Xu[l + 1, :, :d] if keep_next else None, accumulate_into=u_acc, beta=1.0)
+            i_next = spmm(AT, u, out=Xi[l + 1, :, :d] if keep_next else None, accumulate_into=i_acc, beta=1.0)
+        u, it = u_next, i_next
+    inv = 1.0 / float(L + 1)
+    u_out = new_padded(n_u, d, dev)
+    i_out = new_padded(n_i, d, dev)
+    _lib.call("gdr_scale_rows", n_u, d, inv, ptr(u_acc), u_acc.stride(0), ptr(u_out), u_out.stride(0), stream())
+    _lib.call("gdr_scale_rows", n_i, d, inv, ptr(i_acc), i_acc.stride(0), ptr(i_out), i_out.stride(0), stream())
+    return u_out, i_out, Xu, Xi
 
 
 def lightgcn_propagate(graph: BipartiteGraph, u0: torch.Tensor, i0: torch.Tensor,
                        num_layers: int) -> Tuple[torch.Tensor, torch.Tensor]:
     """Forward of distill_recsys.py:337-353 (no autograd)."""
-    u = padded_rows(u0.detach().to(torch.float32))
-    it = padded_rows(i0.detach().to(torch.float32))
-    d = u.shape[1]
-    dev = u.device
-    u_acc = new_padded(graph.num_u, d, dev)
-    i_acc = new_padded(graph.num_i, d, dev)
-    u_acc.copy_(u)
-    i_acc.copy_(it)
-    for _ in range(int(num_layers)):
-        u_next = spmm(graph.A, it, accumulate_into=u_acc, beta=1.0)
-        i_next = spmm(graph.AT, u, accumulate_into=i_acc, beta=1.0)
-        u, it = u_next, i_next
-    inv = 1.0 / float(num_layers + 1)
-    u_out = new_padded(graph.num_u, d, dev)
-    i_out = new_padded(graph.num_i, d, dev)
-    _lib.call("gdr_scale_rows", graph.num_u, d, inv, ptr(u_acc), u_acc.stride(0), ptr(u_out), u_out.stride(0), stream())
-    _lib.call("gdr_scale_rows", graph.num_i, d, inv, ptr(i_acc), i_acc.stride(0), ptr(i_out), i_out.stride(0), stream())
+    u_out, i_out, _, _ = _layer_loop(graph.A, graph.AT, u0, i0, num_layers)
     return u_out, i_out
 
 
@@ -117,6 +196,64 @@ class BipartitePropagate(torch.autograd.Function):
         # the same alternating propagation applied to (gu, gi) because [[0, A], [A^T, 0]] is symmetric.
         du, di = lightgcn_propagate(ctx.graph, gu.contiguous(), gi.contiguous(), ctx.num_layers)
         return du, di, None, None
+
+
+class LightGCNPropagate(torch.autograd.Function):
+    """``u_out, i_out = LightGCNPropagate.apply(u0, i0, edge_weight, graph, num_layers)``: the condensed model's
+    propagation (distill_recsys.py:319-353) differentiable w.r.t. the embeddings AND the edge weights.
+
+    ``edge_weight`` is f32 [E] in the order of the graph's ``edge_index`` (``model.edge_weight()``); the forward
+    reweights ``graph`` in place (``set_edge_weight``) and runs the layer loop of ``lightgcn_propagate`` (same bits).
+    It keeps its own copy of the normalised values and degrees, so reweighting the graph again before ``backward``
+    (a second forward, say) does not change this call's gradients.  Backward: the adjoint propagation gives
+    d u0 / d i0 (the same calls as ``BipartitePropagate``), then gdr_lightgcn_edge_grad and
+    gdr_bipartite_normalize_backward give d edge_weight.  Deterministic; no double backward."""
+
+    @staticmethod
+    def forward(ctx, u0, i0, edge_weight, graph: BipartiteGraph, num_layers: int):
+        L = int(num_layers)
+        if L < 0:
+            raise ValueError("num_layers must be >= 0")
+        if u0.dim() != 2 or i0.dim() != 2 or u0.shape[1] != i0.shape[1]:
+            raise ValueError("u0 [num_u, d] and i0 [num_i, d] need the same d")
+        if u0.shape[0] != graph.num_u or i0.shape[0] != graph.num_i:
+            raise ValueError(f"u0 / i0 have {u0.shape[0]} / {i0.shape[0]} rows, the graph {graph.num_u} / {graph.num_i}")
+        graph.set_edge_weight(edge_weight)
+        A, AT = graph.A, graph.AT
+        ctx.A = CSR(A.rowptr, A.colidx, A.vals.clone(), A.shape, _plan=A.spmm_plan())
+        ctx.AT = CSR(AT.rowptr, AT.colidx, AT.vals.clone(), AT.shape, _plan=AT.spmm_plan())
+        ctx.deg_u, ctx.deg_i = graph.deg_u.clone(), graph.deg_i.clone()
+        ctx.graph, ctx.num_layers, ctx.w_dtype = graph, L, edge_weight.dtype
+        u_out, i_out, ctx.Xu, ctx.Xi = _layer_loop(ctx.A, ctx.AT, u0, i0, L, keep=ctx.needs_input_grad[2])
+        return u_out, i_out
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, gu, gi):
+        need_w = ctx.needs_input_grad[2]
+        du, di, Yu, Yi = _layer_loop(ctx.A, ctx.AT, gu.contiguous(), gi.contiguous(), ctx.num_layers, keep=need_w)
+        dw = _edge_weight_grad(ctx, Yu, Yi, du.shape[1]).to(ctx.w_dtype) if need_w else None
+        ctx.Xu = ctx.Xi = None
+        return du, di, dw, None, None
+
+
+def _edge_weight_grad(ctx, Yu, Yi, d: int) -> torch.Tensor:
+    """dL/dw [E] in input edge order from the kept forward layers (ctx.Xu, ctx.Xi) and adjoint layers (Yu, Yi)."""
+    g, A, AT, L = ctx.graph, ctx.A, ctx.AT, ctx.num_layers
+    E, nnz = g.num_edges, A.nnz
+    dev = A.device
+    dw = torch.empty(E, dtype=torch.float32, device=dev)
+    if E == 0:
+        return dw
+    G = torch.empty(nnz, dtype=torch.float32, device=dev)
+    S_u = torch.empty(g.num_u, dtype=torch.float64, device=dev)
+    _lib.call("gdr_lightgcn_edge_grad", g.num_u, g.num_i, nnz, ptr(A.rowptr), ptr(A.colidx), ptr(A.vals), L, d,
+              ptr(ctx.Xu), ptr(ctx.Xi), ptr(Yu), ptr(Yi), pad4(d), 1.0 / float(L + 1), ptr(G), ptr(S_u), stream())
+    ws = workspace(_lib.query("gdr_bipartite_normalize_backward_ws_bytes", g.num_i, nnz), dev)
+    _lib.call("gdr_bipartite_normalize_backward", g.num_u, g.num_i, nnz, ptr(A.rowptr), ptr(A.colidx),
+              ptr(AT.rowptr), ptr(g.t_perm), ptr(A.vals), ptr(ctx.deg_u), ptr(ctx.deg_i), g.eps, ptr(G), ptr(S_u), E,
+              ptr(g.edge_positions()), ptr(dw), ptr(ws), ws.numel(), stream())
+    return dw
 
 
 # ---------------------------------------------------------------------------------------------------------------

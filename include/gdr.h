@@ -161,6 +161,38 @@ int gdr_bipartite_normalize(int64_t n_u, int64_t n_i, int64_t nnz,
                             float eps, float* norm_out, float* t_norm_out,
                             float* deg_u, float* deg_i, gdr_stream_t stream);
 
+/* Backward of the bipartite LightGCN propagation w.r.t. the edge weights (the condensed model's trained edge
+ * weights, distill_recsys.py:319-353 under the refinement loop :684-733).  Notation: CSR entry e = (a, b) of the
+ * n_u x n_i weight matrix, A_ab = norm_e, M = [[0, A], [A^T, 0]], X_l = M^l [u0; i0], out = c sum_{l<=L} X_l,
+ * Y_m = M^m dL/dout (the adjoint propagation: gdr_spmm_prop on A / A^T), c = 1/(L+1).
+ *
+ * gdr_csr_locate: edge_pos_out[k] = position of the pair (row[k], col[k]) in the CSR (columns sorted inside a row),
+ *   -1 when missing.  status_dev (device int32, zeroed by the caller): bit 0 = a pair outside the matrix,
+ *   bit 1 = a pair not stored.  With E == nnz and status 0, edge_pos is a permutation of [0, nnz).
+ * gdr_lightgcn_edge_grad: from the stacked layers Xu [L][n_u][ld], Xi [L][n_i][ld] (X_0 .. X_{L-1}) and Yu, Yi
+ *   (Y_0 .. Y_{L-1}), all 16-byte aligned with ld a multiple of 4:
+ *     G_out[e]   = dL/dA_ab = c sum_{j<L} ( Xi_j[b] . PY_{L-1-j}[a] + Yi_j[b] . PX_{L-1-j}[a] ),
+ *                  PY_k = sum_{m<=k} Yu_m, PX_k = sum_{m<=k} Xu_m   (fp32)
+ *     S_u_out[a] = sum_{e in row a} G_e norm_e                                  (fp64)
+ *   L == 0 or d == 0 gives zeros.  Deterministic: one fixed summation order, no float atomics.
+ * gdr_bipartite_normalize_backward: with the forward's norm and fp32 degrees (gdr_bipartite_normalize),
+ *     S_i[b] = sum over the transposed row b, ascending, of G_e norm_e                 (fp64)
+ *     dw_out[k] = G_e / (sqrt(du[a]+eps) sqrt(di[b]+eps)) - S_u[a] / (2 (du[a]+eps)) - S_i[b] / (2 (di[b]+eps)),
+ *   e = edge_pos[k], evaluated in fp64 and rounded once; dw_out is in input edge order. */
+int     gdr_csr_locate(int64_t n_rows, int64_t n_cols, int64_t nnz, const int32_t* rowptr, const int32_t* colidx,
+                       int64_t E, const int64_t* row, const int64_t* col, int32_t* edge_pos_out,
+                       int32_t* status_dev, gdr_stream_t stream);
+int     gdr_lightgcn_edge_grad(int64_t n_u, int64_t n_i, int64_t nnz, const int32_t* rowptr, const int32_t* colidx,
+                               const float* norm, int num_layers, int64_t d, const float* Xu, const float* Xi,
+                               const float* Yu, const float* Yi, int64_t ld, float c, float* G_out,
+                               double* S_u_out, gdr_stream_t stream);
+int64_t gdr_bipartite_normalize_backward_ws_bytes(int64_t n_i, int64_t nnz);
+int     gdr_bipartite_normalize_backward(int64_t n_u, int64_t n_i, int64_t nnz, const int32_t* rowptr,
+                                         const int32_t* colidx, const int32_t* t_rowptr, const int32_t* t_perm,
+                                         const float* norm, const float* deg_u, const float* deg_i, float eps,
+                                         const float* G, const double* S_u, int64_t E, const int32_t* edge_pos,
+                                         float* dw_out, void* ws, int64_t ws_bytes, gdr_stream_t stream);
+
 /* Rankformer GCN edge weights (Rankformer/code/rec.py:118-124, the teacher's propagation the
  * reference's LightGCN mirrors): du / di = interaction counts clamped to >= 1,
  *   out_e = w_e / du^a / di^b   (users <- items),   t_out = w_e / du^b / di^a (items <- users,
