@@ -144,6 +144,9 @@ _SIGNATURES = {
     "gdr_topk_scores": (i32, [i64, i64, i64, i64, i64, vp, i64, vp, vp, i64, vp, vp, vp, i64, vp, i64, vp, vp, i64, vp]),
     "gdr_ranking_metrics_ws_bytes": (i64, [i64, i32]),
     "gdr_ranking_metrics": (i32, [i64, i64, i64, vp, i64, vp, vp, vp, i32, vp, vp, vp, vp, vp, i64, vp]),
+    "gdr_bpr_sample": (i32, [i64, i64, vp, vp, i64, vp, C.c_uint64, i64, i64, vp, vp, vp, vp]),
+    "gdr_bpr_loss_ws_bytes": (i64, [i64, i64, i64]),
+    "gdr_bpr_loss": (i32, [i64, i64, i64, i64, vp, i64, vp, i64, vp, vp, vp, vp, vp, i64, vp, i64, vp, vp, i64, vp]),
 }
 
 ERROR_NAMES = {-1: "GDR_EINVAL", -2: "GDR_EWORKSPACE", -3: "GDR_ECUDA", -4: "GDR_ERANGE",

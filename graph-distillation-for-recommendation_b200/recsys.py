@@ -7,7 +7,8 @@ Forward semantics of ``LightGCNCondensed.propagate`` (distill_recsys.py:319-353)
 The two scatter-adds per layer become two CSR SpMMs (the cu x ci matrix and its
 transpose).  ``BipartitePropagate`` is differentiable w.r.t. the embeddings;
 ``LightGCNPropagate`` also w.r.t. the edge weights (the condensed model's trained weights),
-on a graph that is built once and reweighted in place every step.
+on a graph that is built once and reweighted in place every step.  ``BPRSampler`` and ``bpr_loss`` are the rest of a
+refinement step (triplet sampling, BPR loss and its gradient) on the device.
 """
 from __future__ import annotations
 
@@ -19,7 +20,7 @@ import torch
 from torch.autograd.function import once_differentiable
 
 from . import _lib
-from ._dev import need_cuda, new_padded, pad4, padded_rows, ptr, stream, to_device_i64, workspace
+from ._dev import device_of, need_cuda, new_padded, pad4, padded_rows, ptr, stream, to_device_i64, workspace
 from .graph import CSR, coo_to_csr
 from .propagation import spmm
 
@@ -373,3 +374,138 @@ def ranking_metrics(items: torch.Tensor, test, ks: Sequence[int] = (20,), rows=N
             out[f"{name}@{K}"] = float(s[3 * q + m] / ne) if ne else float("nan")
     out.update(n_eval=ne, n_skipped=n_rows - ne)
     return out
+
+
+# ---------------------------------------------------------------------------------------------------------------
+# BPR training step (distill_recsys.py:684-733): device triplet sampler and the fused BPR loss + gradient
+# ---------------------------------------------------------------------------------------------------------------
+_BPR_MAX_BATCH = (1 << 31) // 3
+
+
+class BPRSampler:
+    """(user, positive, negative) triplets drawn on the device (``gdr_bpr_sample``).
+
+    ``R`` is the n_users x n_items interaction matrix (``gdr.CSR`` with sorted, unique columns per row, a torch sparse
+    tensor or a scipy sparse matrix; values are ignored: a positive is a distinct stored item), e.g.
+    ``BipartiteGraph.W``, the condensed CSR of ``build_condensed_bipartite(..., return_device=True)`` or the full
+    training CSR.  A user is eligible when 0 < deg(u) < n_items.  Triplet b of a step: user uniform over the eligible
+    users, positive uniform over the user's row, negative uniform over the items outside it (the distribution of
+    LightGCN's rejection sampler, drawn without rejection).  Random numbers: Philox4x32-10 keyed by ``seed`` with
+    counter (b, step, j, 0), so a step is a pure function of (R, seed, step): identical on every run and every GPU,
+    and any step can be regenerated on its own (``tests/bpr_ref.py`` mirrors it bit for bit).
+
+    The constructor checks the columns and builds the eligible list once (a few synchronisations, at construction only); raises ValueError
+    when no user is eligible.  ``sample`` does not synchronise."""
+
+    def __init__(self, R, seed: int):
+        if isinstance(R, CSR):
+            dev = R.device
+        elif isinstance(R, torch.Tensor) and R.is_cuda:
+            dev = R.device
+        else:
+            dev = device_of(None)
+        self.R = _as_csr(R, tuple(R.shape), "R", dev)
+        self.seed = int(seed)
+        if not 0 <= self.seed < 1 << 64:
+            raise ValueError("seed must lie in [0, 2^64)")
+        n_users, n_items = (int(x) for x in self.R.shape)
+        rowptr, colidx = self.R.rowptr, self.R.colidx
+        deg = (rowptr[1:] - rowptr[:-1]).to(torch.int64)
+        if self.R.nnz:
+            row = torch.repeat_interleave(torch.arange(n_users, device=dev), deg)
+            c = colidx.to(torch.int64)
+            bad = bool(((c < 0) | (c >= n_items)).any())
+            if self.R.nnz > 1:
+                bad |= bool(((c[1:] <= c[:-1]) & (row[1:] == row[:-1])).any())
+            if bad:
+                raise ValueError("R needs column indices in [0, n_items), sorted and unique inside each row")
+        self.eligible = torch.nonzero((deg > 0) & (deg < n_items)).reshape(-1).to(torch.int32)
+        self.n_eligible = int(self.eligible.shape[0])
+        if self.n_eligible == 0:
+            raise ValueError("no user is eligible for BPR sampling (every user has no item or every item)")
+
+    def sample(self, batch_size: int, step: int) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+        """``(users, pos, neg)``: three int64 device tensors of length ``batch_size`` (in [1, 2^31/3]) for ``step``
+        (in [0, 2^32))."""
+        B, step = int(batch_size), int(step)
+        if not 1 <= B <= _BPR_MAX_BATCH:
+            raise ValueError(f"batch_size={B} must lie in [1, {_BPR_MAX_BATCH}]")
+        if not 0 <= step < 1 << 32:
+            raise ValueError(f"step={step} must lie in [0, 2^32)")
+        R, dev = self.R, self.R.device
+        out = torch.empty((3, B), dtype=torch.int64, device=dev)
+        _lib.call("gdr_bpr_sample", R.shape[0], R.shape[1], ptr(R.rowptr), ptr(R.colidx), self.n_eligible,
+                  ptr(self.eligible), self.seed, step, B, ptr(out[0]), ptr(out[1]), ptr(out[2]), stream())
+        return out[0], out[1], out[2]
+
+
+def _bpr_operand(x: torch.Tensor, name: str) -> torch.Tensor:
+    need_cuda(x, name)
+    if x.dim() != 2:
+        raise ValueError(f"{name} must be [rows, d]")
+    return padded_rows(x.detach().to(torch.float32))   # LightGCNPropagate's padded outputs pass without a copy
+
+
+def _bpr_forward(U, I, users, pos, neg, want_gU: bool, want_gI: bool):
+    Uf, If = _bpr_operand(U, "U"), _bpr_operand(I, "I")
+    if Uf.shape[1] != If.shape[1]:
+        raise ValueError("U [n_u, d] and I [n_i, d] need the same d")
+    dev = Uf.device
+    if If.device != dev:
+        raise ValueError("U and I must be on the same device")
+    n_u, d = Uf.shape
+    n_i = If.shape[0]
+    t = [to_device_i64(x, dev).reshape(-1) for x in (users, pos, neg)]
+    B = int(t[0].shape[0])
+    if t[1].shape[0] != B or t[2].shape[0] != B:
+        raise ValueError("users, pos and neg need the same length")
+    if B == 0:
+        raise ValueError("bpr_loss needs at least one triplet")
+    if B > _BPR_MAX_BATCH:
+        raise ValueError(f"bpr_loss takes at most {_BPR_MAX_BATCH} triplets")
+    if n_u == 0 or n_i == 0 or d == 0:
+        raise ValueError("bpr_loss needs n_u, n_i and d >= 1")
+    loss = torch.empty((), dtype=torch.float32, device=dev)
+    gU = new_padded(n_u, d, dev) if want_gU else None
+    gI = new_padded(n_i, d, dev) if want_gI else None
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    ws = workspace(_lib.query("gdr_bpr_loss_ws_bytes", B, n_u, n_i), dev)
+    _lib.call("gdr_bpr_loss", B, n_u, n_i, d, ptr(Uf), Uf.stride(0), ptr(If), If.stride(0), ptr(t[0]), ptr(t[1]),
+              ptr(t[2]), ptr(loss), ptr(gU), gU.stride(0) if gU is not None else 0, ptr(gI),
+              gI.stride(0) if gI is not None else 0, ptr(status), ptr(ws), ws.numel(), stream())
+    st = int(status.item())
+    if st & 1:
+        raise ValueError(f"bpr_loss: a user id outside [0, {n_u}) or an item id outside [0, {n_i})")
+    if st & 2:
+        raise ValueError("bpr_loss: U or I holds a non-finite value in a row a triplet uses")
+    return loss, gU, gI
+
+
+class BPRLoss(torch.autograd.Function):
+    """``loss = BPRLoss.apply(U, I, users, pos, neg)``: ``mean_b softplus(-x_b)`` with
+    ``x_b = <U[u_b], I[p_b]> - <U[u_b], I[n_b]>`` (``-logsigmoid(x).mean()``), fused in ``gdr_bpr_loss``.
+
+    ``U`` [n_u, d] and ``I`` [n_i, d] are typically ``LightGCNPropagate``'s outputs (padded strides are read in
+    place); the triplets are int64 ids (``BPRSampler.sample``).  The forward computes the gradients too when an
+    input needs them; backward scales them by the incoming scalar on the device (exact when it is 1).  Every sum has
+    a fixed order: the loss and the gradients are bit-identical from run to run.  Raises ValueError for no triplets,
+    ids out of range or a non-finite value in a used row (reading the status synchronises once per call).
+    Once-differentiable.  No regularisation term: add it on the ego embeddings in torch."""
+
+    @staticmethod
+    def forward(ctx, U, I, users, pos, neg):
+        loss, ctx.gU, ctx.gI = _bpr_forward(U, I, users, pos, neg, ctx.needs_input_grad[0], ctx.needs_input_grad[1])
+        return loss
+
+    @staticmethod
+    @once_differentiable
+    def backward(ctx, g):
+        gU = ctx.gU * g if ctx.gU is not None else None
+        gI = ctx.gI * g if ctx.gI is not None else None
+        ctx.gU = ctx.gI = None
+        return gU, gI, None, None, None
+
+
+def bpr_loss(U: torch.Tensor, I: torch.Tensor, users, pos, neg) -> torch.Tensor:
+    """``BPRLoss.apply(U, I, users, pos, neg)``: the fused BPR loss, differentiable w.r.t. ``U`` and ``I``."""
+    return BPRLoss.apply(U, I, users, pos, neg)

@@ -691,6 +691,41 @@ int     gdr_ranking_metrics(int64_t n_rows, int64_t n_users, int64_t k, const in
                             double* sums_out_dev, int64_t* n_eval_dev, float* per_row_out /*nullable*/,
                             void* ws, int64_t ws_bytes, gdr_stream_t stream);
 
+/* ---- BPR training step: triplet sampling and the fused BPR loss + gradient -------------------------------------
+ * The sampler, loss and gradient of the refinement loop (distill_recsys.py:684-733); with LightGCNPropagate a step
+ * needs no host round trip.  Neither entry point synchronises.
+ *
+ * gdr_bpr_sample: R = the n_users x n_items interaction CSR, columns sorted and unique inside each row (values are
+ *   not read).  eligible[0..n_eligible) = the users with 0 < deg(u) < n_items (the caller builds it once).  Triplet b
+ *   of `step`, b < batch:
+ *     Philox4x32-10, key = (seed & 0xffffffff, seed >> 32), counter = (b, step, j, 0); a 64-bit word x gives an
+ *     integer in [0, n) as umulhi64(x, n).  Call j = 0 -> (w0..w3): user = eligible[draw((w1<<32)|w0, n_eligible)],
+ *     pos = the draw((w3<<32)|w2, deg)-th entry of the user's row.  Call j = 1 -> (v0..v3): r = draw((v1<<32)|v0,
+ *     n_items - deg), neg = r + #{t : c_t - t <= r} over the row's columns c_0 < ... < c_{deg-1} (the r-th item
+ *     outside the row: the distribution of a rejection sampler, found by binary search).
+ *   users_out, pos_out, neg_out: int64 [batch].  Output depends on (R, eligible, seed, step, b) only: the same on
+ *   every run and every GPU.  batch in [1, 2^31/3], step in [0, 2^32), n_items >= 2.
+ * gdr_bpr_loss: U [n_u][ldu], I [n_i][ldi] f32 (16-byte aligned, ld a multiple of 4 and >= d), triplets
+ *   users / pos / neg int64 [batch], batch in [1, 2^31/3].  Per triplet
+ *     x_b = dot(U[u], I[p]) - dot(U[u], I[n]), each dot the fp32 chain acc = fmaf(U[u,t], I[., t], acc), t ascending;
+ *     l_b = softplus(-x_b) (fp32, max(z,0) + log1p(exp(-|z|))),  c_b = -sigmoid(-x_b) / B (fp32, one rounding).
+ *   *loss_out (device f32) = (fp64 sum of l_b: per-CTA partials in a fixed tree, then a fixed-order combine) / B.
+ *   gU / gI (each nullable; ld a multiple of 4, >= d, 16-byte aligned): overwritten with
+ *     gU[u] = sum_b c_b (I[p_b] - I[n_b]) over u_b = u,  gI[j] = sum_{p_b = j} c_b U[u_b] - sum_{n_b = j} c_b U[u_b],
+ *   zero in untouched rows.  Each row's terms are added in fp64 in (b, role) order and rounded once (rows with > 2048
+ *   terms: fixed chunks in that order, fp64 partials added in chunk order), from a stable sort of the 3B
+ *   (row, 3b + role) slots; no float atomics, so the gradients are bit-identical from run to run.
+ *   status_dev (device int32, zeroed by the caller): bit 0 = an id out of range, bit 1 = a non-finite x_b (a
+ *   non-finite value in a used row).  Such triplets add nothing; the outputs are then not meaningful. */
+int     gdr_bpr_sample(int64_t n_users, int64_t n_items, const int32_t* rowptr, const int32_t* colidx,
+                       int64_t n_eligible, const int32_t* eligible, uint64_t seed, int64_t step, int64_t batch,
+                       int64_t* users_out, int64_t* pos_out, int64_t* neg_out, gdr_stream_t stream);
+int64_t gdr_bpr_loss_ws_bytes(int64_t batch, int64_t n_u, int64_t n_i);
+int     gdr_bpr_loss(int64_t batch, int64_t n_u, int64_t n_i, int64_t d, const float* U, int64_t ldu,
+                     const float* I, int64_t ldi, const int64_t* users, const int64_t* pos, const int64_t* neg,
+                     float* loss_out, float* gU /*nullable*/, int64_t ldgu, float* gI /*nullable*/, int64_t ldgi,
+                     int32_t* status_dev, void* ws, int64_t ws_bytes, gdr_stream_t stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
