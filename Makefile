@@ -10,7 +10,7 @@ OBJS     := $(patsubst $(CSRC)/%.cu,build/%.o,$(SRCS))
 
 all: $(OUT)
 
-build/%.o: $(CSRC)/%.cu $(CSRC)/common.cuh $(CSRC)/comm.cuh $(CSRC)/tc_common.cuh include/gdr.h
+build/%.o: $(CSRC)/%.cu $(CSRC)/common.cuh $(CSRC)/comm.cuh $(CSRC)/tc_common.cuh $(CSRC)/topk_common.cuh include/gdr.h
 	@mkdir -p build
 	$(NVCC) $(NVFLAGS) -c $< -o $@ 2> build/$*.ptxas.log || (cat build/$*.ptxas.log; false)
 

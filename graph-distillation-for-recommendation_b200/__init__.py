@@ -6,7 +6,8 @@ Four stages behind the reference's own call signatures (see SURVEY.md §8):
   3. k-means / WCSS         kmeans.py       (sklearn KMeans call sites)
   4. coarsened graph        coarsen.py      (graph_compress, build_condensed_bipartite)
   +  edge scoring / top-k   sparsify.py     (ER_estimator, attaw_ER_estimator, graph_sparse; SURVEY §8f item 1)
-  +  top-K evaluation       recsys.py       (recommend_topk, ranking_metrics: recall_at_k, distill_recsys.py:446-497)
+  +  top-K evaluation       recsys.py       (recommend_topk, ranking_metrics: recall_at_k, distill_recsys.py:446-497;
+                                            recommend_topk_condensed: the same ranking from a condensed model's tables)
   +  condensed-model training recsys.py     (LightGCNPropagate: gradients w.r.t. embeddings and edge weights, :684-733;
                                             BPRSampler, bpr_loss: triplet sampling and the BPR loss + gradient)
 All arithmetic runs in libgdr_b200.so (hand-written sm_100a CUDA, C ABI in include/gdr.h).
@@ -35,7 +36,7 @@ from .sparsify import (  # noqa: E402
 )
 from .recsys import (  # noqa: E402
     BipartiteGraph, lightgcn_propagate, BipartitePropagate, LightGCNPropagate, RankformerGCNGraph,
-    rankformer_gcn_forward, recommend_topk, ranking_metrics, BPRSampler, BPRLoss, bpr_loss,
+    rankformer_gcn_forward, recommend_topk, recommend_topk_condensed, ranking_metrics, BPRSampler, BPRLoss, bpr_loss,
 )
 from .io import (  # noqa: E402
     induced_subgraph, load_graphsaint, load_rankformer_dataset, read_ui_txt, save_condensed, load_condensed,
@@ -53,7 +54,7 @@ __all__ = [
     "ER_estimator", "attaw_ER_estimator", "graph_sparse", "er_lower", "cosine_reweight", "softmax_rows",
     "class_edge_weight", "topk_filter", "row_degree", "BipartiteGraph", "lightgcn_propagate", "BipartitePropagate", "LightGCNPropagate",
     "RankformerGCNGraph",
-    "rankformer_gcn_forward", "recommend_topk", "ranking_metrics", "BPRSampler", "BPRLoss", "bpr_loss",
+    "rankformer_gcn_forward", "recommend_topk", "recommend_topk_condensed", "ranking_metrics", "BPRSampler", "BPRLoss", "bpr_loss",
     "induced_subgraph", "load_graphsaint", "load_rankformer_dataset", "read_ui_txt",
     "save_condensed", "load_condensed", "RecDataset", "GraphSaintData", "compute_svd_embeddings", "truncated_svd",
     "parallel",

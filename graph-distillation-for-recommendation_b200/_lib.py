@@ -142,6 +142,9 @@ _SIGNATURES = {
     "gdr_coarsen_scale": (i32, [i64, vp, vp, vp, vp, vp, vp, vp]),
     "gdr_topk_scores_ws_bytes": (i64, [i64, i64, i64, i64]),
     "gdr_topk_scores": (i32, [i64, i64, i64, i64, i64, vp, i64, vp, vp, i64, vp, vp, vp, i64, vp, i64, vp, vp, i64, vp]),
+    "gdr_topk_condensed_ws_bytes": (i64, [i64, i64, i64, i64, i64, i64, i64]),
+    "gdr_topk_condensed": (i32, [i64, i64, i64, i64, i64, i64, i64, vp, i64, vp, i64, vp, vp, vp, vp, vp, vp, i64, vp, i64,
+                                 vp, vp, i64, vp]),
     "gdr_ranking_metrics_ws_bytes": (i64, [i64, i32]),
     "gdr_ranking_metrics": (i32, [i64, i64, i64, vp, i64, vp, vp, vp, i32, vp, vp, vp, vp, vp, i64, vp]),
     "gdr_bpr_sample": (i32, [i64, i64, vp, vp, i64, vp, C.c_uint64, i64, i64, vp, vp, vp, vp]),

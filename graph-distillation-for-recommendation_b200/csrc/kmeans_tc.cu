@@ -45,6 +45,7 @@ static const int32_t* g_last_count1 = nullptr;   // device counter of the last t
 int g_tc_ablate = 0;   // experiment: 1 no epilogue math, 2 no tcgen05.ld either, 3 no MMAs, 4 one K-block of MMAs only
 int g_tc_gate = 1;      // gdr_debug_set("tc_gate", v): first-level epilogue gate — 0 off (exact running top-2 over all columns), 1 (default) gate on the running best, 2 also seeded with the previous label's score (measured at config E: the seed pass costs 0.9 ms and returns 0.1)
 extern int64_t g_topk_last_overflow;   // topk.cu
+extern int64_t g_topk_condensed_last_fallback;   // topk_condensed.cu
 int g_tc_screen = 0;    // gdr_debug_set("tc_screen", v): 0 auto, 1 direct 3xTF32, 2 two-level with 256-row x 128-centre CTA tiles, 3 two-level with 128 x 256 tiles, 4 two-level on CTA pairs (cta_group::2, 256 x 256), 6 two-level with the row tile in tensor memory (A operand from TMEM, 128 x 192 tiles)
 
 // smallest TF32 value >= v (v finite); used where a bound must not shrink under the operand rounding
@@ -1861,6 +1862,10 @@ int gdr_debug_get(const char* key, int64_t* value_host) {
   }
   if (!strcmp(key, "topk_overflow_rows")) {
     *value_host = gdr::g_topk_last_overflow;
+    return GDR_OK;
+  }
+  if (!strcmp(key, "topk_condensed_fallback_rows")) {
+    *value_host = gdr::g_topk_condensed_last_fallback;
     return GDR_OK;
   }
   gdr::set_error("debug_get: unknown key %s", key);

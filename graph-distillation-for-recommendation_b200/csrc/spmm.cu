@@ -48,6 +48,7 @@ extern int g_rs_match;            // primitives.cu
 extern int g_rs_max_bits;         // primitives.cu
 extern int g_tc_ablate;
 extern int g_topk_path;           // topk.cu
+extern int g_topk_condensed_path; // topk_condensed.cu
 }  // namespace gdr
 extern "C" int g_sparsify_batch_cap;   // sparsify.cu
 namespace gdr {
@@ -444,6 +445,7 @@ int gdr_debug_set(const char* key, int value) {
   else if (!strcmp(key, "lloyd_graph")) gdr::g_lloyd_graph = value;
   else if (!strcmp(key, "tc_screen")) gdr::g_tc_screen = value;
   else if (!strcmp(key, "topk_path")) gdr::g_topk_path = value;
+  else if (!strcmp(key, "topk_condensed_path")) gdr::g_topk_condensed_path = value;
   else if (!strcmp(key, "coarsen_dense")) gdr::g_coarsen_dense = value;
   else if (!strcmp(key, "tc_ablate")) gdr::g_tc_ablate = value;
   else if (!strcmp(key, "tc_gate")) gdr::g_tc_gate = value;

@@ -18,6 +18,7 @@
 // (3xTF32 tcgen05 + TMA screen whose epilogue keeps a bounded candidate list per user row), k_topk_tc_finish (exact
 // re-score of the candidates, sort); rows whose list overflows (ties) are finished by the exact path.
 #include "tc_common.cuh"
+#include "topk_common.cuh"
 
 namespace gdr {
 
@@ -27,19 +28,8 @@ constexpr int TK_BK = 16;           // contraction step held in shared memory
 constexpr int TK_SEL_THREADS = 512;
 constexpr int TK_SMEM_K = 2048;     // k up to this sorts in shared memory; larger k sorts in workspace
 constexpr int64_t TK_SLAB_BYTES = 384ll << 20;   // score scratch of one row slab
-constexpr uint32_t TK_EXCLUDED = 0xFFFFFFFFu;    // NaN pattern fmaf never produces: marks an excluded item
 constexpr int TK_MAX_KS = 32;
 
-static inline int64_t next_pow2(int64_t x) {
-  int64_t p = 1;
-  while (p < x) p <<= 1;
-  return p;
-}
-__device__ __forceinline__ int64_t next_pow2_dev(int64_t x) {
-  int64_t p = 1;
-  while (p < x) p <<= 1;
-  return p;
-}
 static inline int64_t tk_ld(int64_t n_items) { return align_up(n_items, 4); }
 static inline int64_t tk_kbuf(int64_t k) { return k > TK_SMEM_K ? next_pow2(k) * 8 : 0; }
 // rows per slab: as many as the scratch budget holds, a multiple of the score tile when more than one tile fits
@@ -146,39 +136,6 @@ __global__ void __launch_bounds__(256) k_topk_score(int64_t nr, int64_t r0, int6
         for (int b = 0; b < 4; ++b)
           if (j + b < n_items) out[j + b] = acc[a][h * 4 + b];
       }
-    }
-  }
-}
-
-// 64-bit selection key: larger = better.  -0 is ordered (and reported) as +0; 0 = excluded.
-__device__ __forceinline__ uint64_t tk_key(uint32_t bits, int64_t j) {
-  if (bits == TK_EXCLUDED) return 0ull;
-  uint32_t b = __float_as_uint(__uint_as_float(bits) + 0.f);
-  b = (b & 0x80000000u) ? ~b : (b | 0x80000000u);
-  return ((uint64_t)b << 32) | (uint32_t)(0xFFFFFFFFu - (uint32_t)j);
-}
-__device__ __forceinline__ float tk_key_score(uint64_t key) {
-  uint32_t b = (uint32_t)(key >> 32);
-  b = (b & 0x80000000u) ? (b & 0x7FFFFFFFu) : ~b;
-  return __uint_as_float(b);
-}
-
-// descending bitonic sort of n (power of two) keys held in shared or global memory by the whole CTA
-__device__ void tk_bitonic_desc(uint64_t* a, int64_t n) {
-  for (int64_t len = 2; len <= n; len <<= 1) {
-    for (int64_t j = len >> 1; j > 0; j >>= 1) {
-      for (int64_t i = threadIdx.x; i < n; i += blockDim.x) {
-        const int64_t p = i ^ j;
-        if (p > i) {
-          const uint64_t x = a[i], y = a[p];
-          const bool desc = (i & len) == 0;
-          if (desc ? x < y : x > y) {
-            a[i] = y;
-            a[p] = x;
-          }
-        }
-      }
-      __syncthreads();
     }
   }
 }
@@ -316,16 +273,24 @@ __global__ void __launch_bounds__(TK_SEL_THREADS) k_topk_select(int64_t nr, int6
   }
 }
 
-static int64_t topk_exact_ws_bytes(int64_t n_rows, int64_t n_items, int64_t k) {
+int64_t topk_exact_ws_bytes(int64_t n_rows, int64_t n_items, int64_t k) {
   const int64_t sr = tk_slab_rows(n_rows, n_items, k);
   return ws_need(sr * tk_ld(n_items), 4) + ws_need(sr * tk_kbuf(k), 1) + 256;
 }
 
+int topk_score_rows(int64_t nr, int64_t r0, int64_t n_users, int64_t n_items, int64_t d, const float* U, int64_t ldu,
+                    const int64_t* rows, const float* I, int64_t ldi, float* S, int64_t lds, cudaStream_t s) {
+  dim3 grid((unsigned)cdiv(n_items, TK_BN), (unsigned)cdiv(nr, TK_BM));
+  k_topk_score<<<grid, 256, 0, s>>>(nr, r0, n_users, n_items, d, U, ldu, rows, nullptr, I, ldi, S, lds);
+  GDR_LAUNCHED();
+  return GDR_OK;
+}
+
 // exact path over n_rows output rows (out_rows: their indices, nullable = 0..n_rows-1)
-static int topk_exact(int64_t n_rows, int64_t n_users, int64_t n_items, int64_t d, int64_t k, const float* U, int64_t ldu,
-                      const int64_t* rows, const int32_t* out_rows, const float* I, int64_t ldi, const int32_t* ex_rowptr,
-                      const int32_t* ex_colidx, float* scores_out, int64_t lds, int32_t* items_out, int64_t ldit,
-                      int32_t* status, void* ws, int64_t ws_bytes, cudaStream_t s) {
+int topk_exact(int64_t n_rows, int64_t n_users, int64_t n_items, int64_t d, int64_t k, const float* U, int64_t ldu,
+               const int64_t* rows, const int32_t* out_rows, const float* I, int64_t ldi, const int32_t* ex_rowptr,
+               const int32_t* ex_colidx, float* scores_out, int64_t lds, int32_t* items_out, int64_t ldit,
+               int32_t* status, void* ws, int64_t ws_bytes, cudaStream_t s) {
   const int64_t sr = tk_slab_rows(n_rows, n_items, k), ld = tk_ld(n_items);
   const int64_t kbuf_n = tk_kbuf(k) / 8;
   Workspace W(ws, ws_bytes);

@@ -329,6 +329,75 @@ def recommend_topk(user_emb: torch.Tensor, item_emb: torch.Tensor, k: int, exclu
     return scores, items.long()
 
 
+def _map_arg(m, n_values: int, name: str, device) -> torch.Tensor:
+    """user_map / item_map (torch or numpy, int32 or int64, 1-D) -> int64 device tensor; range checked on the device."""
+    dt = m.dtype if isinstance(m, (torch.Tensor, np.ndarray)) else None
+    if dt not in (torch.int32, torch.int64, np.dtype(np.int32), np.dtype(np.int64)):
+        raise ValueError(f"{name} must be an int32 or int64 torch tensor or numpy array")
+    if m.ndim != 1:
+        raise ValueError(f"{name} must be 1-D")
+    if n_values == 0 and m.shape[0]:
+        raise ValueError(f"{name} has values but its embedding table has no rows")
+    return to_device_i64(m, device)
+
+
+def recommend_topk_condensed(user_emb: torch.Tensor, item_emb: torch.Tensor, k: int, user_map, item_map,
+                             exclude=None, rows=None) -> Tuple[torch.Tensor, torch.Tensor]:
+    """``recommend_topk`` of a condensed model, from its cluster tables: ``(scores [n_rows, k] f32, items [n_rows, k]
+    int64)``, byte-identical to ``recommend_topk(user_emb[user_map], item_emb[item_map], k, exclude, rows)``.
+
+    ``user_emb`` [n_cu, d] and ``item_emb`` [n_ci, d] are the super-user and super-item rows (``LightGCNPropagate``'s
+    outputs, say); ``user_map`` [n_users] and ``item_map`` [n_items] (``u2cu``, ``i2ci``: int32 or int64, torch or
+    numpy) give every original user and item its row.  ``exclude`` (n_users x n_items) and ``rows`` are those of
+    ``recommend_topk``, and item ids are original ids, so the result feeds ``ranking_metrics`` unchanged.  Only the
+    n_cu x n_ci distinct scores are computed; rows whose ranking hits a tie of more than 32 clusters (a zero
+    super-user) are finished on ``recommend_topk``'s exact path.  Raises ValueError for a non-finite value in a
+    super-user row an evaluated row uses or in a super-item row with a member, for user ids or map values out of
+    range, and for k outside [1, n_items].  Synchronises; no autograd."""
+    need_cuda(user_emb, "user_emb")
+    need_cuda(item_emb, "item_emb")
+    if user_emb.dim() != 2 or item_emb.dim() != 2 or user_emb.shape[1] != item_emb.shape[1]:
+        raise ValueError("user_emb [n_cu, d] and item_emb [n_ci, d] need the same d")
+    U = user_emb.detach().to(torch.float32).contiguous()
+    I = item_emb.detach().to(torch.float32).contiguous()
+    dev = U.device
+    if I.device != dev:
+        raise ValueError("user_emb and item_emb must be on the same device")
+    n_cu, d = U.shape
+    n_ci = I.shape[0]
+    um = _map_arg(user_map, n_cu, "user_map", dev)
+    im = _map_arg(item_map, n_ci, "item_map", dev)
+    n_users, n_items = int(um.shape[0]), int(im.shape[0])
+    k = int(k)
+    if not 1 <= k <= n_items:
+        raise ValueError(f"k={k} must lie in [1, n_items={n_items}]")
+    if d == 0:
+        raise ValueError("the embeddings need d >= 1")
+    ex = None if exclude is None else _as_csr(exclude, (n_users, n_items), "exclude", dev)
+    rows_d, n_rows = _rows_arg(rows, n_users, dev)
+    scores = torch.empty((n_rows, k), dtype=torch.float32, device=dev)
+    items = torch.empty((n_rows, k), dtype=torch.int32, device=dev)
+    if n_rows == 0:
+        return scores, items.long()
+    if n_users == 0:
+        raise ValueError("recommend_topk_condensed: rows given but user_map is empty")
+    status = torch.zeros(1, dtype=torch.int32, device=dev)
+    ws = workspace(_lib.query("gdr_topk_condensed_ws_bytes", n_rows, n_users, n_items, n_cu, n_ci, d, k), dev)
+    _lib.call("gdr_topk_condensed", n_rows, n_users, n_items, n_cu, n_ci, d, k, ptr(U), U.stride(0), ptr(I),
+              I.stride(0), ptr(um), ptr(im), ptr(rows_d), ptr(ex.rowptr) if ex is not None else 0,
+              ptr(ex.colidx) if ex is not None else 0, ptr(scores), k, ptr(items), k, ptr(status), ptr(ws), ws.numel(),
+              stream())
+    st = int(status.item())
+    if st & 4:
+        raise ValueError(f"recommend_topk_condensed: a user_map value outside [0, {n_cu}) or an item_map value "
+                         f"outside [0, {n_ci})")
+    if st & 2:
+        raise ValueError(f"recommend_topk_condensed: a user id in rows lies outside [0, {n_users})")
+    if st & 1:
+        raise ValueError("recommend_topk_condensed: user_emb or item_emb holds a non-finite value in a used row")
+    return scores, items.long()
+
+
 def ranking_metrics(items: torch.Tensor, test, ks: Sequence[int] = (20,), rows=None) -> Dict[str, float]:
     """Recall@K, Precision@K and NDCG@K of a top-k list (``recommend_topk``'s ``items``) against held-out items.
 

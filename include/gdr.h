@@ -74,11 +74,14 @@ int gdr_profile_collect(double* total_ms_host, int64_t* launches_host);
  * with the previous label's score; every setting produces the same labels);
  * "rs_match" (radix-sort ranking: 0 [default] per-bit warp ballots, 1 MATCH.ANY); "topk_path" (gdr_topk_scores: 1 exact
  * SIMT path, 2 tensor-core screen);
+ * "topk_condensed_path" (gdr_topk_condensed: 1 every row on the exact fallback);
  * value 0 / -1 = automatic. */
 int gdr_debug_set(const char* key, int value);
 /* Debug read-back (synchronises the device).  keys: "tc_level2_rows" = rows the last two-level
  * tensor-core screen (gdr_kmeans_assign_tc) handed to its 3xTF32 second level; -1 if none ran.
- * "topk_overflow_rows" = rows the last tensor-core gdr_topk_scores finished on the exact path; -1 if none ran. */
+ * "topk_overflow_rows" = rows the last tensor-core gdr_topk_scores finished on the exact path; -1 if none ran.
+ * "topk_condensed_fallback_rows" = rows the last gdr_topk_condensed finished on the exact path; -1 if it wrote
+ * nothing. */
 int gdr_debug_get(const char* key, int64_t* value_host);
 /* Tensor-pipe micro-probe: SM cycles for `iters` back-to-back tcgen05.mma of shape 128 x N x (32 bytes of K)
  * issued by one CTA (variant bit 0: kind::f16 instead of kind::tf32, bit 1: two accumulators, bit 2: no K advance). */
@@ -690,6 +693,29 @@ int     gdr_ranking_metrics(int64_t n_rows, int64_t n_users, int64_t k, const in
                             const int32_t* test_colidx, int n_ks, const int32_t* ks_host,
                             double* sums_out_dev, int64_t* n_eval_dev, float* per_row_out /*nullable*/,
                             void* ws, int64_t ws_bytes, gdr_stream_t stream);
+/* gdr_topk_condensed: gdr_topk_scores for a condensed model, from its cluster tables.  U [n_cu][ldu] and I [n_ci][ldi]
+ *   are the super-user and super-item rows; user_map [n_users] and item_map [n_items] (int64) give each original user
+ *   and item its row, values in [0, n_cu) and [0, n_ci).  rows, the exclusion CSR (n_users x n_items, columns sorted
+ *   inside each row) and the outputs are those of gdr_topk_scores, and the output bytes are those of gdr_topk_scores
+ *   on the expanded tables U[user_map], I[item_map] (either of its paths): (score desc, item asc) across clusters,
+ *   -0 reported as +0, (-1, -inf) padding.  Only the n_cu x n_ci distinct scores of the used super-users are
+ *   computed: each super-user orders the clusters its rows can need, and each row walks that order, expanding
+ *   clusters to their members in id order.  A row that meets a tie run of more than 32 clusters before it has k
+ *   items is finished on gdr_topk_scores' exact path with its expanded row (debug key "topk_condensed_path": 1 sends
+ *   every row there; gdr_debug_get("topk_condensed_fallback_rows") reads back how many rows the last call sent).
+ *   status_dev (device int32, zeroed by the caller): bit 0 = a non-finite value in a super-user row of an evaluated
+ *   row or in a super-item row with at least one member (a super-item without members is never read), bit 1 = a user
+ *   id in rows outside [0, n_users), bit 2 = a map value outside its range; when any bit is set nothing is written.
+ *   The workspace depends on the shapes only (slabs of super-users); the call SYNCHRONISES the stream twice (to size
+ *   the slabs from the number of used super-users, and the fallback from its row count). */
+int64_t gdr_topk_condensed_ws_bytes(int64_t n_rows, int64_t n_users, int64_t n_items, int64_t n_cu, int64_t n_ci,
+                                    int64_t d, int64_t k);
+int     gdr_topk_condensed(int64_t n_rows, int64_t n_users, int64_t n_items, int64_t n_cu, int64_t n_ci, int64_t d,
+                           int64_t k, const float* U, int64_t ldu, const float* I, int64_t ldi,
+                           const int64_t* user_map, const int64_t* item_map, const int64_t* rows /*nullable*/,
+                           const int32_t* ex_rowptr, const int32_t* ex_colidx /*both nullable*/,
+                           float* scores_out, int64_t lds, int32_t* items_out, int64_t ldit,
+                           int32_t* status_dev, void* ws, int64_t ws_bytes, gdr_stream_t stream);
 
 /* ---- BPR training step: triplet sampling and the fused BPR loss + gradient -------------------------------------
  * The sampler, loss and gradient of the refinement loop (distill_recsys.py:684-733); with LightGCNPropagate a step
