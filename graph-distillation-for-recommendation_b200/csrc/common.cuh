@@ -113,6 +113,24 @@ int spmm_launch(int64_t rows, int64_t F, const int32_t* rowptr, const int32_t* c
 
 __device__ __forceinline__ int lane_id() { return threadIdx.x & 31; }
 
+// The exact fp32 distance of the E-step, d(i, j) = fmaf(-2, acc, |c_j|^2) with acc = fmaf(x_k, c_jk, acc) for k
+// ascending from acc = 0.  Every kernel that decides a label exactly (k_assign_simt, k_refine_partial,
+// k_tc_cand_resolve) builds its distances from these two steps, so that they agree bit for bit.
+__device__ __forceinline__ float ed_chain(float acc, float x, float c) { return fmaf(x, c, acc); }
+__device__ __forceinline__ float ed_finish(float acc, float cnorm) { return fmaf(-2.f, acc, cnorm); }
+
+// (distance, centre) as one 64-bit key whose unsigned order is (distance, then lowest index)
+__device__ __forceinline__ unsigned long long rf_pack(float d, int j) {
+  unsigned u = __float_as_uint(d);
+  u = (u >> 31) ? ~u : (u | 0x80000000u);   // monotone map float -> uint32
+  return ((unsigned long long)u << 32) | (unsigned)j;
+}
+__device__ __forceinline__ float rf_unpack(unsigned long long key) {
+  unsigned u = (unsigned)(key >> 32);
+  u = (u >> 31) ? (u & 0x7fffffffu) : ~u;
+  return __uint_as_float(u);
+}
+
 __device__ __forceinline__ float4 ldg_nc_f4(const float* p) {
   float4 r;
   asm volatile("ld.global.nc.L1::no_allocate.v4.f32 {%0,%1,%2,%3}, [%4];"

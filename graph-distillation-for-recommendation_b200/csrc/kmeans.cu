@@ -204,7 +204,7 @@ k_assign_simt(int64_t N, int K, int D, const float* __restrict__ X, int64_t ldx,
 #pragma unroll
         for (int i = 0; i < 8; ++i)
 #pragma unroll
-          for (int j = 0; j < 8; ++j) acc[i][j] = fmaf(a[i], b[j], acc[i][j]);
+          for (int j = 0; j < 8; ++j) acc[i][j] = ed_chain(acc[i][j], a[i], b[j]);
       }
       __syncthreads();
     }
@@ -216,7 +216,7 @@ k_assign_simt(int64_t N, int K, int D, const float* __restrict__ X, int64_t ldx,
         float cn = __ldg(cnorm + col);
 #pragma unroll
         for (int i = 0; i < 8; ++i) {
-          float d = fmaf(-2.f, acc[i][j], cn);
+          float d = ed_finish(acc[i][j], cn);
           if (d < best[i]) {
             best[i] = d;
             bidx[i] = col;
@@ -276,12 +276,6 @@ int launch_row_sqnorm(int64_t K, int D, const float* C, int64_t ldc, float* out,
 constexpr int RF_THREADS = 128;
 constexpr int RF_ROWS = 8;
 
-__device__ __forceinline__ unsigned long long rf_pack(float d, int j) {
-  unsigned u = __float_as_uint(d);
-  u = (u >> 31) ? ~u : (u | 0x80000000u);   // monotone map float -> uint32
-  return ((unsigned long long)u << 32) | (unsigned)j;
-}
-
 __global__ void __launch_bounds__(RF_THREADS) k_refine_partial(int K, int D, const float* __restrict__ X,
                                                                int64_t ldx, const float* __restrict__ CT,
                                                                int64_t ldct, const float* __restrict__ cnorm,
@@ -320,18 +314,18 @@ __global__ void __launch_bounds__(RF_THREADS) k_refine_partial(int K, int D, con
       for (int k = 0; k < D; ++k) {
         const float c = s_ct[k * RF_THREADS + threadIdx.x];
         const float4 xa = s_x4[2 * k], xb = s_x4[2 * k + 1];
-        acc[0] = fmaf(xa.x, c, acc[0]);
-        acc[1] = fmaf(xa.y, c, acc[1]);
-        acc[2] = fmaf(xa.z, c, acc[2]);
-        acc[3] = fmaf(xa.w, c, acc[3]);
-        acc[4] = fmaf(xb.x, c, acc[4]);
-        acc[5] = fmaf(xb.y, c, acc[5]);
-        acc[6] = fmaf(xb.z, c, acc[6]);
-        acc[7] = fmaf(xb.w, c, acc[7]);
+        acc[0] = ed_chain(acc[0], xa.x, c);
+        acc[1] = ed_chain(acc[1], xa.y, c);
+        acc[2] = ed_chain(acc[2], xa.z, c);
+        acc[3] = ed_chain(acc[3], xa.w, c);
+        acc[4] = ed_chain(acc[4], xb.x, c);
+        acc[5] = ed_chain(acc[5], xb.y, c);
+        acc[6] = ed_chain(acc[6], xb.z, c);
+        acc[7] = ed_chain(acc[7], xb.w, c);
       }
 #pragma unroll
       for (int r = 0; r < RF_ROWS; ++r) {
-        const float d = fmaf(-2.f, acc[r], cn);
+        const float d = ed_finish(acc[r], cn);
         unsigned long long key = (j < K && d == d) ? rf_pack(d, j) : ~0ull;
 #pragma unroll
         for (int o = 16; o > 0; o >>= 1) {
@@ -356,10 +350,8 @@ __global__ void __launch_bounds__(256) k_refine_commit(const int32_t* __restrict
     const int64_t row = rows[q];
     int l = (int)(unsigned)(key & 0xffffffffull);
     if (key == ~0ull) l = 0;
-    unsigned u = (unsigned)(key >> 32);
-    u = (u >> 31) ? (u & 0x7fffffffu) : ~u;
     labels[row] = l;
-    if (best_out) best_out[row] = __uint_as_float(u);
+    if (best_out) best_out[row] = rf_unpack(key);
     if (n_changed && labels_prev && labels_prev[row] != l) atomicAdd(n_changed, 1);
   }
 }

@@ -46,6 +46,9 @@ int g_tc_ablate = 0;   // experiment: 1 no epilogue math, 2 no tcgen05.ld either
 int g_tc_gate = 1;      // gdr_debug_set("tc_gate", v): first-level epilogue gate — 0 off (exact running top-2 over all columns), 1 (default) gate on the running best, 2 also seeded with the previous label's score (measured at config E: the seed pass costs 0.9 ms and returns 0.1)
 extern int64_t g_topk_last_overflow;   // topk.cu
 extern int64_t g_topk_condensed_last_fallback;   // topk_condensed.cu
+int g_tc_cand = 1;      // gdr_debug_set("tc_cand", v): second level of the default two-level screen — 1 (default) seeded candidate pass + exact re-score of the candidates, 0 3xTF32 + exact re-score over all centres
+int g_tc_cand_cap = 0;  // gdr_debug_set("tc_cand_cap", v): candidate list capacity per row and column half, 1..TC_CAND_CAP (0: TC_CAND_CAP)
+static const int32_t* g_last_cand = nullptr;     // candidate counters of the last run that used the candidate level (debug read-back)
 int g_tc_screen = 0;    // gdr_debug_set("tc_screen", v): 0 auto, 1 direct 3xTF32, 2 two-level with 256-row x 128-centre CTA tiles, 3 two-level with 128 x 256 tiles, 4 two-level on CTA pairs (cta_group::2, 256 x 256), 6 two-level with the row tile in tensor memory (A operand from TMEM, 128 x 192 tiles)
 
 // smallest TF32 value >= v (v finite); used where a bound must not shrink under the operand rounding
@@ -123,11 +126,12 @@ __global__ void __launch_bounds__(256) k_split_tf32(int64_t rows, int64_t rows_p
   }
 }
 
-// cmax = max_j |c_j| over the real centres, |c_j| per centre (0 on padding); also resets the list lengths
+// cmax = max_j |c_j| over the real centres, |c_j| per centre (0 on padding); also resets the list lengths and counters
 __global__ void __launch_bounds__(1024) k_cnorm_finish(int64_t K, int64_t Kp, const float* __restrict__ cnorm,
                                                        const float* __restrict__ cdnorm /*nullable*/,
                                                        float* __restrict__ cnorm_sqrt, float* __restrict__ cmax /*[2]*/,
-                                                       int32_t* __restrict__ amb_count, int32_t* __restrict__ count1) {
+                                                       int32_t* __restrict__ amb_count, int32_t* __restrict__ count1,
+                                                       int32_t* __restrict__ zero /*nullable*/, int n_zero) {
   __shared__ float s_m[1024];
   __shared__ float s_d[1024];
   float m = 0.f, md = 0.f;
@@ -135,6 +139,7 @@ __global__ void __launch_bounds__(1024) k_cnorm_finish(int64_t K, int64_t Kp, co
     if (amb_count) amb_count[0] = 0;
     if (count1) count1[0] = 0;
   }
+  if (zero && (int)threadIdx.x < n_zero) zero[threadIdx.x] = 0;
   for (int64_t j = threadIdx.x; j < Kp; j += 1024) {
     const float c2 = j < K ? cnorm[j] : 0.f;
     m = fmaxf(m, c2);
@@ -225,6 +230,43 @@ __device__ __forceinline__ void epi_chunk32(const uint32_t (&v)[32], int jbase, 
   }
 }
 
+// slack of the candidate pass's starting limit over the level-1 best it is seeded with: the two passes multiply the
+// same operands but may accumulate differently (same bound as k_tc_seed's 2^-18 term)
+__device__ __forceinline__ float tc_cand_slack(float xn, float cm) { return 3.814697265625e-06f * (xn * cm + cm * cm); }
+
+// Candidate-pass epilogue step (k_tc_cand): as epi_chunk32 with the gate always on, plus every per-element score below
+// the limit in force is appended to this (row, column half)'s list.  The limit only falls, from seed + slack + tolmax
+// to best-so-far + tolmax, so every centre with d < min(seed + slack, final best) + tolmax is recorded.
+__device__ __forceinline__ void epi_chunk32_rec(const uint32_t (&v)[32], int jbase, float tolmax, float& limt,
+                                                float& best, int& n, int2* rec, int cap) {
+  float m8[4];
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    const int u0 = 8 * q;
+    const float m = fmaxf(fmaxf(__uint_as_float(v[u0]), __uint_as_float(v[u0 + 1])),
+                          fmaxf(__uint_as_float(v[u0 + 2]), __uint_as_float(v[u0 + 3])));
+    m8[q] = fmaxf(m, fmaxf(fmaxf(__uint_as_float(v[u0 + 4]), __uint_as_float(v[u0 + 5])),
+                           fmaxf(__uint_as_float(v[u0 + 6]), __uint_as_float(v[u0 + 7]))));
+  }
+  const float m32 = fmaxf(fmaxf(m8[0], m8[1]), fmaxf(m8[2], m8[3]));
+  if (!__any_sync(0xffffffffu, -m32 < limt)) return;
+#pragma unroll
+  for (int q = 0; q < 4; ++q) {
+    if (__any_sync(0xffffffffu, -m8[q] < limt)) {
+#pragma unroll
+      for (int u = 8 * q; u < 8 * q + 8; ++u) {
+        const float d = -__uint_as_float(v[u]);
+        if (d < limt) {
+          if (n < cap) rec[n] = make_int2(jbase + u, __float_as_int(d));
+          ++n;
+        }
+        best = fminf(best, d);
+      }
+      limt = fminf(limt, best + tolmax);
+    }
+  }
+}
+
 template <int NPASS, int BN, int SUB>
 struct TcCfg {
   static constexpr int kXCopies = NPASS == 3 ? 2 : 1;                        // hi (+ lo) copy of the row tile
@@ -244,17 +286,27 @@ struct TcCfg {
   __host__ __device__ static constexpr int total(int nkb) { return bars(nkb) + kTail + 1024; }
 };
 
-template <int NPASS, int BN, int SUB>
-__global__ void __launch_bounds__(TC_THREADS, 1)
-k_assign_tc(const __grid_constant__ CUtensorMap map_xhi, const __grid_constant__ CUtensorMap map_xlo,
-            const __grid_constant__ CUtensorMap map_chi, const __grid_constant__ CUtensorMap map_clo,
-            int64_t N_host, const int32_t* __restrict__ n_rows_dev /*nullable: row count on the device*/,
-            int D /*contraction width incl. the 3 augmented columns for NPASS 1*/, int n_col_tiles, int nkb,
-            const float* __restrict__ cnorm /*NPASS 3: |c_j|^2*/,
-            float* __restrict__ best_out, float* __restrict__ second_out, int32_t* __restrict__ idx_out, int ablate,
-            TcGate gate) {
+// Candidate recording of the seeded first-level pass (k_tc_cand): per (compacted row, column half) the centres whose
+// negated score is below the row's limit, in column order; count[] may exceed cap (overflow: the row takes the fallback).
+struct TcCand {
+  int2* list;       // [rows][2][cap] (centre, negated score bits)
+  int32_t* count;   // [rows][2] centres met below the limit per column half
+  int cap;
+};
+
+// The kernel body, shared by the first level / 3xTF32 level (k_assign_tc) and the seeded candidate pass (k_tc_cand,
+// REC = true).  REC: the gate is always on, the limit starts at the row's seed and every per-element score below it
+// is recorded; best / second / argmin are not written.
+template <int NPASS, int BN, int SUB, bool REC>
+__device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const CUtensorMap& map_xlo,
+                                               const CUtensorMap& map_chi, const CUtensorMap& map_clo, int64_t N_host,
+                                               const int32_t* __restrict__ n_rows_dev, int D, int n_col_tiles, int nkb,
+                                               const float* __restrict__ cnorm, float* __restrict__ best_out,
+                                               float* __restrict__ second_out, int32_t* __restrict__ idx_out, int ablate,
+                                               TcGate gate, TcCand cand) {
   using Cfg = TcCfg<NPASS, BN, SUB>;
   static_assert(Cfg::kTmemCols <= 512 && (NPASS == 1 || SUB == 1) && (SUB == 1 || SUB == 2), "tile plan");
+  static_assert(!REC || (NPASS == 1 && SUB == 1), "candidate recording: first-level shape only");
   const int S = Cfg::stages(nkb);
   constexpr int ROWS = TC_BM * SUB;            // rows per CTA tile
   extern __shared__ uint8_t smem_raw[];
@@ -451,7 +503,7 @@ k_assign_tc(const __grid_constant__ CUtensorMap map_xhi, const __grid_constant__
     constexpr int COLS = SUB == 1 ? BN / 2 : BN;                       // columns per warp and accumulator
     float* s_merge = reinterpret_cast<float*>(tmem_base_smem + 4);   // [3][128] exchange buffer after the barriers
     const int rl = quarter * 32 + lane;
-    const bool chunk_skip = n_col_tiles * BN >= 4096;   // the vote only pays once most chunks can be skipped
+    const bool chunk_skip = REC || n_col_tiles * BN >= 4096;   // the vote only pays once most chunks can be skipped
     uint32_t g = 0;
     for (int rt = blockIdx.x; rt < (ablate == 8 ? 0 : n_row_tiles); rt += gridDim.x) {
       const int64_t row = (int64_t)rt * ROWS + (SUB == 2 ? half * TC_BM : 0) + rl;
@@ -462,14 +514,18 @@ k_assign_tc(const __grid_constant__ CUtensorMap map_xhi, const __grid_constant__
       // gate (NPASS 1): limt = (lower bound of the final best, as a negated score) + tolmax_i; a chunk whose smallest
       // negated score is not below limt for any lane cannot hold the row's best nor anything within tol of it
       float tolmax = 0.f, limt = INFINITY;
-      const bool gated = NPASS == 1 && chunk_skip && gate.xnorm != nullptr;
+      const bool gated = REC || (NPASS == 1 && chunk_skip && gate.xnorm != nullptr);
       if (gated) {
         const float xn = row < N ? gate.xnorm[row] : 0.f, xd = row < N ? gate.xdnorm[row] : 0.f;
         const float cm = gate.cscal[0], cdm = gate.cscal[1];
         tolmax = 1.001f * (2.02f * (xd * cm + xn * (cdm + 3.0517578125e-05f * cm) + 1.52587890625e-05f * cm * cm) +
                            gate.band * xn * cm + 9.5367431640625e-07f * (xn * cm + cm * cm));
-        if (gate.seed != nullptr && row < N) limt = gate.seed[row] + tolmax;
+        if constexpr (REC) limt = row < N ? gate.seed[row] + tc_cand_slack(xn, cm) + tolmax : -INFINITY;   // padding rows record nothing
+        else if (gate.seed != nullptr && row < N) limt = gate.seed[row] + tolmax;
       }
+      int n_rec = 0;   // REC: this (row, column half)'s list
+      int2* rec = nullptr;
+      if constexpr (REC) rec = cand.list + ((int64_t)row * 2 + half) * cand.cap;
       for (int ct = 0; ct < n_col_tiles; ++ct, ++g) {
         const uint32_t a = g & 1, aph = (g >> 1) & 1;
         mbar_wait(&t_full[a], aph);
@@ -491,7 +547,9 @@ k_assign_tc(const __grid_constant__ CUtensorMap map_xhi, const __grid_constant__
 #pragma unroll
           for (int c = 0; c < 2; ++c) {
             const int jbase = ct * BN + col0 + c * 32;
-            if (NPASS == 1) {
+            if constexpr (REC) {
+              epi_chunk32_rec(v[c], jbase, tolmax, limt, best, n_rec, rec, cand.cap);
+            } else if (NPASS == 1) {
               epi_chunk32(v[c], jbase, chunk_skip, gated, tolmax, limt, best, second, bidx);
             } else {
               const float4* cn4 = reinterpret_cast<const float4*>(cnorm + jbase);
@@ -513,7 +571,9 @@ k_assign_tc(const __grid_constant__ CUtensorMap map_xhi, const __grid_constant__
         tc_fence_before();
         mbar_arrive(&t_empty[a]);
       }
-      if (SUB == 2) {
+      if constexpr (REC) {
+        if (row < N) cand.count[row * 2 + half] = n_rec;
+      } else if (SUB == 2) {
         if (row < N) {
           best_out[row] = best;
           second_out[row] = second;
@@ -549,6 +609,28 @@ k_assign_tc(const __grid_constant__ CUtensorMap map_xhi, const __grid_constant__
     __syncwarp();
     asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(Cfg::kTmemCols) : "memory");
   }
+}
+
+template <int NPASS, int BN, int SUB>
+__global__ void __launch_bounds__(TC_THREADS, 1)
+k_assign_tc(const __grid_constant__ CUtensorMap map_xhi, const __grid_constant__ CUtensorMap map_xlo,
+            const __grid_constant__ CUtensorMap map_chi, const __grid_constant__ CUtensorMap map_clo,
+            int64_t N_host, const int32_t* __restrict__ n_rows_dev /*nullable: row count on the device*/,
+            int D /*contraction width incl. the 3 augmented columns for NPASS 1*/, int n_col_tiles, int nkb,
+            const float* __restrict__ cnorm /*NPASS 3: |c_j|^2*/,
+            float* __restrict__ best_out, float* __restrict__ second_out, int32_t* __restrict__ idx_out, int ablate,
+            TcGate gate) {
+  assign_tc_body<NPASS, BN, SUB, false>(map_xhi, map_xlo, map_chi, map_clo, N_host, n_rows_dev, D, n_col_tiles, nkb, cnorm,
+                                        best_out, second_out, idx_out, ablate, gate, TcCand{nullptr, nullptr, 0});
+}
+
+// Seeded candidate pass over the compacted undecided rows: k_assign_tc<1, 256, 1>'s schedule and arithmetic on the
+// compacted augmented rows (row count on the device), with gate.seed / xnorm / xdnorm indexed by compacted slot.
+__global__ void __launch_bounds__(TC_THREADS, 1)
+k_tc_cand(const __grid_constant__ CUtensorMap map_x1, const __grid_constant__ CUtensorMap map_c1, int64_t N_host,
+          const int32_t* __restrict__ n_rows_dev, int D, int n_col_tiles, int nkb, TcGate gate, TcCand cand) {
+  assign_tc_body<1, 256, 1, true>(map_x1, map_x1, map_c1, map_c1, N_host, n_rows_dev, D, n_col_tiles, nkb, nullptr,
+                                  nullptr, nullptr, nullptr, 0, gate, cand);
 }
 
 // ---------------------------------------------------------------------------------
@@ -1369,6 +1451,181 @@ __global__ void __launch_bounds__(256) k_tc_gather(const int32_t* __restrict__ l
   }
 }
 
+// ---------------------------------------------------------------------------------
+// second level on candidate centres (the default two-level screen)
+// ---------------------------------------------------------------------------------
+// For every row level 1 left undecided, k_tc_cand re-runs the first-level product over the compacted rows with the
+// limit fixed from the start at seed + slack + tolmax_i (seed = the row's level-1 best, as a negated score) and records
+// each centre j met below the limit in force; k_tc_cand_resolve then decides the row on those centres alone.
+//
+// Why that is exact.  Let b = the smallest recorded negated score, l its centre (lowest index on ties), and tol(i, l)
+// the expression of k_tc_select1 (with 2^-21 max(|b|, |d_j|) as its last term).  For a centre j with
+// d_j - b > tol(i, l), i.e. s_l - s_j > tol(i, l), the inequality k_tc_select1 relies on gives, for this pair,
+//   t_j <= s_j < s_l - 2 rad_l - eta <= t_l - eta,
+// so j loses to l in the exact fp32 chain, ties included: such a j is excluded.  Every other centre is recorded:
+// the limit in force is min(seed + slack, running best) + tolmax_i >= b + tolmax_i whenever b <= seed + slack (then b
+// is also the row's true minimum, which the limit always admits), and tol(i, .) < tolmax_i.  k_tc_cand_resolve checks
+// b <= seed + slack itself — it does not assume that the two TF32 passes produce the same bits — and sends a row that
+// fails it, a row with an empty list and a row whose list overflowed in either column half to the fallback list,
+// which takes the 3xTF32 level and the exact re-score over all centres as before.  The kept centres are re-scored with
+// the exact fp32 chain of k_assign_simt / k_refine_partial (ed_chain) and the (distance, index) minimum of rf_pack.
+
+// compact the first-level operand rows, |x|, |x - tf32(x)| and the level-1 best (the seed) of the listed rows
+__global__ void __launch_bounds__(256) k_tc_gather_cand(const int32_t* __restrict__ list1, const int32_t* __restrict__ count1,
+                                                        int Dp1, const float* __restrict__ x1, const float* __restrict__ xnorm,
+                                                        const float* __restrict__ xdnorm, const float* __restrict__ best,
+                                                        float* __restrict__ gx1, float* __restrict__ gnorm,
+                                                        float* __restrict__ gdnorm, float* __restrict__ gseed) {
+  const int n = count1[0];
+  const int wpg = (gridDim.x * blockDim.x) >> 5;
+  for (int slot = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; slot < n; slot += wpg) {
+    const int64_t r = list1[slot];
+    const float4* a = reinterpret_cast<const float4*>(x1 + r * Dp1);
+    float4* g = reinterpret_cast<float4*>(gx1 + (int64_t)slot * Dp1);
+    for (int c = lane_id(); c < (Dp1 >> 2); c += 32) g[c] = __ldg(a + c);
+    if (lane_id() == 0) {
+      gnorm[slot] = xnorm[r];
+      gdnorm[slot] = xdnorm[r];
+      gseed[slot] = best[r];
+    }
+  }
+}
+
+// cand_ctr: [0] fallback rows, [1] candidate rows whose exact margin lies inside the band, [2] rows decided on their
+// candidates, [3] rows whose list overflowed, [4..5] recorded entries (uint64)
+constexpr int TC_CAND_CTRS = 6;
+
+// one warp per compacted row: merge the two half lists, filter, exact re-score of the kept centres, label.  The row and
+// up to RS_BATCH kept centre rows are staged in shared memory by the whole warp (coalesced, all loads in flight), then
+// one lane per kept centre runs the exact chain from there.
+constexpr int RS_BATCH = 8;
+constexpr int RS_LD = 132;   // floats per staged row (D <= 128; rows 4 banks apart)
+__global__ void __launch_bounds__(256) k_tc_cand_resolve(
+    const int32_t* __restrict__ list1, const int32_t* __restrict__ count1, const int2* __restrict__ cand,
+    const int32_t* __restrict__ cand_n, int cap, const float* __restrict__ gseed, const float* __restrict__ gnorm,
+    const float* __restrict__ gdnorm, int D, const float* __restrict__ X, int64_t ldx, const float* __restrict__ C,
+    int64_t ldc, const float* __restrict__ cnorm, const float* __restrict__ cnorm_sqrt, const float* __restrict__ cdnorm,
+    const float* __restrict__ cmax, float band, int32_t* __restrict__ labels, const int32_t* __restrict__ labels_prev,
+    int32_t* __restrict__ n_changed, int32_t* __restrict__ list2, int32_t* __restrict__ ctr) {
+  __shared__ __align__(16) float s_rows[8][(1 + RS_BATCH) * RS_LD];   // per warp: [0] x row, [1 + b] kept centre b
+  __shared__ int s_j[8][32];                                          // per warp: kept centres
+  const int n = count1[0];
+  const int lane = lane_id();
+  const int wpg = (gridDim.x * blockDim.x) >> 5;
+  float* sx = s_rows[threadIdx.x >> 5];
+  float* sc = sx + RS_LD;
+  int* sj = s_j[threadIdx.x >> 5];
+  const int D4 = (D + 3) >> 2;   // rows of X and C are 16-byte aligned with ld % 4 == 0
+  int changed = 0;
+  for (int slot = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; slot < n; slot += wpg) {
+    const int32_t row = list1[slot];
+    const int n0 = cand_n[2 * slot], n1 = cand_n[2 * slot + 1];
+    bool fallback = n0 > cap || n1 > cap || n0 + n1 == 0;
+    // lane holds merged entries lane and lane + 32 (half 0 first; 2 cap <= 64)
+    unsigned long long key[2] = {~0ull, ~0ull};
+    if (!fallback) {
+#pragma unroll
+      for (int h = 0; h < 2; ++h) {
+        const int e = lane + 32 * h;
+        if (e < n0 + n1) {
+          const int2 p = e < n0 ? cand[(int64_t)(2 * slot) * cap + e] : cand[(int64_t)(2 * slot + 1) * cap + (e - n0)];
+          key[h] = rf_pack(__int_as_float(p.y), p.x);
+        }
+      }
+    }
+    if (lane == 0 && !fallback) atomicAdd(reinterpret_cast<unsigned long long*>(ctr + 4), (unsigned long long)(n0 + n1));
+    unsigned long long kmin = key[0] < key[1] ? key[0] : key[1];
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const unsigned long long other = __shfl_xor_sync(0xffffffffu, kmin, o);
+      kmin = other < kmin ? other : kmin;
+    }
+    const int l = (int)(unsigned)(kmin & 0xffffffffull);
+    const float b = rf_unpack(kmin);
+    const float xn = gnorm[slot], cm = cmax[0];
+    if (!fallback && !(b <= gseed[slot] + tc_cand_slack(xn, cm))) fallback = true;   // also catches NaN
+    if (fallback) {
+      if (lane == 0) {
+        list2[atomicAdd(ctr, 1)] = row;
+        if (n0 > cap || n1 > cap) atomicAdd(ctr + 3, 1);
+      }
+      continue;
+    }
+    // tol(i, l) of k_tc_select1 without its last term, which is taken per candidate below
+    const float cr = cnorm_sqrt[l];
+    const float E = gdnorm[slot] * cr + xn * (cdnorm[l] + 3.0517578125e-05f * cr);
+    const float tol0 = 2.02f * (E + 1.52587890625e-05f * cnorm[l]) + band * xn * cm;
+    bool keep[2];
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const float d = rf_unpack(key[h]);
+      const float tol = tol0 + 4.76837158e-07f * fmaxf(fabsf(b), fabsf(d));
+      keep[h] = key[h] != ~0ull && !(d - b > tol);   // an excluded centre loses to l in the exact chain
+    }
+    const unsigned m0 = __ballot_sync(0xffffffffu, keep[0]), m1 = __ballot_sync(0xffffffffu, keep[1]);
+    const unsigned lt = (1u << lane) - 1u;
+    __syncwarp();   // the previous row's chains have read sx / sc / sj
+    if (keep[0]) sj[__popc(m0 & lt)] = (int)(unsigned)(key[0] & 0xffffffffull);
+    if (keep[1]) sj[__popc(m0) + __popc(m1 & lt)] = (int)(unsigned)(key[1] & 0xffffffffull);
+    for (int q = lane; q < D4; q += 32)
+      reinterpret_cast<float4*>(sx)[q] = __ldg(reinterpret_cast<const float4*>(X + (int64_t)row * ldx) + q);
+    const int nk = __popc(m0) + __popc(m1);
+    unsigned long long k1 = ~0ull, k2 = ~0ull;   // two smallest exact keys of this lane
+    for (int t0 = 0; t0 < nk; t0 += RS_BATCH) {
+      const int nb = min(RS_BATCH, nk - t0);
+      __syncwarp();
+      for (int bb = 0; bb < nb; ++bb) {
+        const float4* c4 = reinterpret_cast<const float4*>(C + (int64_t)sj[t0 + bb] * ldc);
+        for (int q = lane; q < D4; q += 32) reinterpret_cast<float4*>(sc + bb * RS_LD)[q] = __ldg(c4 + q);
+      }
+      __syncwarp();
+      if (lane < nb) {
+        const int j = sj[t0 + lane];
+        const float* c = sc + lane * RS_LD;
+        float acc = 0.f;
+#pragma unroll 4
+        for (int k = 0; k < D; ++k) acc = ed_chain(acc, sx[k], c[k]);
+        const float dist = ed_finish(acc, cnorm[j]);
+        const unsigned long long kk = dist == dist ? rf_pack(dist, j) : ~0ull;
+        if (kk < k1) {
+          k2 = k1;
+          k1 = kk;
+        } else if (kk < k2) {
+          k2 = kk;
+        }
+      }
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) {
+      const unsigned long long o1 = __shfl_xor_sync(0xffffffffu, k1, o), o2 = __shfl_xor_sync(0xffffffffu, k2, o);
+      const unsigned long long lo = k1 < o1 ? k1 : o1, hi = k1 < o1 ? o1 : k1;
+      const unsigned long long s2 = k2 < o2 ? k2 : o2;
+      k1 = lo;
+      k2 = hi < s2 ? hi : s2;
+    }
+    if (k1 == ~0ull) {   // no finite exact distance: leave the row to the full exact path
+      if (lane == 0) list2[atomicAdd(ctr, 1)] = row;
+      continue;
+    }
+    if (lane == 0) {
+      const int lab = (int)(unsigned)(k1 & 0xffffffffull);
+      labels[row] = lab;
+      if (labels_prev && labels_prev[row] != lab) ++changed;
+      const float d1 = rf_unpack(k1), d2 = k2 == ~0ull ? INFINITY : rf_unpack(k2);
+      if (!(d2 - d1 > band * xn * cm)) atomicAdd(ctr + 1, 1);
+      atomicAdd(ctr + 2, 1);
+    }
+  }
+  if (n_changed) {
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) changed += __shfl_xor_sync(0xffffffffu, changed, o);
+    if (lane == 0 && changed) atomicAdd(n_changed, changed);
+  }
+}
+
+// *dst += *src (the candidate rows' band count joins the re-scored rows' count in *n_refined)
+__global__ void k_add_i32(int32_t* __restrict__ dst, const int32_t* __restrict__ src) { *dst += *src; }
+
 // second-level decision on the compacted rows (slot -> row through list1): same band as k_tc_select
 __global__ void __launch_bounds__(256) k_tc_select2(const int32_t* __restrict__ list1, const int32_t* __restrict__ count1,
                                                     const float* __restrict__ best, const float* __restrict__ second,
@@ -1533,6 +1790,11 @@ constexpr int TC_AUG = 4;   // augmented columns of the first-level operands
 static inline int dpad1(int64_t D) { return (int)align_up(D + TC_AUG, TC_BK); }
 constexpr int TC_KPAD = 256;   // centres padded to the widest accumulator tile
 constexpr int TC_TS_BN = 192;  // accumulator width of the A-in-TMEM first level (its last tile may reach past Kp)
+// candidates recorded per row and column half.  tools/cand_estimate.py, config-E-shaped data after one Lloyd update,
+// 20 000-row sample: 3.7 % (D = 100) / 3.0 % (D = 47) of the rows undecided, 2.2 recorded per row on average, at most 4
+// in one column half (profiles/r3_cand_estimate_configE.txt): 16 leaves ample room at 256 bytes of list per row
+constexpr int TC_CAND_CAP = 16;
+static_assert(TC_CAND_CAP <= 32, "k_tc_cand_resolve holds the two half lists in two entries per lane");
 
 int64_t kmeans_tc_xsplit_bytes(int64_t N, int64_t D) {
   return 2 * ws_need(N * dpad(D), 4) + 2 * ws_need(N, 4) + ws_need(N * dpad1(D), 4) + 256;
@@ -1577,7 +1839,9 @@ int64_t kmeans_assign_tc_ws_bytes(int64_t N, int64_t K, int64_t D) {
          3 * ws_need(Kp, 4) /*|c|^2, |c|, |c - tf32(c)|*/ + 256 /*cmax*/ +
          3 * ws_need(N, 4) /*best, second, idx*/ + ws_need(N, 4) /*amb list*/ + ws_need(N, 8) /*amb packed*/ +
          256 /*amb count*/ + ws_need(N, 4) /*second-level list*/ + 256 /*its count*/ +
-         2 * ws_need(N * Dp, 4) + ws_need(N, 4) /*compacted hi, lo, |x|*/ + 256;
+         2 * ws_need(N * Dp, 4) + ws_need(N, 4) /*compacted hi, lo, |x|*/ + 2 * ws_need(N, 4) /*compacted |dx|, seed*/ +
+         ws_need(2 * N, 4) + ws_need(2 * N * TC_CAND_CAP, 8) /*candidate counts, lists*/ + ws_need(N, 4) /*fallback list*/ +
+         256 /*candidate counters*/ + 256;
 }
 
 // D_eff = contraction width (D, or D + 4 for the augmented first level); nkb = its 32-float K-blocks
@@ -1604,6 +1868,28 @@ static int launch_assign_tc(const CUtensorMap& m_xhi, const CUtensorMap& m_xlo, 
   const int grid = (int)(tiles < sms ? tiles : sms);
   k_assign_tc<NPASS, BN, SUB><<<grid, TC_THREADS, Cfg::total(nkb), s>>>(m_xhi, m_xlo, m_chi, m_clo, N_max, n_rows_dev, D_eff,
                                                                   (int)(Kp / BN), nkb, cnorm, best, second, idx, g_tc_ablate, gate);
+  GDR_LAUNCHED();
+  return GDR_OK;
+}
+
+static int launch_tc_cand(const CUtensorMap& m_x1, const CUtensorMap& m_c1, int64_t N_max, const int32_t* n_rows_dev,
+                          int D_eff, int64_t Kp, int nkb, TcGate gate, TcCand cand, cudaStream_t s) {
+  using Cfg = TcCfg<1, 256, 1>;
+  static PerDevice<bool> attr_set_dev;
+  bool& attr_set = attr_set_dev.get();
+  if (!attr_set) {
+    GDR_CUDA(cudaFuncSetAttribute(k_tc_cand, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_LIMIT));
+    attr_set = true;
+  }
+  int sms = kSMs;
+  {
+    int dev = 0;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
+  }
+  const int64_t tiles = cdiv(N_max, TC_BM);
+  const int grid = (int)(tiles < sms ? tiles : sms);
+  k_tc_cand<<<grid, TC_THREADS, Cfg::total(nkb), s>>>(m_x1, m_c1, N_max, n_rows_dev, D_eff, (int)(Kp / 256), nkb, gate, cand);
   GDR_LAUNCHED();
   return GDR_OK;
 }
@@ -1711,6 +1997,12 @@ int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_
   float* g_hi = W.take<float>(N * Dp);
   float* g_lo = W.take<float>(N * Dp);
   float* g_norm = W.take<float>(N);
+  float* g_dnorm = W.take<float>(N);
+  float* g_seed = W.take<float>(N);
+  int32_t* cand_n = W.take<int32_t>(2 * N);
+  int2* cand_list = W.take<int2>(2 * N * TC_CAND_CAP);
+  int32_t* list2 = W.take<int32_t>(N);
+  int32_t* cand_ctr = W.take<int32_t>(TC_CAND_CTRS);
   int32_t* amb_count = n_refined_dev ? n_refined_dev : amb_count_ws;
   if (!W.ok()) {
     set_error("kmeans_assign(tc): workspace too small");
@@ -1722,7 +2014,8 @@ int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_
                                                            two_level ? c1 : nullptr, Dp1, 2, cdnorm);
   GDR_LAUNCHED();
   int rc;
-  k_cnorm_finish<<<1, 1024, 0, s>>>(K, Kp, cnorm, two_level ? cdnorm : nullptr, cnorm_sqrt, cmax, amb_count, count1);
+  k_cnorm_finish<<<1, 1024, 0, s>>>(K, Kp, cnorm, two_level ? cdnorm : nullptr, cnorm_sqrt, cmax, amb_count, count1,
+                                    two_level ? cand_ctr : nullptr, TC_CAND_CTRS);
   GDR_LAUNCHED();
 
   CUtensorMap m_xhi, m_xlo, m_chi, m_clo;
@@ -1746,6 +2039,7 @@ int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_
     // the profile scope spans the whole tensor-core screen: level 1, decision, compaction, level 2
     ProfileScope prof(PROF_ASSIGN, s);
     CUtensorMap m_x1, m_c1;
+    bool cand_level = false;   // second level on candidate centres (default screen only)
     if ((rc = make_map(&m_x1, xs.x1, N, Dp1, TC_BM))) return rc;
     if (g_tc_screen == 2) {
       if ((rc = make_map(&m_c1, c1, Kp, Dp1, 128))) return rc;
@@ -1764,6 +2058,7 @@ int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_
       // whether A comes from shared or tensor memory, and 192-centre tiles pay the per-tile hand-shakes 53 times instead of 40
       const int ka = (int)align_up(D + TC_AUG, 8);
       const int ts_bn = (g_tc_screen == 6 && ka <= 512 - 2 * TC_TS_BN) ? TC_TS_BN : 0;
+      cand_level = g_tc_cand != 0 && ts_bn == 0;
       const int64_t k_rows = ts_bn == TC_TS_BN ? align_up(K, TC_TS_BN) : Kp;
       if (k_rows > Kp) {
         k_pad_aug<<<(unsigned)cdiv((k_rows - Kp) * Dp1, 256), 256, 0, s>>>(c1, Kp, k_rows, Dp1, (int)D);
@@ -1797,21 +2092,47 @@ int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_
                                                        cdnorm, cmax, TC_BAND, labels, labels_prev, n_changed_dev,
                                                        list1, count1);
     GDR_LAUNCHED();
-    k_tc_gather<<<4 * kSMs, 256, 0, s>>>(list1, count1, Dp, xs.hi, xs.lo, xs.norm, g_hi, g_lo, g_norm);
+    // rows (and their count, on the device) that take the 3xTF32 level over all centres
+    const int32_t* list_f = list1;
+    const int32_t* count_f = count1;
+    g_last_cand = cand_level ? cand_ctr : nullptr;
+    if (cand_level) {
+      float* g_x1 = g_hi;   // N Dp1 <= 2 N Dp floats: g_hi and g_lo are free until the fallback gathers into them
+      k_tc_gather_cand<<<4 * kSMs, 256, 0, s>>>(list1, count1, Dp1, xs.x1, xs.norm, xs.dnorm, best, g_x1, g_norm, g_dnorm,
+                                                g_seed);
+      GDR_LAUNCHED();
+      CUtensorMap m_gx1;
+      if ((rc = make_map(&m_gx1, g_x1, N, Dp1, TC_BM))) return rc;
+      const int cap = g_tc_cand_cap > 0 ? std::min(g_tc_cand_cap, TC_CAND_CAP) : TC_CAND_CAP;
+      if ((rc = launch_tc_cand(m_gx1, m_c1, N, count1, (int)D + TC_AUG, Kp, nkb1, TcGate{g_norm, g_dnorm, cmax, g_seed, TC_BAND},
+                               TcCand{cand_list, cand_n, cap}, s)))
+        return rc;
+      k_tc_cand_resolve<<<4 * kSMs, 256, 0, s>>>(list1, count1, cand_list, cand_n, cap, g_seed, g_norm, g_dnorm, (int)D, X, ldx,
+                                                 C, ldc, cnorm, cnorm_sqrt, cdnorm, cmax, TC_BAND, labels, labels_prev,
+                                                 n_changed_dev, list2, cand_ctr);
+      GDR_LAUNCHED();
+      list_f = list2;
+      count_f = cand_ctr;   // [0]: fallback rows
+    }
+    k_tc_gather<<<4 * kSMs, 256, 0, s>>>(list_f, count_f, Dp, xs.hi, xs.lo, xs.norm, g_hi, g_lo, g_norm);
     GDR_LAUNCHED();
     CUtensorMap m_ghi, m_glo;
     if ((rc = make_map(&m_ghi, g_hi, N, Dp, TC_BM))) return rc;
     if ((rc = make_map(&m_glo, g_lo, N, Dp, TC_BM))) return rc;
-    if ((rc = launch_assign_tc<3, 128, 1>(m_ghi, m_glo, m_chi, m_clo, N, count1, (int)D, Kp, nkb, cnorm, best, second, idx,
+    if ((rc = launch_assign_tc<3, 128, 1>(m_ghi, m_glo, m_chi, m_clo, N, count_f, (int)D, Kp, nkb, cnorm, best, second, idx,
                                        s)))
       return rc;
-    k_tc_select2<<<2 * kSMs, 256, 0, s>>>(list1, count1, best, second, idx, g_norm, cmax, TC_BAND, labels,
+    k_tc_select2<<<2 * kSMs, 256, 0, s>>>(list_f, count_f, best, second, idx, g_norm, cmax, TC_BAND, labels,
                                          labels_prev, n_changed_dev, amb_list, amb_count, amb_packed);
     GDR_LAUNCHED();
   }
   // exact fp32 re-score of the ambiguous rows (list length stays on the device)
-  return launch_assign_simt_rows(N, K, D, X, ldx, c_t, Kp, cnorm, amb_list, amb_count, amb_packed, labels,
-                                 labels_prev, n_changed_dev, best_out, s);
+  rc = launch_assign_simt_rows(N, K, D, X, ldx, c_t, Kp, cnorm, amb_list, amb_count, amb_packed, labels, labels_prev,
+                               n_changed_dev, best_out, s);
+  if (rc || !two_level || !g_last_cand || !n_refined_dev) return rc;
+  k_add_i32<<<1, 1, 0, s>>>(n_refined_dev, cand_ctr + 1);   // + candidate rows whose exact margin lies in the band
+  GDR_LAUNCHED();
+  return GDR_OK;
 }
 
 // gdr_kmeans_assign(precision_mode = 1): split X into the tail of the workspace, then run
@@ -1858,6 +2179,15 @@ int gdr_debug_get(const char* key, int64_t* value_host) {
     int32_t v = -1;
     if (gdr::g_last_count1) GDR_CUDA(cudaMemcpy(&v, gdr::g_last_count1, 4, cudaMemcpyDeviceToHost));
     *value_host = v;
+    return GDR_OK;
+  }
+  if (!strcmp(key, "tc_cand_rows") || !strcmp(key, "tc_cand_overflow_rows") || !strcmp(key, "tc_cand_entries")) {
+    int32_t h[gdr::TC_CAND_CTRS];
+    for (int i = 0; i < gdr::TC_CAND_CTRS; ++i) h[i] = -1;
+    if (gdr::g_last_cand) GDR_CUDA(cudaMemcpy(h, gdr::g_last_cand, sizeof(h), cudaMemcpyDeviceToHost));
+    long long e = -1;
+    if (gdr::g_last_cand) memcpy(&e, h + 4, 8);
+    *value_host = !strcmp(key, "tc_cand_rows") ? h[2] : (!strcmp(key, "tc_cand_overflow_rows") ? h[3] : e);
     return GDR_OK;
   }
   if (!strcmp(key, "topk_overflow_rows")) {

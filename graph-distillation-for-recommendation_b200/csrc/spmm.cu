@@ -43,6 +43,8 @@ static int g_spmm_split = 0;      // number of column windows (1, 2, 4)
 extern int g_lloyd_graph;         // lloyd.cu
 extern int g_tc_screen;           // kmeans_tc.cu
 extern int g_tc_gate;             // kmeans_tc.cu
+extern int g_tc_cand;             // kmeans_tc.cu
+extern int g_tc_cand_cap;         // kmeans_tc.cu
 extern int g_coarsen_dense;       // graph.cu
 extern int g_rs_match;            // primitives.cu
 extern int g_rs_max_bits;         // primitives.cu
@@ -449,6 +451,8 @@ int gdr_debug_set(const char* key, int value) {
   else if (!strcmp(key, "coarsen_dense")) gdr::g_coarsen_dense = value;
   else if (!strcmp(key, "tc_ablate")) gdr::g_tc_ablate = value;
   else if (!strcmp(key, "tc_gate")) gdr::g_tc_gate = value;
+  else if (!strcmp(key, "tc_cand")) gdr::g_tc_cand = value;
+  else if (!strcmp(key, "tc_cand_cap")) gdr::g_tc_cand_cap = value;
   else if (!strcmp(key, "rs_match")) gdr::g_rs_match = value;
   else if (!strcmp(key, "rs_max_bits")) gdr::g_rs_max_bits = value;
   else if (!strcmp(key, "sparsify_batch")) g_sparsify_batch_cap = value;

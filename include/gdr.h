@@ -71,14 +71,19 @@ int gdr_profile_collect(double* total_ms_host, int64_t* launches_host);
  * inputs], 4: CTA pairs with 2-SM TMA, 5: CTA pairs with forwarded 1-SM TMA), "tc_ablate" (role ablations of the
  * first-level kernel for tools/estep_probe.py / tools/mma_rate_probe.py; results are garbage while it is set);
  * "tc_gate" (first-level epilogue gate of the two-level screen: 0 off, 1 [default] on the running best, 2 also seeded
- * with the previous label's score; every setting produces the same labels);
+ * with the previous label's score; every setting produces the same labels); "tc_cand" (second level of the default
+ * two-level screen: 1 [default] seeded 1xTF32 candidate pass + exact re-score of the candidates, 0 3xTF32 over all
+ * centres; same labels); "tc_cand_cap" (candidate list capacity per row and column half, 1..16; 0 = 16);
  * "rs_match" (radix-sort ranking: 0 [default] per-bit warp ballots, 1 MATCH.ANY); "topk_path" (gdr_topk_scores: 1 exact
  * SIMT path, 2 tensor-core screen);
  * "topk_condensed_path" (gdr_topk_condensed: 1 every row on the exact fallback);
  * value 0 / -1 = automatic. */
 int gdr_debug_set(const char* key, int value);
 /* Debug read-back (synchronises the device).  keys: "tc_level2_rows" = rows the last two-level
- * tensor-core screen (gdr_kmeans_assign_tc) handed to its 3xTF32 second level; -1 if none ran.
+ * tensor-core screen (gdr_kmeans_assign_tc) left undecided after its first level; -1 if none ran.
+ * "tc_cand_rows" / "tc_cand_overflow_rows" / "tc_cand_entries" = of those, the rows the last run decided on their
+ * candidate centres / the rows whose candidate list overflowed (they took the 3xTF32 fallback) / the candidates
+ * recorded for the rows read (-1 if the last two-level run did not use candidate lists).
  * "topk_overflow_rows" = rows the last tensor-core gdr_topk_scores finished on the exact path; -1 if none ran.
  * "topk_condensed_fallback_rows" = rows the last gdr_topk_condensed finished on the exact path; -1 if it wrote
  * nothing. */
@@ -303,7 +308,9 @@ int     gdr_kmeans_assign(int64_t N, int64_t K, int64_t D,
  *   prepare: X -> (X_hi, X_lo) TF32 pair, rows zero-padded to a multiple of 32 floats, + |x_i|.
  *   assign_tc: 3xTF32 tcgen05/TMA GEMM with fused |c|^2 add and (best, second, argmin)
  *   epilogue; rows whose margin second-best is within 2^-15 |x_i| max|c_j| are re-scored by
- *   the exact fp32 kernel.  *n_refined_dev (nullable) receives how many rows that was.
+ *   the exact fp32 kernel.  *n_refined_dev (nullable) receives how many rows have their margin between the
+ *   two nearest centres within that band: judged on the exact fp32 distances for the rows the two-level screen
+ *   decides on candidate centres, on the 3xTF32 distances for every other row.
  *   Supports D <= 128 (GDR_EUNSUPPORTED otherwise). */
 int64_t gdr_kmeans_tc_xsplit_bytes(int64_t N, int64_t D);
 int     gdr_kmeans_tc_prepare(int64_t N, int64_t D, const float* X, int64_t ldx,
