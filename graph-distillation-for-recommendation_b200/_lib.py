@@ -83,6 +83,8 @@ _SIGNATURES = {
     "gdr_kmeans_lloyd": (i32, [i64, i64, i64, vp, i64, vp, i64, vp, i32, C.c_double, i32, vp, vp, vp, i32, vp, i64, vp]),
     "gdr_kmeans_plusplus_ws_bytes": (i64, [i64, i64, i64, i32]),
     "gdr_kmeans_plusplus": (i32, [i64, i64, i64, vp, i64, i64, vp, i32, vp, i64, vp, vp, i64, vp]),
+    "gdr_kmeans_plusplus_dist_ws_bytes": (i64, [i64, i64, i64, i32, i32]),
+    "gdr_kmeans_plusplus_dist": (i32, [vp, i64, i64, i64, vp, i64, i64, vp, i32, vp, i64, vp, vp, i64, vp]),
     "gdr_minibatch_update": (i32, [i64, i64, i64, vp, i64, vp, vp, i64, vp, i64, vp, vp]),
     "gdr_segment_sum_ws_bytes": (i64, [i64, i64, i64]),
     "gdr_segment_sum": (i32, [i64, i64, i64, vp, i64, vp, vp, i64, vp, vp, i64, vp]),

@@ -41,6 +41,7 @@ static int g_spmm_unroll = 0;     // 4 or 8
 static int g_spmm_hints = -1;     // 0 off, 1 streaming hints on colidx/vals/T/Y
 static int g_spmm_split = 0;      // number of column windows (1, 2, 4)
 extern int g_lloyd_graph;         // lloyd.cu
+extern int g_kpp_skip_score;      // kmeans_init.cu
 extern int g_tc_screen;           // kmeans_tc.cu
 extern int g_tc_gate;             // kmeans_tc.cu
 extern int g_tc_cand;             // kmeans_tc.cu
@@ -445,6 +446,7 @@ int gdr_debug_set(const char* key, int value) {
   else if (!strcmp(key, "spmm_hints")) gdr::g_spmm_hints = value;
   else if (!strcmp(key, "spmm_split")) gdr::g_spmm_split = value;
   else if (!strcmp(key, "lloyd_graph")) gdr::g_lloyd_graph = value;
+  else if (!strcmp(key, "kpp_dist_skip_score")) gdr::g_kpp_skip_score = value;
   else if (!strcmp(key, "tc_screen")) gdr::g_tc_screen = value;
   else if (!strcmp(key, "topk_path")) gdr::g_topk_path = value;
   else if (!strcmp(key, "topk_condensed_path")) gdr::g_topk_condensed_path = value;

@@ -623,6 +623,20 @@ class CudaOps:
         self.last_info = (bool(info[0]), int(info[1]))
         return labels, float(inertia.value), centers, int(n_iter.value)
 
+    def kmeans_plusplus_dist(self, comm, Xc, n_clusters, first, rand, n_trials):
+        """k-means++ seeding of the row-partitioned Xc (gdr_kmeans_plusplus_dist; collective).  Returns the replicated
+        centres [K, D] (padded rows) and their global row ids."""
+        n_local, D = Xc.shape
+        K = int(n_clusters)
+        dev = Xc.device
+        centers = self.new_padded(K, D, dev, zero=True)
+        indices = torch.empty(K, dtype=torch.int64, device=dev)
+        ws = self.workspace(self._lib.query("gdr_kmeans_plusplus_dist_ws_bytes", n_local, K, D, n_trials, comm.world), dev)
+        self._lib.call("gdr_kmeans_plusplus_dist", comm.lib_handle(), n_local, K, D, self.ptr(Xc) if n_local else 0,
+                       Xc.stride(0) if n_local else self._pad4(D), int(first), rand.ctypes.data, int(n_trials),
+                       self.ptr(centers), centers.stride(0), self.ptr(indices), self.ptr(ws), ws.numel(), self.stream())
+        return centers, indices
+
     @staticmethod
     def _pad4(d):
         return (int(d) + 3) // 4 * 4
@@ -1018,13 +1032,33 @@ def _propagate_row_chunks(comm, part, A_local, x, target, T, alpha, one_minus, o
 # ------------------------------------------------------------------------------------------
 # stage 3
 # ------------------------------------------------------------------------------------------
+def dist_kmeans_plusplus(comm: Comm, part: RowPartition, Xc_local: torch.Tensor, n_clusters: int, random_state,
+                         ops=None, return_indices: bool = False):
+    """k-means++ seeding (sklearn's ``_kmeans_plusplus``) of the row-partitioned ``Xc_local`` without gathering X.
+    Collective.  ``part.n`` is the global row count; the ranks' blocks in rank order are the global rows.  The host
+    draws are ``kmeans_init.kmeans_plusplus_device``'s (one ``choice``, then ``uniform(size=n_local_trials)`` per
+    round), so every rank must pass the same ``random_state``; a mismatch raises GdrError on every rank.  With one rank
+    the result is bit-identical to ``kmeans_plusplus_device``; with more, only the fp64 potentials are grouped by rank.
+    Returns the replicated centres [K, D] (and their global row ids with ``return_indices``)."""
+    from .kmeans_init import draw_plusplus
+    ops = ops or CudaOps()
+    if not hasattr(ops, "kmeans_plusplus_dist"):
+        raise NotImplementedError(f"{type(ops).__name__} has no distributed k-means++ seeding")
+    first, rand, n_trials = draw_plusplus(random_state, int(part.n), int(n_clusters))
+    centers, indices = ops.kmeans_plusplus_dist(comm, Xc_local, n_clusters, first, rand, n_trials)
+    return (centers, indices) if return_indices else centers
+
+
 class DistKMeans:
-    """Lloyd k-means on row-partitioned X with replicated centres (init must be an array that
-    is identical on every rank)."""
+    """Lloyd k-means on row-partitioned X with replicated centres.  ``init`` is an array identical on every rank,
+    "k-means++" (greedy D^2 seeding of the centred rows, ``dist_kmeans_plusplus``) or "random" (the centred rows
+    ``RandomState(random_state).permutation(N)[:K]``, copied from their owners).  A string init needs the same
+    ``random_state`` (seed or RandomState) on every rank; one init per fit."""
 
     def __init__(self, n_clusters: int, init, max_iter: int = 300, tol: float = 1e-4, ops=None, comm: Comm = None,
-                 verbose: bool = False, python_loop: bool = False):
+                 verbose: bool = False, python_loop: bool = False, random_state=None):
         self.n_clusters, self.init, self.max_iter, self.tol = int(n_clusters), init, int(max_iter), tol
+        self.random_state = random_state
         self.ops = ops or CudaOps()
         self.comm = comm or Comm()
         self.verbose = verbose
@@ -1032,6 +1066,13 @@ class DistKMeans:
 
     def fit(self, X_local: torch.Tensor):
         ops, comm, K = self.ops, self.comm, self.n_clusters
+        if isinstance(self.init, str):
+            if self.init not in ("k-means++", "random"):
+                raise ValueError(f"init should be 'k-means++', 'random' or an array, got {self.init!r}")
+            if self.random_state is None:
+                raise ValueError("a string init needs the same random_state on every rank")
+            if not hasattr(ops, "kmeans_plusplus_dist"):
+                raise NotImplementedError(f"{type(ops).__name__} has no distributed init {self.init!r}")
         X = ops.prep_rows(X_local)
         n_local, D = X.shape
         dev = X.device
@@ -1047,22 +1088,26 @@ class DistKMeans:
         mean = m64.to(torch.float32)
         tol_abs = 0.0 if self.tol == 0 else var_mean * float(self.tol)
         Xc = ops.center(X, mean)
-        C0 = torch.as_tensor(np.asarray(self.init) if not isinstance(self.init, torch.Tensor) else self.init,
-                             dtype=torch.float32).to(dev)
-        if tuple(C0.shape) != (K, D):
-            raise ValueError("init has the wrong shape")
+        if isinstance(self.init, str):
+            C0c = self._string_init(Xc, N)
+        else:
+            C0 = torch.as_tensor(np.asarray(self.init) if not isinstance(self.init, torch.Tensor) else self.init,
+                                 dtype=torch.float32).to(dev)
+            if tuple(C0.shape) != (K, D):
+                raise ValueError("init has the wrong shape")
+            C0c = ops.centers_like(C0 - mean, dev)
         if hasattr(ops, "lloyd_native") and (comm.world == 1 or comm.backend == "nccl") and not self.python_loop:
-            lab, inertia, cen, n_iter = ops.lloyd_native(comm, Xc, N, ops.centers_like(C0 - mean, dev), self.max_iter,
-                                                         tol_abs, self.verbose)
+            lab, inertia, cen, n_iter = ops.lloyd_native(comm, Xc, N, C0c, self.max_iter, tol_abs, self.verbose)
             self.labels_ = lab
             self.cluster_centers_ = (cen + mean).contiguous()
             self.inertia_ = inertia
             self.n_iter_ = n_iter
             self._centers_centered, self._mean = cen, mean
             return self
-        centers = [ops.centers_like(C0 - mean, dev), ops.centers_like(torch.zeros_like(C0), dev)]
+        zeros = torch.zeros((K, D), dtype=torch.float32, device=dev)
+        centers = [C0c, ops.centers_like(zeros, dev)]
         labels = [torch.full((n_local,), -1, dtype=torch.int32, device=dev) for _ in range(2)]
-        psums = ops.centers_like(torch.zeros_like(C0), dev)
+        psums = ops.centers_like(zeros, dev)
         ints = torch.zeros(K + 1, dtype=torch.int32, device=dev)   # [counts | n_changed]
         ops.prepare_kmeans(Xc, K)
         cur, nxt, ln, lo_ = 0, 1, 0, 1
@@ -1098,6 +1143,31 @@ class DistKMeans:
         self._centers_centered = centers[cur]
         self._mean = mean
         return self
+
+    def _string_init(self, Xc, N):
+        """Centred initial centres of a string init (replicated on every rank)."""
+        from .kmeans import _check_random_state
+        comm, ops, K = self.comm, self.ops, self.n_clusters
+        rs = _check_random_state(self.random_state)
+        if self.init == "k-means++":
+            return dist_kmeans_plusplus(comm, RowPartition(N, comm.world, comm.rank), Xc, K, rs, ops=ops)
+        # "random": every rank fills the chosen rows it owns; the owner's copy of each row is taken (never summed)
+        n_local, D = Xc.shape
+        dev = Xc.device
+        cnt = torch.tensor([[n_local]], dtype=torch.int64, device=dev)
+        counts = torch.empty((comm.world, 1), dtype=torch.int64, device=dev)
+        comm.all_gather_rows(cnt, counts)
+        offs = np.concatenate([[0], np.cumsum(counts.flatten().cpu().numpy())])
+        seeds = rs.permutation(N)[:K]
+        lo = int(offs[comm.rank])
+        mine = np.nonzero((seeds >= lo) & (seeds < lo + n_local))[0]
+        part = torch.zeros((K, D), dtype=torch.float32, device=dev)
+        if mine.size:
+            part[torch.from_numpy(mine).to(dev)] = Xc[torch.from_numpy(seeds[mine] - lo).to(dev)]
+        allp = torch.empty((comm.world * K, D), dtype=torch.float32, device=dev)
+        comm.all_gather_rows(part, allp)
+        owner = np.searchsorted(offs, seeds, side="right") - 1
+        return ops.centers_like(allp[torch.from_numpy(owner * K + np.arange(K)).to(dev)], dev)
 
     def _relocate(self, Xc, C_old, labels, sums, counts, part_lo):
         """_relocate_empty_clusters_dense across ranks: every rank proposes its n_empty farthest

@@ -613,6 +613,27 @@ int gdr_kmeans_lloyd_dist(gdr_comm_t* comm, int64_t N_local, int64_t N_total, in
                           int max_iter, double tol_abs, int precision_mode, double* inertia_out_host,
                           int32_t* n_iter_out_host, int32_t* info_out_host, int verbose, void* ws, int64_t ws_bytes,
                           gdr_stream_t stream);
+/* gdr_kmeans_plusplus on a row partition: the same greedy D^2 seeding without gathering X.  COLLECTIVE over comm.
+ * X_local = this rank's N_local rows (N_local = 0 allowed); the ranks' blocks in rank order are the global row order
+ * (the call all-gathers N_local once and derives every rank's row offset and N_total).  first_center and
+ * indices_out_dev hold global row ids.  Every rank passes the same first_center, n_trials, K, D and host draws
+ * (rand_vals_host as for gdr_kmeans_plusplus); this is checked at entry and a mismatch, or an argument any rank
+ * rejects, returns GDR_EINVAL on every rank.  Same checks as gdr_kmeans_plusplus: n_trials <= 16, K <= N_total, and
+ * the shared-memory plan for n_trials * D.  centers_out [K][ldc] (device) comes out bit-identical on every rank.
+ * Per round: the owner of each draw (first rank with rows whose prefix P_r + T_r reaches u * pot) finds the row with
+ * gdr_kmeans_plusplus's search and publishes it (all-gather A; the rows are copied, never summed); one pass over
+ * X_local scores all candidates; each rank's fp64 totals per candidate are all-gathered (B) and added in rank order.
+ * Every per-row fp32 distance has the one-GPU bits; only the fp64 totals are grouped by rank, so picks can differ
+ * from gdr_kmeans_plusplus only where a draw or a comparison of two candidate potentials falls within fp64 rounding.
+ * With one rank the indices and centres are bit-identical to gdr_kmeans_plusplus.  A draw no row reaches becomes row
+ * N_total - 1 (np.clip).  One round is captured into a CUDA graph and replayed.  Synchronises the stream twice: after
+ * the entry check and at the end. */
+int64_t gdr_kmeans_plusplus_dist_ws_bytes(int64_t N_local, int64_t K, int64_t D, int n_trials, int world);
+int     gdr_kmeans_plusplus_dist(gdr_comm_t* comm, int64_t N_local, int64_t K, int64_t D,
+                                 const float* X_local, int64_t ldx, int64_t first_center,
+                                 const double* rand_vals_host, int n_trials,
+                                 float* centers_out, int64_t ldc, int64_t* indices_out_dev,
+                                 void* ws, int64_t ws_bytes, gdr_stream_t stream);
 
 /* ---- dense fp64 steps of the truncated SVD embeddings (distill_recsys.py:124-155 compute_svd_embeddings; the reference
  * calls scipy's ARPACK svds on the host).  The block Krylov Rayleigh-Ritz of svd.py runs its sparse products on
