@@ -65,12 +65,17 @@ _SIGNATURES = {
     "gdr_row_sums_f32": (i32, [i64, vp, vp, vp, vp]),
     "gdr_er_lower": (i32, [i64, i64, vp, vp, vp, vp, vp, vp]),
     "gdr_edge_cosine_scale": (i32, [i64, i64, i64, vp, vp, vp, vp, i64, f32, vp, vp, vp]),
+    "gdr_er_lower_rows": (i32, [i64, i64, i64, vp, vp, vp, vp, vp, vp]),
+    "gdr_edge_cosine_scale_rows": (i32, [i64, i64, i64, i64, i64, vp, vp, vp, vp, i64, f32, vp, vp, vp]),
     "gdr_softmax_rows": (i32, [i64, i64, vp, i64, vp, i64, vp]),
     "gdr_class_edge_weight": (i32, [i64, i64, vp, vp, vp, vp, i64, i64, vp, vp]),
     "gdr_induced_subgraph_ws_bytes": (i64, [i64, i64]),
     "gdr_induced_subgraph_coo": (i32, [i64, vp, vp, vp, i64, vp, vp, vp, vp, vp, vp, i64, vp]),
     "gdr_sparsify_classes_ws_bytes": (i64, [i64, i64, i64]),
     "gdr_sparsify_classes": (i32, [i64, i64, i64, vp, vp, vp, vp, vp, i64, i64, vp, vp, vp, vp, vp, i64, vp]),
+    "gdr_sparsify_classes_dist_ws_bytes": (i64, [i64, i64, i64, i32]),
+    "gdr_sparsify_classes_dist": (i32, [vp, i64, i64, i64, i64, i64, vp, vp, vp, vp, vp, i64, i64, vp, vp, vp, vp, vp, i64,
+                                        vp]),
     "gdr_topk_filter_ws_bytes": (i64, [i64, i64]),
     "gdr_topk_filter_csr": (i32, [i64, i64, vp, vp, vp, vp, i64, vp, vp, vp, vp, vp, i64, vp]),
     "gdr_kmeans_assign_ws_bytes": (i64, [i64, i64, i64, i32]),

@@ -100,6 +100,18 @@ int comm_allreduce_f64(gdr_comm* c, double* buf, int64_t n, int op_max, cudaStre
   return GDR_OK;
 }
 
+int comm_allreduce_i64(gdr_comm* c, const int64_t* send, int64_t* recv, int64_t n, cudaStream_t s) {
+  if (!c || c->world == 1) {
+    if (send != recv && n > 0) GDR_CUDA(cudaMemcpyAsync(recv, send, (size_t)n * 8, cudaMemcpyDeviceToDevice, s));
+    return GDR_OK;
+  }
+  const NcclApi* api = nccl_api();
+  if (!api) return GDR_ECUDA;
+  GDR_NCCL(api->AllReduce(send, recv, (size_t)n, ncclInt64, ncclSum, c->nccl, s));
+  count_launch(1);
+  return GDR_OK;
+}
+
 int comm_allgather(gdr_comm* c, const void* send, void* recv, int64_t bytes_per_rank, cudaStream_t s) {
   if (!c || c->world == 1) {
     if (send != recv && bytes_per_rank > 0)

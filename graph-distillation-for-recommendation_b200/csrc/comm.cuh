@@ -43,6 +43,8 @@ const NcclApi* nccl_api();   // nullptr (+ error string) when libnccl cannot be 
 // [sums f32 | ints i32] summed over the ranks as ONE grouped NCCL operation (no-op for world 1 / null comm)
 int comm_allreduce_lloyd(gdr_comm* c, float* sums, int64_t n_floats, int32_t* ints, int64_t n_ints, cudaStream_t s);
 int comm_allreduce_f64(gdr_comm* c, double* buf, int64_t n, int op_max, cudaStream_t s);
+// int64 sums over the ranks, send -> recv (a copy for world 1 / null comm)
+int comm_allreduce_i64(gdr_comm* c, const int64_t* send, int64_t* recv, int64_t n, cudaStream_t s);
 int comm_allgather(gdr_comm* c, const void* send, void* recv, int64_t bytes_per_rank, cudaStream_t s);
 
 }  // namespace gdr

@@ -11,7 +11,10 @@
 // device: the k-th largest weight comes from a 4-pass radix select on the order-preserving integer
 // image of the fp32 weights, the selection is compacted with two scans (CSR order is kept, so the
 // output is a sorted CSR without any sort).  All of it is HBM-bound integer / elementwise work.
+#include <vector>
+
 #include "common.cuh"
+#include "comm.cuh"
 
 namespace gdr {
 
@@ -29,13 +32,13 @@ __global__ void k_row_sums(int64_t n, const int32_t* __restrict__ rowptr, const 
   }
 }
 
-// one warp per row: er[j] = v/deg[r] + v/deg[c]
-__global__ void __launch_bounds__(256) k_er_lower(int64_t n, const int32_t* __restrict__ rowptr,
+// one warp per row: er[j] = v/deg[row_lo + r] + v/deg[c]  (rows of a block starting at global row row_lo; deg global)
+__global__ void __launch_bounds__(256) k_er_lower(int64_t n, int64_t row_lo, const int32_t* __restrict__ rowptr,
                                                   const int32_t* __restrict__ colidx, const float* __restrict__ vals,
                                                   const float* __restrict__ deg, float* __restrict__ er) {
   int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (r >= n) return;
-  const float dr = deg[r];
+  const float dr = deg[row_lo + r];
   for (int j = rowptr[r] + lane_id(); j < rowptr[r + 1]; j += 32) {
     const float v = vals[j];
     er[j] = __fadd_rn(__fdiv_rn(v, dr), __fdiv_rn(v, deg[colidx[j]]));
@@ -52,8 +55,8 @@ __global__ void k_inv_norm(int64_t n, int C, const float* __restrict__ E, int64_
   }
 }
 
-// 8 lanes per edge: out[j] = vals[j] * cos(e_r, e_c)
-__global__ void __launch_bounds__(256) k_edge_cosine_scale(int64_t n, int C, const int32_t* __restrict__ rowptr,
+// 8 lanes per edge: out[j] = vals[j] * cos(e_{row_lo + r}, e_c)  (E and inv indexed by global row)
+__global__ void __launch_bounds__(256) k_edge_cosine_scale(int64_t n, int64_t row_lo, int C, const int32_t* __restrict__ rowptr,
                                                            const int32_t* __restrict__ colidx,
                                                            const float* __restrict__ vals,
                                                            const float* __restrict__ E, int64_t ld,
@@ -61,8 +64,8 @@ __global__ void __launch_bounds__(256) k_edge_cosine_scale(int64_t n, int C, con
   int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (r >= n) return;
   const int lane = lane_id(), g = lane >> 3, gl = lane & 7;
-  const float* er = E + r * ld;
-  const float ir = inv[r];
+  const float* er = E + (row_lo + r) * ld;
+  const float ir = inv[row_lo + r];
   const int b = rowptr[r], e = rowptr[r + 1];
   for (int j0 = b; j0 < e; j0 += 4) {
     const int j = j0 + g;
@@ -120,8 +123,7 @@ __device__ __forceinline__ uint32_t f32_key(float f) {
 struct SelState {
   uint32_t prefix;    // bytes of the k-th largest key fixed so far (high to low)
   uint32_t mask;      // which bits of prefix are fixed
-  int32_t k_rem;      // how many entries >= the final key are still to be taken among the candidates
-  int32_t pad;
+  int64_t k_rem;      // how many entries >= the final key are still to be taken among the candidates
 };
 
 __global__ void k_sel_init(SelState* st, int32_t* hist, int32_t k) {
@@ -206,7 +208,7 @@ __global__ void k_sel_compact(int64_t n_rows, int64_t nnz, const int32_t* __rest
 // traffic per pass — a launch, not a bandwidth problem — so the per-class loop of ~20 short launches
 // is replaced by ~20 launches per BATCH of classes.
 // ---------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) k_class_weight_b(int64_t n, int64_t nnz, const int32_t* __restrict__ rowptr,
+__global__ void __launch_bounds__(256) k_class_weight_b(int64_t n, int64_t nnz, int64_t row_lo, const int32_t* __restrict__ rowptr,
                                                         const int32_t* __restrict__ colidx, const float* __restrict__ er,
                                                         const float* __restrict__ P, int64_t ldp, int cls0,
                                                         float* __restrict__ w /*[classes][nnz]*/) {
@@ -214,12 +216,12 @@ __global__ void __launch_bounds__(256) k_class_weight_b(int64_t n, int64_t nnz, 
   if (r >= n) return;
   const int cls = cls0 + blockIdx.y;
   float* wc = w + (int64_t)blockIdx.y * nnz;
-  const float pr = P[r * ldp + cls];
+  const float pr = P[(row_lo + r) * ldp + cls];
   for (int j = rowptr[r] + lane_id(); j < rowptr[r + 1]; j += 32)
     wc[j] = __fmul_rn(__fmul_rn(pr, P[(int64_t)colidx[j] * ldp + cls]), er[j]);
 }
 
-__global__ void k_sel_init_b(SelState* st, int32_t* hist, int32_t k) {
+__global__ void k_sel_init_b(SelState* st, int32_t* hist, int64_t k) {
   if (threadIdx.x == 0) {
     st[blockIdx.x].prefix = 0;
     st[blockIdx.x].mask = 0;
@@ -316,6 +318,50 @@ __global__ void k_sel_compact_b(int64_t n_rows, int64_t nnz, int64_t k, const in
 __global__ void k_copy_i32_to_i64(const int32_t* src, int64_t* dst) { dst[0] = src[0]; }
 
 // ---------------------------------------------------------------------------------
+// the class-batched select on a row partition (gdr_sparsify_classes_dist).  The local passes are the kernels above;
+// these three carry what is global: 64-bit histogram counts, k_rem, and each rank's share of the threshold ties.
+// ---------------------------------------------------------------------------------
+// local int32 histograms -> int64 (the all-reduce operand); the int32 ones are cleared for the next pass
+__global__ void k_seld_widen(int32_t* __restrict__ hist, int64_t* __restrict__ hl) {
+  const int64_t i = (int64_t)blockIdx.x * 256 + threadIdx.x;
+  hl[i] = hist[i];
+  hist[i] = 0;
+}
+
+// k_sel_pick_b on the global histograms hg; after the last byte (shift 0) the local histogram's count of the threshold
+// key is this rank's number of ties
+__global__ void k_seld_pick(SelState* st, const int64_t* __restrict__ hg, const int64_t* __restrict__ hl, int shift,
+                            int64_t* __restrict__ ties_mine) {
+  __shared__ int64_t sh[256];
+  sh[threadIdx.x] = hg[blockIdx.x * 256 + threadIdx.x];
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    SelState* s = st + blockIdx.x;
+    int64_t k = s->k_rem;
+    int d = 255;
+    for (; d > 0; --d) {
+      if (sh[d] >= k) break;
+      k -= sh[d];
+    }
+    s->prefix |= (uint32_t)d << shift;
+    s->mask |= 0xffu << shift;
+    s->k_rem = k;
+    if (shift == 0) ties_mine[blockIdx.x] = hl[blockIdx.x * 256 + d];
+  }
+}
+
+// the blocks in rank order are the global stored order, so the first k_rem ties overall are rank p's first
+// clamp(k_rem - sum_{q<p} ties_q, 0, ties_p); k_rem becomes that local quota, which k_sel_flag_b then applies
+__global__ void k_seld_quota(SelState* st, const int64_t* __restrict__ ties /*[world][nb]*/, int nb, int rank) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c >= nb) return;
+  int64_t before = 0;
+  for (int q = 0; q < rank; ++q) before += ties[(int64_t)q * nb + c];
+  const int64_t left = st[c].k_rem - before;
+  st[c].k_rem = left < 0 ? 0 : (left < ties[(int64_t)rank * nb + c] ? left : ties[(int64_t)rank * nb + c]);
+}
+
+// ---------------------------------------------------------------------------------
 // induced subgraph  adj[np.ix_(idx, idx)]  (utils_graphsaint.py:34-36, utils.py:127-129)
 // ---------------------------------------------------------------------------------
 __global__ void k_sub_map(int64_t m, const int64_t* __restrict__ idx, int32_t* __restrict__ map) {
@@ -353,6 +399,44 @@ __global__ void __launch_bounds__(256) k_sub_rows(int64_t m, const int64_t* __re
 
 using namespace gdr;
 
+namespace {
+
+constexpr int kSpdMeta = 10;   // int64 words per rank in the entry check of gdr_sparsify_classes_dist
+
+struct SpdBuffers {
+  int64_t* meta;     // [world][kSpdMeta]  entry check (first in the workspace: see gdr_sparsify_classes_dist)
+  float* w;          // [bmax][nnz]        class weights of the batch
+  int32_t* a;        // [bmax][nnz + 1]    tie flags -> their local ranks
+  int32_t* b;        // [bmax][nnz + 1]    selection flags -> output positions
+  int32_t* hist;     // [bmax][256]        local pass histograms
+  int64_t* hl;       // [bmax][256]        the same widened (all-reduce send buffer)
+  int64_t* hg;       // [bmax][256]        global histograms
+  int64_t* ties;     // [world][bmax]      ties per rank and class (all-gathered in place)
+  SelState* st;      // [bmax]
+  void* sws;
+  int64_t sws_b, off;
+};
+
+SpdBuffers spd_carve(void* ws, int64_t nnz, int64_t bmax, int world) {
+  Workspace W(ws, INT64_MAX);
+  SpdBuffers B;
+  B.meta = W.take<int64_t>((int64_t)world * kSpdMeta);
+  B.w = W.take<float>(bmax * nnz);
+  B.a = W.take<int32_t>(bmax * (nnz + 1) + 1);
+  B.b = W.take<int32_t>(bmax * (nnz + 1) + 1);
+  B.hist = W.take<int32_t>(bmax * 256);
+  B.hl = W.take<int64_t>(bmax * 256);
+  B.hg = W.take<int64_t>(bmax * 256);
+  B.ties = W.take<int64_t>((int64_t)world * bmax);
+  B.st = W.take<SelState>(bmax);
+  B.sws_b = scan_ws_bytes(bmax * (nnz + 1));
+  B.sws = W.take<char>(B.sws_b);
+  B.off = W.off + 256;
+  return B;
+}
+
+}  // namespace
+
 extern "C" {
 
 int gdr_row_sums_f32(int64_t n, const int32_t* rowptr, const float* vals, float* deg_out, gdr_stream_t stream) {
@@ -370,7 +454,35 @@ int gdr_er_lower(int64_t n, int64_t nnz, const int32_t* rowptr, const int32_t* c
   k_row_sums<<<grid_for(n), 256, 0, s>>>(n, rowptr, vals, deg_scratch);
   GDR_LAUNCHED();
   if (nnz == 0) return GDR_OK;
-  k_er_lower<<<(unsigned)cdiv(n * 32, 256), 256, 0, s>>>(n, rowptr, colidx, vals, deg_scratch, er_out);
+  k_er_lower<<<(unsigned)cdiv(n * 32, 256), 256, 0, s>>>(n, 0, rowptr, colidx, vals, deg_scratch, er_out);
+  GDR_LAUNCHED();
+  return GDR_OK;
+}
+
+int gdr_er_lower_rows(int64_t n_local, int64_t nnz, int64_t row_lo, const int32_t* rowptr, const int32_t* colidx,
+                      const float* vals, const float* deg, float* er_out, gdr_stream_t stream) {
+  GDR_CHECK_ARG(n_local > 0 && nnz >= 0 && row_lo >= 0 && rowptr && deg, "er_lower_rows: bad arguments");
+  GDR_CHECK_ARG(nnz == 0 || (colidx && vals && er_out), "er_lower_rows: null pointer");
+  if (nnz == 0) return GDR_OK;
+  k_er_lower<<<(unsigned)cdiv(n_local * 32, 256), 256, 0, (cudaStream_t)stream>>>(n_local, row_lo, rowptr, colidx, vals,
+                                                                                  deg, er_out);
+  GDR_LAUNCHED();
+  return GDR_OK;
+}
+
+int gdr_edge_cosine_scale_rows(int64_t n_local, int64_t nnz, int64_t C, int64_t row_lo, int64_t n_global,
+                               const int32_t* rowptr, const int32_t* colidx, const float* vals, const float* ebd,
+                               int64_t ld, float eps, float* inv_norm_scratch, float* vals_out, gdr_stream_t stream) {
+  GDR_CHECK_ARG(n_local > 0 && nnz >= 0 && C > 0 && row_lo >= 0 && row_lo + n_local <= n_global && rowptr && ebd &&
+                    ld >= C && inv_norm_scratch,
+                "edge_cosine_scale: bad arguments");
+  GDR_CHECK_ARG(nnz == 0 || (colidx && vals && vals_out), "edge_cosine_scale: null pointer");
+  cudaStream_t s = (cudaStream_t)stream;
+  k_inv_norm<<<grid_for(n_global), 256, 0, s>>>(n_global, (int)C, ebd, ld, eps, inv_norm_scratch);
+  GDR_LAUNCHED();
+  if (nnz == 0) return GDR_OK;
+  k_edge_cosine_scale<<<(unsigned)cdiv(n_local * 32, 256), 256, 0, s>>>(n_local, row_lo, (int)C, rowptr, colidx, vals,
+                                                                        ebd, ld, inv_norm_scratch, vals_out);
   GDR_LAUNCHED();
   return GDR_OK;
 }
@@ -378,17 +490,8 @@ int gdr_er_lower(int64_t n, int64_t nnz, const int32_t* rowptr, const int32_t* c
 int gdr_edge_cosine_scale(int64_t n, int64_t nnz, int64_t C, const int32_t* rowptr, const int32_t* colidx,
                           const float* vals, const float* ebd, int64_t ld, float eps, float* inv_norm_scratch,
                           float* vals_out, gdr_stream_t stream) {
-  GDR_CHECK_ARG(n > 0 && nnz >= 0 && C > 0 && rowptr && ebd && ld >= C && inv_norm_scratch,
-                "edge_cosine_scale: bad arguments");
-  GDR_CHECK_ARG(nnz == 0 || (colidx && vals && vals_out), "edge_cosine_scale: null pointer");
-  cudaStream_t s = (cudaStream_t)stream;
-  k_inv_norm<<<grid_for(n), 256, 0, s>>>(n, (int)C, ebd, ld, eps, inv_norm_scratch);
-  GDR_LAUNCHED();
-  if (nnz == 0) return GDR_OK;
-  k_edge_cosine_scale<<<(unsigned)cdiv(n * 32, 256), 256, 0, s>>>(n, (int)C, rowptr, colidx, vals, ebd, ld,
-                                                                 inv_norm_scratch, vals_out);
-  GDR_LAUNCHED();
-  return GDR_OK;
+  return gdr_edge_cosine_scale_rows(n, nnz, C, 0, n, rowptr, colidx, vals, ebd, ld, eps, inv_norm_scratch, vals_out,
+                                    stream);
 }
 
 int gdr_softmax_rows(int64_t n, int64_t C, const float* X, int64_t ld, float* out, int64_t ldo, gdr_stream_t stream) {
@@ -553,9 +656,10 @@ int gdr_sparsify_classes(int64_t n, int64_t nnz, int64_t C, const int32_t* rowpt
   for (int64_t c0 = 0; c0 < C; c0 += bmax) {
     const unsigned nb = (unsigned)std::min<int64_t>(bmax, C - c0);
     const int64_t tot = (int64_t)nb * (nnz + 1);
-    k_class_weight_b<<<dim3((unsigned)cdiv(n * 32, 256), nb), 256, 0, s>>>(n, nnz, rowptr, colidx, er, prob, ldp, (int)c0, w);
+    k_class_weight_b<<<dim3((unsigned)cdiv(n * 32, 256), nb), 256, 0, s>>>(n, nnz, 0, rowptr, colidx, er, prob, ldp, (int)c0,
+                                                                         w);
     GDR_LAUNCHED();
-    k_sel_init_b<<<nb, 256, 0, s>>>(st, hist, (int32_t)k);
+    k_sel_init_b<<<nb, 256, 0, s>>>(st, hist, k);
     GDR_LAUNCHED();
     for (int shift = 24; shift >= 0; shift -= 8) {
       k_sel_hist_b<<<dim3(gx, nb), 256, 0, s>>>(nnz, w, st, shift, hist);
@@ -573,6 +677,143 @@ int gdr_sparsify_classes(int64_t n, int64_t nnz, int64_t C, const int32_t* rowpt
     k_sel_compact_b<<<dim3(grid_for(std::max(nnz, n + 1)), nb), 256, 0, s>>>(
         n, nnz, k, rowptr, colidx, vals, b, rowptr_out + c0 * (n + 1), colidx_out + c0 * k, vals_out + c0 * k,
         nnz_out_dev + c0);
+    GDR_LAUNCHED();
+  }
+  return GDR_OK;
+}
+
+/* gdr_sparsify_classes on a row partition (see gdr.h).  One class batch:
+ *   weights   k_class_weight_b on the local rows (global row ids for prob), or er itself without prob
+ *   4 passes  k_sel_hist_b (local, int32) -> widen to int64 -> all-reduce -> k_seld_pick on every rank
+ *   quota     each rank's ties of the threshold (local histogram bin) all-gathered; rank p keeps its first
+ *             clamp(k_rem - sum_{q<p} ties_q, 0, ties_p)
+ *   compact   k_sel_eqflag_b, scan, k_sel_flag_b, scan, k_sel_compact_b as on one GPU
+ * The batch size comes from the LARGEST local nnz so that every rank issues the same collectives; the workspace of
+ * gdr_sparsify_classes_dist_ws_bytes (sized with the local nnz's batch, which is never smaller) holds it. */
+int64_t gdr_sparsify_classes_dist_ws_bytes(int64_t n_local, int64_t nnz_local, int64_t C, int world) {
+  (void)n_local;
+  return spd_carve(nullptr, nnz_local, sparsify_batch(nnz_local, C), world).off;
+}
+
+int gdr_sparsify_classes_dist(gdr_comm_t* comm, int64_t n_local, int64_t nnz, int64_t row_lo, int64_t n_global, int64_t C,
+                              const int32_t* rowptr, const int32_t* colidx, const float* vals, const float* er,
+                              const float* prob, int64_t ldp, int64_t k, int32_t* rowptr_out, int32_t* colidx_out,
+                              float* vals_out, int64_t* nnz_out_dev, void* ws, int64_t ws_bytes, gdr_stream_t stream) {
+  GDR_CHECK_ARG(comm, "sparsify_classes_dist: null communicator");
+  const int world = comm->world, rank = comm->rank;
+  cudaStream_t s = (cudaStream_t)stream;
+  // local checks are decided collectively below: a rank that returned early would leave the others in a collective
+  int local_rc = GDR_OK;
+  if (!(n_local >= 0 && nnz >= 0 && row_lo >= 0 && C > 0 && k >= 0 && (prob ? C <= ldp : C == 1) &&
+        rowptr_out && nnz_out_dev && ws && (n_local == 0 || rowptr) &&
+        (nnz == 0 || (n_local > 0 && colidx && vals && er && colidx_out && vals_out)))) {
+    set_error("sparsify_classes_dist: bad arguments");
+    local_rc = GDR_EINVAL;
+  } else if (nnz >= (1ll << 31) - 1) {
+    set_error("sparsify_classes_dist: local nnz exceeds the int32 CSR limit");
+    local_rc = GDR_ERANGE;
+  } else if (ws_bytes < gdr_sparsify_classes_dist_ws_bytes(n_local, nnz, C, world)) {
+    set_error("sparsify_classes_dist: workspace too small");
+    local_rc = GDR_EWORKSPACE;
+  }
+  // entry check: the same C, k, n_global, prob presence and batch cap everywhere; blocks contiguous in rank order
+  int64_t mine[kSpdMeta] = {C, k, n_global, row_lo, n_local, nnz, local_rc, prob != nullptr, g_sparsify_batch_cap, 0};
+  std::vector<int64_t> all((size_t)world * kSpdMeta);
+  const int64_t meta_bytes = (int64_t)all.size() * 8;
+  // the gather buffer is the head of the workspace; a rank whose workspace cannot hold it still takes part in the
+  // check (through a temporary buffer: a rejected call only) so that every rank learns the verdict
+  int64_t* meta = ws && ws_bytes >= meta_bytes ? (int64_t*)ws : nullptr;   // spd_carve's first block
+  int64_t* meta_tmp = nullptr;
+  if (!meta) {
+    GDR_CUDA(cudaMalloc(&meta_tmp, meta_bytes));
+    meta = meta_tmp;
+  }
+  int rc = GDR_OK;
+  if (cudaMemcpyAsync(meta + rank * kSpdMeta, mine, sizeof(mine), cudaMemcpyHostToDevice, s) != cudaSuccess) {
+    set_error("sparsify_classes_dist: copy of the argument check failed");
+    rc = GDR_ECUDA;
+  }
+  if (rc == GDR_OK) rc = comm_allgather(comm, meta + rank * kSpdMeta, meta, sizeof(mine), s);
+  if (rc == GDR_OK && (cudaMemcpyAsync(all.data(), meta, meta_bytes, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+                       cudaStreamSynchronize(s) != cudaSuccess)) {
+    set_error("sparsify_classes_dist: read-back of the argument check failed");
+    rc = GDR_ECUDA;
+  }
+  if (meta_tmp) cudaFree(meta_tmp);
+  if (rc != GDR_OK) return rc;
+  if (local_rc != GDR_OK) return local_rc;
+  int64_t next_lo = 0, nnz_global = 0, nnz_max = 0;
+  for (int r = 0; r < world; ++r) {
+    const int64_t* m = &all[(size_t)r * kSpdMeta];
+    if (m[6] != GDR_OK) {
+      set_error("sparsify_classes_dist: rank %d rejected its arguments", r);
+      return GDR_EINVAL;
+    }
+    if (m[0] != C || m[1] != k || m[2] != n_global || m[7] != mine[7] || m[8] != mine[8]) {
+      set_error("sparsify_classes_dist: rank %d passed a different C, k, n_global, prob or batch cap", r);
+      return GDR_EINVAL;
+    }
+    if (m[3] != next_lo) {
+      set_error("sparsify_classes_dist: the row block of rank %d does not follow the previous rank's", r);
+      return GDR_EINVAL;
+    }
+    next_lo += m[4];
+    nnz_global += m[5];
+    nnz_max = std::max(nnz_max, m[5]);
+  }
+  GDR_CHECK_ARG(next_lo == n_global, "sparsify_classes_dist: the row blocks hold %lld rows, n_global is %lld",
+                (long long)next_lo, (long long)n_global);
+  GDR_CHECK_ARG(k <= nnz_global, "sparsify_classes_dist: k = %lld exceeds the %lld stored entries", (long long)k,
+                (long long)nnz_global);
+
+  if (k == 0 || nnz == 0) {
+    GDR_CUDA(cudaMemsetAsync(rowptr_out, 0, C * (n_local + 1) * 4, s));
+    GDR_CUDA(cudaMemsetAsync(nnz_out_dev, 0, C * 8, s));
+  }
+  if (k == 0) return GDR_OK;   // the same k on every rank: no rank enters a collective
+  const int64_t cap = std::min(k, nnz);   // output slice per class
+  const int64_t bmax = sparsify_batch(nnz_max, C);
+  SpdBuffers B = spd_carve(ws, nnz, bmax, world);
+  const unsigned gx = grid_for(nnz);
+  for (int64_t c0 = 0; c0 < C; c0 += bmax) {
+    const unsigned nb = (unsigned)std::min<int64_t>(bmax, C - c0);
+    const int64_t tot = (int64_t)nb * (nnz + 1);
+    int64_t* ties_mine = B.ties + (int64_t)rank * nb;
+    const float* w = er;
+    if (prob) {
+      if (nnz > 0) {
+        k_class_weight_b<<<dim3((unsigned)cdiv(n_local * 32, 256), nb), 256, 0, s>>>(n_local, nnz, row_lo, rowptr, colidx,
+                                                                                   er, prob, ldp, (int)c0, B.w);
+        GDR_LAUNCHED();
+      }
+      w = B.w;
+    }
+    k_sel_init_b<<<nb, 256, 0, s>>>(B.st, B.hist, k);
+    GDR_LAUNCHED();
+    for (int shift = 24; shift >= 0; shift -= 8) {
+      if (nnz > 0) {
+        k_sel_hist_b<<<dim3(gx, nb), 256, 0, s>>>(nnz, w, B.st, shift, B.hist);
+        GDR_LAUNCHED();
+      }
+      k_seld_widen<<<nb, 256, 0, s>>>(B.hist, B.hl);
+      GDR_LAUNCHED();
+      if ((rc = comm_allreduce_i64(comm, B.hl, B.hg, (int64_t)nb * 256, s))) return rc;
+      k_seld_pick<<<nb, 256, 0, s>>>(B.st, B.hg, B.hl, shift, ties_mine);
+      GDR_LAUNCHED();
+    }
+    if ((rc = comm_allgather(comm, ties_mine, B.ties, (int64_t)nb * 8, s))) return rc;
+    k_seld_quota<<<(unsigned)cdiv(nb, 256), 256, 0, s>>>(B.st, B.ties, (int)nb, rank);
+    GDR_LAUNCHED();
+    if (nnz == 0) continue;
+    k_sel_eqflag_b<<<dim3(gx, nb), 256, 0, s>>>(nnz, w, B.st, B.a);
+    GDR_LAUNCHED();
+    if ((rc = exclusive_scan_i32(B.a, B.a, tot, B.sws, B.sws_b, s))) return rc;
+    k_sel_flag_b<<<dim3(gx, nb), 256, 0, s>>>(nnz, w, B.st, B.a, B.b);
+    GDR_LAUNCHED();
+    if ((rc = exclusive_scan_i32(B.b, B.b, tot, B.sws, B.sws_b, s))) return rc;
+    k_sel_compact_b<<<dim3(grid_for(std::max(nnz, n_local + 1)), nb), 256, 0, s>>>(
+        n_local, nnz, cap, rowptr, colidx, vals, B.b, rowptr_out + c0 * (n_local + 1), colidx_out + c0 * cap,
+        vals_out + c0 * cap, nnz_out_dev + c0);
     GDR_LAUNCHED();
   }
   return GDR_OK;

@@ -12,6 +12,8 @@ so nothing is ported here — the exchanges are the ones the algorithm needs:
   stage 3  per Lloyd iteration ONE all-reduce of the [K x D] partial sums and ONE of the
            packed int32 [counts | n_changed]; every rank finalises identically, so the
            replicated centres stay bit-identical across ranks;
+  sparsify all-gather of the degree vector and the logits; per radix pass of the top-k one all-reduce
+           of the per-rank histograms, then one all-gather of the tie counts (dist_graph_sparse);
   stage 4  all-gather of the labels, local segmented edge counting, dense n x n all-reduce of
            (int32 counts, f32 sums), compaction back to CSR.
 
@@ -653,6 +655,52 @@ class CudaOps:
     def row_dist(self, Xc, C, labels):
         return ((Xc - C[labels.long()]) ** 2).sum(dim=1)  # rare relocation path only
 
+    # -- edge sparsification (between stages 3 and 4) --
+    def er_lower_rows(self, A, deg, row_lo):
+        """v/deg[row_lo + r] + v/deg[c] for the local block A with the global degree vector (gdr_er_lower_rows)."""
+        er = torch.empty(max(A.nnz, 1), dtype=torch.float32, device=A.device)
+        self._lib.call("gdr_er_lower_rows", A.shape[0], A.nnz, int(row_lo), self.ptr(A.rowptr), self.ptr(A.colidx),
+                       self.ptr(A.vals), self.ptr(deg), self.ptr(er), self.stream())
+        return er[: A.nnz]
+
+    def cosine_reweight_rows(self, A, ebd, row_lo, eps=1e-8):
+        """vals * cos(ebd[row_lo + r], ebd[c]) for the local block A, ``ebd`` global (gdr_edge_cosine_scale_rows)."""
+        inv = torch.empty(ebd.shape[0], dtype=torch.float32, device=A.device)
+        out = torch.empty(max(A.nnz, 1), dtype=torch.float32, device=A.device)
+        self._lib.call("gdr_edge_cosine_scale_rows", A.shape[0], A.nnz, ebd.shape[1], int(row_lo), ebd.shape[0],
+                       self.ptr(A.rowptr), self.ptr(A.colidx), self.ptr(A.vals), self.ptr(ebd), ebd.stride(0), float(eps),
+                       self.ptr(inv), self.ptr(out), self.stream())
+        return self._g.CSR(A.rowptr, A.colidx, out[: A.nnz], A.shape)
+
+    def softmax_rows(self, x):
+        from .sparsify import softmax_rows
+        return softmax_rows(x)
+
+    def sparsify_classes_dist(self, comm, A, row_lo, n_global, er, prob, k):
+        """This rank's kept edges of every class (gdr_sparsify_classes_dist; collective).  ``A`` None: a rank without
+        rows, which still joins.  ``prob`` None: one graph, weights ``er``.  Returns one local CSR per class (None for a
+        rank without rows)."""
+        C = 1 if prob is None else int(prob.shape[1])
+        dev = er.device
+        n_local, nnz = (0, 0) if A is None else (A.shape[0], A.nnz)
+        cap = min(int(k), nnz)
+        rowptr = torch.empty((C, n_local + 1), dtype=torch.int32, device=dev)
+        colidx = torch.empty((C, max(cap, 1)), dtype=torch.int32, device=dev)
+        vals = torch.empty((C, max(cap, 1)), dtype=torch.float32, device=dev)
+        nnz_out = torch.zeros(C, dtype=torch.int64, device=dev)
+        ws = self.workspace(self._lib.query("gdr_sparsify_classes_dist_ws_bytes", n_local, nnz, C, comm.world), dev)
+        have = nnz > 0
+        self._lib.call("gdr_sparsify_classes_dist", comm.lib_handle(), n_local, nnz, int(row_lo), int(n_global), C,
+                       self.ptr(A.rowptr) if n_local else 0, self.ptr(A.colidx) if have else 0,
+                       self.ptr(A.vals) if have else 0, self.ptr(er) if have else 0,
+                       0 if prob is None else self.ptr(prob), 0 if prob is None else prob.stride(0), int(k),
+                       self.ptr(rowptr), self.ptr(colidx) if have else 0, self.ptr(vals) if have else 0, self.ptr(nnz_out),
+                       self.ptr(ws), ws.numel(), self.stream())
+        if A is None:
+            return [None] * C
+        counts = nnz_out.tolist()
+        return [self._g.CSR(rowptr[c], colidx[c, : counts[c]], vals[c, : counts[c]], A.shape) for c in range(C)]
+
     # -- stage 4 --
     def label_counts(self, labels, n):
         return self._co.label_counts(labels, n)
@@ -1206,6 +1254,54 @@ class DistKMeans:
 
 
 # ------------------------------------------------------------------------------------------
+# edge sparsification (between stages 3 and 4)
+# ------------------------------------------------------------------------------------------
+def dist_graph_sparse(comm: Comm, part: RowPartition, A_local, ratio: float, ebd_local: Optional[torch.Tensor] = None,
+                      sp_type: str = "vanilla", ops=None):
+    """``sparsify.graph_sparse`` (ClustGDD.graph_sparse, clustgdd_agent_transduct.py:131-232) on a row partition.
+    Collective.  ``A_local`` is this rank's row block of A_hat with global column ids (``dist_build_adjacency``; None on a
+    rank without rows, which still joins), ``ebd_local`` its rows of the logits.  Returns this rank's row blocks of the
+    sparsified graphs as CSR with global column ids (None on a rank without rows): one for 'vanilla' / 'single' /
+    'no_sp', one per class for 'attaw'.  The blocks concatenated in rank order are byte-identical to the one-GPU
+    ``graph_sparse`` on the whole graph, for any number of ranks.  'rand' is not supported here: its draws are
+    ``torch.randperm`` over the global edge list on the host generator."""
+    if sp_type == "no_sp":
+        return [A_local]
+    if sp_type == "rand":
+        raise NotImplementedError("sp_type='rand' has no row-partitioned form")
+    if sp_type not in ("vanilla", "single", "attaw"):
+        raise ValueError(f"unknown sp_type {sp_type!r}")
+    if sp_type != "vanilla" and ebd_local is None:
+        raise ValueError(f"sp_type={sp_type!r} needs ebd")
+    ops = ops or CudaOps()
+    if not hasattr(ops, "sparsify_classes_dist"):
+        raise NotImplementedError(f"{type(ops).__name__} has no distributed sparsification")
+    dev = ebd_local.device if ebd_local is not None else torch.device("cuda", torch.cuda.current_device())
+    sizes = _block_sizes(part)
+    nnz = torch.tensor([0 if A_local is None else A_local.nnz], dtype=torch.int64, device=dev)
+    k = int(int(comm.all_reduce(nnz, "sum").item()) * ratio)     # graph_sparse's int(nedges * ratio)
+
+    def global_er(A):
+        # the degree vector of A's rows is needed at every column: row sums, all-gathered
+        deg = comm.all_gather_var(ops.row_sums(A) if A is not None else torch.zeros(0, dtype=torch.float32, device=dev),
+                                  sizes)
+        return ops.er_lower_rows(A, deg, part.lo) if A is not None else torch.zeros(0, dtype=torch.float32, device=dev)
+
+    if sp_type == "vanilla":
+        return ops.sparsify_classes_dist(comm, A_local, part.lo, part.n, global_er(A_local), None, k)
+    from ._dev import need_cuda
+    e = need_cuda(ebd_local, "ebd").to(torch.float32).contiguous()
+    if e.dim() != 2 or e.shape[0] != part.n_local:
+        raise ValueError("ebd_local must be [rows of this rank, n_classes]")
+    C = int(e.shape[1])
+    ebd = comm.all_gather_var(e.reshape(-1), [s * C for s in sizes]).view(part.n, C)
+    R = ops.cosine_reweight_rows(A_local, ebd, part.lo) if A_local is not None else None
+    er = global_er(R)
+    prob = ops.softmax_rows(ebd) if sp_type == "attaw" else None
+    return ops.sparsify_classes_dist(comm, R, part.lo, part.n, er, prob, k)
+
+
+# ------------------------------------------------------------------------------------------
 # stage 4
 # ------------------------------------------------------------------------------------------
 def dist_graph_compress(comm: Comm, part: RowPartition, labels_local: torch.Tensor, A_local, ops=None, replicate: bool = True,
@@ -1223,8 +1319,6 @@ def dist_graph_compress(comm: Comm, part: RowPartition, labels_local: torch.Tens
     the wall-clock milliseconds of every section (synchronising; tools/stage4_probe.py)."""
     import time as _time
     ops = ops or CudaOps()
-    dev = labels_local.device
-    rows_per, world = part.rows_per, part.world
     _t = [_time.perf_counter()]
 
     def mark(name):
@@ -1234,6 +1328,27 @@ def dist_graph_compress(comm: Comm, part: RowPartition, labels_local: torch.Tens
             now = _time.perf_counter()
             timing[name] = timing.get(name, 0.0) + (now - _t[0]) * 1e3
             _t[0] = now
+    labels = _compress_labels(comm, part, labels_local, ops)
+    mark("labels_allgather_sizes")
+    return _dist_compress_graph(comm, ops, A_local, *labels, replicate, merge, mark)
+
+
+def dist_graph_compress_list(comm: Comm, part: RowPartition, labels_local: torch.Tensor, A_local, adj_list_local,
+                             ops=None, replicate: bool = True, merge: str = "route"):
+    """graph_compress (clustgdd_agent_transduct.py:234-250) with the reference's shape: every graph of
+    ``adj_list_local`` (this rank's row blocks, e.g. from ``dist_graph_sparse``) and ``A_local`` coarsened by the same
+    labels.  Returns (compressed_list, adj_syn); each element is what ``dist_graph_compress`` returns for that graph.
+    The labels all-gather, n and the cluster sizes are computed once per call."""
+    ops = ops or CudaOps()
+    labels = _compress_labels(comm, part, labels_local, ops)
+    compressed = [_dist_compress_graph(comm, ops, a, *labels, replicate, merge) for a in adj_list_local]
+    return compressed, _dist_compress_graph(comm, ops, A_local, *labels, replicate, merge)
+
+
+def _compress_labels(comm: Comm, part: RowPartition, labels_local: torch.Tensor, ops):
+    """(this rank's labels int32, all labels, n, cluster sizes): the per-call part of stage 4."""
+    dev = labels_local.device
+    rows_per, world = part.rows_per, part.world
     block = torch.full((rows_per,), -1, dtype=torch.int32, device=dev)
     block[: labels_local.shape[0]] = labels_local.to(torch.int32)
     gathered = torch.empty(rows_per * world, dtype=torch.int32, device=dev)
@@ -1244,11 +1359,15 @@ def dist_graph_compress(comm: Comm, part: RowPartition, labels_local: torch.Tens
     nmax = labels_all.max().to(torch.int64).reshape(1)
     n = int(comm.all_reduce(nmax, "max").item()) + 1
     sizes = ops.label_counts(labels_all, n)
-    mark("labels_allgather_sizes")
+    return labels_local.to(torch.int32).contiguous(), labels_all, n, sizes
+
+
+def _dist_compress_graph(comm: Comm, ops, A_local, lab_l, labels_all, n, sizes, replicate, merge, mark=lambda name: None):
+    """The per-graph part of stage 4: route (or records) exchange, merge, scale, and the replication."""
+    world = comm.world
     cr = (n + world - 1) // world
     a_lo = min(n, comm.rank * cr)
     n_rows = min(n, a_lo + cr) - a_lo
-    lab_l = labels_local.to(torch.int32).contiguous()
     if merge == "route" and hasattr(ops, "coarsen_route"):
         # every edge goes to the owner of its coarse row once; the owner sorts + reduces (one sort per edge, sums in CSR order)
         keys, w, send_counts = ops.coarsen_route(A_local, lab_l, labels_all, n, world)

@@ -470,13 +470,23 @@ int gdr_remap_chunk_major(int64_t nnz, const int32_t* colidx_in, int64_t rows_pe
  *   gdr_topk_filter_csr     torch.topk(weight, k) + COO rebuild        clustgdd_agent_transduct.py:142-151,168-181
  *                           keeps every entry above the k-th largest weight plus the first entries (stored
  *                           order) equal to it, exactly k in total; output is a sorted CSR (capacity k);
- *                           radix select + two scans, no host synchronisation, no sort. */
+ *                           radix select + two scans, no host synchronisation, no sort.
+ * Row-block forms (one rank's rows [row_lo, row_lo + n_local) of a row-partitioned graph, column ids global): per-row
+ * operands are read at row_lo + r, per-column operands at colidx[j]; every value has the bits of the whole-graph call.
+ *   gdr_er_lower_rows           er with a caller-supplied GLOBAL degree vector deg [n_global]
+ *   gdr_edge_cosine_scale_rows  global ebd [n_global][ld]; inv_norm_scratch: n_global floats (all norms are computed)
+ * gdr_sparsify_classes_dist (below, with gdr_sparsify_classes) runs the top-k across the ranks. */
 int gdr_row_sums_f32(int64_t n, const int32_t* rowptr, const float* vals, float* deg_out, gdr_stream_t stream);
 int gdr_er_lower(int64_t n, int64_t nnz, const int32_t* rowptr, const int32_t* colidx, const float* vals,
                  float* deg_scratch, float* er_out, gdr_stream_t stream);
 int gdr_edge_cosine_scale(int64_t n, int64_t nnz, int64_t C, const int32_t* rowptr, const int32_t* colidx,
                           const float* vals, const float* ebd, int64_t ld, float eps,
                           float* inv_norm_scratch, float* vals_out, gdr_stream_t stream);
+int gdr_er_lower_rows(int64_t n_local, int64_t nnz, int64_t row_lo, const int32_t* rowptr, const int32_t* colidx,
+                      const float* vals, const float* deg, float* er_out, gdr_stream_t stream);
+int gdr_edge_cosine_scale_rows(int64_t n_local, int64_t nnz, int64_t C, int64_t row_lo, int64_t n_global,
+                               const int32_t* rowptr, const int32_t* colidx, const float* vals, const float* ebd,
+                               int64_t ld, float eps, float* inv_norm_scratch, float* vals_out, gdr_stream_t stream);
 int gdr_softmax_rows(int64_t n, int64_t C, const float* X, int64_t ld, float* out, int64_t ldo,
                      gdr_stream_t stream);
 int gdr_class_edge_weight(int64_t n, int64_t nnz, const int32_t* rowptr, const int32_t* colidx,
@@ -677,6 +687,26 @@ int     gdr_sparsify_classes(int64_t n, int64_t nnz, int64_t C, const int32_t* r
                              const float* vals, const float* er, const float* prob, int64_t ldp, int64_t k,
                              int32_t* rowptr_out, int32_t* colidx_out, float* vals_out, int64_t* nnz_out_dev,
                              void* ws, int64_t ws_bytes, gdr_stream_t stream);
+/* gdr_sparsify_classes on a row partition.  COLLECTIVE over comm.  Each rank passes its local CSR block (n_local rows
+ * from global row row_lo, nnz local entries, global column ids; n_local = 0 and nnz = 0 allowed), the global er of its
+ * local edges, the GLOBAL prob [n_global][ldp] (or NULL: the weight is er itself and C must be 1, for 'vanilla' /
+ * 'single') and the GLOBAL k (0 <= k <= total nnz).  Output per class c: this rank's kept edges as a local CSR, slice
+ * c of rowptr_out [C][n_local+1] and of colidx_out / vals_out [C][min(k, nnz)], count in nnz_out_dev[c].  The blocks
+ * concatenated in rank order are byte-identical to gdr_sparsify_classes / gdr_topk_filter_csr on the whole graph for
+ * any number of ranks: the row blocks in rank order are the global stored order, each radix pass sums the ranks'
+ * histograms (64-bit counts, one all-reduce per pass and class batch), and the ties at the threshold are shared out
+ * in rank order (one all-gather of the per-rank tie counts per batch): rank p keeps its first
+ * clamp(k_rem - sum_{q<p} ties_q, 0, ties_p).  At entry every rank all-gathers C, k, n_global, row_lo, n_local, nnz,
+ * whether prob is given, the "sparsify_batch" cap and its argument verdict; a mismatch, blocks that are not contiguous
+ * in rank order, or an argument any rank rejects returns GDR_EINVAL on every rank.  The class batch is sized from the
+ * largest local nnz.  The local nnz keeps the int32 CSR limit (GDR_ERANGE).  Synchronises the stream once, after the
+ * entry check. */
+int64_t gdr_sparsify_classes_dist_ws_bytes(int64_t n_local, int64_t nnz_local, int64_t C, int world);
+int     gdr_sparsify_classes_dist(gdr_comm_t* comm, int64_t n_local, int64_t nnz_local, int64_t row_lo,
+                                  int64_t n_global, int64_t C, const int32_t* rowptr, const int32_t* colidx,
+                                  const float* vals, const float* er, const float* prob, int64_t ldp, int64_t k,
+                                  int32_t* rowptr_out, int32_t* colidx_out, float* vals_out, int64_t* nnz_out_dev,
+                                  void* ws, int64_t ws_bytes, gdr_stream_t stream);
 int64_t gdr_topk_filter_ws_bytes(int64_t n, int64_t nnz);
 int     gdr_topk_filter_csr(int64_t n, int64_t nnz, const int32_t* rowptr, const int32_t* colidx,
                             const float* vals, const float* weight, int64_t k, int32_t* rowptr_out,
