@@ -23,7 +23,6 @@ _SIGNATURES = {
     "gdr_launch_count": (i64, []),
     "gdr_debug_set": (i32, [cp, i32]),
     "gdr_debug_get": (i32, [cp, vp]),
-    "gdr_debug_mma_probe": (i32, [i32, i32, i32, vp]),
     "gdr_profile_enable": (i32, [i32]),
     "gdr_profile_collect": (i32, [vp, vp]),
     "gdr_sort_pairs_ws_bytes": (i64, [i64]),

@@ -20,7 +20,6 @@
 #include "tc_common.cuh"
 #include <cuda.h>
 #include <string.h>
-#include <stdlib.h>
 
 namespace gdr {
 
@@ -42,14 +41,13 @@ constexpr float TC_BAND = 3.0517578125e-05f;      // 2^-15
 // first-level screen: one TF32 product over the augmented operands of k_split_tf32; its error radius is built
 // from the measured rounding residuals |x - tf32(x)|, |c - tf32(c)| (see k_split_tf32 / k_tc_select1).
 static const int32_t* g_last_count1 = nullptr;   // device counter of the last two-level run (debug read-back)
-int g_tc_ablate = 0;   // experiment: 1 no epilogue math, 2 no tcgen05.ld either, 3 no MMAs, 4 one K-block of MMAs only
-int g_tc_gate = 1;      // gdr_debug_set("tc_gate", v): first-level epilogue gate — 0 off (exact running top-2 over all columns), 1 (default) gate on the running best, 2 also seeded with the previous label's score (measured at config E: the seed pass costs 0.9 ms and returns 0.1)
+int g_tc_gate = 1;      // gdr_debug_set("tc_gate", v): first-level epilogue gate — 0 off (exact running top-2 over all columns), otherwise (default) gate on the running best
 extern int64_t g_topk_last_overflow;   // topk.cu
 extern int64_t g_topk_condensed_last_fallback;   // topk_condensed.cu
 int g_tc_cand = 1;      // gdr_debug_set("tc_cand", v): second level of the default two-level screen — 1 (default) seeded candidate pass + exact re-score of the candidates, 0 3xTF32 + exact re-score over all centres
 int g_tc_cand_cap = 0;  // gdr_debug_set("tc_cand_cap", v): candidate list capacity per row and column half, 1..TC_CAND_CAP (0: TC_CAND_CAP)
 static const int32_t* g_last_cand = nullptr;     // candidate counters of the last run that used the candidate level (debug read-back)
-int g_tc_screen = 0;    // gdr_debug_set("tc_screen", v): 0 auto, 1 direct 3xTF32, 2 two-level with 256-row x 128-centre CTA tiles, 3 two-level with 128 x 256 tiles, 4 two-level on CTA pairs (cta_group::2, 256 x 256), 6 two-level with the row tile in tensor memory (A operand from TMEM, 128 x 192 tiles)
+int g_tc_screen = 0;    // gdr_debug_set("tc_screen", v): 0 auto, 1 direct 3xTF32, >= 2 two-level
 
 // smallest TF32 value >= v (v finite); used where a bound must not shrink under the operand rounding
 __device__ __forceinline__ float tf32_up(float v) {
@@ -170,30 +168,20 @@ __global__ void __launch_bounds__(1024) k_cnorm_finish(int64_t K, int64_t Kp, co
 //            k_split_tf32 (aug_mode 1 / 2), whose accumulator is directly the score s_ij >= x_i.c_j - |c_j|^2/2;
 //            the epilogue is a bare running (max, second max, argmax) — no norm add, no per-centre loads —
 //            and k_tc_select1 accepts the row when s_best - s_second exceeds twice the error radius.
-// BN      = centres per accumulator tile (UMMA N): 128 or 256.
-// SUB     = 128-row sub-tiles resident per CTA.  Every SM streams the WHOLE centre matrix from L2 once per row
-//           tile, so the L2 -> SMEM traffic of a launch is (N / (128 SUB)) * Kp * Dp * 4 bytes: at one TF32
-//           product per K-step that stream, not the tensor pipe, bounds the kernel (measured: 9.8 TB/s at
-//           SUB = 1), and SUB = 2 halves it — each centre K-block feeds the MMAs of both sub-tiles.
+// BN      = centres per accumulator tile (UMMA N): 128 (NPASS 3) or 256 (NPASS 1); a CTA tile holds TC_BM = 128 rows.
 constexpr int TC_MAX_STAGES = 8;
 constexpr int TC_SMEM_LIMIT = 227 * 1024;
-__device__ long long g_tc_probe[4];   // ablation runs: MMA-thread cycles / nanoseconds / MMAs issued of CTA 0
-// k_assign_tc_ts with tc_ablate bit 16, CTA 0, cycles: [0] MMA warp total, [1] its waits for a centre stage, [2] for an
-// accumulator, [3] for the A operand, [4] issue + commits; [5] producer total, [6] its waits for a free stage;
-// [7] epilogue warp 2 total, [8] its waits for an accumulator, [9] tcgen05.ld + arithmetic, [10] arrive, [11] A store
-__device__ long long g_ts_probe[16];
 
 // First-level epilogue gate.  k_tc_select1 only needs to know (a) the best score of a row and (b) whether ANY other
 // centre comes within tol(i, best) of it, and tol(i, j) <= tolmax_i = the same expression with max_j |c_j|, max_j |dc_j|.
 // So the running top-2 has to look only at chunks that hold a score within tolmax_i of a lower bound of the row's
-// final best: the running best, and — from the second Lloyd iteration on — the score of the row's PREVIOUS label
-// against the new centres (k_tc_seed), which is already the final best for the rows that keep their label.  A warp
-// (32 rows) then takes the per-element path for a few percent of the 8-column chunks instead of ~a third.
+// final best: the running best (k_tc_cand starts from the row's level-1 best instead).  A warp (32 rows) then takes
+// the per-element path for a few percent of the 8-column chunks instead of ~a third.
 struct TcGate {
   const float* xnorm;    // |x_i|           (nullptr: gate off, exact running top-2 over all columns)
   const float* xdnorm;   // |x_i - tf32(x_i)|
   const float* cscal;    // [0] = max_j |c_j|, [1] = max_j (|c_j - tf32(c_j)|)
-  const float* seed;     // upper bound of the row's final best (negated score), +inf when unknown; nullable
+  const float* seed;     // k_tc_cand only: the row's level-1 best (negated score)
   float band;
 };
 
@@ -231,7 +219,7 @@ __device__ __forceinline__ void epi_chunk32(const uint32_t (&v)[32], int jbase, 
 }
 
 // slack of the candidate pass's starting limit over the level-1 best it is seeded with: the two passes multiply the
-// same operands but may accumulate differently (same bound as k_tc_seed's 2^-18 term)
+// same operands but may accumulate differently
 __device__ __forceinline__ float tc_cand_slack(float xn, float cm) { return 3.814697265625e-06f * (xn * cm + cm * cm); }
 
 // Candidate-pass epilogue step (k_tc_cand): as epi_chunk32 with the gate always on, plus every per-element score below
@@ -267,15 +255,15 @@ __device__ __forceinline__ void epi_chunk32_rec(const uint32_t (&v)[32], int jba
   }
 }
 
-template <int NPASS, int BN, int SUB>
+template <int NPASS, int BN>
 struct TcCfg {
   static constexpr int kXCopies = NPASS == 3 ? 2 : 1;                        // hi (+ lo) copy of the row tile
   static constexpr int kStageBytes = kXCopies * BN * TC_BK * 4;              // one centre K-block (hi [+ lo])
-  static constexpr int kTmemCols = 2 * SUB * BN;                             // two buffers of SUB accumulators
+  static constexpr int kTmemCols = 2 * BN;                                   // two accumulators
   static constexpr int kTail = 512 /*barriers*/ + 1536 /*epilogue merge buffer*/;
-  __host__ __device__ static constexpr int x_hi(int nkb, int sub, int kb) { return (sub * nkb + kb) * TC_KBLK_BYTES; }
-  __host__ __device__ static constexpr int x_lo(int nkb, int kb) { return (nkb + kb) * TC_KBLK_BYTES; }   // NPASS 3, SUB 1
-  __host__ __device__ static constexpr int x_bytes(int nkb) { return SUB * kXCopies * nkb * TC_KBLK_BYTES; }
+  __host__ __device__ static constexpr int x_hi(int kb) { return kb * TC_KBLK_BYTES; }
+  __host__ __device__ static constexpr int x_lo(int nkb, int kb) { return (nkb + kb) * TC_KBLK_BYTES; }   // NPASS 3
+  __host__ __device__ static constexpr int x_bytes(int nkb) { return kXCopies * nkb * TC_KBLK_BYTES; }
   __host__ __device__ static constexpr int c_stage(int nkb, int s) { return x_bytes(nkb) + s * kStageBytes; }
   // as many centre stages as fit beside the resident rows (<= TC_MAX_STAGES)
   __host__ __device__ static constexpr int stages(int nkb) {
@@ -297,18 +285,17 @@ struct TcCand {
 // The kernel body, shared by the first level / 3xTF32 level (k_assign_tc) and the seeded candidate pass (k_tc_cand,
 // REC = true).  REC: the gate is always on, the limit starts at the row's seed and every per-element score below it
 // is recorded; best / second / argmin are not written.
-template <int NPASS, int BN, int SUB, bool REC>
+template <int NPASS, int BN, bool REC>
 __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const CUtensorMap& map_xlo,
                                                const CUtensorMap& map_chi, const CUtensorMap& map_clo, int64_t N_host,
                                                const int32_t* __restrict__ n_rows_dev, int D, int n_col_tiles, int nkb,
                                                const float* __restrict__ cnorm, float* __restrict__ best_out,
-                                               float* __restrict__ second_out, int32_t* __restrict__ idx_out, int ablate,
+                                               float* __restrict__ second_out, int32_t* __restrict__ idx_out,
                                                TcGate gate, TcCand cand) {
-  using Cfg = TcCfg<NPASS, BN, SUB>;
-  static_assert(Cfg::kTmemCols <= 512 && (NPASS == 1 || SUB == 1) && (SUB == 1 || SUB == 2), "tile plan");
-  static_assert(!REC || (NPASS == 1 && SUB == 1), "candidate recording: first-level shape only");
+  using Cfg = TcCfg<NPASS, BN>;
+  static_assert(Cfg::kTmemCols <= 512, "tile plan");
+  static_assert(!REC || NPASS == 1, "candidate recording: first-level shape only");
   const int S = Cfg::stages(nkb);
-  constexpr int ROWS = TC_BM * SUB;            // rows per CTA tile
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::bars(nkb));
@@ -323,7 +310,7 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
   const int warp = threadIdx.x >> 5;
   const int lane = threadIdx.x & 31;
   const int64_t N = n_rows_dev ? (int64_t)n_rows_dev[0] : N_host;
-  const int n_row_tiles = (int)((N + ROWS - 1) / ROWS);
+  const int n_row_tiles = (int)((N + TC_BM - 1) / TC_BM);
 
   if (warp == 0 && lane == 0) {
     for (int i = 0; i < TC_BAR_KB; ++i) {
@@ -355,7 +342,7 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
   // instructions.  (Running the loops inside `if (lane == 0)` makes every descriptor a per-thread value: the
   // compiler then wraps each UTCHMMA in an ELECT / R2UR.BROADCAST waterfall and the issue path — ~350 cycles per
   // MMA, measured with clock64 inside the kernel — becomes the bottleneck instead of the tensor pipe, which runs a
-  // 128 x 256 x 8 TF32 MMA in 171 cycles: tools/mma_issue_probe.py.)
+  // 128 x 256 x 8 TF32 MMA in 171 cycles.)
   if (warp == 0) {
     // ================= TMA producer =================
     uint32_t tile_it = 0;
@@ -365,27 +352,20 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
       for (int kb = 0; kb < nkb; ++kb) {
         mbar_wait(&x_empty[kb], (tile_it & 1) ^ 1);
         if (elect_one()) {
-          mbar_expect_tx(&x_full[kb], SUB * Cfg::kXCopies * TC_KBLK_BYTES);
-#pragma unroll
-          for (int sub = 0; sub < SUB; ++sub)
-            tma_load_2d(smem + Cfg::x_hi(nkb, sub, kb), &map_xhi, kb * TC_BK, rt * ROWS + sub * TC_BM, &x_full[kb]);
-          if (NPASS == 3) tma_load_2d(smem + Cfg::x_lo(nkb, kb), &map_xlo, kb * TC_BK, rt * ROWS, &x_full[kb]);
+          mbar_expect_tx(&x_full[kb], Cfg::kXCopies * TC_KBLK_BYTES);
+          tma_load_2d(smem + Cfg::x_hi(kb), &map_xhi, kb * TC_BK, rt * TC_BM, &x_full[kb]);
+          if (NPASS == 3) tma_load_2d(smem + Cfg::x_lo(nkb, kb), &map_xlo, kb * TC_BK, rt * TC_BM, &x_full[kb]);
         }
         __syncwarp();
       }
       for (int ct = 0; ct < n_col_tiles; ++ct) {
         for (int kb = 0; kb < nkb; ++kb) {
-          if (ablate >= 6) continue;   // experiment: raw MMA issue rate, no stage barriers at all
           mbar_wait(&c_empty[s], ph ^ 1);
           if (elect_one()) {
-            if (ablate == 5) {   // experiment: MMAs on stale shared memory, no centre stream
-              mbar_arrive(&c_full[s]);
-            } else {
-              mbar_expect_tx(&c_full[s], Cfg::kStageBytes);
-              uint8_t* dst = smem + Cfg::c_stage(nkb, s);
-              tma_load_2d(dst, &map_chi, kb * TC_BK, ct * BN, &c_full[s]);
-              if (NPASS == 3) tma_load_2d(dst + BN * TC_BK * 4, &map_clo, kb * TC_BK, ct * BN, &c_full[s]);
-            }
+            mbar_expect_tx(&c_full[s], Cfg::kStageBytes);
+            uint8_t* dst = smem + Cfg::c_stage(nkb, s);
+            tma_load_2d(dst, &map_chi, kb * TC_BK, ct * BN, &c_full[s]);
+            if (NPASS == 3) tma_load_2d(dst + BN * TC_BK * 4, &map_clo, kb * TC_BK, ct * BN, &c_full[s]);
           }
           __syncwarp();
           if (++s == S) {
@@ -400,7 +380,7 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
     // The per-K-block issue path is kept to a handful of uniform instructions (descriptor = base + offset, ring
     // position advanced incrementally, K steps unrolled): at ~128 cycles per 128 x 256 x 8 MMA the tensor pipe
     // drains a K-block in ~500 cycles, and a path with integer divisions and descriptor rebuilds took longer
-    // than that (measured: 250 cycles per MMA with every wait removed, 128 in tools/mma_issue_probe.py).
+    // than that (measured: 250 cycles per MMA with every wait removed, 128 on a bare stream of MMAs).
     constexpr uint32_t idesc = umma_idesc_tf32(TC_BM, BN);
     uint32_t tile_it = 0, g = 0;
     int s = 0;
@@ -408,26 +388,20 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
     const uint64_t dx0 = umma_desc_sw128(smem_u32(smem));                                  // row tile, K-block 0
     const uint64_t dc0 = umma_desc_sw128(smem_u32(smem + Cfg::c_stage(nkb, 0)));             // centre stage 0
     constexpr uint64_t kKb = TC_KBLK_BYTES >> 4, kStage = Cfg::kStageBytes >> 4, kLo = (uint64_t)(BN * TC_BK * 4) >> 4;
-    long long pc0 = 0, pn0 = 0, n_mma = 0;
-    if (ablate && blockIdx.x == 0) {
-      pc0 = clock64();
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(pn0));
-    }
     for (int rt = blockIdx.x; rt < n_row_tiles; rt += gridDim.x, ++tile_it) {
       for (int ct = 0; ct < n_col_tiles; ++ct, ++g) {
         const uint32_t a = g & 1, aph = (g >> 1) & 1;
-        if (ablate != 8) mbar_wait(&t_empty[a], aph ^ 1);   // 8: no accumulator hand-shake with the epilogue either
+        mbar_wait(&t_empty[a], aph ^ 1);
         tc_fence_after();
-        const uint32_t tmem_d = tmem_base + a * (SUB * BN);
+        const uint32_t tmem_d = tmem_base + a * BN;
         const bool last_ct = ct == n_col_tiles - 1;
         for (int kb = 0; kb < nkb; ++kb) {
           if (ct == 0) mbar_wait(&x_full[kb], tile_it & 1);
-          if (ablate < 6) mbar_wait(&c_full[s], ph);
+          mbar_wait(&c_full[s], ph);
           tc_fence_after();
           const uint64_t d_chi = dc0 + (uint64_t)s * kStage;
           // K = 8 steps that still hold real columns (the rest of the 32-float block is zero padding)
           const int ksteps = min(TC_BK / 8, (D - kb * TC_BK + 7) >> 3);
-          if (ablate) n_mma += ksteps;
           if (elect_one()) {
             if (NPASS == 3) {
               const uint64_t d_xhi = dx0 + (uint64_t)kb * kKb;
@@ -451,32 +425,23 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
                 }
               }
             } else {
+              const uint64_t d_x = dx0 + (uint64_t)kb * kKb;
+              if (ksteps == 4) {
 #pragma unroll
-              for (int sub = 0; sub < SUB; ++sub) {
-                const uint64_t d_x = dx0 + (uint64_t)(sub * nkb + kb) * kKb;
-                const uint32_t td = tmem_d + sub * BN;
-                if (ablate != 3 && ablate != 4 && ablate != 7 && ksteps == 4) {
-#pragma unroll
-                  for (int k = 0; k < 4; ++k) {
-                    const uint64_t adv = (uint64_t)((k * 8 * 4) >> 4);
-                    tc_mma_tf32(td, d_x + adv, d_chi + adv, idesc, (kb | k) != 0);
-                  }
-                } else {
-                  for (int k = 0; k < ((ablate == 3 || (ablate == 4 && kb > 0)) ? 0 : ksteps); ++k) {
-                    const uint64_t adv = (uint64_t)((k * 8 * 4) >> 4);
-                    if (ablate == 7) {   // D = F32, A = B = BF16 (format code 1), same N / M fields
-                      constexpr uint32_t idesc_bf16 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(TC_BM >> 4) << 24);
-                      tc_mma_bf16(td, d_x + adv, d_chi + adv, idesc_bf16, (kb | k) != 0);
-                    } else {
-                      tc_mma_tf32(td, d_x + adv, d_chi + adv, idesc, (kb | k) != 0);
-                    }
-                  }
+                for (int k = 0; k < 4; ++k) {
+                  const uint64_t adv = (uint64_t)((k * 8 * 4) >> 4);
+                  tc_mma_tf32(tmem_d, d_x + adv, d_chi + adv, idesc, (kb | k) != 0);
+                }
+              } else {
+                for (int k = 0; k < ksteps; ++k) {
+                  const uint64_t adv = (uint64_t)((k * 8 * 4) >> 4);
+                  tc_mma_tf32(tmem_d, d_x + adv, d_chi + adv, idesc, (kb | k) != 0);
                 }
               }
             }
-            if (ablate < 6) tc_commit(&c_empty[s]);                  // frees the centre stage
-            if (last_ct) tc_commit(&x_empty[kb]);                    // X K-block no longer needed
-            if (kb == nkb - 1 && ablate != 8) tc_commit(&t_full[a]); // accumulators ready
+            tc_commit(&c_empty[s]);                          // frees the centre stage
+            if (last_ct) tc_commit(&x_empty[kb]);            // X K-block no longer needed
+            if (kb == nkb - 1) tc_commit(&t_full[a]);        // accumulator ready
           }
           __syncwarp();
           if (++s == S) {
@@ -486,27 +451,20 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
         }
       }
     }
-    if (ablate && blockIdx.x == 0 && lane == 0) {
-      long long pn1;
-      asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(pn1));
-      g_tc_probe[0] = clock64() - pc0;
-      g_tc_probe[1] = pn1 - pn0;
-      g_tc_probe[2] = n_mma * (NPASS == 3 ? 3 : SUB);
-    }
   } else {
-    // ================= epilogue: 8 warps; warp w reads TMEM lanes [32*(w%4), +32).  SUB = 1: the two
-    //                    warps of a lane quarter take one column half of the accumulator each (merged at the
-    //                    end of the row tile); SUB = 2: one row sub-tile each, no merge.  Two warps per SM
-    //                    sub-partition hide each other's tcgen05.ld and min-chain latencies =================
+    // ================= epilogue: 8 warps; warp w reads TMEM lanes [32*(w%4), +32).  The two warps of a lane
+    //                    quarter take one column half of the accumulator each (merged at the end of the row
+    //                    tile); two warps per SM sub-partition hide each other's tcgen05.ld and min-chain
+    //                    latencies =================
     const int quarter = warp & 3;
     const int half = (warp - 2) >> 2;
-    constexpr int COLS = SUB == 1 ? BN / 2 : BN;                       // columns per warp and accumulator
+    constexpr int COLS = BN / 2;                                      // columns per warp and accumulator
     float* s_merge = reinterpret_cast<float*>(tmem_base_smem + 4);   // [3][128] exchange buffer after the barriers
     const int rl = quarter * 32 + lane;
     const bool chunk_skip = REC || n_col_tiles * BN >= 4096;   // the vote only pays once most chunks can be skipped
     uint32_t g = 0;
-    for (int rt = blockIdx.x; rt < (ablate == 8 ? 0 : n_row_tiles); rt += gridDim.x) {
-      const int64_t row = (int64_t)rt * ROWS + (SUB == 2 ? half * TC_BM : 0) + rl;
+    for (int rt = blockIdx.x; rt < n_row_tiles; rt += gridDim.x) {
+      const int64_t row = (int64_t)rt * TC_BM + rl;
       // NPASS 3: (best, second) = two smallest distances; NPASS 1: two largest scores, stored negated so that
       // both variants share the min-tracking code and the merge below
       float best = INFINITY, second = INFINITY;
@@ -521,7 +479,6 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
         tolmax = 1.001f * (2.02f * (xd * cm + xn * (cdm + 3.0517578125e-05f * cm) + 1.52587890625e-05f * cm * cm) +
                            gate.band * xn * cm + 9.5367431640625e-07f * (xn * cm + cm * cm));
         if constexpr (REC) limt = row < N ? gate.seed[row] + tc_cand_slack(xn, cm) + tolmax : -INFINITY;   // padding rows record nothing
-        else if (gate.seed != nullptr && row < N) limt = gate.seed[row] + tolmax;
       }
       int n_rec = 0;   // REC: this (row, column half)'s list
       int2* rec = nullptr;
@@ -532,18 +489,12 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
         tc_fence_after();
 #pragma unroll 1
         for (int h2 = 0; h2 < COLS / 64; ++h2) {
-          const int col0 = (SUB == 1 ? half * COLS : 0) + h2 * 64;   // column inside the centre tile
-          const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + a * (SUB * BN) +
-                                 (SUB == 2 ? half * BN : 0) + col0;
+          const int col0 = half * COLS + h2 * 64;   // column inside the centre tile
+          const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + a * BN + col0;
           uint32_t v[2][32];
-          if (ablate == 2) continue;
           tc_ld_32x32(taddr, v[0]);
           tc_ld_32x32(taddr + 32, v[1]);          // both chunks in flight before the first is consumed
           tc_wait_ld();
-          if (ablate == 1) {
-            if (v[0][0] == 0x7fc12345u && v[1][31] == 0x7fc54321u) bidx = 1;   // keep the loads alive
-            continue;
-          }
 #pragma unroll
           for (int c = 0; c < 2; ++c) {
             const int jbase = ct * BN + col0 + c * 32;
@@ -573,12 +524,6 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
       }
       if constexpr (REC) {
         if (row < N) cand.count[row * 2 + half] = n_rec;
-      } else if (SUB == 2) {
-        if (row < N) {
-          best_out[row] = best;
-          second_out[row] = second;
-          idx_out[row] = bidx;
-        }
       } else {
         // merge the two column halves of each row: lower columns win ties
         if (half == 1) {
@@ -611,745 +556,25 @@ __device__ __forceinline__ void assign_tc_body(const CUtensorMap& map_xhi, const
   }
 }
 
-template <int NPASS, int BN, int SUB>
+template <int NPASS, int BN>
 __global__ void __launch_bounds__(TC_THREADS, 1)
 k_assign_tc(const __grid_constant__ CUtensorMap map_xhi, const __grid_constant__ CUtensorMap map_xlo,
             const __grid_constant__ CUtensorMap map_chi, const __grid_constant__ CUtensorMap map_clo,
             int64_t N_host, const int32_t* __restrict__ n_rows_dev /*nullable: row count on the device*/,
             int D /*contraction width incl. the 3 augmented columns for NPASS 1*/, int n_col_tiles, int nkb,
             const float* __restrict__ cnorm /*NPASS 3: |c_j|^2*/,
-            float* __restrict__ best_out, float* __restrict__ second_out, int32_t* __restrict__ idx_out, int ablate,
-            TcGate gate) {
-  assign_tc_body<NPASS, BN, SUB, false>(map_xhi, map_xlo, map_chi, map_clo, N_host, n_rows_dev, D, n_col_tiles, nkb, cnorm,
-                                        best_out, second_out, idx_out, ablate, gate, TcCand{nullptr, nullptr, 0});
+            float* __restrict__ best_out, float* __restrict__ second_out, int32_t* __restrict__ idx_out, TcGate gate) {
+  assign_tc_body<NPASS, BN, false>(map_xhi, map_xlo, map_chi, map_clo, N_host, n_rows_dev, D, n_col_tiles, nkb, cnorm,
+                                   best_out, second_out, idx_out, gate, TcCand{nullptr, nullptr, 0});
 }
 
-// Seeded candidate pass over the compacted undecided rows: k_assign_tc<1, 256, 1>'s schedule and arithmetic on the
+// Seeded candidate pass over the compacted undecided rows: k_assign_tc<1, 256>'s schedule and arithmetic on the
 // compacted augmented rows (row count on the device), with gate.seed / xnorm / xdnorm indexed by compacted slot.
 __global__ void __launch_bounds__(TC_THREADS, 1)
 k_tc_cand(const __grid_constant__ CUtensorMap map_x1, const __grid_constant__ CUtensorMap map_c1, int64_t N_host,
           const int32_t* __restrict__ n_rows_dev, int D, int n_col_tiles, int nkb, TcGate gate, TcCand cand) {
-  assign_tc_body<1, 256, 1, true>(map_x1, map_x1, map_c1, map_c1, N_host, n_rows_dev, D, n_col_tiles, nkb, nullptr,
-                                  nullptr, nullptr, nullptr, 0, gate, cand);
-}
-
-// ---------------------------------------------------------------------------------
-// first level with the row tile in TENSOR MEMORY (tcgen05.mma with the A operand from TMEM)
-// ---------------------------------------------------------------------------------
-// A 128 x BN x 8 TF32 MMA whose operands both come from shared memory reads 4 KB (A) + BN * 32 B (B) of it; the tensor
-// pipe's operand port moves ~64 B per cycle, so at BN = 256 the MMA takes ~171 cycles instead of the 128 the B operand
-// alone needs (tools/mma_issue_probe.py), while the TMA writes of the centre stream compete for the same shared memory.
-// The row tile is the same for all Kp / BN column tiles: it is copied ONCE per row tile into tensor memory (lane = row,
-// one column per TF32 element — the layout of an accumulator) and every MMA reads A from there.  TMEM plan (512
-// columns): two BN-column accumulators + ceil8(D + 4) columns of A  ->  BN = 192 for D + 4 <= 128, BN = 128 up to 256.
-// Roles as in k_assign_tc (warp 0 TMA, warp 1 MMA, warps 2-9 epilogue); in addition the epilogue warps move the next
-// row tile shared -> registers -> TMEM (tcgen05.st) as soon as the LAST accumulator of the current row tile is
-// complete (its commit covers every MMA that read the old A), before they drain that accumulator.
-__device__ __forceinline__ void tc_mma_tf32_ts(uint32_t tmem_d, uint32_t tmem_a, uint64_t bdesc, uint32_t idesc,
-                                               uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::tf32 [%0], [%1], %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "r"(tmem_a), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-__device__ __forceinline__ void tc_st_32x8(uint32_t taddr, const uint32_t (&v)[8]) {
-  asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1, %2, %3, %4, %5, %6, %7, %8};" ::"r"(taddr), "r"(v[0]),
-               "r"(v[1]), "r"(v[2]), "r"(v[3]), "r"(v[4]), "r"(v[5]), "r"(v[6]), "r"(v[7])
-               : "memory");
-}
-__device__ __forceinline__ void tc_wait_st() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
-
-template <int BN>
-struct TsCfg {
-  static constexpr int kStageBytes = BN * TC_BK * 4;
-  static constexpr int kACol = 2 * BN;                        // first TMEM column of the A operand
-  static constexpr int kMaxK8 = (512 - kACol) / 8;            // K = 8 steps the A operand has room for
-  static constexpr int kTail = 512 /*barriers*/ + 1536 /*epilogue merge buffer*/;
-  static constexpr int kStages = (TC_SMEM_LIMIT - 1024 - kTail) / kStageBytes;   // the whole shared memory is the centre ring
-  __host__ __device__ static constexpr int c_stage(int s) { return s * kStageBytes; }
-  __host__ __device__ static constexpr int bars() { return c_stage(kStages); }
-  __host__ __device__ static constexpr int total() { return bars() + kTail + 1024; }
-};
-
-template <int BN>
-__global__ void __launch_bounds__(TC_THREADS, 1)
-k_assign_tc_ts(const float* __restrict__ x1 /*[N][ldx1] augmented TF32 rows*/, int ldx1,
-               const __grid_constant__ CUtensorMap map_c, int64_t N_host, const int32_t* __restrict__ n_rows_dev,
-               int D /*contraction width incl. the augmented columns*/, int n_col_tiles, int nkb,
-               float* __restrict__ best_out, float* __restrict__ second_out, int32_t* __restrict__ idx_out, int ablate,
-               TcGate gate) {
-  using Cfg = TsCfg<BN>;
-  static_assert(BN % 64 == 0 && Cfg::kMaxK8 >= 1 && Cfg::kStages <= 16, "tile plan");
-  constexpr int S = Cfg::kStages;
-  constexpr int NK8H = (Cfg::kMaxK8 + 1) / 2;           // K = 8 steps of a row held by one thread (the other half: its twin warp)
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::bars());
-  uint64_t* a_full = bars;                              // [1] the A operand of the row tile is in TMEM
-  uint64_t* c_full = bars + 1;                          // [16]
-  uint64_t* c_empty = c_full + 16;                      // [16]
-  uint64_t* t_full = c_empty + 16;                      // [2]
-  uint64_t* t_empty = t_full + 2;                       // [2]
-  uint32_t* tmem_base_smem = reinterpret_cast<uint32_t*>(t_empty + 2);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const int64_t N = n_rows_dev ? (int64_t)n_rows_dev[0] : N_host;
-  const int n_row_tiles = (int)((N + TC_BM - 1) / TC_BM);
-  const int k8_total = (D + 7) >> 3;                    // K = 8 steps that hold real columns
-  // experiments (gdr_debug_set("tc_ablate", mask)): 1 no epilogue arithmetic, 2 no tcgen05.ld either, 4 no MMAs, 8 no centre stream
-  const int ab = ablate > 0 ? ablate : 0;
-
-  if (warp == 0 && lane == 0) {
-    mbar_init(a_full, TC_EPI_THREADS);
-    for (int i = 0; i < S; ++i) {
-      mbar_init(&c_full[i], 1);
-      mbar_init(&c_empty[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&t_full[i], 1);
-      mbar_init(&t_empty[i], TC_EPI_THREADS);
-    }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_base_smem)), "r"(512)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_base_smem;
-
-  if (warp == 0) {
-    // ================= TMA producer: nothing but the centre stream =================
-    int s = 0;
-    uint32_t ph = 0;
-    const bool probe = (ab & 16) && blockIdx.x == 0;
-    long long p_tot = probe ? clock64() : 0, p_wait = 0;
-    for (int rt = blockIdx.x; rt < n_row_tiles; rt += gridDim.x) {
-      for (int ct = 0; ct < n_col_tiles; ++ct) {
-        for (int kb = 0; kb < nkb; ++kb) {
-          long long t0 = probe ? clock64() : 0;
-          mbar_wait(&c_empty[s], ph ^ 1);
-          if (probe) p_wait += clock64() - t0;
-          if (elect_one()) {
-            if (ab & 8) {
-              mbar_arrive(&c_full[s]);
-            } else {
-              mbar_expect_tx(&c_full[s], Cfg::kStageBytes);
-              tma_load_2d(smem + Cfg::c_stage(s), &map_c, kb * TC_BK, ct * BN, &c_full[s]);
-            }
-          }
-          __syncwarp();
-          if (++s == S) {
-            s = 0;
-            ph ^= 1;
-          }
-        }
-      }
-    }
-    if (probe && lane == 0) {
-      g_ts_probe[5] = clock64() - p_tot;
-      g_ts_probe[6] = p_wait;
-    }
-  } else if (warp == 1) {
-    // ================= MMA issuer (uniform control flow, one elected lane issues) =================
-    constexpr uint32_t idesc = umma_idesc_tf32(TC_BM, BN);
-    uint32_t tile_it = 0, g = 0;
-    int s = 0;
-    uint32_t ph = 0;
-    const uint64_t dc0 = umma_desc_sw128(smem_u32(smem));
-    constexpr uint64_t kStage = Cfg::kStageBytes >> 4;
-    const uint32_t tmem_a = tmem_base + Cfg::kACol;
-    const bool probe = (ab & 16) && blockIdx.x == 0;
-    long long m_tot = probe ? clock64() : 0, m_wc = 0, m_wt = 0, m_wa = 0, m_is = 0, t0 = 0, t1 = 0;
-    for (int rt = blockIdx.x; rt < n_row_tiles; rt += gridDim.x, ++tile_it) {
-      if (probe) t0 = clock64();
-      mbar_wait(a_full, tile_it & 1);
-      tc_fence_after();
-      if (probe) m_wa += clock64() - t0;
-      for (int ct = 0; ct < n_col_tiles; ++ct, ++g) {
-        const uint32_t a = g & 1, aph = (g >> 1) & 1;
-        if (probe) t0 = clock64();
-        mbar_wait(&t_empty[a], aph ^ 1);
-        tc_fence_after();
-        if (probe) m_wt += clock64() - t0;
-        const uint32_t tmem_d = tmem_base + a * BN;
-        for (int kb = 0; kb < nkb; ++kb) {
-          if (probe) t0 = clock64();
-          mbar_wait(&c_full[s], ph);
-          tc_fence_after();
-          if (probe) {
-            t1 = clock64();
-            m_wc += t1 - t0;
-          }
-          const uint64_t d_c = dc0 + (uint64_t)s * kStage;
-          const int ksteps = min(TC_BK / 8, k8_total - kb * (TC_BK / 8));
-          if (elect_one()) {
-            const uint32_t ta = tmem_a + kb * TC_BK;
-            if (!(ab & 4) && ksteps == 4) {
-#pragma unroll
-              for (int k = 0; k < 4; ++k)
-                tc_mma_tf32_ts(tmem_d, ta + k * 8, d_c + (uint64_t)((k * 8 * 4) >> 4), idesc, (kb | k) != 0);
-            } else {
-              for (int k = 0; k < ((ab & 4) ? 0 : ksteps); ++k)
-                tc_mma_tf32_ts(tmem_d, ta + k * 8, d_c + (uint64_t)((k * 8 * 4) >> 4), idesc, (kb | k) != 0);
-            }
-            tc_commit(&c_empty[s]);
-            if (kb == nkb - 1) tc_commit(&t_full[a]);
-          }
-          __syncwarp();
-          if (probe) m_is += clock64() - t1;
-          if (++s == S) {
-            s = 0;
-            ph ^= 1;
-          }
-        }
-      }
-    }
-    if (probe && lane == 0) {
-      g_ts_probe[0] = clock64() - m_tot;
-      g_ts_probe[1] = m_wc;
-      g_ts_probe[2] = m_wt;
-      g_ts_probe[3] = m_wa;
-      g_ts_probe[4] = m_is;
-    }
-  } else {
-    // ================= epilogue (8 warps; warp w owns TMEM lanes [32 (w % 4), +32) and one column half) =================
-    const int quarter = warp & 3;
-    const int half = (warp - 2) >> 2;
-    constexpr int COLS = BN / 2;
-    float* s_merge = reinterpret_cast<float*>(tmem_base_smem + 4);
-    const int rl = quarter * 32 + lane;
-    const uint32_t lane_addr = tmem_base + ((uint32_t)(quarter * 32) << 16);
-    const bool chunk_skip = n_col_tiles * BN >= 4096;
-    // The row tile travels global -> registers -> TMEM: thread (quarter, lane) owns row rl and, of its K = 8 steps, those
-    // of its warp's parity (the twin warp of the lane quarter takes the others).  The loads of the NEXT row tile are
-    // issued at the start of the current one and rest in registers until its last accumulator is complete.
-    uint32_t xa[NK8H][8];
-    auto load_a = [&](int rt) {
-      const int64_t row = (int64_t)rt * TC_BM + rl;
-      const uint4* src = reinterpret_cast<const uint4*>(x1 + row * ldx1);
-#pragma unroll
-      for (int i = 0; i < NK8H; ++i) {
-        const int k8 = 2 * i + half;
-        uint4 lo = make_uint4(0, 0, 0, 0), hi = lo;
-        if (k8 < k8_total && row < N) {
-          lo = __ldg(src + 2 * k8);
-          hi = __ldg(src + 2 * k8 + 1);
-        }
-        xa[i][0] = lo.x, xa[i][1] = lo.y, xa[i][2] = lo.z, xa[i][3] = lo.w;
-        xa[i][4] = hi.x, xa[i][5] = hi.y, xa[i][6] = hi.z, xa[i][7] = hi.w;
-      }
-    };
-    auto store_a = [&]() {
-#pragma unroll
-      for (int i = 0; i < NK8H; ++i) {
-        const int k8 = 2 * i + half;
-        if (k8 < k8_total) tc_st_32x8(lane_addr + Cfg::kACol + k8 * 8, xa[i]);
-      }
-      tc_wait_st();
-      tc_fence_before();
-      mbar_arrive(a_full);
-    };
-    uint32_t g = 0;
-    const bool probe = (ab & 16) && blockIdx.x == 0 && warp == 2;
-    long long e_tot = probe ? clock64() : 0, e_wt = 0, e_ld = 0, e_ar = 0, e_st = 0, t0 = 0, t1 = 0;
-    if ((int)blockIdx.x < n_row_tiles) {
-      load_a(blockIdx.x);
-      store_a();
-    }
-    for (int rt = blockIdx.x; rt < n_row_tiles; rt += gridDim.x) {
-      const int64_t row = (int64_t)rt * TC_BM + rl;
-      const bool has_next = rt + (int)gridDim.x < n_row_tiles;
-      if (has_next) load_a(rt + gridDim.x);
-      float best = INFINITY, second = INFINITY;
-      int bidx = 0;
-      float tolmax = 0.f, limt = INFINITY;
-      const bool gated = chunk_skip && gate.xnorm != nullptr;
-      if (gated) {
-        const float xn = row < N ? gate.xnorm[row] : 0.f, xd = row < N ? gate.xdnorm[row] : 0.f;
-        const float cm = gate.cscal[0], cdm = gate.cscal[1];
-        tolmax = 1.001f * (2.02f * (xd * cm + xn * (cdm + 3.0517578125e-05f * cm) + 1.52587890625e-05f * cm * cm) +
-                           gate.band * xn * cm + 9.5367431640625e-07f * (xn * cm + cm * cm));
-        if (gate.seed != nullptr && row < N) limt = gate.seed[row] + tolmax;
-      }
-      for (int ct = 0; ct < n_col_tiles; ++ct, ++g) {
-        const uint32_t a = g & 1, aph = (g >> 1) & 1;
-        if (probe) t0 = clock64();
-        mbar_wait(&t_full[a], aph);
-        tc_fence_after();
-        if (probe) {
-          t1 = clock64();
-          e_wt += t1 - t0;
-        }
-        // every MMA of this row tile is complete: the next one takes its place in TMEM before this accumulator is read
-        if (ct == n_col_tiles - 1 && has_next) store_a();
-        if (probe) {
-          t0 = clock64();
-          e_st += t0 - t1;
-        }
-        const uint32_t tacc = lane_addr + a * BN + half * COLS;
-        const int j0 = ct * BN + half * COLS;
-        if (!(ab & 2)) {
-#pragma unroll 1
-          for (int h2 = 0; h2 < COLS / 64; ++h2) {
-            uint32_t v[2][32];
-            tc_ld_32x32(tacc + h2 * 64, v[0]);
-            tc_ld_32x32(tacc + h2 * 64 + 32, v[1]);
-            tc_wait_ld();
-            if (ab & 1) {
-              if (v[0][0] == 0x7fc12345u && v[1][31] == 0x7fc54321u) bidx = 1;
-              continue;
-            }
-            epi_chunk32(v[0], j0 + h2 * 64, chunk_skip, gated, tolmax, limt, best, second, bidx);
-            epi_chunk32(v[1], j0 + h2 * 64 + 32, chunk_skip, gated, tolmax, limt, best, second, bidx);
-          }
-          if (COLS % 64) {
-            uint32_t v[32];
-            tc_ld_32x32(tacc + (COLS / 64) * 64, v);
-            tc_wait_ld();
-            if (ab & 1) {
-              if (v[0] == 0x7fc12345u) bidx = 1;
-            } else {
-              epi_chunk32(v, j0 + (COLS / 64) * 64, chunk_skip, gated, tolmax, limt, best, second, bidx);
-            }
-          }
-        }
-        if (probe) {
-          t1 = clock64();
-          e_ld += t1 - t0;
-        }
-        tc_fence_before();
-        mbar_arrive(&t_empty[a]);
-        if (probe) e_ar += clock64() - t1;
-      }
-      // merge the two column halves of each row: lower columns win ties
-      if (half == 1) {
-        s_merge[rl] = best;
-        s_merge[128 + rl] = second;
-        reinterpret_cast<int*>(s_merge)[256 + rl] = bidx;
-      }
-      asm volatile("bar.sync 1, %0;" ::"n"(TC_EPI_THREADS) : "memory");
-      if (half == 0) {
-        const float b1 = s_merge[rl], s1 = s_merge[128 + rl];
-        const int i1 = reinterpret_cast<int*>(s_merge)[256 + rl];
-        const float nb = fminf(best, b1);
-        const float ns = fminf(fminf(second, s1), fmaxf(best, b1));
-        const int ni = b1 < best ? i1 : bidx;
-        if (row < N) {
-          best_out[row] = nb;
-          second_out[row] = ns;
-          idx_out[row] = ni;
-        }
-      }
-      asm volatile("bar.sync 1, %0;" ::"n"(TC_EPI_THREADS) : "memory");
-    }
-    if (probe && lane == 0) {
-      g_ts_probe[7] = clock64() - e_tot;
-      g_ts_probe[8] = e_wt;
-      g_ts_probe[9] = e_ld;
-      g_ts_probe[10] = e_ar;
-      g_ts_probe[11] = e_st;
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 1) {
-    __syncwarp();
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
-}
-
-// ---------------------------------------------------------------------------------
-// first level on CTA pairs: tcgen05.mma.cta_group::2, M = 256 (128 rows per CTA), N = 256
-// ---------------------------------------------------------------------------------
-// The single-CTA first level is bound by the stream of centre tiles (L2 -> SMEM at ~9 TB/s chip-wide and the
-// SMEM operand reads of N = 128 shapes).  A CTA pair shares every centre tile: each CTA loads HALF of it
-// (128 centres) and the pair's MMA reads both halves, so L2 traffic and B-operand SMEM reads per flop halve
-// while each CTA still owns a full 128 x 256 accumulator.  Protocol (leader = cluster rank 0):
-//   * both producers TMA into their own SMEM but complete the transaction bytes on the LEADER's full barriers;
-//   * only the leader's thread issues MMAs; its tcgen05.commit multicasts the arrive to both CTAs' barriers
-//     (stage free, row tile free, accumulator ready);
-//   * one lane per epilogue warp of BOTH CTAs arrives on the leader's accumulator-empty barrier (count 16).
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-  asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t smem_addr, uint32_t cta_rank) {
-  uint32_t r;
-  asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(cta_rank));
-  return r;
-}
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-  asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
-}
-// TMA load into this CTA's shared memory, transaction bytes completed on a barrier given by its cluster address
-__device__ __forceinline__ void tma_load_2d_2sm(void* smem_dst, const CUtensorMap* map, int c0, int c1,
-                                                uint32_t bar_cluster_addr) {
-  asm volatile(
-      "cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-      ::"r"(smem_u32(smem_dst)), "l"(reinterpret_cast<uint64_t>(map)), "r"(c0), "r"(c1), "r"(bar_cluster_addr)
-      : "memory");
-}
-__device__ __forceinline__ void tc_commit_2sm(uint64_t* bar, uint16_t cta_mask) {
-  asm volatile(
-      "tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-      ::"r"(smem_u32(bar)), "h"(cta_mask)
-      : "memory");
-}
-__device__ __forceinline__ void tc_mma_tf32_2sm(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                                uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::2.kind::tf32 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
-
-struct Tc2Cfg {
-  static constexpr int BN = 256;                                  // centres per accumulator (pair-wide MMA N)
-  static constexpr int kStageBytes = (BN / 2) * TC_BK * 4;        // this CTA's half of one centre K-block: 16 KB
-  static constexpr int kStages = 8;
-  static constexpr int kTmemCols = 2 * BN;
-  static constexpr int kTail = 512;                               // barriers + TMEM base slot
-  __host__ __device__ static constexpr int x_blk(int kb) { return kb * TC_KBLK_BYTES; }
-  __host__ __device__ static constexpr int c_stage(int nkb, int s) { return nkb * TC_KBLK_BYTES + s * kStageBytes; }
-  __host__ __device__ static constexpr int bars(int nkb) { return c_stage(nkb, kStages); }
-  __host__ __device__ static constexpr int total(int nkb) { return bars(nkb) + kTail + 1024; }
-};
-
-__global__ void __launch_bounds__(TC_THREADS, 1)
-k_assign_tc_pair(const __grid_constant__ CUtensorMap map_x, const __grid_constant__ CUtensorMap map_c,
-                 int64_t N_host, const int32_t* __restrict__ n_rows_dev, int D, int n_col_tiles, int nkb,
-                 float* __restrict__ best_out, float* __restrict__ second_out, int32_t* __restrict__ idx_out, int ablate,
-                 int fwd /*1: ordinary 1-SM TMA on each CTA's own barriers, the peer forwards "stage landed" to the leader*/) {
-  using Cfg = Tc2Cfg;
-  constexpr int S = Cfg::kStages;
-  constexpr int BN = Cfg::BN;
-  extern __shared__ uint8_t smem_raw[];
-  // identical offsets in both CTAs: the dynamic shared memory base is the same for every CTA of a kernel
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::bars(nkb));
-  uint64_t* x_full = bars;                              // [TC_BAR_KB]  used in the leader
-  uint64_t* x_empty = bars + TC_BAR_KB;                 // [TC_BAR_KB]  each CTA its own
-  uint64_t* c_full = bars + 2 * TC_BAR_KB;              // [S]          used in the leader
-  uint64_t* c_empty = c_full + S;                       // [S]          each CTA its own
-  uint64_t* t_full = c_empty + S;                       // [2]          each CTA its own
-  uint64_t* t_empty = t_full + 2;                       // [2]          used in the leader
-  uint64_t* c_peer = t_empty + 2;                       // [S]          leader: "the peer's half of stage s has landed" (fwd)
-  uint64_t* x_peer = c_peer + S;                        // [TC_BAR_KB]  leader: same for the peer's row-tile K-blocks (fwd)
-  uint32_t* tmem_base_smem = reinterpret_cast<uint32_t*>(x_peer + TC_BAR_KB);
-
-  const int warp = threadIdx.x >> 5;
-  const int lane = threadIdx.x & 31;
-  const uint32_t crank = cluster_ctarank();
-  const bool leader = crank == 0;
-  const int64_t N = n_rows_dev ? (int64_t)n_rows_dev[0] : N_host;
-  const int n_row_tiles = (int)((N + TC_BM - 1) / TC_BM);
-  const int n_units = (n_row_tiles + 1) / 2;            // a unit = two consecutive row tiles, one per CTA
-  const int unit0 = (int)blockIdx.x >> 1, unit_stride = (int)gridDim.x >> 1;
-
-  if (warp == 0 && lane == 0) {
-    for (int i = 0; i < TC_BAR_KB; ++i) {
-      mbar_init(&x_full[i], 1);
-      mbar_init(&x_empty[i], 1);
-    }
-    for (int i = 0; i < S; ++i) {
-      mbar_init(&c_full[i], 1);
-      mbar_init(&c_empty[i], 1);
-    }
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&t_full[i], 1);
-      mbar_init(&t_empty[i], 16);       // one lane of each of the 8 epilogue warps of both CTAs
-    }
-    for (int i = 0; i < S; ++i) mbar_init(&c_peer[i], 1);
-    for (int i = 0; i < TC_BAR_KB; ++i) mbar_init(&x_peer[i], 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (warp == 1) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(tmem_base_smem)),
-                 "r"(Cfg::kTmemCols)
-                 : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();                   // peer barriers initialised, both TMEM allocations done
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_base_smem;
-
-  if (warp == 0) {
-    // ================= TMA producer (both CTAs; warp-uniform loop, one elected lane issues) =================
-    uint32_t tile_it = 0;
-    int s = 0;
-    uint32_t ph = 0;
-    const uint32_t x_full0 = mapa_u32(smem_u32(&x_full[0]), 0), c_full0 = mapa_u32(smem_u32(&c_full[0]), 0);   // leader's barriers
-    for (int un = unit0; un < n_units; un += unit_stride, ++tile_it) {
-      const int rt = 2 * un + (int)crank;
-      for (int kb = 0; kb < nkb; ++kb) {
-        mbar_wait(&x_empty[kb], (tile_it & 1) ^ 1);
-        if (elect_one()) {
-          if (fwd) {
-            mbar_expect_tx(&x_full[kb], TC_KBLK_BYTES);
-            tma_load_2d(smem + Cfg::x_blk(kb), &map_x, kb * TC_BK, rt * TC_BM, &x_full[kb]);
-          } else {
-            if (leader) mbar_expect_tx(&x_full[kb], 2 * TC_KBLK_BYTES);
-            tma_load_2d_2sm(smem + Cfg::x_blk(kb), &map_x, kb * TC_BK, rt * TC_BM, x_full0 + 8u * (uint32_t)kb);
-          }
-        }
-        __syncwarp();
-      }
-      for (int ct = 0; ct < n_col_tiles; ++ct) {
-        for (int kb = 0; kb < nkb; ++kb) {
-          if (ablate >= 6) continue;
-          mbar_wait(&c_empty[s], ph ^ 1);
-          if (elect_one()) {
-            if (ablate == 5) {
-              if (leader || fwd) mbar_arrive(&c_full[s]);
-            } else if (fwd) {
-              mbar_expect_tx(&c_full[s], Cfg::kStageBytes);
-              tma_load_2d(smem + Cfg::c_stage(nkb, s), &map_c, kb * TC_BK, ct * BN + (int)crank * (BN / 2), &c_full[s]);
-            } else {
-              if (leader) mbar_expect_tx(&c_full[s], 2 * Cfg::kStageBytes);
-              tma_load_2d_2sm(smem + Cfg::c_stage(nkb, s), &map_c, kb * TC_BK, ct * BN + (int)crank * (BN / 2),
-                              c_full0 + 8u * (uint32_t)s);
-            }
-          }
-          __syncwarp();
-          if (++s == S) {
-            s = 0;
-            ph ^= 1;
-          }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ================= MMA issuer (leader CTA only; warp-uniform loop, one elected lane issues) =================
-    if (leader) {
-      constexpr uint32_t idesc = umma_idesc_tf32(2 * TC_BM, BN);
-      uint32_t tile_it = 0, g = 0;
-      int s = 0;
-      uint32_t ph = 0;
-      const uint64_t dx0 = umma_desc_sw128(smem_u32(smem));
-      const uint64_t dc0 = umma_desc_sw128(smem_u32(smem + Cfg::c_stage(nkb, 0)));
-      constexpr uint64_t kKb = TC_KBLK_BYTES >> 4, kStage = Cfg::kStageBytes >> 4;
-      for (int un = unit0; un < n_units; un += unit_stride, ++tile_it) {
-        for (int ct = 0; ct < n_col_tiles; ++ct, ++g) {
-          const uint32_t a = g & 1, aph = (g >> 1) & 1;
-          if (ablate != 8) mbar_wait(&t_empty[a], aph ^ 1);
-          tc_fence_after();
-          const uint32_t tmem_d = tmem_base + a * BN;
-          const bool last_ct = ct == n_col_tiles - 1;
-          for (int kb = 0; kb < nkb; ++kb) {
-            if (ct == 0) {
-              mbar_wait(&x_full[kb], tile_it & 1);
-              if (fwd) mbar_wait(&x_peer[kb], tile_it & 1);
-            }
-            if (ablate < 6) {
-              mbar_wait(&c_full[s], ph);
-              if (fwd) mbar_wait(&c_peer[s], ph);
-            }
-            tc_fence_after();
-            const uint64_t d_x = dx0 + (uint64_t)kb * kKb;
-            const uint64_t d_c = dc0 + (uint64_t)s * kStage;
-            const int ksteps = min(TC_BK / 8, (D - kb * TC_BK + 7) >> 3);
-            if (elect_one()) {
-              if (ablate != 3 && ablate != 4 && ksteps == 4) {
-#pragma unroll
-                for (int k = 0; k < 4; ++k) {
-                  const uint64_t adv = (uint64_t)((k * 8 * 4) >> 4);
-                  tc_mma_tf32_2sm(tmem_d, d_x + adv, d_c + adv, idesc, (kb | k) != 0);
-                }
-              } else {
-                for (int k = 0; k < ((ablate == 3 || (ablate == 4 && kb > 0)) ? 0 : ksteps); ++k) {
-                  const uint64_t adv = (uint64_t)((k * 8 * 4) >> 4);
-                  tc_mma_tf32_2sm(tmem_d, d_x + adv, d_c + adv, idesc, (kb | k) != 0);
-                }
-              }
-              if (ablate < 6) tc_commit_2sm(&c_empty[s], 3);              // frees the stage in both CTAs
-              if (last_ct) tc_commit_2sm(&x_empty[kb], 3);                // row-tile K-block free in both CTAs
-              if (kb == nkb - 1 && ablate != 8) tc_commit_2sm(&t_full[a], 3);   // accumulator ready in both CTAs
-            }
-            __syncwarp();
-            if (++s == S) {
-              s = 0;
-              ph ^= 1;
-            }
-          }
-        }
-      }
-    } else if (fwd) {
-      // peer CTA: forward "my half of the stage / my row-tile K-block has landed" to the leader's barriers
-      uint32_t tile_it = 0;
-      int s = 0;
-      uint32_t ph = 0;
-      const uint32_t c_peer0 = mapa_u32(smem_u32(&c_peer[0]), 0), x_peer0 = mapa_u32(smem_u32(&x_peer[0]), 0);
-      for (int un = unit0; un < n_units; un += unit_stride, ++tile_it) {
-        for (int ct = 0; ct < n_col_tiles; ++ct) {
-          for (int kb = 0; kb < nkb; ++kb) {
-            if (ct == 0) {
-              mbar_wait(&x_full[kb], tile_it & 1);
-              if (elect_one()) mbar_arrive_cluster(x_peer0 + 8u * (uint32_t)kb);
-              __syncwarp();
-            }
-            mbar_wait(&c_full[s], ph);
-            if (elect_one()) mbar_arrive_cluster(c_peer0 + 8u * (uint32_t)s);
-            __syncwarp();
-            if (++s == S) {
-              s = 0;
-              ph ^= 1;
-            }
-          }
-        }
-      }
-    }
-  } else {
-    // ================= epilogue (both CTAs): as k_assign_tc<1, 256, 1> =================
-    const int quarter = warp & 3;
-    const int half = (warp - 2) >> 2;
-    const int rl = quarter * 32 + lane;
-    const uint32_t t_empty_leader[2] = {mapa_u32(smem_u32(&t_empty[0]), 0), mapa_u32(smem_u32(&t_empty[1]), 0)};
-    __shared__ float s_mb[3][TC_BM];
-    uint32_t g = 0;
-    for (int un = unit0; un < (ablate == 8 ? 0 : n_units); un += unit_stride) {
-      const int rt = 2 * un + (int)crank;
-      const int64_t row = (int64_t)rt * TC_BM + rl;
-      float best = INFINITY, second = INFINITY;   // negated scores
-      int bidx = 0;
-      for (int ct = 0; ct < n_col_tiles; ++ct, ++g) {
-        const uint32_t a = g & 1, aph = (g >> 1) & 1;
-        mbar_wait(&t_full[a], aph);
-        tc_fence_after();
-#pragma unroll 1
-        for (int h2 = 0; h2 < (ablate == 2 ? 0 : BN / 128); ++h2) {
-          const int col0 = half * (BN / 2) + h2 * 64;
-          const uint32_t taddr = tmem_base + ((uint32_t)(quarter * 32) << 16) + a * BN + col0;
-          uint32_t v[2][32];
-          tc_ld_32x32(taddr, v[0]);
-          tc_ld_32x32(taddr + 32, v[1]);
-          tc_wait_ld();
-#pragma unroll
-          for (int c = 0; c < 2; ++c) {
-            const int jbase = ct * BN + col0 + c * 32;
-#pragma unroll
-            for (int u0 = 0; u0 < 32; u0 += 8) {               // chunk skip as in k_assign_tc<1, *, *>
-              float m = fmaxf(fmaxf(__uint_as_float(v[c][u0]), __uint_as_float(v[c][u0 + 1])),
-                              fmaxf(__uint_as_float(v[c][u0 + 2]), __uint_as_float(v[c][u0 + 3])));
-              m = fmaxf(m, fmaxf(fmaxf(__uint_as_float(v[c][u0 + 4]), __uint_as_float(v[c][u0 + 5])),
-                                 fmaxf(__uint_as_float(v[c][u0 + 6]), __uint_as_float(v[c][u0 + 7]))));
-              if (__any_sync(0xffffffffu, -m < second)) {
-#pragma unroll
-                for (int u = u0; u < u0 + 8; ++u) {
-                  const float d = -__uint_as_float(v[c][u]);
-                  second = fminf(second, fmaxf(d, best));
-                  bidx = d < best ? jbase + u : bidx;
-                  best = fminf(best, d);
-                }
-              }
-            }
-          }
-        }
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive_cluster(t_empty_leader[a]);
-      }
-      // merge the two column halves of each row
-      if (half == 1) {
-        s_mb[0][rl] = best;
-        s_mb[1][rl] = second;
-        reinterpret_cast<int*>(s_mb[2])[rl] = bidx;
-      }
-      asm volatile("bar.sync 1, %0;" ::"n"(TC_EPI_THREADS) : "memory");
-      if (half == 0) {
-        const float b1 = s_mb[0][rl], s1 = s_mb[1][rl];
-        const int i1 = reinterpret_cast<int*>(s_mb[2])[rl];
-        const float nb = fminf(best, b1);
-        const float ns = fminf(fminf(second, s1), fmaxf(best, b1));
-        const int ni = b1 < best ? i1 : bidx;
-        if (row < N) {
-          best_out[row] = nb;
-          second_out[row] = ns;
-          idx_out[row] = ni;
-        }
-      }
-      asm volatile("bar.sync 1, %0;" ::"n"(TC_EPI_THREADS) : "memory");
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();   // neither CTA frees TMEM / leaves while the pair's MMAs, multicasts or remote arrives can still land
-  if (warp == 1) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(Cfg::kTmemCols) : "memory");
-  }
-}
-
-// micro-probe of the pair MMA (tools/mma_issue_probe.py): a 2-CTA cluster, the leader issues `iters`
-// tcgen05.mma.cta_group::2 of shape 256 x 256 x (32 bytes of K) in the production pattern (4-4-4-1 per tile, four
-// A / B tiles, alternating accumulators) on zero-filled operands; cycles until the last one has completed.
-__global__ void __launch_bounds__(128, 1) k_mma_probe_pair(int iters, long long* __restrict__ cycles) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  __shared__ uint64_t bar;
-  __shared__ uint32_t tmem_slot;
-  for (int i = threadIdx.x; i < 8 * 128 * 128 / 4; i += blockDim.x) reinterpret_cast<float*>(smem)[i] = 0.f;
-  const bool leader = cluster_ctarank() == 0;
-  if (threadIdx.x == 0) {
-    mbar_init(&bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (threadIdx.x < 32) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-  }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  tc_fence_after();
-  const uint32_t tmem_base = tmem_slot;
-  if (leader && threadIdx.x < 32) {
-    constexpr uint32_t idesc = umma_idesc_tf32(256, 256);
-    const long long t0 = clock64();
-    int issued = 0;
-    for (int t = 0; issued < iters; ++t) {
-      const uint32_t d = tmem_base + (uint32_t)(t & 1) * 256u;
-      for (int kb = 0; kb < 4; ++kb) {
-        const uint64_t da = umma_desc_sw128(smem_u32(smem + kb * 16384));
-        const uint64_t db = umma_desc_sw128(smem_u32(smem + 65536 + ((t * 4 + kb) & 3) * 16384));
-        const int ks = kb < 3 ? 4 : 1;
-        tc_fence_after();
-        if (elect_one()) {
-          for (int k = 0; k < ks; ++k) {
-            const uint64_t adv = (uint64_t)((k * 32) >> 4);
-            tc_mma_tf32_2sm(d, da + adv, db + adv, idesc, (kb | k) != 0);
-          }
-        }
-        __syncwarp();
-        issued += ks;
-      }
-    }
-    if (elect_one()) tc_commit_2sm(&bar, 1);
-    __syncwarp();
-    mbar_wait(&bar, 0);
-    if (threadIdx.x == 0) cycles[0] = clock64() - t0;
-  }
-  tc_fence_before();
-  __syncthreads();
-  cluster_sync_all();
-  if (threadIdx.x < 32) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
+  assign_tc_body<1, 256, true>(map_x1, map_x1, map_c1, map_c1, N_host, n_rows_dev, D, n_col_tiles, nkb, nullptr,
+                               nullptr, nullptr, nullptr, gate, cand);
 }
 
 // first-level decision.  best = -s_idx, second = -s_second (negated scores of the first-level kernel).  With
@@ -1394,38 +619,6 @@ __global__ void __launch_bounds__(256) k_tc_select1(int64_t N, const float* __re
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) changed += __shfl_xor_sync(0xffffffffu, changed, o);
     if (lane_id() == 0 && changed) atomicAdd(n_changed, changed);
-  }
-}
-
-// Seed of the first-level gate: the score of row i against the NEW centre of its previous label, evaluated on the
-// same augmented TF32 operands the GEMM multiplies (fp32 FMA chain instead of the TMEM accumulation: the two agree to
-// ~(D + 4) 2^-23 |x||c|, covered by the 2^-18 slack).  seed_i >= the row's final best negated score.
-__global__ void __launch_bounds__(256) k_tc_seed(int64_t N, int64_t K, int Dp1, const float* __restrict__ x1,
-                                                 const float* __restrict__ c1, const int32_t* __restrict__ hint,
-                                                 const float* __restrict__ xnorm, const float* __restrict__ cscal,
-                                                 float* __restrict__ seed) {
-  const int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
-  if (r >= N) return;
-  const int j = hint[r];
-  if (j < 0 || j >= K) {
-    if (lane_id() == 0) seed[r] = INFINITY;
-    return;
-  }
-  const float4* a = reinterpret_cast<const float4*>(x1 + r * Dp1);
-  const float4* b = reinterpret_cast<const float4*>(c1 + (int64_t)j * Dp1);
-  float acc = 0.f;
-  for (int c = lane_id(); c < (Dp1 >> 2); c += 32) {
-    const float4 p = __ldg(a + c), q = __ldg(b + c);
-    acc = fmaf(p.x, q.x, acc);
-    acc = fmaf(p.y, q.y, acc);
-    acc = fmaf(p.z, q.z, acc);
-    acc = fmaf(p.w, q.w, acc);
-  }
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
-  if (lane_id() == 0) {
-    const float xn = xnorm[r], cm = cscal[0];
-    seed[r] = -acc + 3.814697265625e-06f * (xn * cm + cm * cm);
   }
 }
 
@@ -1695,101 +888,12 @@ __global__ void __launch_bounds__(256) k_tc_select(int64_t N, const float* __res
 }
 
 // ---------------------------------------------------------------------------------
-// tensor-pipe micro-probe (tools/mma_rate_probe.py): one CTA issues `iters` back-to-back tcgen05.mma of shape
-// 128 x N x (32 bytes of K) on zero-filled, 128B-swizzled operand tiles and reports the cycles until the
-// last one has completed.  variant bit 0: kind::f16 (BF16) instead of kind::tf32; bit 1: alternate between
-// two accumulators; bit 2: same K offset every time (no advance inside the swizzle atom).
-// ---------------------------------------------------------------------------------
-__global__ void __launch_bounds__(128, 1) k_mma_probe(int N, int iters, int variant, long long* __restrict__ cycles) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-  __shared__ uint64_t bar;
-  __shared__ uint32_t tmem_slot;
-  // variant bit 3: non-zero operands (a hash of the index, |v| < 1)
-  for (int i = threadIdx.x; i < 4 * (128 + 256) * 128 / 4; i += blockDim.x)
-    reinterpret_cast<float*>(smem)[i] = (variant & 8) ? (float)((i * 2654435761u) >> 8) * 5.9604645e-8f - 0.5f : 0.f;
-  __shared__ uint64_t bar2;
-  if (threadIdx.x == 0) {
-    mbar_init(&bar2, 1);
-    mbar_init(&bar, 1);
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-  }
-  if (threadIdx.x < 32) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(&tmem_slot)), "r"(512) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-  }
-  asm volatile("fence.proxy.async.shared::cta;" ::: "memory");   // generic-proxy zero fill -> async-proxy MMA reads
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = tmem_slot;
-  if (threadIdx.x < 32) {   // warp-uniform loop, one elected lane issues (as the production kernels do)
-    const uint32_t fmt = (variant & 1) ? 1u : 2u;
-    const uint32_t idesc = (1u << 4) | (fmt << 7) | (fmt << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
-    const long long t0 = clock64();
-    if (variant & 256) {
-      // bit 8: the production pattern — per "tile" four elect blocks of 4, 4, 4 and 1 MMAs on four different A / B
-      // tiles, accumulator overwritten by the first, accumulators alternating per tile (+ bit 4: commits as there)
-      int issued = 0;
-      for (int t = 0; issued < iters; ++t) {
-        const uint32_t d = tmem_base + (uint32_t)(t & 1) * 256u;
-        for (int kb = 0; kb < 4; ++kb) {
-          const uint64_t da = umma_desc_sw128(smem_u32(smem + kb * 16384));
-          const uint64_t db = umma_desc_sw128(smem_u32(smem + 65536 + ((t * 4 + kb) & 3) * 32768));
-          const int ks = kb < 3 ? 4 : ((variant & 512) ? 4 : 1);     // bit 9: no K tail (4, 4, 4, 4)
-          tc_fence_after();
-          if (elect_one()) {
-            for (int k = 0; k < ks; ++k) {
-              const uint64_t adv = (uint64_t)((k * 32) >> 4);
-              tc_mma_tf32(d, da + adv, db + adv, idesc, (kb | k) != 0);
-            }
-            if (variant & 16) tc_commit(&bar2);
-          }
-          __syncwarp();
-          issued += ks;
-        }
-      }
-    } else
-    for (int i = 0; i < iters; i += 4) {
-      // bit 7: a different A tile and B tile for every group of 4 MMAs (4 of each in shared memory), as a real
-      // K loop has; otherwise the same two tiles are re-used by every MMA
-      const int tsel = (variant & 128) ? ((i >> 2) & 3) : 0;
-      const uint64_t da = umma_desc_sw128(smem_u32(smem + tsel * 16384));
-      const uint64_t db = umma_desc_sw128(smem_u32(smem + 65536 + tsel * 32768));
-      if (variant & 64) tc_fence_after();                      // bit 6: tcgen05.fence::after_thread_sync every 4 MMAs
-      const uint32_t d = tmem_base + ((variant & 2) ? (uint32_t)((i >> 2) & 1) * 256u : 0u);
-      if (elect_one()) {
-#pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          const uint64_t adv = (variant & 4) ? 0 : (uint64_t)((k * 32) >> 4);
-          const uint32_t acc = (variant & 32) ? (uint32_t)(((i + k) % 16) != 0) : (uint32_t)(i + k > 1);
-          if (variant & 1) tc_mma_bf16(d, da + adv, db + adv, idesc, acc);
-          else tc_mma_tf32(d, da + adv, db + adv, idesc, acc);
-        }
-        if (variant & 16) tc_commit(&bar2);                    // bit 4: a commit every 4 MMAs
-      }
-      __syncwarp();
-    }
-    if (elect_one()) tc_commit(&bar);
-    __syncwarp();
-    mbar_wait(&bar, 0);
-    if (threadIdx.x == 0) cycles[0] = clock64() - t0;
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (threadIdx.x < 32) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
-  }
-}
-
-// ---------------------------------------------------------------------------------
 // host side
 // ---------------------------------------------------------------------------------
 static inline int dpad(int64_t D) { return (int)align_up(D, TC_BK); }
 constexpr int TC_AUG = 4;   // augmented columns of the first-level operands
 static inline int dpad1(int64_t D) { return (int)align_up(D + TC_AUG, TC_BK); }
 constexpr int TC_KPAD = 256;   // centres padded to the widest accumulator tile
-constexpr int TC_TS_BN = 192;  // accumulator width of the A-in-TMEM first level (its last tile may reach past Kp)
 // candidates recorded per row and column half.  tools/cand_estimate.py, config-E-shaped data after one Lloyd update,
 // 20 000-row sample: 3.7 % (D = 100) / 3.0 % (D = 47) of the rows undecided, 2.2 recorded per row on average, at most 4
 // in one column half (profiles/r3_cand_estimate_configE.txt): 16 leaves ample room at 256 bytes of list per row
@@ -1835,7 +939,7 @@ static bool tc_two_level(int64_t N, bool want_best) {
 int64_t kmeans_assign_tc_ws_bytes(int64_t N, int64_t K, int64_t D) {
   int Dp = dpad(D);
   int64_t Kp = align_up(K, TC_KPAD);
-  return 3 * ws_need(Kp * Dp, 4) /*c_hi, c_lo, c^T*/ + ws_need((Kp + TC_TS_BN) * dpad1(D), 4) /*augmented centres*/ +
+  return 3 * ws_need(Kp * Dp, 4) /*c_hi, c_lo, c^T*/ + ws_need(Kp * dpad1(D), 4) /*augmented centres*/ +
          3 * ws_need(Kp, 4) /*|c|^2, |c|, |c - tf32(c)|*/ + 256 /*cmax*/ +
          3 * ws_need(N, 4) /*best, second, idx*/ + ws_need(N, 4) /*amb list*/ + ws_need(N, 8) /*amb packed*/ +
          256 /*amb count*/ + ws_need(N, 4) /*second-level list*/ + 256 /*its count*/ +
@@ -1845,17 +949,16 @@ int64_t kmeans_assign_tc_ws_bytes(int64_t N, int64_t K, int64_t D) {
 }
 
 // D_eff = contraction width (D, or D + 4 for the augmented first level); nkb = its 32-float K-blocks
-template <int NPASS, int BN, int SUB>
+template <int NPASS, int BN>
 static int launch_assign_tc(const CUtensorMap& m_xhi, const CUtensorMap& m_xlo, const CUtensorMap& m_chi,
                             const CUtensorMap& m_clo, int64_t N_max, const int32_t* n_rows_dev, int D_eff, int64_t Kp,
                             int nkb, const float* cnorm, float* best, float* second, int32_t* idx, cudaStream_t s,
                             TcGate gate = TcGate{nullptr, nullptr, nullptr, nullptr, 0.f}) {
-  using Cfg = TcCfg<NPASS, BN, SUB>;
+  using Cfg = TcCfg<NPASS, BN>;
   static PerDevice<bool> attr_set_dev;
   bool& attr_set = attr_set_dev.get();
   if (!attr_set) {
-    GDR_CUDA(cudaFuncSetAttribute(k_assign_tc<NPASS, BN, SUB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  TC_SMEM_LIMIT));
+    GDR_CUDA(cudaFuncSetAttribute(k_assign_tc<NPASS, BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_LIMIT));
     attr_set = true;
   }
   int sms = kSMs;
@@ -1864,17 +967,17 @@ static int launch_assign_tc(const CUtensorMap& m_xhi, const CUtensorMap& m_xlo, 
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   }
-  const int64_t tiles = cdiv(N_max, TC_BM * SUB);
+  const int64_t tiles = cdiv(N_max, TC_BM);
   const int grid = (int)(tiles < sms ? tiles : sms);
-  k_assign_tc<NPASS, BN, SUB><<<grid, TC_THREADS, Cfg::total(nkb), s>>>(m_xhi, m_xlo, m_chi, m_clo, N_max, n_rows_dev, D_eff,
-                                                                  (int)(Kp / BN), nkb, cnorm, best, second, idx, g_tc_ablate, gate);
+  k_assign_tc<NPASS, BN><<<grid, TC_THREADS, Cfg::total(nkb), s>>>(m_xhi, m_xlo, m_chi, m_clo, N_max, n_rows_dev, D_eff,
+                                                                   (int)(Kp / BN), nkb, cnorm, best, second, idx, gate);
   GDR_LAUNCHED();
   return GDR_OK;
 }
 
 static int launch_tc_cand(const CUtensorMap& m_x1, const CUtensorMap& m_c1, int64_t N_max, const int32_t* n_rows_dev,
                           int D_eff, int64_t Kp, int nkb, TcGate gate, TcCand cand, cudaStream_t s) {
-  using Cfg = TcCfg<1, 256, 1>;
+  using Cfg = TcCfg<1, 256>;
   static PerDevice<bool> attr_set_dev;
   bool& attr_set = attr_set_dev.get();
   if (!attr_set) {
@@ -1894,76 +997,10 @@ static int launch_tc_cand(const CUtensorMap& m_x1, const CUtensorMap& m_c1, int6
   return GDR_OK;
 }
 
-template <int BN>
-static int launch_assign_tc_ts(const float* x1, int ldx1, const CUtensorMap& m_c, int64_t N_max, const int32_t* n_rows_dev,
-                               int D_eff, int n_col_tiles, int nkb, float* best, float* second, int32_t* idx, cudaStream_t s,
-                               TcGate gate) {
-  using Cfg = TsCfg<BN>;
-  static PerDevice<bool> attr_set_dev;
-  bool& attr_set = attr_set_dev.get();
-  if (!attr_set) {
-    GDR_CUDA(cudaFuncSetAttribute(k_assign_tc_ts<BN>, cudaFuncAttributeMaxDynamicSharedMemorySize, TC_SMEM_LIMIT));
-    attr_set = true;
-  }
-  int sms = kSMs;
-  {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  }
-  const int64_t tiles = cdiv(N_max, TC_BM);
-  const int grid = (int)(tiles < sms ? tiles : sms);
-  k_assign_tc_ts<BN><<<grid, TC_THREADS, Cfg::total(), s>>>(x1, ldx1, m_c, N_max, n_rows_dev, D_eff, n_col_tiles, nkb, best,
-                                                          second, idx, g_tc_ablate, gate);
-  GDR_LAUNCHED();
-  return GDR_OK;
-}
-
-// rows [r0, r1) of the augmented centre matrix as padding centres (score -1e30 for every row of X)
-__global__ void k_pad_aug(float* __restrict__ aug, int64_t r0, int64_t r1, int Dp1, int D) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x, n = (r1 - r0) * Dp1;
-  if (i < n) aug[r0 * Dp1 + i] = (int)(i % Dp1) == D + 2 ? to_tf32(-1e30f) : 0.f;
-}
-
-static int launch_assign_tc_pair(const CUtensorMap& m_x, const CUtensorMap& m_c, int64_t N_max, const int32_t* n_rows_dev,
-                                 int D_eff, int64_t Kp, int nkb, float* best, float* second, int32_t* idx, int fwd,
-                                 cudaStream_t s) {
-  static PerDevice<bool> attr_set_dev;
-  bool& attr_set = attr_set_dev.get();
-  if (!attr_set) {
-    GDR_CUDA(cudaFuncSetAttribute(k_assign_tc_pair, cudaFuncAttributeMaxDynamicSharedMemorySize, Tc2Cfg::total(TC_BAR_KB)));
-    attr_set = true;
-  }
-  int sms = kSMs;
-  {
-    int dev = 0;
-    cudaGetDevice(&dev);
-    cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  }
-  const int64_t units = cdiv(cdiv(N_max, TC_BM), 2);
-  const int pairs = (int)(units < sms / 2 ? units : sms / 2);
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * pairs);
-  cfg.blockDim = dim3(TC_THREADS);
-  cfg.dynamicSmemBytes = Tc2Cfg::total(nkb);
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  GDR_CUDA(cudaLaunchKernelEx(&cfg, k_assign_tc_pair, m_x, m_c, N_max, n_rows_dev, D_eff, (int)(Kp / Tc2Cfg::BN), nkb, best,
-                              second, idx, g_tc_ablate, fwd));
-  GDR_LAUNCHED();
-  return GDR_OK;
-}
-
-int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_t ldx, const void* xsplit,
-                         const float* C, int64_t ldc, int32_t* labels, const int32_t* labels_prev,
-                         int32_t* n_changed_dev, float* best_out, int32_t* n_refined_dev, void* ws,
-                         int64_t ws_bytes, cudaStream_t s, const int32_t* labels_hint) {
+static int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_t ldx, const void* xsplit,
+                                const float* C, int64_t ldc, int32_t* labels, const int32_t* labels_prev,
+                                int32_t* n_changed_dev, float* best_out, int32_t* n_refined_dev, void* ws,
+                                int64_t ws_bytes, cudaStream_t s) {
   if (D > TC_MAX_KB * TC_BK) {
     set_error("kmeans_assign(tc): D=%lld > %d is not supported by the tensor-core path", (long long)D,
               TC_MAX_KB * TC_BK);
@@ -1981,7 +1018,7 @@ int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_
   float* c_hi = W.take<float>(Kp * Dp);
   float* c_lo = W.take<float>(Kp * Dp);
   float* c_t = W.take<float>(Kp * Dp);   // fp32 centres transposed [Dp][Kp] for the re-score kernel
-  float* c1 = W.take<float>((Kp + TC_TS_BN) * Dp1);   // augmented first-level centres (+ padding rows of the last 192-tile)
+  float* c1 = W.take<float>(Kp * Dp1);   // augmented first-level centres
   float* cnorm = W.take<float>(Kp);
   float* cnorm_sqrt = W.take<float>(Kp);
   float* cdnorm = W.take<float>(Kp);
@@ -2027,7 +1064,7 @@ int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_
     if ((rc = make_map(&m_xlo, xs.lo, N, Dp, TC_BM))) return rc;
     {
       ProfileScope prof(PROF_ASSIGN, s);
-      if ((rc = launch_assign_tc<3, 128, 1>(m_xhi, m_xlo, m_chi, m_clo, N, nullptr, (int)D, Kp, nkb, cnorm, best, second,
+      if ((rc = launch_assign_tc<3, 128>(m_xhi, m_xlo, m_chi, m_clo, N, nullptr, (int)D, Kp, nkb, cnorm, best, second,
                                          idx, s)))
         return rc;
     }
@@ -2039,54 +1076,18 @@ int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_
     // the profile scope spans the whole tensor-core screen: level 1, decision, compaction, level 2
     ProfileScope prof(PROF_ASSIGN, s);
     CUtensorMap m_x1, m_c1;
-    bool cand_level = false;   // second level on candidate centres (default screen only)
     if ((rc = make_map(&m_x1, xs.x1, N, Dp1, TC_BM))) return rc;
-    if (g_tc_screen == 2) {
-      if ((rc = make_map(&m_c1, c1, Kp, Dp1, 128))) return rc;
-      if ((rc = launch_assign_tc<1, 128, 2>(m_x1, m_x1, m_c1, m_c1, N, nullptr, (int)D + TC_AUG, Kp, nkb1, cnorm, best, second,
-                                         idx, s)))
-        return rc;
-    } else if (g_tc_screen == 4 || g_tc_screen == 5) {
-      if ((rc = make_map(&m_c1, c1, Kp, Dp1, 128))) return rc;   // each CTA of a pair loads 128 of the 256 centres
-      if ((rc = launch_assign_tc_pair(m_x1, m_c1, N, nullptr, (int)D + TC_AUG, Kp, nkb1, best, second, idx,
-                                      g_tc_screen == 5 ? 1 : 0, s)))
-        return rc;
-    } else {
-      // default: both operands from shared memory (k_assign_tc<1, 256, 1>).  tc_screen 6 (D + 4 <= 128): the row tile in
-      // tensor memory (k_assign_tc_ts, 192-centre tiles, all of shared memory is the centre ring) — measured at config E:
-      // 8.2 vs 7.6 ms (D = 100), 6.1 vs 5.4 ms (D = 47): the TF32 MMA runs at ~0.65 cycles per accumulator column
-      // whether A comes from shared or tensor memory, and 192-centre tiles pay the per-tile hand-shakes 53 times instead of 40
-      const int ka = (int)align_up(D + TC_AUG, 8);
-      const int ts_bn = (g_tc_screen == 6 && ka <= 512 - 2 * TC_TS_BN) ? TC_TS_BN : 0;
-      cand_level = g_tc_cand != 0 && ts_bn == 0;
-      const int64_t k_rows = ts_bn == TC_TS_BN ? align_up(K, TC_TS_BN) : Kp;
-      if (k_rows > Kp) {
-        k_pad_aug<<<(unsigned)cdiv((k_rows - Kp) * Dp1, 256), 256, 0, s>>>(c1, Kp, k_rows, Dp1, (int)D);
-        GDR_LAUNCHED();
-      }
-      if ((rc = make_map(&m_c1, c1, std::max(Kp, k_rows), Dp1, ts_bn ? ts_bn : 256))) return rc;
-      TcGate gate{nullptr, nullptr, nullptr, nullptr, TC_BAND};
-      if (g_tc_gate) {
-        gate.xnorm = xs.norm;
-        gate.xdnorm = xs.dnorm;
-        gate.cscal = cmax;
-        const int32_t* hint = labels_hint ? labels_hint : labels_prev;
-        if (hint && g_tc_gate >= 2) {
-          float* seed = g_norm;   // free until k_tc_gather fills it after the first level
-          k_tc_seed<<<(unsigned)cdiv(N * 32, 256), 256, 0, s>>>(N, K, Dp1, xs.x1, c1, hint, xs.norm, cmax, seed);
-          GDR_LAUNCHED();
-          gate.seed = seed;
-        }
-      }
-      if (ts_bn == TC_TS_BN)
-        rc = launch_assign_tc_ts<TC_TS_BN>(xs.x1, Dp1, m_c1, N, nullptr, (int)D + TC_AUG, (int)(k_rows / TC_TS_BN), nkb1, best,
-                                           second, idx, s, gate);
-      else
-        rc = launch_assign_tc<1, 256, 1>(m_x1, m_x1, m_c1, m_c1, N, nullptr, (int)D + TC_AUG, Kp, nkb1, cnorm, best, second,
-                                         idx, s, gate);
-      if (rc) return rc;
+    if ((rc = make_map(&m_c1, c1, Kp, Dp1, 256))) return rc;
+    TcGate gate{nullptr, nullptr, nullptr, nullptr, TC_BAND};
+    if (g_tc_gate) {
+      gate.xnorm = xs.norm;
+      gate.xdnorm = xs.dnorm;
+      gate.cscal = cmax;
     }
-    if (g_tc_ablate) return GDR_OK;   // timing experiment: first-level kernel only
+    if ((rc = launch_assign_tc<1, 256>(m_x1, m_x1, m_c1, m_c1, N, nullptr, (int)D + TC_AUG, Kp, nkb1, cnorm, best, second, idx,
+                                       s, gate)))
+      return rc;
+    const bool cand_level = g_tc_cand != 0;   // second level on candidate centres
     g_last_count1 = count1;
     k_tc_select1<<<(unsigned)cdiv(N, 256), 256, 0, s>>>(N, best, second, idx, xs.norm, xs.dnorm, cnorm, cnorm_sqrt,
                                                        cdnorm, cmax, TC_BAND, labels, labels_prev, n_changed_dev,
@@ -2119,7 +1120,7 @@ int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_
     CUtensorMap m_ghi, m_glo;
     if ((rc = make_map(&m_ghi, g_hi, N, Dp, TC_BM))) return rc;
     if ((rc = make_map(&m_glo, g_lo, N, Dp, TC_BM))) return rc;
-    if ((rc = launch_assign_tc<3, 128, 1>(m_ghi, m_glo, m_chi, m_clo, N, count_f, (int)D, Kp, nkb, cnorm, best, second, idx,
+    if ((rc = launch_assign_tc<3, 128>(m_ghi, m_glo, m_chi, m_clo, N, count_f, (int)D, Kp, nkb, cnorm, best, second, idx,
                                        s)))
       return rc;
     k_tc_select2<<<2 * kSMs, 256, 0, s>>>(list_f, count_f, best, second, idx, g_norm, cmax, TC_BAND, labels,
@@ -2151,7 +1152,7 @@ int kmeans_assign_tc(int64_t N, int64_t K, int64_t D, const float* X, int64_t ld
   int rc = kmeans_tc_prepare(N, D, X, ldx, xsplit, s);
   if (rc) return rc;
   return kmeans_assign_tc_run(N, K, D, X, ldx, xsplit, C, ldc, labels, labels_prev, n_changed_dev, best_out,
-                              nullptr, ws, kmeans_assign_tc_ws_bytes(N, K, D), s, nullptr);
+                              nullptr, ws, kmeans_assign_tc_ws_bytes(N, K, D), s);
 }
 
 }  // namespace gdr
@@ -2161,20 +1162,6 @@ extern "C" {
 // debug read-back (synchronises the device): "tc_level2_rows" = rows the last two-level screen sent to level 2
 int gdr_debug_get(const char* key, int64_t* value_host) {
   GDR_CHECK_ARG(key && value_host, "debug_get: bad arguments");
-  if (!strncmp(key, "ts_probe_", 9)) {
-    long long h[16];
-    GDR_CUDA(cudaMemcpyFromSymbol(h, gdr::g_ts_probe, sizeof(h)));
-    const int i = atoi(key + 9);
-    GDR_CHECK_ARG(i >= 0 && i < 16, "debug_get: ts_probe index");
-    *value_host = h[i];
-    return GDR_OK;
-  }
-  if (!strcmp(key, "tc_probe_cycles") || !strcmp(key, "tc_probe_ns") || !strcmp(key, "tc_probe_mmas")) {
-    long long h[4] = {0, 0, 0, 0};
-    GDR_CUDA(cudaMemcpyFromSymbol(h, gdr::g_tc_probe, sizeof(h)));
-    *value_host = !strcmp(key, "tc_probe_cycles") ? h[0] : (!strcmp(key, "tc_probe_ns") ? h[1] : h[2]);
-    return GDR_OK;
-  }
   if (!strcmp(key, "tc_level2_rows")) {
     int32_t v = -1;
     if (gdr::g_last_count1) GDR_CUDA(cudaMemcpy(&v, gdr::g_last_count1, 4, cudaMemcpyDeviceToHost));
@@ -2200,44 +1187,6 @@ int gdr_debug_get(const char* key, int64_t* value_host) {
   }
   gdr::set_error("debug_get: unknown key %s", key);
   return GDR_EINVAL;
-}
-
-// cycles for `iters` back-to-back MMAs of shape 128 x N x 32 B on one SM (see k_mma_probe); synchronises
-int gdr_debug_mma_probe(int N, int iters, int variant, int64_t* cycles_host) {
-  GDR_CHECK_ARG((N == 64 || N == 128 || N == 256) && iters > 0 && cycles_host, "mma_probe: bad arguments");
-  long long* d = nullptr;
-  GDR_CUDA(cudaMalloc(&d, 8));
-  if (variant == 1024) {   // the CTA-pair probe (N is ignored: 256 x 256 x 8)
-    const int smem2 = 8 * 128 * 128 + 1024;
-    GDR_CUDA(cudaFuncSetAttribute(gdr::k_mma_probe_pair, cudaFuncAttributeMaxDynamicSharedMemorySize, smem2));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3(2);
-    cfg.blockDim = dim3(128);
-    cfg.dynamicSmemBytes = smem2;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = 2;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    GDR_CUDA(cudaLaunchKernelEx(&cfg, gdr::k_mma_probe_pair, iters, d));
-    GDR_CUDA(cudaDeviceSynchronize());
-    long long h2 = 0;
-    GDR_CUDA(cudaMemcpy(&h2, d, 8, cudaMemcpyDeviceToHost));
-    cudaFree(d);
-    *cycles_host = h2;
-    return GDR_OK;
-  }
-  const int smem = 4 * (128 + 256) * 128 + 1024;
-  GDR_CUDA(cudaFuncSetAttribute(gdr::k_mma_probe, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-  gdr::k_mma_probe<<<1, 128, smem>>>(N, iters, variant, d);
-  GDR_CUDA(cudaDeviceSynchronize());
-  long long h = 0;
-  GDR_CUDA(cudaMemcpy(&h, d, 8, cudaMemcpyDeviceToHost));
-  cudaFree(d);
-  *cycles_host = h;
-  return GDR_OK;
 }
 
 int64_t gdr_kmeans_tc_xsplit_bytes(int64_t N, int64_t D) { return gdr::kmeans_tc_xsplit_bytes(N, D); }
@@ -2270,7 +1219,7 @@ int gdr_kmeans_assign_tc(int64_t N, int64_t K, int64_t D, const float* X, int64_
     return GDR_EWORKSPACE;
   }
   return gdr::kmeans_assign_tc_run(N, K, D, X, ldx, xsplit, C, ldc, labels, labels_prev, n_changed_dev, best_out,
-                                   n_refined_dev, ws, ws_bytes, (cudaStream_t)stream, nullptr);
+                                   n_refined_dev, ws, ws_bytes, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -22,11 +22,6 @@ using namespace gdr;
 namespace gdr {
 int64_t kmeans_assign_tc_ws_bytes(int64_t N, int64_t K, int64_t D);
 int64_t kmeans_tc_xsplit_bytes(int64_t N, int64_t D);
-// kmeans_tc.cu: the E-step with an explicit label hint for the first-level gate (labels_hint may alias `labels`:
-// it is read before any label is written)
-int kmeans_assign_tc_run(int64_t N, int64_t K, int64_t D, const float* X, int64_t ldx, const void* xsplit, const float* C,
-                         int64_t ldc, int32_t* labels, const int32_t* labels_prev, int32_t* n_changed_dev, float* best_out,
-                         int32_t* n_refined_dev, void* ws, int64_t ws_bytes, cudaStream_t s, const int32_t* labels_hint);
 int g_lloyd_graph = 1;  // gdr_debug_set("lloyd_graph", 0) disables graph replay
 bool profiling_enabled();
 // kmeans.cu: distributed empty-cluster relocation (candidate records / application of the global choice)
@@ -313,14 +308,8 @@ int lloyd_run(gdr_comm* comm, int64_t N, int64_t N_total, int64_t K, int64_t D, 
   // (max_iter == 0: centres[0], labels undefined -> the E-step below fills them)
   int32_t* labels = n_iter == 0 ? B.labels[0] : B.labels[1 - p];
   if (!strict) {
-    // rerun the E-step so that the labels match the final centres (:742-754); the labels of the last iteration
-    // (still in `labels`) seed the first-level gate
-    if (precision_mode == 1 && N > 0 && n_iter > 0)
-      rc = kmeans_assign_tc_run(N, K, D, Xc, ldx, B.xsplit, B.centers[p], ldw, labels, nullptr, nullptr, nullptr, nullptr,
-                                B.ws_assign, B.ws_assign_b, s, labels);
-    else
-      rc = assign(B.centers[p], labels, nullptr, nullptr);
-    if (rc) return rc;
+    // rerun the E-step so that the labels match the final centres (:742-754)
+    if ((rc = assign(B.centers[p], labels, nullptr, nullptr))) return rc;
   }
   double* inertia_dev = B.stats;
   if (N > 0) {

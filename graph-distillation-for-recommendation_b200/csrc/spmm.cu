@@ -17,11 +17,7 @@
 //   * the row's (colidx, val) pairs are read coalesced, LPR at a time, and
 //     broadcast with warp shuffles; UNROLL gathers are in flight per lane
 //     before the first FMA consumes one (MLP); accumulation order stays CSR
-//     order, one fp32 chain per output element => deterministic;
-//   * streamed operands (colidx, vals, T, Y) use no-allocate / streaming cache
-//     hints so that they do not evict the gathered X rows from L1/L2;
-//   * wide feature matrices can be processed in column windows (col_split) so
-//     that the window of X stays L2-resident across the whole pass.
+//     order, one fp32 chain per output element => deterministic.
 #include "common.cuh"
 #include "comm.cuh"
 #include <stdlib.h>
@@ -36,10 +32,6 @@ constexpr int SPMM_BLOCK_WEIGHT = 2048;   // plan: weight(row) = nnz(row) + SPMM
 constexpr int SPMM_ROW_COST = 16;         // => at most SPMM_BLOCK_WEIGHT / SPMM_ROW_COST = 128 rows per block
 constexpr int SPMM_HEAVY_NNZ = 1024;   // rows longer than this are processed by the whole CTA
 
-// run-time tuning (gdr_debug_set): 0 = automatic choice
-static int g_spmm_unroll = 0;     // 4 or 8
-static int g_spmm_hints = -1;     // 0 off, 1 streaming hints on colidx/vals/T/Y
-static int g_spmm_split = 0;      // number of column windows (1, 2, 4)
 extern int g_lloyd_graph;         // lloyd.cu
 extern int g_kpp_skip_score;      // kmeans_init.cu
 extern int g_tc_screen;           // kmeans_tc.cu
@@ -49,31 +41,11 @@ extern int g_tc_cand_cap;         // kmeans_tc.cu
 extern int g_coarsen_dense;       // graph.cu
 extern int g_rs_match;            // primitives.cu
 extern int g_rs_max_bits;         // primitives.cu
-extern int g_tc_ablate;
 extern int g_topk_path;           // topk.cu
 extern int g_topk_condensed_path; // topk_condensed.cu
 }  // namespace gdr
 extern "C" int g_sparsify_batch_cap;   // sparsify.cu
 namespace gdr {
-
-__device__ __forceinline__ int ld_stream_i32(const int32_t* p) {
-  int v;
-  asm volatile("ld.global.nc.L1::no_allocate.s32 %0, [%1];" : "=r"(v) : "l"(p));
-  return v;
-}
-__device__ __forceinline__ float ld_stream_f32(const float* p) {
-  float v;
-  asm volatile("ld.global.nc.L1::no_allocate.f32 %0, [%1];" : "=f"(v) : "l"(p));
-  return v;
-}
-__device__ __forceinline__ float4 ld_cs_f4(const float* p) {
-  float4 r;
-  asm volatile("ld.global.cs.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(r.x), "=f"(r.y), "=f"(r.z), "=f"(r.w) : "l"(p));
-  return r;
-}
-__device__ __forceinline__ void st_cs_f4(float* p, const float4& v) {
-  asm volatile("st.global.cs.v4.f32 [%0], {%1,%2,%3,%4};" ::"l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
 
 // Multicast epilogue (multi-GPU hop fused with its all-gather): besides Y, every output row is stored into the gathered
 // operand of the NEXT hop on every rank — dst[p] are peer-mapped (NVLink) pointers to rank p's copy of that matrix, row
@@ -85,7 +57,7 @@ struct SpmmPeers {
   int64_t ld;
 };
 
-template <int LPR, int NCH, int UNROLL, bool HINTS>
+template <int LPR, int NCH, int UNROLL>
 __device__ __forceinline__ void spmm_row(const int32_t* __restrict__ colidx,
                                          const float* __restrict__ vals, float alpha,
                                          const float* __restrict__ X, int64_t ldx, int start, int end,
@@ -100,8 +72,8 @@ __device__ __forceinline__ void spmm_row(const int32_t* __restrict__ colidx,
     int c_l = 0;
     float v_l = 0.f;
     if (my < end) {
-      c_l = HINTS ? ld_stream_i32(colidx + my) : __ldg(colidx + my);
-      v_l = vals ? __fmul_rn(HINTS ? ld_stream_f32(vals + my) : __ldg(vals + my), alpha) : alpha;
+      c_l = __ldg(colidx + my);
+      v_l = vals ? __fmul_rn(__ldg(vals + my), alpha) : alpha;
     }
     int cnt = min(LPR, end - k);
 #pragma unroll 1
@@ -144,8 +116,8 @@ __device__ __forceinline__ void spmm_row(const int32_t* __restrict__ colidx,
   }
 }
 
-template <int LPR, int NCH, int UNROLL, bool HINTS, bool MC>
-__global__ void __launch_bounds__(SPMM_THREADS, MC ? (NCH == 1 ? 4 : 1) : ((NCH == 1 && UNROLL <= 2) ? 8 : ((NCH == 1 && UNROLL <= 4) ? 6 : 1)))
+template <int LPR, int NCH, bool MC>
+__global__ void __launch_bounds__(SPMM_THREADS, NCH == 1 ? (MC ? 4 : 6) : 1)
 k_spmm(int64_t rows, int c4_end, const int32_t* __restrict__ rowptr, const int32_t* __restrict__ colidx,
        const float* __restrict__ vals, float alpha, const float* __restrict__ X, int64_t ldx,
        float* __restrict__ Y, int64_t ldy, float* __restrict__ T, int64_t ldt, float beta,
@@ -154,6 +126,7 @@ k_spmm(int64_t rows, int c4_end, const int32_t* __restrict__ rowptr, const int32
   __shared__ int s_heavy[SPMM_MAX_ROWS];
   __shared__ int s_next, s_nheavy;
   constexpr int GROUPS = 32 / LPR;  // rows processed concurrently by one warp
+  constexpr int UNROLL = NCH >= 8 ? 1 : (NCH >= 4 ? 2 : 4);   // gathers in flight per lane (each carries NCH float4)
   // row block of this CTA: from the nnz-balanced plan when there is one, else 64 consecutive rows
   const int64_t row0 = bounds ? (int64_t)bounds[blockIdx.x] : (int64_t)blockIdx.x * SPMM_ROWS_PER_CTA;
   const int nrows = bounds ? (bounds[blockIdx.x + 1] - (int)row0)
@@ -171,24 +144,19 @@ k_spmm(int64_t rows, int c4_end, const int32_t* __restrict__ rowptr, const int32
 
   // epilogue of one float4 column chunk: Y = acc ; T += beta * acc (two roundings, as the reference)
   auto store = [&](int64_t row, int c4, const float4& a) {
-    if (Y) {
-      float* yp = Y + row * ldy + 4 * c4;
-      if (HINTS) st_cs_f4(yp, a);
-      else *reinterpret_cast<float4*>(yp) = a;
-    }
+    if (Y) *reinterpret_cast<float4*>(Y + row * ldy + 4 * c4) = a;
     if (MC) {
       for (int p = 0; p < mc.n; ++p)   // posted NVLink stores: the row lands in every rank's gathered operand
         *reinterpret_cast<float4*>(mc.dst[p] + (mc.row_off + row) * mc.ld + 4 * c4) = a;
     }
     if (T) {
       float* tp = T + row * ldt + 4 * c4;
-      float4 t = HINTS ? ld_cs_f4(tp) : *reinterpret_cast<float4*>(tp);
+      float4 t = *reinterpret_cast<float4*>(tp);
       t.x = __fadd_rn(t.x, __fmul_rn(beta, a.x));
       t.y = __fadd_rn(t.y, __fmul_rn(beta, a.y));
       t.z = __fadd_rn(t.z, __fmul_rn(beta, a.z));
       t.w = __fadd_rn(t.w, __fmul_rn(beta, a.w));
-      if (HINTS) st_cs_f4(tp, t);
-      else *reinterpret_cast<float4*>(tp) = t;
+      *reinterpret_cast<float4*>(tp) = t;
     }
   };
 
@@ -211,7 +179,7 @@ k_spmm(int64_t rows, int c4_end, const int32_t* __restrict__ rowptr, const int32
       }
     }
     float4 acc[NCH];
-    spmm_row<LPR, NCH, UNROLL, HINTS>(colidx, vals, alpha, X, ldx, start, end, c4_end, gl, gmask, col4_base, acc);
+    spmm_row<LPR, NCH, UNROLL>(colidx, vals, alpha, X, ldx, start, end, c4_end, gl, gmask, col4_base, acc);
     if (live) {
 #pragma unroll
       for (int c = 0; c < NCH; ++c) {
@@ -236,7 +204,7 @@ k_spmm(int64_t rows, int c4_end, const int32_t* __restrict__ rowptr, const int32
     chunk = (chunk + LPR - 1) / LPR * LPR;
     const int cs = min(he, hs + part * chunk), ce = min(he, cs + chunk);
     float4 acc[NCH];
-    spmm_row<LPR, NCH, UNROLL, HINTS>(colidx, vals, alpha, X, ldx, cs, ce, c4_end, gl, gmask, col4_base, acc);
+    spmm_row<LPR, NCH, UNROLL>(colidx, vals, alpha, X, ldx, cs, ce, c4_end, gl, gmask, col4_base, acc);
 #pragma unroll
     for (int c = 0; c < NCH; ++c) s_part[part][c * LPR + gl] = acc[c];
     __syncthreads();
@@ -277,58 +245,20 @@ struct SpmmArgs {
   SpmmPeers mc;
 };
 
-template <int LPR, int NCH, int UNROLL, bool HINTS>
+// one column window [col4_base, c4_end) in float4 units; mc.n > 0: the multi-GPU hop fused with its all-gather
+template <int LPR, int NCH>
 static int launch_spmm(const SpmmArgs& a, int col4_base, int c4_end) {
   unsigned grid = a.bounds ? (unsigned)a.n_blocks : (unsigned)cdiv(a.rows, SPMM_ROWS_PER_CTA);
   {
     ProfileScope prof(PROF_SPMM, a.s);
-    if constexpr (!HINTS && UNROLL == (NCH >= 8 ? 1 : (NCH >= 4 ? 2 : 4))) {
-      if (a.mc.n > 0) {   // multi-GPU hop fused with its all-gather (built for the default tuning of every width)
-        k_spmm<LPR, NCH, UNROLL, HINTS, true><<<grid, SPMM_THREADS, 0, a.s>>>(a.rows, c4_end, a.rowptr, a.colidx, a.vals,
-                                                                              a.alpha, a.X, a.ldx, a.Y, a.ldy, a.T, a.ldt,
-                                                                              a.beta, col4_base, a.bounds, a.mc);
-        GDR_LAUNCHED();
-        return GDR_OK;
-      }
-    }
-    if (a.mc.n > 0) {
-      set_error("spmm: the fused all-gather epilogue is built for the default tuning only (spmm_unroll / spmm_hints unset)");
-      return GDR_EUNSUPPORTED;
-    }
-    k_spmm<LPR, NCH, UNROLL, HINTS, false><<<grid, SPMM_THREADS, 0, a.s>>>(a.rows, c4_end, a.rowptr, a.colidx, a.vals, a.alpha,
-                                                                           a.X, a.ldx, a.Y, a.ldy, a.T, a.ldt, a.beta,
-                                                                           col4_base, a.bounds, a.mc);
+    if (a.mc.n > 0)
+      k_spmm<LPR, NCH, true><<<grid, SPMM_THREADS, 0, a.s>>>(a.rows, c4_end, a.rowptr, a.colidx, a.vals, a.alpha, a.X, a.ldx,
+                                                             a.Y, a.ldy, a.T, a.ldt, a.beta, col4_base, a.bounds, a.mc);
+    else
+      k_spmm<LPR, NCH, false><<<grid, SPMM_THREADS, 0, a.s>>>(a.rows, c4_end, a.rowptr, a.colidx, a.vals, a.alpha, a.X, a.ldx,
+                                                              a.Y, a.ldy, a.T, a.ldt, a.beta, col4_base, a.bounds, a.mc);
   }
   GDR_LAUNCHED();
-  return GDR_OK;
-}
-
-template <int LPR, int NCH>
-static int dispatch_tuning(const SpmmArgs& a, int base, int c4_end, int unroll, bool hints) {
-  if constexpr (NCH == 1) {
-    if (unroll == 2)
-      return hints ? launch_spmm<LPR, NCH, 2, true>(a, base, c4_end) : launch_spmm<LPR, NCH, 2, false>(a, base, c4_end);
-  }
-  if constexpr (NCH <= 2) {
-    if (unroll >= 8)
-      return hints ? launch_spmm<LPR, NCH, 8, true>(a, base, c4_end) : launch_spmm<LPR, NCH, 8, false>(a, base, c4_end);
-  }
-  constexpr int U = NCH >= 8 ? 1 : (NCH >= 4 ? 2 : 4);
-  return hints ? launch_spmm<LPR, NCH, U, true>(a, base, c4_end) : launch_spmm<LPR, NCH, U, false>(a, base, c4_end);
-}
-
-// one column window [base, base + width) in float4 units
-static int spmm_window(const SpmmArgs& a, int base, int width, int unroll, bool hints) {
-  const int c4_end = base + width;
-  if (width <= 8) return dispatch_tuning<8, 1>(a, base, c4_end, unroll, hints);
-  if (width <= 16) return dispatch_tuning<16, 1>(a, base, c4_end, unroll, hints);
-  if (width <= 32) return dispatch_tuning<32, 1>(a, base, c4_end, unroll, hints);
-  if (width <= 64) return dispatch_tuning<32, 2>(a, base, c4_end, unroll, hints);
-  if (width <= 128) return dispatch_tuning<32, 4>(a, base, c4_end, unroll, hints);
-  for (int b = base; b < c4_end; b += 256) {
-    int rc = dispatch_tuning<32, 8>(a, b, std::min(c4_end, b + 256), unroll, hints);
-    if (rc) return rc;
-  }
   return GDR_OK;
 }
 
@@ -380,18 +310,17 @@ int spmm_launch_mc(int64_t rows, int64_t F, const int32_t* rowptr, const int32_t
   if (rows == 0 || F == 0) return GDR_OK;
   const int F4 = (int)cdiv(F, 4);
   SpmmArgs a{rows, rowptr, colidx, vals, alpha, X, ldx, Y, ldy, T, ldt, beta, s, bounds, n_blocks, mc};
-  const int unroll = g_spmm_unroll > 0 ? g_spmm_unroll : 4;
-  const bool hints = g_spmm_hints >= 0 ? g_spmm_hints != 0 : false;
-  int split = g_spmm_split > 0 ? g_spmm_split : 1;
-  if (split > 1 && F4 >= 8 * split) {
-    const int w = (int)cdiv(F4, split);
-    for (int b = 0; b < F4; b += w) {
-      int rc = spmm_window(a, b, std::min(w, F4 - b), unroll, hints);
-      if (rc) return rc;
-    }
-    return GDR_OK;
+  // lanes per row and float4 columns per lane from the width
+  if (F4 <= 8) return launch_spmm<8, 1>(a, 0, F4);
+  if (F4 <= 16) return launch_spmm<16, 1>(a, 0, F4);
+  if (F4 <= 32) return launch_spmm<32, 1>(a, 0, F4);
+  if (F4 <= 64) return launch_spmm<32, 2>(a, 0, F4);
+  if (F4 <= 128) return launch_spmm<32, 4>(a, 0, F4);
+  for (int b = 0; b < F4; b += 256) {
+    int rc = launch_spmm<32, 8>(a, b, std::min(F4, b + 256));
+    if (rc) return rc;
   }
-  return spmm_window(a, 0, F4, unroll, hints);
+  return GDR_OK;
 }
 
 __global__ void k_scale_rows(int64_t rows, int F4, float a, const float* __restrict__ X, int64_t ldx,
@@ -439,19 +368,15 @@ int gdr_remap_chunk_major(int64_t nnz, const int32_t* colidx_in, int64_t rows_pe
   return GDR_OK;
 }
 
-// Tuning / experiment knobs (not part of the stable surface; see tools/spmm_sweep.py).
+// Path selectors and test knobs (not part of the stable surface; see include/gdr.h).
 int gdr_debug_set(const char* key, int value) {
   GDR_CHECK_ARG(key, "debug_set: null key");
-  if (!strcmp(key, "spmm_unroll")) gdr::g_spmm_unroll = value;
-  else if (!strcmp(key, "spmm_hints")) gdr::g_spmm_hints = value;
-  else if (!strcmp(key, "spmm_split")) gdr::g_spmm_split = value;
-  else if (!strcmp(key, "lloyd_graph")) gdr::g_lloyd_graph = value;
+  if (!strcmp(key, "lloyd_graph")) gdr::g_lloyd_graph = value;
   else if (!strcmp(key, "kpp_dist_skip_score")) gdr::g_kpp_skip_score = value;
   else if (!strcmp(key, "tc_screen")) gdr::g_tc_screen = value;
   else if (!strcmp(key, "topk_path")) gdr::g_topk_path = value;
   else if (!strcmp(key, "topk_condensed_path")) gdr::g_topk_condensed_path = value;
   else if (!strcmp(key, "coarsen_dense")) gdr::g_coarsen_dense = value;
-  else if (!strcmp(key, "tc_ablate")) gdr::g_tc_ablate = value;
   else if (!strcmp(key, "tc_gate")) gdr::g_tc_gate = value;
   else if (!strcmp(key, "tc_cand")) gdr::g_tc_cand = value;
   else if (!strcmp(key, "tc_cand_cap")) gdr::g_tc_cand_cap = value;

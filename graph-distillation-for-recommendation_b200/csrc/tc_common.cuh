@@ -70,16 +70,6 @@ __device__ __forceinline__ void tc_mma_tf32(uint32_t tmem_d, uint64_t adesc, uin
       ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
       : "memory");
 }
-// experiment only (tc_ablate 7): the same bytes issued as kind::f16 / BF16 operands — is the TF32 kind itself the slow part?
-__device__ __forceinline__ void tc_mma_bf16(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc,
-                                            uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-      ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate)
-      : "memory");
-}
 // 32 lanes x 32 columns of fp32 accumulators -> 32 registers per thread
 __device__ __forceinline__ void tc_ld_32x32(uint32_t taddr, uint32_t (&v)[32]) {
   asm volatile(

@@ -65,19 +65,19 @@ int64_t     gdr_launch_count(void);
 int gdr_profile_enable(int kind);
 int gdr_profile_collect(double* total_ms_host, int64_t* launches_host);
 
-/* Experiment knobs for kernel tuning sweeps (tools/spmm_sweep.py); not a stable surface.
- * keys: "spmm_unroll" (4|8), "spmm_hints" (0|1), "spmm_split" (1|2|4), "lloyd_graph" (0|1),
- * "sparsify_batch" (cap on the classes per batch of gdr_sparsify_classes), "tc_screen" (1 direct 3xTF32; two-level screen with 2: 256x128 CTA tiles, 3: 128x256 CTA tiles [default for large
- * inputs], 4: CTA pairs with 2-SM TMA, 5: CTA pairs with forwarded 1-SM TMA), "tc_ablate" (role ablations of the
- * first-level kernel for tools/estep_probe.py / tools/mma_rate_probe.py; results are garbage while it is set);
- * "tc_gate" (first-level epilogue gate of the two-level screen: 0 off, 1 [default] on the running best, 2 also seeded
- * with the previous label's score; every setting produces the same labels); "tc_cand" (second level of the default
- * two-level screen: 1 [default] seeded 1xTF32 candidate pass + exact re-score of the candidates, 0 3xTF32 over all
- * centres; same labels); "tc_cand_cap" (candidate list capacity per row and column half, 1..16; 0 = 16);
- * "rs_match" (radix-sort ranking: 0 [default] per-bit warp ballots, 1 MATCH.ANY); "topk_path" (gdr_topk_scores: 1 exact
- * SIMT path, 2 tensor-core screen);
- * "topk_condensed_path" (gdr_topk_condensed: 1 every row on the exact fallback);
- * value 0 / -1 = automatic. */
+/* Path selectors and test knobs; not a stable surface: keys may change between versions, and an unknown key
+ * fails with GDR_EINVAL.  keys:
+ * "tc_screen" (E-step of gdr_kmeans_assign_tc: 0 [default] automatic, 1 direct 3xTF32, any value >= 2 the
+ * two-level screen whatever N); "tc_gate" (first-level epilogue gate of the two-level screen: 0 off, any other
+ * value [default 1] on; the same labels either way); "tc_cand" (second level of the two-level screen: 1 [default]
+ * seeded 1xTF32 candidate pass + exact re-score of the candidates, 0 3xTF32 over all centres; same labels);
+ * "tc_cand_cap" (candidate list capacity per row and column half, 1..16; 0 = 16);
+ * "lloyd_graph" (0: no CUDA-graph replay of the Lloyd iteration); "coarsen_dense" (0: stage 4 always on the sort
+ * path); "sparsify_batch" (cap on the classes per batch of gdr_sparsify_classes); "kpp_dist_skip_score" (1: the
+ * k-means++ rounds of gdr_kmeans_plusplus_dist without their score pass, for exchange timing only);
+ * "rs_match" (radix-sort ranking: 0 [default] per-bit warp ballots, 1 MATCH.ANY); "rs_max_bits" (digit width cap
+ * of large sorts; 0 [default] = 9); "topk_path" (gdr_topk_scores: 0 automatic, 1 exact SIMT path,
+ * 2 tensor-core screen); "topk_condensed_path" (gdr_topk_condensed: 1 every row on the exact fallback). */
 int gdr_debug_set(const char* key, int value);
 /* Debug read-back (synchronises the device).  keys: "tc_level2_rows" = rows the last two-level
  * tensor-core screen (gdr_kmeans_assign_tc) left undecided after its first level; -1 if none ran.
@@ -86,11 +86,8 @@ int gdr_debug_set(const char* key, int value);
  * recorded for the rows read (-1 if the last two-level run did not use candidate lists).
  * "topk_overflow_rows" = rows the last tensor-core gdr_topk_scores finished on the exact path; -1 if none ran.
  * "topk_condensed_fallback_rows" = rows the last gdr_topk_condensed finished on the exact path; -1 if it wrote
- * nothing. */
+ * nothing.  An unknown key fails with GDR_EINVAL. */
 int gdr_debug_get(const char* key, int64_t* value_host);
-/* Tensor-pipe micro-probe: SM cycles for `iters` back-to-back tcgen05.mma of shape 128 x N x (32 bytes of K)
- * issued by one CTA (variant bit 0: kind::f16 instead of kind::tf32, bit 1: two accumulators, bit 2: no K advance). */
-int gdr_debug_mma_probe(int N, int iters, int variant, int64_t* cycles_host);
 
 /* ---- generic device primitives (used by stages 1, 3, 4) -------------- */
 /* Stable LSD radix sort of (uint64 key, uint32 payload) pairs on the low

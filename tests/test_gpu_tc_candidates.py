@@ -164,7 +164,7 @@ def test_candidate_counts_identical_across_gate_modes(gdr, knob):
     knob("tc_screen", 3)
     ref = None
     truth = None
-    for gate in (0, 1, 2):
+    for gate in (0, 1):
         knob("tc_gate", gate)
         for prev in ((None,) if truth is None else (None, truth, torch.zeros(N, dtype=torch.int32, device=DEV))):
             lab, _, n_ref = assign(gdr, Xd, Cd, prev)

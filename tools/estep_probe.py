@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""E-step alone at a BASELINE shape: direct 3xTF32 vs the two-level screen (128- / 256-centre tiles).
+"""E-step alone at a BASELINE shape: direct 3xTF32 (tc_screen 1) vs the two-level screen (tc_screen 3).
 Run on the GPU box:  python tools/estep_probe.py [B|E]"""
 import ctypes, os, sys
 import numpy as np, torch
@@ -26,7 +26,7 @@ C = padded_rows(Xc[perm].clone())
 op = TcOperand(Xc)
 ws = torch.empty(_lib.query("gdr_kmeans_assign_tc_ws_bytes", n, K, f), dtype=torch.uint8, device=dev)
 flush = torch.empty(256 << 20, dtype=torch.uint8, device=dev)
-MODES = tuple(int(m) for m in os.environ.get("PROBE_MODES", "1,2,3,4,5").split(","))
+MODES = (1, 3)
 for it in range(int(os.environ.get("PROBE_ITERS", "4"))):
     res = {}
     for mode in MODES:
@@ -50,44 +50,4 @@ for it in range(int(os.environ.get("PROBE_ITERS", "4"))):
     print(f"iter {it}: " + "  ".join(f"mode{m}: {res[m][0]*1e3:.0f} us (level2 {res[m][1]}, exact {res[m][2]})" for m in MODES) + f"  labels equal: {same}", flush=True)
     sums, counts = segment_sum(Xc, res[MODES[0]][3], K)
     C = padded_rows((sums / counts.clamp_min(1).unsqueeze(1)).contiguous())
-if os.environ.get("PROBE_ABLATE"):
-    # which role bounds the first-level kernel?  (results are garbage in these runs)
-    for mode in MODES:
-        _lib.call("gdr_debug_set", b"tc_screen", mode)
-        for ab in (0, 2, 3, 5, 8):
-            _lib.call("gdr_debug_set", b"tc_ablate", ab)
-            lab = torch.empty(n, dtype=torch.int32, device=dev)
-            ts = []
-            for rep in range(3):
-                flush.fill_(1)
-                a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                a.record(); assign_labels(Xc, C, lab, tc_operand=op, ws=ws); b.record()
-                torch.cuda.synchronize(); ts.append(a.elapsed_time(b))
-            print(f"mode {mode} ablate {ab}: {min(ts[1:])*1e3:.0f} us", flush=True)
-    _lib.call("gdr_debug_set", b"tc_ablate", 0)
 _lib.call("gdr_debug_set", b"tc_screen", 0)
-if os.environ.get("PROBE_CLOCKS"):
-    # SM clock / power while each variant runs back to back for ~2 s (is the tensor pipe power-capped?)
-    import threading, time, pynvml
-    pynvml.nvmlInit()
-    h = pynvml.nvmlDeviceGetHandleByIndex(0)
-    for mode in MODES:
-        _lib.call("gdr_debug_set", b"tc_screen", mode)
-        lab = torch.empty(n, dtype=torch.int32, device=dev)
-        samples, stop = [], threading.Event()
-        def samp():
-            while not stop.is_set():
-                samples.append((pynvml.nvmlDeviceGetClockInfo(h, pynvml.NVML_CLOCK_SM), pynvml.nvmlDeviceGetPowerUsage(h) / 1000.0))
-                time.sleep(0.05)
-        th = threading.Thread(target=samp); th.start()
-        t0 = time.perf_counter(); reps = 0
-        a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        a.record()
-        while time.perf_counter() - t0 < 2.0:
-            assign_labels(Xc, C, lab, tc_operand=op, ws=ws); reps += 1
-            if reps % 8 == 0: torch.cuda.synchronize()
-        b.record(); torch.cuda.synchronize()
-        stop.set(); th.join()
-        clk = sorted(s[0] for s in samples[len(samples)//2:]); pw = sorted(s[1] for s in samples[len(samples)//2:])
-        print(f"mode {mode}: {a.elapsed_time(b)/reps*1e3:.0f} us/E-step back to back, SM clock median {clk[len(clk)//2]} MHz (min {clk[0]}), power median {pw[len(pw)//2]:.0f} W", flush=True)
-    _lib.call("gdr_debug_set", b"tc_screen", 0)
