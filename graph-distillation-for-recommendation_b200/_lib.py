@@ -125,6 +125,8 @@ _SIGNATURES = {
     "gdr_standardize_apply": (i32, [i64, i64, vp, i64, vp, vp, vp, i64, vp]),
     "gdr_dense_gram_ws_bytes": (i64, [i64, i64, i64]),
     "gdr_dense_gram": (i32, [i64, i64, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp]),
+    "gdr_dense_gram_dist_ws_bytes": (i64, [i64, i64, i64, i32]),
+    "gdr_dense_gram_dist": (i32, [vp, i64, i64, i64, i64, i64, vp, i64, vp, i64, vp, i64, vp, i64, vp]),
     "gdr_dense_chol": (i32, [i64, vp, i64, vp, i64, vp, C.c_double, vp]),
     "gdr_dense_trsm_rows": (i32, [i64, i64, vp, i64, vp, i64, vp]),
     "gdr_dense_gemm_small": (i32, [i64, i64, i64, C.c_double, vp, i64, vp, i64, C.c_double, vp, i64, vp, i64, vp, vp]),

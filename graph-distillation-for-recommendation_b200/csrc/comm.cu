@@ -125,6 +125,38 @@ int comm_allgather(gdr_comm* c, const void* send, void* recv, int64_t bytes_per_
   return GDR_OK;
 }
 
+int comm_send(gdr_comm* c, const void* buf, int64_t bytes, int peer, cudaStream_t s) {
+  const NcclApi* api = nccl_api();
+  if (!api) return GDR_ECUDA;
+  GDR_NCCL(api->Send(buf, (size_t)bytes, ncclInt8, peer, c->nccl, s));
+  count_launch(1);
+  return GDR_OK;
+}
+
+int comm_recv(gdr_comm* c, void* buf, int64_t bytes, int peer, cudaStream_t s) {
+  const NcclApi* api = nccl_api();
+  if (!api) return GDR_ECUDA;
+  GDR_NCCL(api->Recv(buf, (size_t)bytes, ncclInt8, peer, c->nccl, s));
+  count_launch(1);
+  return GDR_OK;
+}
+
+int comm_broadcast(gdr_comm* c, void* buf, int64_t bytes, int root, cudaStream_t s) {
+  if (!c || c->world == 1) return GDR_OK;
+  const NcclApi* api = nccl_api();
+  if (!api) return GDR_ECUDA;
+  GDR_NCCL(api->GroupStart());
+  if (c->rank == root) {
+    for (int p = 0; p < c->world; ++p)
+      if (p != root) GDR_NCCL(api->Send(buf, (size_t)bytes, ncclInt8, p, c->nccl, s));
+  } else {
+    GDR_NCCL(api->Recv(buf, (size_t)bytes, ncclInt8, root, c->nccl, s));
+  }
+  GDR_NCCL(api->GroupEnd());
+  count_launch(1);
+  return GDR_OK;
+}
+
 }  // namespace gdr
 
 

@@ -46,5 +46,10 @@ int comm_allreduce_f64(gdr_comm* c, double* buf, int64_t n, int op_max, cudaStre
 // int64 sums over the ranks, send -> recv (a copy for world 1 / null comm)
 int comm_allreduce_i64(gdr_comm* c, const int64_t* send, int64_t* recv, int64_t n, cudaStream_t s);
 int comm_allgather(gdr_comm* c, const void* send, void* recv, int64_t bytes_per_rank, cudaStream_t s);
+// NCCL point-to-point: the matching comm_recv / comm_send runs on rank `peer` (world > 1 only)
+int comm_send(gdr_comm* c, const void* buf, int64_t bytes, int peer, cudaStream_t s);
+int comm_recv(gdr_comm* c, void* buf, int64_t bytes, int peer, cudaStream_t s);
+// buf of rank `root` -> buf of every other rank, as one group of sends (no-op for world 1 / null comm)
+int comm_broadcast(gdr_comm* c, void* buf, int64_t bytes, int root, cudaStream_t s);
 
 }  // namespace gdr

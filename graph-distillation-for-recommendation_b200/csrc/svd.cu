@@ -8,8 +8,12 @@
 //   gdr_dense_trsm_rows    Y <- Y L^-T, one thread per row                   (CholeskyQR)
 //   gdr_dense_gemm_small   Z <- beta Z + alpha A P, A tall, P small           (block Gram-Schmidt, Ritz vectors)
 //   gdr_sym_eig_jacobi     eigen-decomposition of a small symmetric matrix    (the (q b)^2 Ritz problem)
+//   gdr_dense_gram_dist    gdr_dense_gram of row blocks split over the ranks, the same bits on every rank
 // All reductions have a fixed order (two-stage partial sums): results are run-to-run deterministic.
 #include "common.cuh"
+#include "comm.cuh"
+#include <algorithm>
+#include <vector>
 
 namespace gdr {
 
@@ -62,6 +66,73 @@ __global__ void k_gram_reduce(int p, int r, int slabs, const double* __restrict_
   double s = 0.0;
   for (int z = 0; z < slabs; ++z) s += part[(int64_t)z * p * r + t];
   C[(t / r) * ldc + (t % r)] = s;
+}
+
+// ---- the Gram on a row partition (gdr_dense_gram_dist) ----
+// A rank's rows cut at the global slab boundaries: segment z (blockIdx.z) runs k_gram_partial's chain over local rows
+// [r0, r1), from 0.0 when it starts its slab or from init (the accumulators the previous rank's part of the slab ended
+// with), and stores the chain's end in out [p][r]: the slab's partial, or the carry for the next rank.  The steps of GR
+// rows start at the segment, not at the slab, so zero rows pad a step at a rank boundary too; they leave a chain as it
+// is (fma(0, 0, c) = c for every c but -0.0, which only an fp64 underflow can produce).
+struct GramSegs {
+  int64_t r0[GRAM_MAX_SLABS], r1[GRAM_MAX_SLABS];
+  const double* init[GRAM_MAX_SLABS];
+  double* out[GRAM_MAX_SLABS];
+};
+
+__global__ void __launch_bounds__(256) k_gram_segments(int p, int r, const double* __restrict__ A, int64_t lda,
+                                                       const double* __restrict__ B, int64_t ldb, GramSegs sg) {
+  __shared__ double sA[GR][GT + 1];
+  __shared__ double sB[GR][GT + 1];
+  const int ti = blockIdx.x * GT, tj = blockIdx.y * GT, z = blockIdx.z;
+  const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
+  const double* init = sg.init[z];
+  double acc[2][2];
+#pragma unroll
+  for (int a = 0; a < 2; ++a)
+#pragma unroll
+    for (int b = 0; b < 2; ++b) {
+      const int i = ti + ty * 2 + a, j = tj + tx * 2 + b;
+      acc[a][b] = (init && i < p && j < r) ? init[(int64_t)i * r + j] : 0.0;
+    }
+  const int64_t r0 = sg.r0[z], r1 = sg.r1[z];
+  for (int64_t rr = r0; rr < r1; rr += GR) {
+    for (int t = threadIdx.x; t < GR * GT; t += 256) {
+      const int row = t / GT, col = t % GT;
+      const int64_t g = rr + row;
+      sA[row][col] = (g < r1 && ti + col < p) ? A[g * lda + ti + col] : 0.0;
+      sB[row][col] = (g < r1 && tj + col < r) ? B[g * ldb + tj + col] : 0.0;
+    }
+    __syncthreads();
+#pragma unroll 8
+    for (int k = 0; k < GR; ++k) {
+      const double a0 = sA[k][ty * 2], a1 = sA[k][ty * 2 + 1];
+      const double b0 = sB[k][tx * 2], b1 = sB[k][tx * 2 + 1];
+      acc[0][0] = fma(a0, b0, acc[0][0]);
+      acc[0][1] = fma(a0, b1, acc[0][1]);
+      acc[1][0] = fma(a1, b0, acc[1][0]);
+      acc[1][1] = fma(a1, b1, acc[1][1]);
+    }
+    __syncthreads();
+  }
+#pragma unroll
+  for (int a = 0; a < 2; ++a)
+#pragma unroll
+    for (int b = 0; b < 2; ++b) {
+      const int i = ti + ty * 2 + a, j = tj + tx * 2 + b;
+      if (i < p && j < r) sg.out[z][(int64_t)i * r + j] = acc[a][b];
+    }
+}
+
+// sum_out = sum_in + part[0] + ... + part[n - 1]: k_gram_reduce's slab-order chain, continued from the running sum of the
+// slabs that ended on earlier ranks (0.0 on the first rank)
+__global__ void k_gram_reduce_dist(int64_t pr, int n, const double* __restrict__ part, const double* __restrict__ sum_in,
+                                   double* __restrict__ sum_out) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= pr) return;
+  double s = sum_in[t];
+  for (int z = 0; z < n; ++z) s += part[(int64_t)z * pr + t];
+  sum_out[t] = s;
 }
 
 // lower Cholesky of an n x n SPD matrix (n <= 128) in shared memory; info[0] = 0 ok, j + 1 = pivot j not positive
@@ -319,9 +390,33 @@ __global__ void k_gather_cols(int n, int kcols, const double* __restrict__ W, co
   Wk[t] = W[(int64_t)i * n + order[k]];
 }
 
+// the slabs of an N-row Gram: contiguous blocks of cdiv(N, slabs) rows, summed in slab order
+static int gram_slabs(int64_t N) { return (int)std::max<int64_t>(1, std::min<int64_t>(GRAM_MAX_SLABS, cdiv(N, 2048))); }
+
 }  // namespace gdr
 
 using namespace gdr;
+
+namespace {
+
+struct GramDistBuffers {
+  int64_t* meta;   // [world][8]  entry check (first in the workspace: see gdr_dense_gram_dist)
+  double* part;    // [slabs][p][r] partials of the slabs that end on this rank, in slab order
+  double* x;       // [4][p][r]  carry in, running sum in | carry out, running sum out
+  int64_t off;
+};
+
+GramDistBuffers gram_dist_carve(void* ws, int64_t N, int64_t p, int64_t r, int world) {
+  Workspace W(ws, INT64_MAX);
+  GramDistBuffers b;
+  b.meta = W.take<int64_t>((int64_t)world * 8);
+  b.part = W.take<double>(gram_slabs(N) * p * r);
+  b.x = W.take<double>(4 * p * r);
+  b.off = W.off + 256;
+  return b;
+}
+
+}  // namespace
 
 extern "C" {
 
@@ -338,13 +433,127 @@ int gdr_dense_gram(int64_t N, int64_t p, int64_t r, const double* A, int64_t lda
     return GDR_EWORKSPACE;
   }
   cudaStream_t s = (cudaStream_t)stream;
-  const int slabs = (int)std::max<int64_t>(1, std::min<int64_t>(GRAM_MAX_SLABS, cdiv(N, 2048)));
+  const int slabs = gram_slabs(N);
   double* part = (double*)ws;
   dim3 grid((unsigned)cdiv(p, GT), (unsigned)cdiv(r, GT), (unsigned)slabs);
   k_gram_partial<<<grid, 256, 0, s>>>(N, (int)p, (int)r, A, lda, B, ldb, slabs, part);
   GDR_LAUNCHED();
   k_gram_reduce<<<(unsigned)cdiv(p * r, 256), 256, 0, s>>>((int)p, (int)r, slabs, part, C, ldc);
   GDR_LAUNCHED();
+  return GDR_OK;
+}
+
+int64_t gdr_dense_gram_dist_ws_bytes(int64_t N_global, int64_t p, int64_t r, int world) {
+  return gram_dist_carve(nullptr, N_global, p, r, world).off;
+}
+
+int gdr_dense_gram_dist(gdr_comm_t* comm, int64_t N_global, int64_t row_lo, int64_t n_local, int64_t p, int64_t r,
+                        const double* A, int64_t lda, const double* B, int64_t ldb, double* C, int64_t ldc, void* ws,
+                        int64_t ws_bytes, gdr_stream_t stream) {
+  GDR_CHECK_ARG(comm, "dense_gram_dist: null communicator");
+  const int world = comm->world, rank = comm->rank;
+  cudaStream_t s = (cudaStream_t)stream;
+  // local checks are decided collectively below: a rank that returned early would leave the others in a collective
+  int local_rc = GDR_OK;
+  if (!(N_global >= 0 && row_lo >= 0 && n_local >= 0 && row_lo + n_local <= N_global && p > 0 && r > 0 && C && ldc >= r &&
+        ws && (n_local == 0 || (A && B && lda >= p && ldb >= r)))) {
+    set_error("dense_gram_dist: bad arguments");
+    local_rc = GDR_EINVAL;
+  } else if (ws_bytes < gdr_dense_gram_dist_ws_bytes(N_global, p, r, world)) {
+    set_error("dense_gram_dist: workspace too small");
+    local_rc = GDR_EWORKSPACE;
+  }
+  // entry check: the same N_global, p and r everywhere, row blocks contiguous in rank order and covering N_global
+  int64_t mine[8] = {N_global, row_lo, n_local, p, r, local_rc, 0, 0};
+  std::vector<int64_t> all((size_t)world * 8);
+  const int64_t meta_bytes = (int64_t)all.size() * 8;
+  // the gather buffer is the head of the workspace; a rank whose workspace cannot hold it still takes part in the
+  // check (through a temporary buffer: a rejected call only) so that every rank learns the verdict
+  int64_t* meta = ws && ws_bytes >= meta_bytes ? (int64_t*)ws : nullptr;
+  int64_t* meta_tmp = nullptr;
+  if (!meta) {
+    GDR_CUDA(cudaMalloc(&meta_tmp, meta_bytes));
+    meta = meta_tmp;
+  }
+  int rc = GDR_OK;
+  if (cudaMemcpyAsync(meta + rank * 8, mine, 64, cudaMemcpyHostToDevice, s) != cudaSuccess) {
+    set_error("dense_gram_dist: copy of the argument check failed");
+    rc = GDR_ECUDA;
+  }
+  if (rc == GDR_OK) rc = comm_allgather(comm, meta + rank * 8, meta, 64, s);
+  if (rc == GDR_OK && (cudaMemcpyAsync(all.data(), meta, meta_bytes, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+                       cudaStreamSynchronize(s) != cudaSuccess)) {
+    set_error("dense_gram_dist: read-back of the argument check failed");
+    rc = GDR_ECUDA;
+  }
+  if (meta_tmp) cudaFree(meta_tmp);
+  if (rc != GDR_OK) return rc;
+  if (local_rc != GDR_OK) return local_rc;
+  int64_t next_lo = 0;
+  for (int q = 0; q < world; ++q) {
+    const int64_t* m = &all[(size_t)q * 8];
+    if (m[5] != GDR_OK) {
+      set_error("dense_gram_dist: rank %d rejected its arguments", q);
+      return GDR_EINVAL;
+    }
+    if (m[0] != N_global || m[3] != p || m[4] != r) {
+      set_error("dense_gram_dist: rank %d passed a different N_global, p or r", q);
+      return GDR_EINVAL;
+    }
+    if (m[1] != next_lo) {
+      set_error("dense_gram_dist: the row block of rank %d does not follow the one of rank %d", q, q - 1);
+      return GDR_EINVAL;
+    }
+    next_lo += m[2];
+  }
+  GDR_CHECK_ARG(next_lo == N_global, "dense_gram_dist: the row blocks hold %lld rows, not N_global = %lld",
+                (long long)next_lo, (long long)N_global);   // the same verdict on every rank
+
+  // this rank's rows cut at the global slab boundaries (gdr_dense_gram's geometry): the segments that start their slab
+  // need nothing from the previous rank; at most one, the first, continues the carry of a slab begun on an earlier rank
+  const int64_t pr = p * r, rows_per = cdiv(N_global, gram_slabs(N_global));
+  GramDistBuffers G = gram_dist_carve(ws, N_global, p, r, world);
+  double *carry_in = G.x, *sum_in = G.x + pr, *carry_out = G.x + 2 * pr, *sum_out = G.x + 3 * pr;
+  GramSegs starts = {}, cont = {};
+  int n_starts = 0, n_cont = 0, n_done = 0;
+  for (int64_t a = row_lo, hi = row_lo + n_local; a < hi;) {
+    const int64_t z0 = a / rows_per * rows_per, z1 = std::min(N_global, z0 + rows_per), b = std::min(hi, z1);
+    GramSegs& g = a == z0 ? starts : cont;
+    int& n = a == z0 ? n_starts : n_cont;
+    g.r0[n] = a - row_lo;
+    g.r1[n] = b - row_lo;
+    g.init[n] = a == z0 ? nullptr : carry_in;
+    g.out[n] = b == z1 ? G.part + (int64_t)(n_done++) * pr : carry_out;
+    ++n;
+    a = b;
+  }
+  const unsigned tx = (unsigned)cdiv(p, GT), ty = (unsigned)cdiv(r, GT);
+  if (n_starts) {
+    k_gram_segments<<<dim3(tx, ty, (unsigned)n_starts), 256, 0, s>>>((int)p, (int)r, A, lda, B, ldb, starts);
+    GDR_LAUNCHED();
+  }
+  // (carry, running sum) from the previous rank; the first rank starts the running sum from 0.0
+  if (rank > 0) {
+    if ((rc = comm_recv(comm, G.x, 2 * pr * 8, rank - 1, s))) return rc;
+  } else {
+    GDR_CUDA(cudaMemsetAsync(G.x, 0, 2 * pr * 8, s));
+  }
+  if (n_cont) {
+    k_gram_segments<<<dim3(tx, ty, 1), 256, 0, s>>>((int)p, (int)r, A, lda, B, ldb, cont);
+    GDR_LAUNCHED();
+  }
+  // an empty rank hands on what it received
+  double* handed = G.x;
+  if (n_local > 0) {
+    k_gram_reduce_dist<<<(unsigned)cdiv(pr, 256), 256, 0, s>>>(pr, n_done, G.part, sum_in, sum_out);
+    GDR_LAUNCHED();
+    handed = carry_out;
+  }
+  if (rank + 1 < world && (rc = comm_send(comm, handed, 2 * pr * 8, rank + 1, s))) return rc;
+  // the last rank's running sum is C: every other rank receives it into its (already sent) running-sum slot
+  double* total = handed + pr;
+  if ((rc = comm_broadcast(comm, total, pr * 8, world - 1, s))) return rc;
+  GDR_CUDA(cudaMemcpy2DAsync(C, (size_t)ldc * 8, total, (size_t)r * 8, (size_t)r * 8, (size_t)p, cudaMemcpyDeviceToDevice, s));
   return GDR_OK;
 }
 

@@ -643,6 +643,19 @@ class CudaOps:
     def _pad4(d):
         return (int(d) + 3) // 4 * 4
 
+    # -- truncated SVD (distill_recsys) --
+    def gram_dist(self, comm, n_global, row_lo, A, B):
+        """AᵀB of the row-partitioned fp64 A [n_local, p], B [n_local, r] (global rows row_lo .. row_lo + n_local of
+        n_global), replicated with gdr_dense_gram's bits on the concatenated rows (gdr_dense_gram_dist; collective)."""
+        n_local, p = A.shape
+        r = B.shape[1]
+        C = torch.empty((p, r), dtype=torch.float64, device=A.device)
+        ws = self.workspace(self._lib.query("gdr_dense_gram_dist_ws_bytes", int(n_global), p, r, comm.world), A.device)
+        self._lib.call("gdr_dense_gram_dist", comm.lib_handle(), int(n_global), int(row_lo), n_local, p, r,
+                       self.ptr(A) if n_local else 0, A.stride(0) if n_local else p, self.ptr(B) if n_local else 0,
+                       B.stride(0) if n_local else r, self.ptr(C), r, self.ptr(ws), ws.numel(), self.stream())
+        return C
+
     def inertia(self, Xc, C, labels):
         out = torch.zeros(1, dtype=torch.float64, device=C.device)
         if Xc.shape[0] == 0:
@@ -1508,6 +1521,69 @@ def dist_lightgcn_propagate(comm: Comm, part_u: RowPartition, part_i: RowPartiti
         u, it = u_next, i_next
     inv = 1.0 / float(num_layers + 1)
     return ops.scale(u_acc, inv), ops.scale(i_acc, inv)
+
+
+def _same_on_every_rank(comm: Comm, device, what: str, *vals):
+    """Raises ValueError on every rank unless every rank passed the same integers (one all-gather)."""
+    mine = torch.tensor([int(v) for v in vals], dtype=torch.int64, device=device)
+    allv = torch.empty(comm.world * mine.numel(), dtype=torch.int64, device=device)
+    comm.all_gather_rows(mine, allv)
+    if not bool((allv.view(comm.world, -1) == mine).all()):
+        raise ValueError(f"{what}: the ranks passed different arguments")
+
+
+def dist_truncated_svd(comm: Comm, part_u: RowPartition, part_i: RowPartition, R_local, RT_local, k: int, seed: int = 42,
+                       block: int = None, n_blocks: int = None, ops=None):
+    """svd.truncated_svd of the row-partitioned interaction matrix (R_local, RT_local as dist_build_interaction returns
+    them) without gathering R.  Collective; every rank passes the same k, seed, block and n_blocks (checked: a mismatch
+    raises ValueError on every rank).  The Krylov blocks Q and the products B = A Q stay row-partitioned: each SpMM runs
+    on this rank's rows against its operand all-gathered in the padded equal-block layout, each Gram is
+    gdr_dense_gram_dist, and the small (q b)² Ritz problem is solved on every rank from identical data.  Returns
+    (U_local [this rank's users, k], S [k] descending, the same on every rank, V_local [this rank's items, k]), fp32
+    on the device; the blocks in rank order are byte-identical to truncated_svd(R) for any number of ranks."""
+    from .svd import krylov_ritz
+    ops = ops or CudaOps()
+    if not hasattr(ops, "gram_dist"):
+        raise NotImplementedError(f"{type(ops).__name__} has no distributed Gram matrix")
+    dev = R_local.device
+    _same_on_every_rank(comm, dev, "dist_truncated_svd", part_u.n, part_i.n, k, seed, -1 if block is None else block,
+                        -1 if n_blocks is None else n_blocks)
+    # Krylov space on the smaller side (truncated_svd's choice): A maps it to the larger one
+    if part_i.n <= part_u.n:
+        A, At, p_s, p_o = R_local, RT_local, part_i, part_u
+    else:
+        A, At, p_s, p_o = RT_local, R_local, part_u, part_i
+
+    def times(M, x_local, part):
+        """This rank's rows of M X, X the whole matrix whose rows ``part`` splits (this rank holds x_local)."""
+        f = x_local.shape[1]
+        blk = ops.empty_rows(part.rows_per, f, x_local)
+        blk[: x_local.shape[0]].copy_(x_local)
+        full = ops.empty_rows(part.rows_per * part.world, f, x_local)      # row index = global id (equal blocks)
+        comm.all_gather_rows(blk, full)
+        return ops.spmm(M, full, 1.0, None, 0.0)
+
+    Uo, S, Vs = krylov_ritz(p_s.n, slice(p_s.lo, p_s.hi), k, seed, block, n_blocks, dev,
+                            lambda X, Y: ops.gram_dist(comm, p_s.n, p_s.lo, X, Y),
+                            lambda X, Y: ops.gram_dist(comm, p_o.n, p_o.lo, X, Y),
+                            lambda X: times(A, X, p_s), lambda Y: times(At, Y, p_o))
+    return (Uo, S, Vs) if part_i.n <= part_u.n else (Vs, S, Uo)
+
+
+def dist_compute_svd_embeddings(comm: Comm, part_u: RowPartition, part_i: RowPartition, R_local, RT_local, dim: int,
+                                seed: int = 42, ops=None):
+    """svd.compute_svd_embeddings (distill_recsys.py:124-155) on the row partition: (U sqrt(S), V sqrt(S)) of this
+    rank's users and items from dist_truncated_svd, as fp32 DEVICE tensors (the input of dist_standard_scale), byte-
+    identical to the rows of the one-GPU embeddings.  Collective; raises the reference's ValueError when no
+    factorisation is possible, and ValueError on every rank when the ranks pass different dim or seed."""
+    _same_on_every_rank(comm, R_local.device, "dist_compute_svd_embeddings", part_u.n, part_i.n, dim, seed)
+    shape = (part_u.n, part_i.n)
+    k = min(int(dim), min(shape) - 1)
+    if k <= 0:
+        raise ValueError(f"Cannot compute SVD with shape={tuple(shape)} and dim={dim}")
+    U, S, V = dist_truncated_svd(comm, part_u, part_i, R_local, RT_local, k, seed=seed, ops=ops)
+    sqrt_s = torch.sqrt(torch.clamp_min(S, 1e-12)).reshape(1, -1)
+    return U * sqrt_s, V * sqrt_s
 
 
 def dist_standard_scale(comm: Comm, x_local: torch.Tensor, ops=None):

@@ -46,14 +46,15 @@ def _gram(A: torch.Tensor, B: torch.Tensor) -> torch.Tensor:
     return C
 
 
-def _cholqr2(Y: torch.Tensor) -> bool:
+def _cholqr2(Y: torch.Tensor, gram=_gram) -> bool:
     """In-place orthonormalisation of the columns of the fp64 block Y [N, b] (CholeskyQR, twice).  False when the block
-    has lost rank (a pivot of the Gram matrix is below 1e-13 of its largest diagonal entry)."""
+    has lost rank (a pivot of the Gram matrix is below 1e-13 of its largest diagonal entry).  ``gram(X, Y)`` is XᵀY
+    over all rows of the block (on a row partition: over every rank's rows, replicated)."""
     N, b = Y.shape
     info = torch.zeros(1, dtype=torch.int32, device=Y.device)
     L = torch.empty((b, b), dtype=torch.float64, device=Y.device)
     for _ in range(2):
-        S = _gram(Y, Y)
+        S = gram(Y, Y)
         _lib.call("gdr_dense_chol", b, ptr(S), b, ptr(L), b, ptr(info), 1e-13, stream())
         if int(info.item()):
             return False
@@ -61,59 +62,56 @@ def _cholqr2(Y: torch.Tensor) -> bool:
     return True
 
 
-def _project_out(Z: torch.Tensor, Q: torch.Tensor):
+def _project_out(Z: torch.Tensor, Q: torch.Tensor, gram=_gram):
     """Z <- Z - Q (Qᵀ Z), twice (block Gram-Schmidt with re-orthogonalisation), Q [N, m] orthonormal."""
     N, b = Z.shape
     m = Q.shape[1]
     for _ in range(2):
-        P = _gram(Q, Z)
-        _lib.call("gdr_dense_gemm_small", N, m, b, -1.0, ptr(Q), Q.stride(0), ptr(P), b, 1.0, ptr(Z), Z.stride(0), 0, 0, 0,
-                  stream())
+        P = gram(Q, Z)
+        if N:
+            _lib.call("gdr_dense_gemm_small", N, m, b, -1.0, ptr(Q), Q.stride(0), ptr(P), b, 1.0, ptr(Z), Z.stride(0), 0, 0,
+                      0, stream())
 
 
-def truncated_svd(R: CSR, k: int, seed: int = 42, block: int = None, n_blocks: int = None
-                  ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
-    """(U [n_rows, k], S [k] descending, V [n_cols, k]) of the k largest singular triplets of the device CSR ``R``."""
-    n_rows, n_cols = R.shape
-    dev = R.device
-    Rt, _ = R.transpose()
-    # Krylov space on the smaller side: A maps it to the larger one
-    if n_cols <= n_rows:
-        A, At, ns = R, Rt, n_cols
-    else:
-        A, At, ns = Rt, R, n_rows
+def krylov_ritz(ns: int, rows: slice, k: int, seed: int, block, n_blocks, dev, gram_s, gram_o, mul_A, mul_At
+                ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """The factorisation of truncated_svd, written for the rows ``rows`` of the small side (ns rows) that this process
+    holds: all of them on one GPU, a row block on a partition (parallel.dist_truncated_svd).  ``gram_s(X, Y)`` / ``gram_o``
+    = XᵀY over all rows of the small / other side; ``mul_A(X)`` = the held rows of the other side of A X for the held
+    fp64 rows X of small-side vectors (fp32 result), ``mul_At(Y)`` = the held small-side rows of Aᵀ Y.  Every branch is
+    decided on replicated data.  Returns (Uo [held other-side rows, k], S [k] fp32 descending, Vs [held small-side rows, k])."""
     k = int(min(k, ns))
+    n_s = rows.stop - rows.start
     if ns <= EXACT_SIDE and block is None and n_blocks is None:
         # the whole space of the smaller side: Q = I, the Ritz problem below is the exact Gram eigen-problem of A
         # (a Krylov space clamped to a few dimensions short of ns interlaces the spectrum instead of matching it)
         m = ns
-        Qm = torch.eye(ns, dtype=torch.float64, device=dev)
+        Qm = torch.eye(ns, dtype=torch.float64, device=dev)[rows]
     else:
         b = int(min(block or (k + 8), ns, 128))
         q = int(n_blocks or max(6, min(14, 600 // b)))
         q = max(1, min(q, ns // b))                              # q b <= ns: the space cannot be larger than the side
         gen = torch.Generator(device="cpu").manual_seed(int(seed))
-        G = torch.randn((ns, b), generator=gen, dtype=torch.float32).to(dev)
-        Q = torch.zeros((ns, q * b), dtype=torch.float64, device=dev)
+        G = torch.randn((ns, b), generator=gen, dtype=torch.float32)[rows].to(dev)
+        Q = torch.zeros((n_s, q * b), dtype=torch.float64, device=dev)
         V = Q[:, :b]
         V.copy_(G)
-        if not _cholqr2(V):
+        if not _cholqr2(V, gram_s):
             raise ValueError("truncated_svd: the random start block is rank deficient")
         m = b
         for j in range(1, q):
-            Vp = Q[:, (j - 1) * b: j * b]
-            Y = spmm(A, Vp.to(torch.float32).contiguous())       # [n_other, b]  sparse x dense on the CSR kernel
-            Z = spmm(At, Y.contiguous())                         # [ns, b]
+            Y = mul_A(Q[:, (j - 1) * b: j * b])                  # [n_other, b]  sparse x dense on the CSR kernel
+            Z = mul_At(Y)                                        # [ns, b]
             Vn = Q[:, j * b: (j + 1) * b]
             Vn.copy_(Z)
-            _project_out(Vn, Q[:, :m])
-            if not _cholqr2(Vn):                                 # Krylov space exhausted: keep the blocks so far
+            _project_out(Vn, Q[:, :m], gram_s)
+            if not _cholqr2(Vn, gram_s):                         # Krylov space exhausted: keep the blocks so far
                 break
             m += b
         Qm = Q[:, :m]
-    B = spmm(A, Qm.to(torch.float32).contiguous()).double()      # [n_other, m] = A Q
+    B = mul_A(Qm).double()                                       # [n_other, m] = A Q
     # Rayleigh-Ritz on the Gram matrix of B (fp64; the leading Ritz values lose nothing to the squared condition number)
-    T = _gram(B, B).contiguous()
+    T = gram_o(B, B).contiguous()
     W = torch.empty((m, m), dtype=torch.float64, device=dev)
     evals = torch.empty(m, dtype=torch.float64, device=dev)
     order = torch.empty(m, dtype=torch.int32, device=dev)
@@ -127,13 +125,28 @@ def truncated_svd(R: CSR, k: int, seed: int = 42, block: int = None, n_blocks: i
     S = evals[:kk].clamp_min(0).sqrt()
     inv_s = torch.where(S > 0, 1.0 / S, torch.zeros_like(S)).contiguous()
     n_other = B.shape[0]
-    Vs = torch.empty((ns, kk), dtype=torch.float32, device=dev)          # small-side vectors  Q W
+    Vs = torch.empty((n_s, kk), dtype=torch.float32, device=dev)         # small-side vectors  Q W
     Uo = torch.empty((n_other, kk), dtype=torch.float32, device=dev)     # other-side vectors  B W / sigma
-    _lib.call("gdr_dense_gemm_small", ns, m, kk, 1.0, ptr(Qm), Qm.stride(0), ptr(Wk), kk, 0.0, 0, 0, ptr(Vs), kk, 0, stream())
-    _lib.call("gdr_dense_gemm_small", n_other, m, kk, 1.0, ptr(B), B.stride(0), ptr(Wk), kk, 0.0, 0, 0, ptr(Uo), kk, ptr(inv_s),
-              stream())
-    S32 = S.to(torch.float32)
-    return (Uo, S32, Vs) if n_cols <= n_rows else (Vs, S32, Uo)
+    if n_s:
+        _lib.call("gdr_dense_gemm_small", n_s, m, kk, 1.0, ptr(Qm), Qm.stride(0), ptr(Wk), kk, 0.0, 0, 0, ptr(Vs), kk, 0,
+                  stream())
+    if n_other:
+        _lib.call("gdr_dense_gemm_small", n_other, m, kk, 1.0, ptr(B), B.stride(0), ptr(Wk), kk, 0.0, 0, 0, ptr(Uo), kk,
+                  ptr(inv_s), stream())
+    return Uo, S.to(torch.float32), Vs
+
+
+def truncated_svd(R: CSR, k: int, seed: int = 42, block: int = None, n_blocks: int = None
+                  ) -> Tuple[torch.Tensor, torch.Tensor, torch.Tensor]:
+    """(U [n_rows, k], S [k] descending, V [n_cols, k]) of the k largest singular triplets of the device CSR ``R``."""
+    n_rows, n_cols = R.shape
+    Rt, _ = R.transpose()
+    # Krylov space on the smaller side: A maps it to the larger one
+    A, At = (R, Rt) if n_cols <= n_rows else (Rt, R)
+    ns = min(n_rows, n_cols)
+    Uo, S, Vs = krylov_ritz(ns, slice(0, ns), k, seed, block, n_blocks, R.device, _gram, _gram,
+                            lambda X: spmm(A, X.to(torch.float32).contiguous()), lambda Y: spmm(At, Y.contiguous()))
+    return (Uo, S, Vs) if n_cols <= n_rows else (Vs, S, Uo)
 
 
 def compute_svd_embeddings(R: Union[sp.spmatrix, CSR], dim: int, seed: int = 42, device=None

@@ -655,6 +655,20 @@ int     gdr_kmeans_plusplus_dist(gdr_comm_t* comm, int64_t N_local, int64_t K, i
 int64_t gdr_dense_gram_ws_bytes(int64_t N, int64_t p, int64_t r);
 int     gdr_dense_gram(int64_t N, int64_t p, int64_t r, const double* A, int64_t lda, const double* B, int64_t ldb,
                        double* C, int64_t ldc, void* ws, int64_t ws_bytes, gdr_stream_t stream);
+/* gdr_dense_gram on a row partition.  COLLECTIVE over comm.  Each rank passes its n_local rows of A and B, global rows
+ * [row_lo, row_lo + n_local) of the N_global (n_local = 0 allowed, A and B may then be NULL); C[p x r] comes out on
+ * every rank with the bits gdr_dense_gram gives on the concatenated rows, for any number of ranks.  The slabs are
+ * gdr_dense_gram's, from N_global; a rank runs each slab's fp64 fma chain over its rows of that slab, continuing the
+ * exact accumulators (the carry) handed on by the previous rank when the slab began there, and adds the slabs that end
+ * on it to the slab-order running sum it receives (0.0 on rank 0).  Rank q sends rank q + 1 the carry and the running
+ * sum (2 p r doubles, NCCL point-to-point); the last rank's sum is C and is sent to all.  Slabs that start on a rank
+ * are summed before it receives anything.  At entry every rank all-gathers N_global, row_lo, n_local, p, r and its
+ * argument verdict; a mismatch, blocks that are not contiguous in rank order or do not cover N_global, or an argument
+ * any rank rejects returns GDR_EINVAL on every rank.  Synchronises the stream once, after the entry check. */
+int64_t gdr_dense_gram_dist_ws_bytes(int64_t N_global, int64_t p, int64_t r, int world);
+int     gdr_dense_gram_dist(gdr_comm_t* comm, int64_t N_global, int64_t row_lo, int64_t n_local, int64_t p, int64_t r,
+                            const double* A, int64_t lda, const double* B, int64_t ldb, double* C, int64_t ldc,
+                            void* ws, int64_t ws_bytes, gdr_stream_t stream);
 int     gdr_dense_chol(int64_t n, const double* S, int64_t lds, double* L, int64_t ldl, int32_t* info_dev, double rel_tol,
                        gdr_stream_t stream);
 int     gdr_dense_trsm_rows(int64_t N, int64_t n, double* Y, int64_t ldy, const double* L, int64_t ldl,
