@@ -78,7 +78,10 @@ def graph_compress(cluster_labels: torch.Tensor, adj_norm, adj_list: Sequence) -
 
     S[a, b] = sum_{i in a, j in b} A_ij / (n_a * n_b) for a != b (diagonal removed), returned as
     torch sparse COO n x n with n = cluster_labels.max() + 1 (trailing empty clusters shrink n,
-    as in the reference).  One result per graph in ``adj_list`` plus one for ``adj_norm``."""
+    as in the reference).  One result per graph in ``adj_list`` plus one for ``adj_norm``.
+    Every off-diagonal cell with at least one edge is stored: a cell whose weights cancel exactly
+    (signed weights, e.g. ``graph_sparse`` outputs) is an explicit 0, where the reference's
+    dense ``.to_sparse()`` drops it."""
     dev = adj_norm.device
     labels = cluster_labels.to(device=dev, dtype=torch.int32).contiguous()
     n = int(labels.max().item()) + 1

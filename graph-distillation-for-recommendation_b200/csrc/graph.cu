@@ -793,11 +793,12 @@ __global__ void k_csr_to_coo(int64_t n_rows, const int32_t* __restrict__ rowptr,
 // accumulates cell (a, b = label[col]) into a dense shared-memory row of n_dst counters:
 //   count[b] += 1 (u32),  sum[b] += round(w / q_a) (i64 fixed point)
 // Integer accumulation is associative, so the result does not depend on the order in which the shared-memory atomics
-// land: bit-reproducible, and the weight sum is rounded to fp32 ONCE (closer to the exact sum than any fp32 summation
-// order).  q_a = pow2(max |w| of the cluster) * pow2(edges of the cluster) * 2^-62 — no overflow, ~2^-48 of the
-// largest weight.  The row is then compacted in column order into a scratch slice (at the cluster's edge offset),
-// and a second small kernel packs the slices into the final CSR.  HBM traffic: the edges once (8 B each), the
-// column labels through L2, the cells twice — against four (key, value) radix passes over all edges before.
+// land: bit-reproducible.  q_a = pow2(max |w| of the cluster) * pow2(edges of the cluster) * 2^-62 — no overflow, ~2^-48
+// of the largest weight.  Each term is rounded to a multiple of q_a, so a cell of n edges is within n * q_a / 2 plus one
+// fp32 rounding of its exact sum: one ulp only when the cell is at least about n * q_a * 2^24.  The row is then compacted
+// in column order into a scratch slice (at the cluster's edge offset), and a second small kernel packs the slices into
+// the final CSR.  HBM traffic: the edges once (8 B each), the column labels through L2, the cells twice — against four
+// (key, value) radix passes over all edges before.
 constexpr int CD_THREADS = 1024;
 constexpr int CD_HUB = 4096;          // rows at least this long are walked by the whole CTA
 

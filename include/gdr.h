@@ -411,7 +411,9 @@ int gdr_add_row_vector(int64_t rows, int64_t D, float* X, int64_t ldx, const flo
  *   counts[a,b] = #edges with that key   (int32, exact)
  *   wsum[a,b]   = sum of w over them     (fp32; nullable).  CSR input whose coarse row fits in shared memory (n_dst
  *                 <= ~17 K with weights): one CTA per coarse row accumulates the cells there, the weights as 64-bit
- *                 fixed-point integers -> the exact sum rounded to fp32 once, bit-reproducible.  Otherwise (COO input,
+ *                 fixed-point integers with a step q ~ 2^-48 of the cluster's largest |w| -> bit-reproducible, within
+ *                 n_cell * q / 2 plus one fp32 rounding of the exact sum (one ulp only when the cell is at least about
+ *                 n_cell * q * 2^24).  Otherwise (COO input,
  *                 wider rows, gdr_debug_set("coarsen_dense", 0)): radix sort by cell, fp32 sums in input order.
  *   replaces  build_condensed_bipartite           distill_recsys.py:184-201
  *             graph_compress (P^T A P)            clustgdd_agent_transduct.py:234-250

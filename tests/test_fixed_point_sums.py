@@ -1,16 +1,14 @@
 """The arithmetic of the shared-memory coarsening (csrc/graph.cu k_cd_accumulate), restated in numpy and checked on the
 CPU: per-cluster fixed-point step q = 2^(e_w + e_n - 62) from (max |w|, edge count), terms round(w / q) accumulated as a
-64-bit integer kept in two 32-bit words with a carry, in ANY order -> the exact sum rounded to fp32 once, no overflow."""
+64-bit integer kept in two 32-bit words with a carry, in ANY order -> bit-reproducible, no overflow, and within
+n_cell * q / 2 plus one fp32 rounding of the exact sum: one ulp when the cell is at least about n_cell * q * 2^24, not for
+a cell small next to the cluster's largest weight."""
 from fractions import Fraction
 
 import numpy as np
 import pytest
 
-
-def _step(wmax: np.float32, n_edges: int):
-    ew = int(np.frexp(np.float32(wmax))[1])          # wmax < 2^ew
-    ee = int(np.frexp(float(max(n_edges, 1)))[1])    # n_edges < 2^ee
-    return ew + ee - 62                              # q = 2^this
+from coarsen_ref import dense_bound, fixed_point_sum, one_ulp_regime, step as _step, ulp32
 
 
 def _accumulate_two_words(terms: np.ndarray, order: np.ndarray) -> int:
@@ -49,10 +47,13 @@ def test_fixed_point_sum_is_the_exact_sum_rounded_once_in_any_order(seed, n, sca
         assert abs(total) < 2 ** 62                            # no overflow, whatever the order
         results.add(total)
         got = np.float32(np.float64(total) * 2.0 ** e)
-        ref = np.float32(float(exact))
-        # the integer sum differs from the exact sum by at most n/2 steps of q ~ 2^-48 of the largest weight: the fp32
-        # rounding of both agrees up to one ulp (and is identical unless the exact sum sits on a rounding boundary)
-        assert abs(float(got) - float(ref)) <= float(np.spacing(np.abs(ref)))
+        assert got == fixed_point_sum(w, e)
+        # the integer sum differs from the exact sum by at most n/2 steps of q ~ 2^-48 of the largest weight; this cell
+        # holds that weight, so it is large next to n*q and its fp32 rounding is within one ulp of the exact sum's
+        S = float(exact)
+        assert abs(Fraction(float(got)) - exact) <= Fraction(float(dense_bound(S, n, 2.0 ** e)))
+        assert one_ulp_regime(S, n, 2.0 ** e)
+        assert abs(float(got) - float(np.float32(S))) <= float(ulp32(S))
     assert len(results) == 1                                   # associative: bit-reproducible
 
 
@@ -61,3 +62,20 @@ def test_step_is_a_function_of_the_global_cluster_stats_only():
     assert _step(np.float32(0.5), 12600) == _step(np.float32(0.5), 12600)
     assert _step(np.float32(0.5), 12600) == 0 + 14 - 62        # 0.5 = 0.5 * 2^0 -> ew 0; 12600 < 2^14 -> ee 14
     assert _step(np.float32(0.0), 0) == 0 + 1 - 62
+
+
+@pytest.mark.parametrize("w_cell,ulps", [(1e-9, 31), (1e-12, 17204)])
+def test_small_cell_next_to_a_large_weight_is_off_by_more_than_one_ulp(w_cell, ulps):
+    """A cluster with a weight-1 self-loop and 12 600 edges: q = 2^-47 for every cell of it.  A one-edge cell of weight
+    1e-9 is rounded to a multiple of q — dozens of ulps from the exact (and fp32-exact) value — so 'within one ulp' does
+    not hold; the bound n*q/2 + one fp32 rounding does."""
+    e = _step(np.float32(1.0), 12600)
+    assert e == -47
+    w = np.array([w_cell], dtype=np.float32)
+    got = fixed_point_sum(w, e)
+    S = float(w[0])                                            # a one-edge cell: the exact sum is the fp32 weight itself
+    err = abs(float(got) - S)
+    assert err <= dense_bound(S, 1, 2.0 ** e)
+    assert not one_ulp_regime(S, 1, 2.0 ** e)
+    assert err > ulp32(S)                                      # the old 'within one ulp of the exact sum' fails here
+    assert round(err / ulp32(S)) == ulps

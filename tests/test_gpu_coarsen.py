@@ -5,6 +5,8 @@ import pytest
 import scipy.sparse as sp
 import torch
 
+import coarsen_ref
+
 pytestmark = pytest.mark.gpu
 DEV = torch.device("cuda", 0) if torch.cuda.is_available() else None
 
@@ -50,7 +52,7 @@ def test_dense_coarsen_equals_sort_path_and_fp64(gdr, n, k, avg_deg, hubs, drop)
     rp_d, ci_d, cnt_d, ws_d = _coarsen(gdr, A, labels, k, dense=True, drop_diag=drop)
     assert torch.equal(rp_s, rp_d) and torch.equal(ci_s, ci_d) and torch.equal(cnt_s, cnt_d)
     torch.testing.assert_close(ws_d, ws_s, rtol=2e-6, atol=0)
-    # fp64 reference: the fixed-point sums are the exact sums rounded once
+    # fp64 reference: the fixed-point sums are within n*q_a/2 plus one fp32 rounding of the exact sums
     As = sp.csr_matrix((A.vals.cpu().numpy().astype(np.float64), A.colidx.cpu().numpy(), A.rowptr.cpu().numpy()), shape=(n, n))
     P = sp.csr_matrix((np.ones(n), (np.arange(n), lab)), shape=(n, k))
     S = (P.T @ As @ P).tocsr()
@@ -59,9 +61,14 @@ def test_dense_coarsen_equals_sort_path_and_fp64(gdr, n, k, avg_deg, hubs, drop)
         S.eliminate_zeros()
     S.sort_indices()
     assert np.array_equal(S.indptr, rp_d.cpu().numpy()) and np.array_equal(S.indices, ci_d.cpu().numpy())
-    ref = S.data.astype(np.float32)
     got = ws_d.cpu().numpy()
-    assert np.all(np.abs(got - ref) <= np.spacing(np.abs(ref)))      # within one fp32 ulp of the exact sum
+    r = coarsen_ref.csr_cells(A.rowptr.cpu().numpy(), A.colidx.cpu().numpy(), A.vals.cpu().numpy(), lab, lab, drop)
+    q = coarsen_ref.steps(A.rowptr.cpu().numpy(), A.vals.cpu().numpy(), lab, k)[r["a"]]
+    assert np.array_equal(r["count"], cnt_d.cpu().numpy())
+    err = np.abs(got.astype(np.float64) - r["sum"])
+    assert np.all(err <= coarsen_ref.dense_bound(r["sum"], r["count"], q))
+    one = coarsen_ref.one_ulp_regime(r["sum"], r["count"], q)      # where n*q_a/2 <= ulp/4: within one ulp of fl32(exact)
+    assert np.all(np.abs(got[one] - r["sum"][one].astype(np.float32)) <= coarsen_ref.ulp32(r["sum"][one]))
     # bit-reproducible although the shared-memory atomics land in any order
     _, _, _, ws_d2 = _coarsen(gdr, A, labels, k, dense=True, drop_diag=drop)
     assert torch.equal(ws_d, ws_d2)

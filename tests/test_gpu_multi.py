@@ -119,7 +119,7 @@ def _worker(rank, world, port):
         kk = int(labels.max()) + 1
         _, _, cnt1, _ = gdr.coarsen_edges(labels, labels, kk, kk, csr=A_full, drop_diag=True)
         # transports: NCCL send/recv (symm False) and posted stores through the symmetric buffer (gdr_symm_scatterv);
-        # forms: cells accumulated in shared memory (dense 1: exact sums rounded once, with the GLOBAL per-cluster fixed-point
+        # forms: cells accumulated in shared memory (dense 1: fixed-point sums with the GLOBAL per-cluster fixed-point
         # step) and the sort (dense 0: fp32 sums in global CSR order) — the routed result equals one GPU's bit for bit in both
         from gdr import _lib as _lib_dbg
         for dense in (1, 0):
