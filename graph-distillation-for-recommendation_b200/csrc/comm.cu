@@ -157,6 +157,53 @@ int comm_broadcast(gdr_comm* c, void* buf, int64_t bytes, int root, cudaStream_t
   return GDR_OK;
 }
 
+int comm_entry_check(gdr_comm* c, cudaStream_t s, const char* call, int local_rc, int64_t row_lo, int64_t n_local,
+                     int64_t n_global, std::initializer_list<int64_t> agreed, const char* agreed_names, int64_t extra,
+                     int64_t* row_off, int64_t* extras) {
+  GDR_CHECK_ARG(agreed.size() <= (size_t)kEntryAgreed, "%s: more than %d agreed words", call, kEntryAgreed);
+  const int world = c->world;
+  int64_t mine[kEntryWords] = {local_rc, row_lo, n_local, extra};
+  std::copy(agreed.begin(), agreed.end(), mine + 4);
+  std::vector<int64_t> all((size_t)world * kEntryWords);
+  int64_t* row = c->entry + (int64_t)c->rank * kEntryWords;
+  if (cudaMemcpyAsync(row, mine, sizeof(mine), cudaMemcpyHostToDevice, s) != cudaSuccess) {
+    set_error("%s: copy of the argument check failed", call);
+    return GDR_ECUDA;
+  }
+  if (int rc = comm_allgather(c, row, c->entry, sizeof(mine), s)) return rc;
+  if (cudaMemcpyAsync(all.data(), c->entry, all.size() * 8, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+      cudaStreamSynchronize(s) != cudaSuccess) {
+    set_error("%s: read-back of the argument check failed", call);
+    return GDR_ECUDA;
+  }
+  if (local_rc != GDR_OK) return local_rc;
+  int64_t next_lo = 0;
+  for (int r = 0; r < world; ++r) {
+    const int64_t* m = &all[(size_t)r * kEntryWords];
+    if (m[0] != GDR_OK) {
+      set_error("%s: rank %d rejected its arguments", call, r);
+      return GDR_EINVAL;
+    }
+    if (!std::equal(mine + 4, mine + kEntryWords, m + 4)) {
+      set_error("%s: rank %d passed a different %s", call, r, agreed_names);
+      return GDR_EINVAL;
+    }
+    if (row_lo >= 0 && m[1] != next_lo) {
+      set_error("%s: the row block of rank %d does not follow the previous rank's", call, r);
+      return GDR_EINVAL;
+    }
+    if (row_off) row_off[r] = next_lo;
+    if (extras) extras[r] = m[3];
+    next_lo += m[2];
+  }
+  if (n_global >= 0 && next_lo != n_global) {
+    set_error("%s: the row blocks hold %lld rows, not %lld", call, (long long)next_lo, (long long)n_global);
+    return GDR_EINVAL;
+  }
+  if (row_off) row_off[world] = next_lo;
+  return GDR_OK;
+}
+
 }  // namespace gdr
 
 
@@ -275,11 +322,19 @@ int gdr_comm_init(gdr_comm_t** comm_out, const void* id128_host, int rank, int w
   c->rank = rank;
   c->world = world;
   c->nccl = nullptr;
+  c->entry = nullptr;
   GDR_CUDA(cudaGetDevice(&c->device));
+  cudaError_t e = cudaMalloc((void**)&c->entry, (size_t)world * kEntryWords * 8);
+  if (e != cudaSuccess) {
+    set_error("comm_init: cudaMalloc of the entry-check buffer -> %s", cudaGetErrorString(e));
+    cudaGetLastError();
+    delete c;
+    return GDR_ECUDA;
+  }
   if (world > 1) {
     const NcclApi* api = nccl_api();
     if (!api || !id128_host) {
-      delete c;
+      gdr_comm_destroy(c);
       if (api) set_error("comm_init: null unique id");
       return api ? GDR_EINVAL : GDR_ECUDA;
     }
@@ -288,7 +343,8 @@ int gdr_comm_init(gdr_comm_t** comm_out, const void* id128_host, int rank, int w
     ncclResult_t r = api->CommInitRank(&c->nccl, world, id, rank);
     if (r != ncclSuccess) {
       set_error("ncclCommInitRank -> %s", api->GetErrorString(r));
-      delete c;
+      c->nccl = nullptr;
+      gdr_comm_destroy(c);
       return GDR_ECUDA;
     }
   }
@@ -302,6 +358,7 @@ int gdr_comm_destroy(gdr_comm_t* comm) {
     const NcclApi* api = nccl_api();
     if (api) api->CommDestroy(comm->nccl);
   }
+  cudaFree(comm->entry);
   delete comm;
   return GDR_OK;
 }

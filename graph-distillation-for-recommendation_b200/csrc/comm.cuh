@@ -1,13 +1,15 @@
-// comm.cuh — internal view of the communicator (comm.cu) for the distributed drivers (lloyd.cu).
+// comm.cuh — internal view of the communicator (comm.cu) for the distributed drivers.
 #pragma once
 #include <cuda_runtime.h>
 #include <nccl.h>   // types and prototypes only: the functions are bound at run time (dlopen), never linked
 #include <stdint.h>
+#include <initializer_list>
 #include "common.cuh"
 
 struct gdr_comm {
   ncclComm_t nccl;
   int rank, world, device;
+  int64_t* entry;   // [world][gdr::kEntryWords] gather buffer of gdr::comm_entry_check
 };
 
 // Symmetric buffer: the same allocation on every rank of the communicator, each rank holding peer-mapped (CUDA IPC over
@@ -51,5 +53,16 @@ int comm_send(gdr_comm* c, const void* buf, int64_t bytes, int peer, cudaStream_
 int comm_recv(gdr_comm* c, void* buf, int64_t bytes, int peer, cudaStream_t s);
 // buf of rank `root` -> buf of every other rank, as one group of sends (no-op for world 1 / null comm)
 int comm_broadcast(gdr_comm* c, void* buf, int64_t bytes, int root, cudaStream_t s);
+
+// The collective entry check of the row-partitioned entry points (return codes: gdr.h, next to gdr_comm_init).  Every
+// rank passes its verdict local_rc, its row block [row_lo, row_lo + n_local) (row_lo < 0 on every rank: the blocks
+// follow one another by construction), the words every rank must pass alike (agreed_names names them in the message),
+// one word `extra` the caller wants back from every rank, and n_global >= 0 when the blocks must cover n_global rows.
+// On GDR_OK, row_off[0..world] (optional) = every rank's first global row and the total, extras[0..world) (optional) =
+// every rank's extra word.  One H2D copy, one all-gather into c->entry, one read-back and a stream synchronisation.
+constexpr int kEntryAgreed = 8, kEntryWords = 4 + kEntryAgreed;
+int comm_entry_check(gdr_comm* c, cudaStream_t s, const char* call, int local_rc, int64_t row_lo, int64_t n_local,
+                     int64_t n_global, std::initializer_list<int64_t> agreed, const char* agreed_names,
+                     int64_t extra = 0, int64_t* row_off = nullptr, int64_t* extras = nullptr);
 
 }  // namespace gdr

@@ -14,7 +14,6 @@
 // uses an fp32 cumsum, so a draw that lands within rounding of a boundary may pick a neighbour.
 #include "common.cuh"
 #include "comm.cuh"
-#include <vector>
 
 namespace gdr {
 
@@ -463,7 +462,6 @@ using namespace gdr;
 namespace {
 
 struct PpdBuffers {
-  int64_t* meta;     // [world][8]     entry check (first in the workspace: see gdr_kmeans_plusplus_dist)
   float* dcol;       // [2][Lmax][N]   candidate columns of the last two passes
   double* bpot;      // [2][Lmax][nb]  their block sums
   double* bprefix;   // [nb + 1]
@@ -479,7 +477,6 @@ PpdBuffers ppd_carve(void* ws, int64_t N, int64_t K, int64_t D, int Lmax, int wo
   Workspace W(ws, INT64_MAX);
   PpdBuffers b;
   b.slot = align_up(Lmax * 8 + (Lmax + 1) * D * 4, 16);
-  b.meta = W.take<int64_t>(world * 8);
   b.dcol = W.take<float>(2 * Lmax * n);
   b.bpot = W.take<double>(2 * Lmax * nb);
   b.bprefix = W.take<double>(nb + 1);
@@ -578,7 +575,7 @@ int gdr_kmeans_plusplus_dist(gdr_comm_t* comm, int64_t N_local, int64_t K, int64
   GDR_CHECK_ARG(comm, "kmeans_plusplus_dist: null communicator");
   const int world = comm->world, rank = comm->rank;
   cudaStream_t caller = (cudaStream_t)stream;
-  // local checks are decided collectively below: a rank that returned early would leave the others in a collective
+  // local checks are decided collectively in comm_entry_check: an early return would leave the others in a collective
   int local_rc = GDR_OK;
   const size_t smem_score = (size_t)n_trials * D * 4;
   if (!(N_local >= 0 && K > 0 && D > 0 && centers_out && ws && (N_local == 0 || X_local) && ldx >= D && ldc >= D &&
@@ -598,50 +595,17 @@ int gdr_kmeans_plusplus_dist(gdr_comm_t* comm, int64_t N_local, int64_t K, int64
     set_error("kmeans_plusplus_dist: workspace too small");
     local_rc = GDR_EWORKSPACE;
   }
-  // entry check: every rank must pass the same first centre, n_trials, K, D and random numbers
   const uint64_t sum = (local_rc == GDR_OK && K > 1) ? fnv1a(rand_vals_host, (size_t)(K - 1) * n_trials * 8) : 0;
-  int64_t mine[8] = {N_local, first_center, n_trials, (int64_t)sum, K, D, local_rc, 0};
-  std::vector<int64_t> all((size_t)world * 8);
-  // the gather buffer is the head of the workspace; a rank whose workspace cannot hold it still takes part in the
-  // check (through a temporary buffer: a rejected call only) so that every rank learns the verdict
-  const int64_t meta_bytes = (int64_t)all.size() * 8;
-  int64_t* meta = ws && ws_bytes >= meta_bytes ? (int64_t*)ws : nullptr;   // ppd_carve's first block
-  int64_t* meta_tmp = nullptr;
-  if (!meta) {
-    GDR_CUDA(cudaMalloc(&meta_tmp, meta_bytes));
-    meta = meta_tmp;
-  }
-  int rc = GDR_OK;
-  if (cudaMemcpyAsync(meta + rank * 8, mine, 64, cudaMemcpyHostToDevice, caller) != cudaSuccess) {
-    set_error("kmeans_plusplus_dist: copy of the argument check failed");
-    rc = GDR_ECUDA;
-  }
-  if (rc == GDR_OK) rc = comm_allgather(comm, meta + rank * 8, meta, 64, caller);
-  if (rc == GDR_OK && (cudaMemcpyAsync(all.data(), meta, meta_bytes, cudaMemcpyDeviceToHost, caller) != cudaSuccess ||
-                       cudaStreamSynchronize(caller) != cudaSuccess)) {
-    set_error("kmeans_plusplus_dist: read-back of the argument check failed");
-    rc = GDR_ECUDA;
-  }
-  if (meta_tmp) cudaFree(meta_tmp);
-  if (rc != GDR_OK) return rc;
-  if (local_rc != GDR_OK) return local_rc;
   PpdState init = {};
+  int rc = comm_entry_check(comm, caller, "kmeans_plusplus_dist", local_rc, -1, N_local, -1,
+                            {first_center, n_trials, (int64_t)sum, K, D}, "first centre, n_trials, K, D or random numbers",
+                            0, init.off);
+  if (rc != GDR_OK) return rc;
   init.world = world;
   init.rank = rank;
   init.last = 0;
-  for (int r = 0; r < world; ++r) {
-    const int64_t* m = &all[(size_t)r * 8];
-    if (m[6] != GDR_OK) {
-      set_error("kmeans_plusplus_dist: rank %d rejected its arguments", r);
-      return GDR_EINVAL;
-    }
-    if (m[1] != mine[1] || m[2] != mine[2] || m[3] != mine[3] || m[4] != mine[4] || m[5] != mine[5]) {
-      set_error("kmeans_plusplus_dist: rank %d passed a different first centre, n_trials, K, D or random numbers", r);
-      return GDR_EINVAL;
-    }
-    init.off[r + 1] = init.off[r] + m[0];
-    if (m[0] > 0) init.last = r;
-  }
+  for (int r = 0; r < world; ++r)
+    if (init.off[r + 1] > init.off[r]) init.last = r;
   const int64_t N_total = init.off[world];
   init.n_total = N_total;
   GDR_CHECK_ARG(K <= N_total, "kmeans_plusplus_dist: n_samples=%lld should be >= n_clusters=%lld", (long long)N_total,

@@ -401,10 +401,7 @@ using namespace gdr;
 
 namespace {
 
-constexpr int kSpdMeta = 10;   // int64 words per rank in the entry check of gdr_sparsify_classes_dist
-
 struct SpdBuffers {
-  int64_t* meta;     // [world][kSpdMeta]  entry check (first in the workspace: see gdr_sparsify_classes_dist)
   float* w;          // [bmax][nnz]        class weights of the batch
   int32_t* a;        // [bmax][nnz + 1]    tie flags -> their local ranks
   int32_t* b;        // [bmax][nnz + 1]    selection flags -> output positions
@@ -420,7 +417,6 @@ struct SpdBuffers {
 SpdBuffers spd_carve(void* ws, int64_t nnz, int64_t bmax, int world) {
   Workspace W(ws, INT64_MAX);
   SpdBuffers B;
-  B.meta = W.take<int64_t>((int64_t)world * kSpdMeta);
   B.w = W.take<float>(bmax * nnz);
   B.a = W.take<int32_t>(bmax * (nnz + 1) + 1);
   B.b = W.take<int32_t>(bmax * (nnz + 1) + 1);
@@ -702,7 +698,7 @@ int gdr_sparsify_classes_dist(gdr_comm_t* comm, int64_t n_local, int64_t nnz, in
   GDR_CHECK_ARG(comm, "sparsify_classes_dist: null communicator");
   const int world = comm->world, rank = comm->rank;
   cudaStream_t s = (cudaStream_t)stream;
-  // local checks are decided collectively below: a rank that returned early would leave the others in a collective
+  // local checks are decided collectively in comm_entry_check: an early return would leave the others in a collective
   int local_rc = GDR_OK;
   if (!(n_local >= 0 && nnz >= 0 && row_lo >= 0 && C > 0 && k >= 0 && (prob ? C <= ldp : C == 1) &&
         rowptr_out && nnz_out_dev && ws && (n_local == 0 || rowptr) &&
@@ -716,53 +712,16 @@ int gdr_sparsify_classes_dist(gdr_comm_t* comm, int64_t n_local, int64_t nnz, in
     set_error("sparsify_classes_dist: workspace too small");
     local_rc = GDR_EWORKSPACE;
   }
-  // entry check: the same C, k, n_global, prob presence and batch cap everywhere; blocks contiguous in rank order
-  int64_t mine[kSpdMeta] = {C, k, n_global, row_lo, n_local, nnz, local_rc, prob != nullptr, g_sparsify_batch_cap, 0};
-  std::vector<int64_t> all((size_t)world * kSpdMeta);
-  const int64_t meta_bytes = (int64_t)all.size() * 8;
-  // the gather buffer is the head of the workspace; a rank whose workspace cannot hold it still takes part in the
-  // check (through a temporary buffer: a rejected call only) so that every rank learns the verdict
-  int64_t* meta = ws && ws_bytes >= meta_bytes ? (int64_t*)ws : nullptr;   // spd_carve's first block
-  int64_t* meta_tmp = nullptr;
-  if (!meta) {
-    GDR_CUDA(cudaMalloc(&meta_tmp, meta_bytes));
-    meta = meta_tmp;
-  }
-  int rc = GDR_OK;
-  if (cudaMemcpyAsync(meta + rank * kSpdMeta, mine, sizeof(mine), cudaMemcpyHostToDevice, s) != cudaSuccess) {
-    set_error("sparsify_classes_dist: copy of the argument check failed");
-    rc = GDR_ECUDA;
-  }
-  if (rc == GDR_OK) rc = comm_allgather(comm, meta + rank * kSpdMeta, meta, sizeof(mine), s);
-  if (rc == GDR_OK && (cudaMemcpyAsync(all.data(), meta, meta_bytes, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-                       cudaStreamSynchronize(s) != cudaSuccess)) {
-    set_error("sparsify_classes_dist: read-back of the argument check failed");
-    rc = GDR_ECUDA;
-  }
-  if (meta_tmp) cudaFree(meta_tmp);
+  std::vector<int64_t> nnz_of((size_t)world);
+  int rc = comm_entry_check(comm, s, "sparsify_classes_dist", local_rc, row_lo, n_local, n_global,
+                            {C, k, n_global, prob != nullptr, g_sparsify_batch_cap}, "C, k, n_global, prob or batch cap",
+                            nnz, nullptr, nnz_of.data());
   if (rc != GDR_OK) return rc;
-  if (local_rc != GDR_OK) return local_rc;
-  int64_t next_lo = 0, nnz_global = 0, nnz_max = 0;
-  for (int r = 0; r < world; ++r) {
-    const int64_t* m = &all[(size_t)r * kSpdMeta];
-    if (m[6] != GDR_OK) {
-      set_error("sparsify_classes_dist: rank %d rejected its arguments", r);
-      return GDR_EINVAL;
-    }
-    if (m[0] != C || m[1] != k || m[2] != n_global || m[7] != mine[7] || m[8] != mine[8]) {
-      set_error("sparsify_classes_dist: rank %d passed a different C, k, n_global, prob or batch cap", r);
-      return GDR_EINVAL;
-    }
-    if (m[3] != next_lo) {
-      set_error("sparsify_classes_dist: the row block of rank %d does not follow the previous rank's", r);
-      return GDR_EINVAL;
-    }
-    next_lo += m[4];
-    nnz_global += m[5];
-    nnz_max = std::max(nnz_max, m[5]);
+  int64_t nnz_global = 0, nnz_max = 0;
+  for (int64_t m : nnz_of) {
+    nnz_global += m;
+    nnz_max = std::max(nnz_max, m);
   }
-  GDR_CHECK_ARG(next_lo == n_global, "sparsify_classes_dist: the row blocks hold %lld rows, n_global is %lld",
-                (long long)next_lo, (long long)n_global);
   GDR_CHECK_ARG(k <= nnz_global, "sparsify_classes_dist: k = %lld exceeds the %lld stored entries", (long long)k,
                 (long long)nnz_global);
 

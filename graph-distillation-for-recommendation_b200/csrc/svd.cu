@@ -13,7 +13,6 @@
 #include "common.cuh"
 #include "comm.cuh"
 #include <algorithm>
-#include <vector>
 
 namespace gdr {
 
@@ -400,16 +399,14 @@ using namespace gdr;
 namespace {
 
 struct GramDistBuffers {
-  int64_t* meta;   // [world][8]  entry check (first in the workspace: see gdr_dense_gram_dist)
   double* part;    // [slabs][p][r] partials of the slabs that end on this rank, in slab order
   double* x;       // [4][p][r]  carry in, running sum in | carry out, running sum out
   int64_t off;
 };
 
-GramDistBuffers gram_dist_carve(void* ws, int64_t N, int64_t p, int64_t r, int world) {
+GramDistBuffers gram_dist_carve(void* ws, int64_t N, int64_t p, int64_t r) {
   Workspace W(ws, INT64_MAX);
   GramDistBuffers b;
-  b.meta = W.take<int64_t>((int64_t)world * 8);
   b.part = W.take<double>(gram_slabs(N) * p * r);
   b.x = W.take<double>(4 * p * r);
   b.off = W.off + 256;
@@ -444,7 +441,8 @@ int gdr_dense_gram(int64_t N, int64_t p, int64_t r, const double* A, int64_t lda
 }
 
 int64_t gdr_dense_gram_dist_ws_bytes(int64_t N_global, int64_t p, int64_t r, int world) {
-  return gram_dist_carve(nullptr, N_global, p, r, world).off;
+  (void)world;
+  return gram_dist_carve(nullptr, N_global, p, r).off;
 }
 
 int gdr_dense_gram_dist(gdr_comm_t* comm, int64_t N_global, int64_t row_lo, int64_t n_local, int64_t p, int64_t r,
@@ -453,7 +451,7 @@ int gdr_dense_gram_dist(gdr_comm_t* comm, int64_t N_global, int64_t row_lo, int6
   GDR_CHECK_ARG(comm, "dense_gram_dist: null communicator");
   const int world = comm->world, rank = comm->rank;
   cudaStream_t s = (cudaStream_t)stream;
-  // local checks are decided collectively below: a rank that returned early would leave the others in a collective
+  // local checks are decided collectively in comm_entry_check: an early return would leave the others in a collective
   int local_rc = GDR_OK;
   if (!(N_global >= 0 && row_lo >= 0 && n_local >= 0 && row_lo + n_local <= N_global && p > 0 && r > 0 && C && ldc >= r &&
         ws && (n_local == 0 || (A && B && lda >= p && ldb >= r)))) {
@@ -463,56 +461,14 @@ int gdr_dense_gram_dist(gdr_comm_t* comm, int64_t N_global, int64_t row_lo, int6
     set_error("dense_gram_dist: workspace too small");
     local_rc = GDR_EWORKSPACE;
   }
-  // entry check: the same N_global, p and r everywhere, row blocks contiguous in rank order and covering N_global
-  int64_t mine[8] = {N_global, row_lo, n_local, p, r, local_rc, 0, 0};
-  std::vector<int64_t> all((size_t)world * 8);
-  const int64_t meta_bytes = (int64_t)all.size() * 8;
-  // the gather buffer is the head of the workspace; a rank whose workspace cannot hold it still takes part in the
-  // check (through a temporary buffer: a rejected call only) so that every rank learns the verdict
-  int64_t* meta = ws && ws_bytes >= meta_bytes ? (int64_t*)ws : nullptr;
-  int64_t* meta_tmp = nullptr;
-  if (!meta) {
-    GDR_CUDA(cudaMalloc(&meta_tmp, meta_bytes));
-    meta = meta_tmp;
-  }
-  int rc = GDR_OK;
-  if (cudaMemcpyAsync(meta + rank * 8, mine, 64, cudaMemcpyHostToDevice, s) != cudaSuccess) {
-    set_error("dense_gram_dist: copy of the argument check failed");
-    rc = GDR_ECUDA;
-  }
-  if (rc == GDR_OK) rc = comm_allgather(comm, meta + rank * 8, meta, 64, s);
-  if (rc == GDR_OK && (cudaMemcpyAsync(all.data(), meta, meta_bytes, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
-                       cudaStreamSynchronize(s) != cudaSuccess)) {
-    set_error("dense_gram_dist: read-back of the argument check failed");
-    rc = GDR_ECUDA;
-  }
-  if (meta_tmp) cudaFree(meta_tmp);
+  int rc = comm_entry_check(comm, s, "dense_gram_dist", local_rc, row_lo, n_local, N_global, {N_global, p, r},
+                            "N_global, p or r");
   if (rc != GDR_OK) return rc;
-  if (local_rc != GDR_OK) return local_rc;
-  int64_t next_lo = 0;
-  for (int q = 0; q < world; ++q) {
-    const int64_t* m = &all[(size_t)q * 8];
-    if (m[5] != GDR_OK) {
-      set_error("dense_gram_dist: rank %d rejected its arguments", q);
-      return GDR_EINVAL;
-    }
-    if (m[0] != N_global || m[3] != p || m[4] != r) {
-      set_error("dense_gram_dist: rank %d passed a different N_global, p or r", q);
-      return GDR_EINVAL;
-    }
-    if (m[1] != next_lo) {
-      set_error("dense_gram_dist: the row block of rank %d does not follow the one of rank %d", q, q - 1);
-      return GDR_EINVAL;
-    }
-    next_lo += m[2];
-  }
-  GDR_CHECK_ARG(next_lo == N_global, "dense_gram_dist: the row blocks hold %lld rows, not N_global = %lld",
-                (long long)next_lo, (long long)N_global);   // the same verdict on every rank
 
   // this rank's rows cut at the global slab boundaries (gdr_dense_gram's geometry): the segments that start their slab
   // need nothing from the previous rank; at most one, the first, continues the carry of a slab begun on an earlier rank
   const int64_t pr = p * r, rows_per = cdiv(N_global, gram_slabs(N_global));
-  GramDistBuffers G = gram_dist_carve(ws, N_global, p, r, world);
+  GramDistBuffers G = gram_dist_carve(ws, N_global, p, r);
   double *carry_in = G.x, *sum_in = G.x + pr, *carry_out = G.x + 2 * pr, *sum_out = G.x + 3 * pr;
   GramSegs starts = {}, cont = {};
   int n_starts = 0, n_cont = 0, n_done = 0;

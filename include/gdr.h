@@ -496,7 +496,15 @@ int gdr_class_edge_weight(int64_t n, int64_t nnz, const int32_t* rowptr, const i
  * these entry points replace nothing in it: they are the exchanges a row partition of the same path needs.
  * NCCL is bound at run time (dlopen of the already mapped libnccl.so.2, else the system copy / $GDR_NCCL_LIB).
  * Protocol: rank 0 calls gdr_comm_unique_id, the host framework broadcasts the 128 bytes, every rank calls
- * gdr_comm_init (collective).  All exchange calls are collective and are enqueued on `stream`. */
+ * gdr_comm_init (collective).  All exchange calls are collective and are enqueued on `stream`.
+ * Collective entry check of the row-partitioned entry points (gdr_kmeans_plusplus_dist, gdr_dense_gram_dist,
+ * gdr_sparsify_classes_dist): a rank does not return on its own argument checks.  Every rank all-gathers its verdict,
+ * its row block and the values every rank must pass alike (listed with each entry point) through a small buffer the
+ * communicator owns (allocated by gdr_comm_init), reads them back and synchronises the stream once.  A rank whose own
+ * arguments are rejected returns its own code (GDR_EINVAL, GDR_EWORKSPACE, GDR_EUNSUPPORTED, GDR_ERANGE), every other
+ * rank GDR_EINVAL.  Values that differ between ranks, a row block that does not start where the previous rank's ends,
+ * or blocks that do not cover the global row count return GDR_EINVAL on every rank.  A failure of the exchange itself
+ * returns GDR_ECUDA.  After any rejection the communicator stays usable. */
 typedef struct gdr_comm gdr_comm_t;
 int gdr_comm_unique_id(void* id128_host);
 int gdr_comm_init(gdr_comm_t** comm_out, const void* id128_host, int rank, int world);
@@ -519,10 +527,11 @@ int gdr_alltoallv(gdr_comm_t* comm, const void* send, const int64_t* send_off_ho
                   void* recv, const int64_t* recv_off_host, const int64_t* recv_cnt_host, int64_t elem_bytes,
                   gdr_stream_t stream);
 /* Symmetric buffers: the same device allocation on every rank, mapped into every peer over NVLink (CUDA IPC), so that a
- * kernel can store straight into the other GPUs' copies.  gdr_symm_create / _destroy are collective (and the only entry
- * points of this library that allocate device memory).  gdr_symm_barrier is stream-ordered: when it completes on a rank,
- * everything every rank enqueued before ITS barrier call — including its stores into this rank's copy — is done and
- * visible.  gdr_symm_put_rows: rows of `src` -> offset dst_offset_bytes of every copy (one read, world posted stores).
+ * kernel can store straight into the other GPUs' copies.  gdr_symm_create / _destroy are collective (and, with
+ * gdr_comm_init's entry-check buffer, the only entry points of this library that allocate device memory).
+ * gdr_symm_barrier is stream-ordered: when it completes on a rank, everything every rank enqueued before ITS barrier
+ * call — including its stores into this rank's copy — is done and visible.  gdr_symm_put_rows: rows of `src` ->
+ * offset dst_offset_bytes of every copy (one read, world posted stores).
  * gdr_symm_scatterv: the variable all-to-all / all-gather of stages 1 and 4 without NCCL — block p of `send`
  * (send_cnt_host[p] elements of elem_bytes at element send_off_host[p]) is stored at BYTE offset dst_off_bytes_host[p]
  * of rank p's copy (its own included), one kernel, 16-byte posted NVLink stores; bracket it with gdr_symm_barrier.
@@ -625,10 +634,10 @@ int gdr_kmeans_lloyd_dist(gdr_comm_t* comm, int64_t N_local, int64_t N_total, in
 /* gdr_kmeans_plusplus on a row partition: the same greedy D^2 seeding without gathering X.  COLLECTIVE over comm.
  * X_local = this rank's N_local rows (N_local = 0 allowed); the ranks' blocks in rank order are the global row order
  * (the call all-gathers N_local once and derives every rank's row offset and N_total).  first_center and
- * indices_out_dev hold global row ids.  Every rank passes the same first_center, n_trials, K, D and host draws
- * (rand_vals_host as for gdr_kmeans_plusplus); this is checked at entry and a mismatch, or an argument any rank
- * rejects, returns GDR_EINVAL on every rank.  Same checks as gdr_kmeans_plusplus: n_trials <= 16, K <= N_total, and
- * the shared-memory plan for n_trials * D.  centers_out [K][ldc] (device) comes out bit-identical on every rank.
+ * indices_out_dev hold global row ids.  Collective entry check (see gdr_comm_init) on first_center, n_trials, K, D and
+ * a checksum of the host draws (rand_vals_host as for gdr_kmeans_plusplus).  Same checks as gdr_kmeans_plusplus:
+ * n_trials <= 16, K <= N_total, and the shared-memory plan for n_trials * D.  centers_out [K][ldc] (device) comes out
+ * bit-identical on every rank.
  * Per round: the owner of each draw (first rank with rows whose prefix P_r + T_r reaches u * pot) finds the row with
  * gdr_kmeans_plusplus's search and publishes it (all-gather A; the rows are copied, never summed); one pass over
  * X_local scores all candidates; each rank's fp64 totals per candidate are all-gathered (B) and added in rank order.
@@ -664,9 +673,9 @@ int     gdr_dense_gram(int64_t N, int64_t p, int64_t r, const double* A, int64_t
  * exact accumulators (the carry) handed on by the previous rank when the slab began there, and adds the slabs that end
  * on it to the slab-order running sum it receives (0.0 on rank 0).  Rank q sends rank q + 1 the carry and the running
  * sum (2 p r doubles, NCCL point-to-point); the last rank's sum is C and is sent to all.  Slabs that start on a rank
- * are summed before it receives anything.  At entry every rank all-gathers N_global, row_lo, n_local, p, r and its
- * argument verdict; a mismatch, blocks that are not contiguous in rank order or do not cover N_global, or an argument
- * any rank rejects returns GDR_EINVAL on every rank.  Synchronises the stream once, after the entry check. */
+ * are summed before it receives anything.  Collective entry check (see gdr_comm_init) on N_global, p and r; the row
+ * blocks must cover N_global.  Synchronises the stream once, after the entry check.  The `world` argument of
+ * gdr_dense_gram_dist_ws_bytes is unused (the workspace does not depend on the rank count); it stays for the ABI. */
 int64_t gdr_dense_gram_dist_ws_bytes(int64_t N_global, int64_t p, int64_t r, int world);
 int     gdr_dense_gram_dist(gdr_comm_t* comm, int64_t N_global, int64_t row_lo, int64_t n_local, int64_t p, int64_t r,
                             const double* A, int64_t lda, const double* B, int64_t ldb, double* C, int64_t ldc,
@@ -709,11 +718,10 @@ int     gdr_sparsify_classes(int64_t n, int64_t nnz, int64_t C, const int32_t* r
  * any number of ranks: the row blocks in rank order are the global stored order, each radix pass sums the ranks'
  * histograms (64-bit counts, one all-reduce per pass and class batch), and the ties at the threshold are shared out
  * in rank order (one all-gather of the per-rank tie counts per batch): rank p keeps its first
- * clamp(k_rem - sum_{q<p} ties_q, 0, ties_p).  At entry every rank all-gathers C, k, n_global, row_lo, n_local, nnz,
- * whether prob is given, the "sparsify_batch" cap and its argument verdict; a mismatch, blocks that are not contiguous
- * in rank order, or an argument any rank rejects returns GDR_EINVAL on every rank.  The class batch is sized from the
- * largest local nnz.  The local nnz keeps the int32 CSR limit (GDR_ERANGE).  Synchronises the stream once, after the
- * entry check. */
+ * clamp(k_rem - sum_{q<p} ties_q, 0, ties_p).  Collective entry check (see gdr_comm_init) on C, k, n_global, whether
+ * prob is given and the "sparsify_batch" cap; the row blocks must cover n_global, and it also gathers every rank's
+ * local nnz.  The class batch is sized from the largest local nnz.  The local nnz keeps the int32 CSR limit
+ * (GDR_ERANGE).  Synchronises the stream once, after the entry check. */
 int64_t gdr_sparsify_classes_dist_ws_bytes(int64_t n_local, int64_t nnz_local, int64_t C, int world);
 int     gdr_sparsify_classes_dist(gdr_comm_t* comm, int64_t n_local, int64_t nnz_local, int64_t row_lo,
                                   int64_t n_global, int64_t C, const int32_t* rowptr, const int32_t* colidx,
