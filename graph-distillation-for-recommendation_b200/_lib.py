@@ -108,6 +108,8 @@ _SIGNATURES = {
     "gdr_allreduce_centroids": (i32, [vp, vp, i64, vp, i64, vp]),
     "gdr_allreduce_f64": (i32, [vp, vp, i64, i32, vp]),
     "gdr_alltoallv": (i32, [vp, vp, vp, vp, vp, vp, vp, i64, vp]),
+    "gdr_minibatch_batch_dist_ws_bytes": (i64, [i64, i64, i64, i32]),
+    "gdr_minibatch_batch_dist": (i32, [vp, i64, vp, vp, vp, i64, i64, i64, i64, vp, i64, vp, i64, vp, i64, vp, vp, i64, vp]),
     "gdr_symm_create": (i32, [vp, i64, vp]),
     "gdr_symm_destroy": (i32, [vp]),
     "gdr_symm_info": (i32, [vp, vp, vp]),

@@ -157,6 +157,33 @@ int comm_broadcast(gdr_comm* c, void* buf, int64_t bytes, int root, cudaStream_t
   return GDR_OK;
 }
 
+int comm_allgatherv_inplace(gdr_comm* c, int n_bufs, void* const* bufs, const int64_t* row_bytes, const int64_t* counts,
+                            cudaStream_t s) {
+  if (!c || c->world == 1) return GDR_OK;
+  const NcclApi* api = nccl_api();
+  if (!api) return GDR_ECUDA;
+  const int me = c->rank;
+  int64_t off_me = 0;
+  for (int p = 0; p < me; ++p) off_me += counts[p];
+  GDR_NCCL(api->GroupStart());
+  int64_t off = 0;
+  for (int p = 0; p < c->world; ++p) {
+    if (p != me) {
+      for (int a = 0; a < n_bufs; ++a) {
+        char* b = (char*)bufs[a];
+        if (counts[me] > 0)
+          GDR_NCCL(api->Send(b + off_me * row_bytes[a], (size_t)(counts[me] * row_bytes[a]), ncclInt8, p, c->nccl, s));
+        if (counts[p] > 0)
+          GDR_NCCL(api->Recv(b + off * row_bytes[a], (size_t)(counts[p] * row_bytes[a]), ncclInt8, p, c->nccl, s));
+      }
+    }
+    off += counts[p];
+  }
+  GDR_NCCL(api->GroupEnd());
+  count_launch(1);
+  return GDR_OK;
+}
+
 int comm_entry_check(gdr_comm* c, cudaStream_t s, const char* call, int local_rc, int64_t row_lo, int64_t n_local,
                      int64_t n_global, std::initializer_list<int64_t> agreed, const char* agreed_names, int64_t extra,
                      int64_t* row_off, int64_t* extras) {

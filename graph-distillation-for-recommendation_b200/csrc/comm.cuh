@@ -53,6 +53,11 @@ int comm_send(gdr_comm* c, const void* buf, int64_t bytes, int peer, cudaStream_
 int comm_recv(gdr_comm* c, void* buf, int64_t bytes, int peer, cudaStream_t s);
 // buf of rank `root` -> buf of every other rank, as one group of sends (no-op for world 1 / null comm)
 int comm_broadcast(gdr_comm* c, void* buf, int64_t bytes, int root, cudaStream_t s);
+// In-place variable all-gather of n_bufs arrays that share one row split: rows [off_p, off_p + counts[p]) of bufs[a]
+// (row_bytes[a] bytes each, off_p = counts[0] + ... + counts[p-1]) go from rank p to the same rows of every other rank,
+// as ONE group of NCCL sends and receives (no-op for world 1 / null comm).
+int comm_allgatherv_inplace(gdr_comm* c, int n_bufs, void* const* bufs, const int64_t* row_bytes, const int64_t* counts,
+                            cudaStream_t s);
 
 // The collective entry check of the row-partitioned entry points (return codes: gdr.h, next to gdr_comm_init).  Every
 // rank passes its verdict local_rc, its row block [row_lo, row_lo + n_local) (row_lo < 0 on every rank: the blocks

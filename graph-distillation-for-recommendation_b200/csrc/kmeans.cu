@@ -11,6 +11,7 @@
 // re-scoring kernel of the tensor-core path in kmeans_tc.cu), the deterministic
 // M-step and the small reductions around them.
 #include "common.cuh"
+#include "comm.cuh"
 #include <vector>
 
 namespace gdr {
@@ -758,6 +759,32 @@ __global__ void __launch_bounds__(256) k_minibatch_update(int64_t B, int64_t K, 
   }
 }
 
+// ---- MiniBatchKMeans batch assembly on a row partition (gdr_minibatch_batch_dist) -----------------------------
+// pack: the n batch positions this rank owns (order[0..n), batch order) -> rows of the compact buffer P [n][ldp],
+// padding columns zero.  One warp per row.  A position whose row lies outside [row_lo, row_lo + n_local) (a plan that
+// does not match the row blocks) packs a zero row instead of reading outside X.
+__global__ void __launch_bounds__(256) k_mb_pack(int64_t n, int D, int ldp, const int64_t* __restrict__ idx,
+                                                 const int32_t* __restrict__ order, int64_t row_lo, int64_t n_local,
+                                                 const float* __restrict__ X, int64_t ldx, float* __restrict__ P) {
+  const int64_t r = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (r >= n) return;
+  const int64_t g = idx[order[r]] - row_lo;
+  const bool own = g >= 0 && g < n_local;
+  for (int c = lane_id(); c < ldp; c += 32) P[r * ldp + c] = (own && c < D) ? X[g * ldx + c] : 0.f;
+}
+
+// place: record k of the exchanged buffers (every rank's compact rows in rank order = the order of `order`) -> batch
+// position order[k]: Xb row (ldb columns, zero beyond ldp) and, when labels travel, its label.  One warp per record.
+__global__ void __launch_bounds__(256) k_mb_place(int64_t m, int ldp, const int32_t* __restrict__ order,
+                                                  const float* __restrict__ P, const int32_t* __restrict__ Lp,
+                                                  float* __restrict__ Xb, int64_t ldb, int32_t* __restrict__ labels_b) {
+  const int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (k >= m) return;
+  const int64_t j = order[k];
+  for (int64_t c = lane_id(); c < ldb; c += 32) Xb[j * ldb + c] = c < ldp ? P[k * ldp + c] : 0.f;
+  if (labels_b && lane_id() == 0) labels_b[j] = Lp[k];
+}
+
 // ---- distributed relocation (lloyd.cu: relocate_distributed) ----------------------------------
 // candidate record: [dist, rank (int bits), old label (int bits), x[0..D)]
 __global__ void __launch_bounds__(256) k_pick_candidate(int nparts, const float* __restrict__ pv,
@@ -1311,6 +1338,70 @@ int gdr_minibatch_update(int64_t B, int64_t K, int64_t D, const float* Xb, int64
   GDR_CHECK_ARG(C_old != C_new, "minibatch_update: in-place update is not supported");
   k_minibatch_update<<<(unsigned)cdiv(K * 32, 256), 256, 0, (cudaStream_t)stream>>>(B, K, (int)D, Xb, ldx, labels, C_old,
                                                                                    ldc_old, C_new, ldc_new, weight_sums);
+  GDR_LAUNCHED();
+  return GDR_OK;
+}
+
+int64_t gdr_minibatch_batch_dist_ws_bytes(int64_t m, int64_t K, int64_t D, int world) {
+  (void)world;
+  const int64_t ldp = align_up(D > 0 ? D : 1, 4);
+  return ws_need(m * ldp, 4) + ws_need(m, 4) + ws_need(K > 0 ? K : 1, 4) + 256;
+}
+
+int gdr_minibatch_batch_dist(gdr_comm_t* comm, int64_t m, const int64_t* idx, const int32_t* order,
+                             const int64_t* counts_host, int64_t row_lo, int64_t n_local, int64_t K, int64_t D,
+                             const float* X_local, int64_t ldx, const float* C, int64_t ldc, float* Xb, int64_t ldb,
+                             int32_t* labels_b, void* ws, int64_t ws_bytes, gdr_stream_t stream) {
+  // every check is local and comes before the exchange; the caller agrees on the arguments once per fit
+  GDR_CHECK_ARG(comm && counts_host && m >= 0 && m < (1ll << 31) && D > 0 && D < (1 << 20),
+                "minibatch_batch_dist: bad arguments");
+  const int world = comm->world, me = comm->rank;
+  int64_t total = 0, off_me = 0;
+  for (int p = 0; p < world; ++p) {
+    GDR_CHECK_ARG(counts_host[p] >= 0, "minibatch_batch_dist: negative count for rank %d", p);
+    if (p < me) off_me += counts_host[p];
+    total += counts_host[p];
+  }
+  GDR_CHECK_ARG(total == m, "minibatch_batch_dist: the counts add up to %lld, not m = %lld", (long long)total,
+                (long long)m);
+  if (m == 0) return GDR_OK;
+  const int64_t n_me = counts_host[me];
+  GDR_CHECK_ARG(idx && order && Xb && ldb >= D, "minibatch_batch_dist: null idx / order / Xb or ldb < D");
+  GDR_CHECK_ARG(row_lo >= 0 && n_local >= 0 && (n_me == 0 || (X_local && ldx >= D)),
+                "minibatch_batch_dist: bad row block");
+  if (C) {
+    GDR_CHECK_ARG(labels_b && K > 0 && K < (1ll << 31) && ldc % 4 == 0 && ldc >= D && ((uintptr_t)C & 15) == 0,
+                  "minibatch_batch_dist: C needs labels_b, 0 < K < 2^31, 16B alignment and ldc %% 4 == 0, ldc >= D");
+  }
+  if (!ws || ws_bytes < gdr_minibatch_batch_dist_ws_bytes(m, K, D, world)) {
+    set_error("minibatch_batch_dist: workspace too small");
+    return GDR_EWORKSPACE;
+  }
+  cudaStream_t s = (cudaStream_t)stream;
+  const int ldp = (int)align_up(D, 4);
+  Workspace W(ws, ws_bytes);
+  float* P = W.take<float>(m * ldp);
+  int32_t* L = W.take<int32_t>(m);
+  float* cnorm = W.take<float>(K > 0 ? K : 1);
+  if (n_me > 0) {
+    k_mb_pack<<<(unsigned)cdiv(n_me * 32, 256), 256, 0, s>>>(n_me, (int)D, ldp, idx, order + off_me, row_lo, n_local,
+                                                            X_local, ldx, P + off_me * ldp);
+    GDR_LAUNCHED();
+    if (C) {
+      // the one-GPU E-step kernels (gdr_kmeans_assign, precision_mode 0) on the owned rows: k_assign_simt scans every
+      // centre for each row tile, so a row's label does not depend on the rows that share the launch
+      k_row_sqnorm<<<(unsigned)cdiv(K, 8), 256, 0, s>>>(K, (int)D, C, ldc, cnorm);
+      GDR_LAUNCHED();
+      k_assign_simt<<<(unsigned)cdiv(n_me, AS_BM), AS_THREADS, 0, s>>>(n_me, (int)K, (int)D, P + off_me * ldp, ldp, C,
+                                                                       ldc, cnorm, L + off_me, nullptr, nullptr,
+                                                                       nullptr, nullptr, nullptr);
+      GDR_LAUNCHED();
+    }
+  }
+  void* bufs[2] = {P, L};
+  const int64_t row_bytes[2] = {(int64_t)ldp * 4, 4};
+  if (int rc = comm_allgatherv_inplace(comm, C ? 2 : 1, bufs, row_bytes, counts_host, s)) return rc;
+  k_mb_place<<<(unsigned)cdiv(m * 32, 256), 256, 0, s>>>(m, ldp, order, P, L, Xb, ldb, C ? labels_b : nullptr);
   GDR_LAUNCHED();
   return GDR_OK;
 }

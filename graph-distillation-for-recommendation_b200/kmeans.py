@@ -398,21 +398,31 @@ class MiniBatchKMeans(KMeans):
     @staticmethod
     def _labels_inertia(Xp: torch.Tensor, C: torch.Tensor, labels: torch.Tensor, mode: int = 0, tc=None):
         assign_labels(Xp, C, labels, precision_mode=0, tc_operand=tc if mode == 1 else None)
+        return MiniBatchKMeans._inertia(Xp, C, labels)
+
+    @staticmethod
+    def _inertia(Xp: torch.Tensor, C: torch.Tensor, labels: torch.Tensor):
         out = torch.zeros(1, dtype=torch.float64, device=Xp.device)
         ws = workspace(_lib.query("gdr_inertia_ws_bytes", Xp.shape[0], Xp.shape[1]), Xp.device)
         _lib.call("gdr_inertia", Xp.shape[0], Xp.shape[1], ptr(Xp), Xp.stride(0), ptr(C), C.stride(0), ptr(labels), ptr(out),
                   ptr(ws), ws.numel(), stream())
         return out
 
-    def _mb_init(self, Xp: torch.Tensor, rs, init_size: int) -> torch.Tensor:
-        """_init_centroids (sklearn/_kmeans.py:985-1060) on an ``init_size`` random subset."""
-        N, D = Xp.shape
+    def _check_fit_args(self, N: int):
+        """The argument checks of fit that depend on the data only through N."""
         K = int(self.n_clusters)
-        Xi = Xp
-        if init_size is not None and init_size < N:
-            idx = torch.from_numpy(rs.randint(0, N, init_size).astype(np.int64)).to(Xp.device)
-            Xi = padded_rows(Xp[idx].contiguous())
-        C0 = new_padded(K, D, Xp.device, zero=True)
+        if K <= 0:
+            raise ValueError("n_clusters must be > 0")
+        if N < K:
+            raise ValueError(f"n_samples={N} should be >= n_clusters={K}.")
+        if self.reassignment_ratio < 0:
+            raise ValueError(f"reassignment_ratio should be >= 0, got {self.reassignment_ratio} instead.")
+
+    def _mb_init(self, rows, N: int, D: int, dev, rs, init_size: int) -> torch.Tensor:
+        """_init_centroids (sklearn/_kmeans.py:985-1060) on an ``init_size`` random subset (``rows``: see minibatch_loop)."""
+        K = int(self.n_clusters)
+        Xi = rows(rs.randint(0, N, init_size).astype(np.int64)) if init_size < N else rows(None)
+        C0 = new_padded(K, D, dev, zero=True)
         if isinstance(self.init, str):
             if self.init == "k-means++":
                 from .kmeans_init import kmeans_plusplus_device
@@ -420,7 +430,7 @@ class MiniBatchKMeans(KMeans):
             elif self.init == "random":
                 n_i = Xi.shape[0]
                 seeds = rs.choice(n_i, size=K, replace=False, p=np.ones(n_i, dtype=np.float32) / np.float32(n_i))
-                C0.copy_(Xi[torch.from_numpy(np.asarray(seeds, dtype=np.int64)).to(Xp.device)])
+                C0.copy_(Xi[torch.from_numpy(np.asarray(seeds, dtype=np.int64)).to(dev)])
             else:
                 raise ValueError(f"init should be 'k-means++', 'random' or an array, got {self.init!r}")
         else:
@@ -429,7 +439,7 @@ class MiniBatchKMeans(KMeans):
             if tuple(arr.shape) != (K, D):
                 raise ValueError(f"The shape of the initial centers {tuple(arr.shape)} does not match "
                                  f"the number of clusters {K} / features {D}.")
-            C0.copy_(arr.to(device=Xp.device, dtype=torch.float32))
+            C0.copy_(arr.to(device=dev, dtype=torch.float32))
         return C0
 
     def fit(self, X, y=None, sample_weight=None):
@@ -437,116 +447,29 @@ class MiniBatchKMeans(KMeans):
             raise NotImplementedError("sample_weight is not supported (the reference never passes it)")
         Xd = self._to_device(X)
         N, D = Xd.shape
-        K = int(self.n_clusters)
-        if K <= 0:
-            raise ValueError("n_clusters must be > 0")
-        if N < K:
-            raise ValueError(f"n_samples={N} should be >= n_clusters={K}.")
-        if self.reassignment_ratio < 0:
-            raise ValueError(f"reassignment_ratio should be >= 0, got {self.reassignment_ratio} instead.")
+        self._check_fit_args(N)
         dev = Xd.device
         rs = _check_random_state(self.random_state)
         Xp = padded_rows(Xd.contiguous())
-        batch = min(int(self.batch_size), N)
-        init_size = self.init_size
-        if init_size is None:
-            init_size = 3 * batch
-            if init_size < K:
-                init_size = 3 * K
-        elif init_size < K:
-            init_size = 3 * K
-        init_size = min(int(init_size), N)
-        init_is_array = not isinstance(self.init, str)
-        n_init = self.n_init
-        if n_init == "auto":
-            n_init = 1 if (init_is_array or self.init == "k-means++") else 3
-        if init_is_array:
-            n_init = 1
-        tol_abs = 0.0
-        if self.tol > 0:       # _tolerance (:285-293): mean of the column variances * tol
-            var_mean = torch.zeros(1, dtype=torch.float64, device=dev)
+
+        def rows(idx):
+            return Xp if idx is None else padded_rows(Xp[torch.from_numpy(idx).to(dev)].contiguous())
+
+        def assemble(idx, C, labels_b):
+            Xb = padded_rows(Xp[torch.from_numpy(idx).to(dev, non_blocking=True)].contiguous())
+            assign_labels(Xb, C, labels_b, precision_mode=0)
+            return Xb
+
+        def var_mean():
+            vm = torch.zeros(1, dtype=torch.float64, device=dev)
             mean = torch.empty(D, dtype=torch.float32, device=dev)
             scratch = new_padded(N, D, dev)
             ws = workspace(_lib.query("gdr_center_columns_ws_bytes", N, D), dev)
-            _lib.call("gdr_center_columns", N, D, ptr(Xp), Xp.stride(0), ptr(mean), ptr(var_mean), ptr(scratch), scratch.stride(0),
+            _lib.call("gdr_center_columns", N, D, ptr(Xp), Xp.stride(0), ptr(mean), ptr(vm), ptr(scratch), scratch.stride(0),
                       ptr(ws), ws.numel(), stream())
-            tol_abs = float(var_mean.item()) * float(self.tol)
-            del scratch
+            return float(vm.item())
 
-        # validation set for the initialisation (:2110-2112)
-        valid_idx = torch.from_numpy(rs.randint(0, N, init_size).astype(np.int64)).to(dev)
-        X_valid = padded_rows(Xp[valid_idx].contiguous())
-        lab_valid = torch.empty(X_valid.shape[0], dtype=torch.int32, device=dev)
-        best_inertia, centers = None, None
-        for _ in range(int(n_init)):
-            cand = self._mb_init(Xp, rs, init_size)
-            inertia = float(self._labels_inertia(X_valid, cand, lab_valid).item())
-            if best_inertia is None or inertia < best_inertia:
-                centers, best_inertia = cand, inertia
-        centers_new = new_padded(K, D, dev, zero=True)
-        counts = torch.zeros(K, dtype=torch.float32, device=dev)
-        ewa, ewa_min, no_improvement, n_since = None, None, 0, 0
-        n_steps = (int(self.max_iter) * N) // batch
-        # RandomState.choice(n, size, p=w / w.sum(), replace=True): cdf = p.cumsum(); cdf /= cdf[-1];
-        # cdf.searchsorted(random_sample(size), side="right") — the same table, built once
-        w32 = np.ones(N, dtype=np.float32)
-        cdf = (w32 / np.sum(w32)).astype(np.float64).cumsum()
-        cdf /= cdf[-1]
-        labels_b = torch.empty(batch, dtype=torch.int32, device=dev)
-        host = torch.empty(2, dtype=torch.float64).pin_memory()
-        step, any_zero = -1, True          # counts start at zero: the first step always reassigns
-        for step in range(n_steps):
-            idx = torch.from_numpy(cdf.searchsorted(rs.random_sample(batch), side="right").astype(np.int64)).to(dev, non_blocking=True)
-            Xb = padded_rows(Xp[idx].contiguous())
-            # _random_reassign (:2039-2053): every 10 * n_clusters samples, or as soon as a centre has no weight
-            n_since += batch
-            inertia_dev = self._labels_inertia(Xb, centers, labels_b)
-            _lib.call("gdr_minibatch_update", batch, K, D, ptr(Xb), Xb.stride(0), ptr(labels_b), ptr(centers), centers.stride(0),
-                      ptr(centers_new), centers_new.stride(0), ptr(counts), stream())
-            # the reassignment decision looks at the counts BEFORE this step's update in sklearn (the flag is an argument
-            # of _mini_batch_step), so it is taken from the previous step's read-back
-            reassign = any_zero or n_since >= 10 * K
-            if reassign:
-                n_since = 0
-                if self.reassignment_ratio > 0:
-                    to_re = counts < float(self.reassignment_ratio) * counts.max()
-                    n_re = int(to_re.sum().item())
-                    if n_re > 0.5 * batch:
-                        keep = torch.argsort(counts)[int(0.5 * batch):]
-                        to_re[keep] = False
-                        n_re = int(to_re.sum().item())
-                    if n_re:
-                        picks = torch.from_numpy(np.asarray(rs.choice(batch, replace=False, size=n_re), dtype=np.int64)).to(dev)
-                        centers_new[to_re] = Xb[picks]
-                    if n_re and n_re < K:
-                        counts[to_re] = counts[~to_re].min()
-            host[0:1].copy_(inertia_dev, non_blocking=True)
-            host[1:2].copy_((counts == 0).any().to(torch.float64).reshape(1), non_blocking=True)
-            csd = float(((centers_new - centers) ** 2).sum().item()) if tol_abs > 0 else 0.0
-            centers, centers_new = centers_new, centers
-            torch.cuda.current_stream().synchronize()
-            any_zero = bool(host[1] > 0)
-            # _mini_batch_convergence (:1974-2037)
-            b_inertia = float(host[0]) / batch
-            if step == 0:
-                continue
-            if ewa is None:
-                ewa = b_inertia
-            else:
-                alpha = min(batch * 2.0 / (N + 1), 1.0)
-                ewa = ewa * (1 - alpha) + b_inertia * alpha
-            if self.verbose:
-                print(f"Minibatch step {step + 1}/{n_steps}: mean batch inertia: {b_inertia}, ewa inertia: {ewa}")
-            if tol_abs > 0.0 and csd <= tol_abs:
-                break
-            if ewa_min is None or ewa < ewa_min:
-                no_improvement, ewa_min = 0, ewa
-            else:
-                no_improvement += 1
-            if self.max_no_improvement is not None and no_improvement >= self.max_no_improvement:
-                break
-        self.n_steps_ = step + 1
-        self.n_iter_ = int(np.ceil(((step + 1) * batch) / N))
+        centers, ewa = minibatch_loop(self, N, D, dev, rs, rows, assemble, var_mean)
         self._centers_dev = centers
         self.n_features_in_ = D
         self.cluster_centers_ = self._out(centers.contiguous() if pad4(D) == D else centers.clone().contiguous())
@@ -560,6 +483,110 @@ class MiniBatchKMeans(KMeans):
         else:
             self.inertia_ = (ewa if ewa is not None else 0.0) * N
         return self
+
+
+def minibatch_loop(est: MiniBatchKMeans, N: int, D: int, dev, rs, rows, assemble, var_mean):
+    """The body of ``MiniBatchKMeans.fit`` between the argument checks and the final E-step, shared by the one-GPU
+    estimator and ``parallel.DistMiniBatchKMeans``.  Every host draw, the EWA / early-stop logic, the centre update and
+    the reassignment are here and run on replicated data; the rows of X enter through three seams:
+      rows(idx)                      padded rows ``idx`` (numpy int64) of X, or X itself for ``idx`` None;
+      assemble(idx, centers, labels) the padded batch rows X[idx], with ``labels[j]`` = the exact-fp32 label
+                                     (precision_mode 0) of row j against ``centers``;
+      var_mean()                     the mean of X's column variances (only called for tol > 0).
+    Sets ``est.n_steps_`` and ``est.n_iter_``; returns (centres [K, D] padded, smoothed batch inertia or None)."""
+    K = int(est.n_clusters)
+    batch = min(int(est.batch_size), N)
+    init_size = est.init_size
+    if init_size is None:
+        init_size = 3 * batch
+        if init_size < K:
+            init_size = 3 * K
+    elif init_size < K:
+        init_size = 3 * K
+    init_size = min(int(init_size), N)
+    init_is_array = not isinstance(est.init, str)
+    n_init = est.n_init
+    if n_init == "auto":
+        n_init = 1 if (init_is_array or est.init == "k-means++") else 3
+    if init_is_array:
+        n_init = 1
+    tol_abs = 0.0
+    if est.tol > 0:       # _tolerance (:285-293): mean of the column variances * tol
+        tol_abs = var_mean() * float(est.tol)
+
+    # validation set for the initialisation (:2110-2112)
+    X_valid = rows(rs.randint(0, N, init_size).astype(np.int64))
+    lab_valid = torch.empty(X_valid.shape[0], dtype=torch.int32, device=dev)
+    best_inertia, centers = None, None
+    for _ in range(int(n_init)):
+        cand = est._mb_init(rows, N, D, dev, rs, init_size)
+        inertia = float(est._labels_inertia(X_valid, cand, lab_valid).item())
+        if best_inertia is None or inertia < best_inertia:
+            centers, best_inertia = cand, inertia
+    centers_new = new_padded(K, D, dev, zero=True)
+    counts = torch.zeros(K, dtype=torch.float32, device=dev)
+    ewa, ewa_min, no_improvement, n_since = None, None, 0, 0
+    n_steps = (int(est.max_iter) * N) // batch
+    # RandomState.choice(n, size, p=w / w.sum(), replace=True): cdf = p.cumsum(); cdf /= cdf[-1];
+    # cdf.searchsorted(random_sample(size), side="right") — the same table, built once
+    w32 = np.ones(N, dtype=np.float32)
+    cdf = (w32 / np.sum(w32)).astype(np.float64).cumsum()
+    cdf /= cdf[-1]
+    labels_b = torch.empty(batch, dtype=torch.int32, device=dev)
+    host = torch.empty(2, dtype=torch.float64).pin_memory()
+    step, any_zero = -1, True          # counts start at zero: the first step always reassigns
+    for step in range(n_steps):
+        Xb = assemble(cdf.searchsorted(rs.random_sample(batch), side="right").astype(np.int64), centers, labels_b)
+        # _random_reassign (:2039-2053): every 10 * n_clusters samples, or as soon as a centre has no weight
+        n_since += batch
+        inertia_dev = est._inertia(Xb, centers, labels_b)
+        _lib.call("gdr_minibatch_update", batch, K, D, ptr(Xb), Xb.stride(0), ptr(labels_b), ptr(centers), centers.stride(0),
+                  ptr(centers_new), centers_new.stride(0), ptr(counts), stream())
+        # the reassignment decision looks at the counts BEFORE this step's update in sklearn (the flag is an argument
+        # of _mini_batch_step), so it is taken from the previous step's read-back
+        reassign = any_zero or n_since >= 10 * K
+        if reassign:
+            n_since = 0
+            if est.reassignment_ratio > 0:
+                to_re = counts < float(est.reassignment_ratio) * counts.max()
+                n_re = int(to_re.sum().item())
+                if n_re > 0.5 * batch:
+                    keep = torch.argsort(counts)[int(0.5 * batch):]
+                    to_re[keep] = False
+                    n_re = int(to_re.sum().item())
+                if n_re:
+                    picks = torch.from_numpy(np.asarray(rs.choice(batch, replace=False, size=n_re), dtype=np.int64)).to(dev)
+                    centers_new[to_re] = Xb[picks]
+                if n_re and n_re < K:
+                    counts[to_re] = counts[~to_re].min()
+        host[0:1].copy_(inertia_dev, non_blocking=True)
+        host[1:2].copy_((counts == 0).any().to(torch.float64).reshape(1), non_blocking=True)
+        csd = float(((centers_new - centers) ** 2).sum().item()) if tol_abs > 0 else 0.0
+        centers, centers_new = centers_new, centers
+        torch.cuda.current_stream().synchronize()
+        any_zero = bool(host[1] > 0)
+        # _mini_batch_convergence (:1974-2037)
+        b_inertia = float(host[0]) / batch
+        if step == 0:
+            continue
+        if ewa is None:
+            ewa = b_inertia
+        else:
+            alpha = min(batch * 2.0 / (N + 1), 1.0)
+            ewa = ewa * (1 - alpha) + b_inertia * alpha
+        if est.verbose:
+            print(f"Minibatch step {step + 1}/{n_steps}: mean batch inertia: {b_inertia}, ewa inertia: {ewa}")
+        if tol_abs > 0.0 and csd <= tol_abs:
+            break
+        if ewa_min is None or ewa < ewa_min:
+            no_improvement, ewa_min = 0, ewa
+        else:
+            no_improvement += 1
+        if est.max_no_improvement is not None and no_improvement >= est.max_no_improvement:
+            break
+    est.n_steps_ = step + 1
+    est.n_iter_ = int(np.ceil(((step + 1) * batch) / N))
+    return centers, ewa
 
 
 def standard_scale(X: torch.Tensor) -> torch.Tensor:

@@ -31,6 +31,8 @@ from typing import Optional, Tuple
 import numpy as np
 import torch
 
+from .kmeans import MiniBatchKMeans
+
 
 @dataclass
 class RowPartition:
@@ -656,6 +658,29 @@ class CudaOps:
                        B.stride(0) if n_local else r, self.ptr(C), r, self.ptr(ws), ws.numel(), self.stream())
         return C
 
+    def minibatch_batch(self, comm, idx, row_off, X, C, Xb, labels_b):
+        """Rows ``idx`` (numpy int64, the same on every rank) of the row-partitioned X into Xb on every rank, with their
+        exact-fp32 labels against C when C is given (gdr_minibatch_batch_dist; a per-step collective)."""
+        import ctypes
+        m = int(idx.shape[0])
+        n_local, D = X.shape
+        K = int(C.shape[0]) if C is not None else 0
+        dev = Xb.device
+        order, counts = batch_plan(idx, row_off)
+        idx_d = torch.from_numpy(idx).to(dev, non_blocking=True)
+        order_d = torch.from_numpy(order).to(dev, non_blocking=True)
+        key = (m, K, D)
+        if getattr(self, "_mb_ws", (None,))[0] != key:
+            self._mb_ws = (key, self.workspace(self._lib.query("gdr_minibatch_batch_dist_ws_bytes", m, K, D, comm.world), dev))
+        ws = self._mb_ws[1]
+        cnt = (ctypes.c_int64 * comm.world)(*[int(c) for c in counts])
+        self._lib.call("gdr_minibatch_batch_dist", comm.lib_handle(), m, self.ptr(idx_d), self.ptr(order_d),
+                       ctypes.addressof(cnt), int(row_off[comm.rank]), n_local, K, D, self.ptr(X) if n_local else 0,
+                       X.stride(0) if n_local else self._pad4(D), self.ptr(C), C.stride(0) if C is not None else 0,
+                       self.ptr(Xb), Xb.stride(0), self.ptr(labels_b) if C is not None else 0, self.ptr(ws), ws.numel(),
+                       self.stream())
+        return Xb
+
     def inertia(self, Xc, C, labels):
         out = torch.zeros(1, dtype=torch.float64, device=C.device)
         if Xc.shape[0] == 0:
@@ -1266,6 +1291,180 @@ class DistKMeans:
             counts[old] -= 1
 
 
+def batch_plan(idx, row_off) -> Tuple[np.ndarray, np.ndarray]:
+    """The host half of gdr_minibatch_batch_dist: ``order`` (int32) lists the batch positions of ``idx`` (global row
+    ids) grouped by owning rank — rank order, ascending within a rank — and ``counts`` (int64 [world]) how many each
+    rank owns.  ``row_off`` [world + 1] are the ranks' first global rows and the total (empty ranks repeat an offset).
+    Pure numpy and stable, so every rank derives the same plan from the same draws."""
+    idx = np.asarray(idx, dtype=np.int64)
+    row_off = np.asarray(row_off, dtype=np.int64)
+    world = row_off.shape[0] - 1
+    if idx.size and (idx.min() < 0 or idx.max() >= row_off[-1]):
+        raise ValueError(f"batch_plan: row ids must lie in [0, {int(row_off[-1])})")
+    owner = np.searchsorted(row_off, idx, side="right") - 1
+    order = np.argsort(owner, kind="stable").astype(np.int32)
+    return order, np.bincount(owner, minlength=world).astype(np.int64)
+
+
+def random_state_digest(rs: np.random.RandomState) -> int:
+    """64-bit digest of a RandomState's whole state (equal states, equal digests), as a signed integer."""
+    import hashlib
+    name, keys, pos, has_gauss, cached = rs.get_state()
+    h = hashlib.blake2b(digest_size=8)
+    h.update(str(name).encode())
+    h.update(np.ascontiguousarray(keys, dtype=np.uint32).tobytes())
+    h.update(np.array([pos, has_gauss], dtype=np.int64).tobytes())
+    h.update(np.float64(cached).tobytes())
+    return int.from_bytes(h.digest(), "little", signed=True)
+
+
+def _array_digest(a) -> int:
+    import hashlib
+    arr = np.ascontiguousarray(a.detach().cpu().numpy() if isinstance(a, torch.Tensor) else np.asarray(a), dtype=np.float32)
+    h = hashlib.blake2b(digest_size=8)
+    h.update(np.array(arr.shape, dtype=np.int64).tobytes())
+    h.update(arr.tobytes())
+    return int.from_bytes(h.digest(), "little", signed=True)
+
+
+def _f64_bits(v) -> int:
+    return int(np.float64(v).view(np.int64))
+
+
+def _agree_on_entry(comm: Comm, device, what: str, err: Optional[Exception], n_local: int, *vals) -> np.ndarray:
+    """The entry agreement of a row-partitioned fit: ONE all-gather of [verdict, n_local, vals...].  A rank whose own
+    arguments were rejected raises its error, every other rank ValueError; so do all ranks when the vals differ.
+    Returns the row offsets [world + 1] (the blocks in rank order)."""
+    mine = torch.tensor([0 if err is None else 1, int(n_local)] + [int(v) for v in vals], dtype=torch.int64, device=device)
+    allv = torch.empty(comm.world * mine.numel(), dtype=torch.int64, device=device)
+    comm.all_gather_rows(mine, allv)
+    allv = allv.view(comm.world, -1).cpu().numpy()
+    if err is not None:
+        raise err
+    if allv[:, 0].any():
+        raise ValueError(f"{what}: rank {int(np.nonzero(allv[:, 0])[0][0])} rejected its arguments")
+    if not (allv[:, 2:] == allv[comm.rank, 2:]).all():
+        raise ValueError(f"{what}: the ranks passed different arguments")
+    return np.concatenate([[0], np.cumsum(allv[:, 1])]).astype(np.int64)
+
+
+class DistMiniBatchKMeans(MiniBatchKMeans):
+    """``MiniBatchKMeans`` on row-partitioned X: the one-GPU bytes for any number of ranks.
+
+    Same constructor as ``MiniBatchKMeans`` plus ``comm`` and ``ops``; ``fit(X_local)`` takes this rank's contiguous row
+    block (the blocks in rank order are X; any sizes, empty ones included).  The step loop is ``kmeans.minibatch_loop``,
+    run on every rank with the same host draws: each batch (and the validation and init subsets) is assembled on every
+    rank by gdr_minibatch_batch_dist — the owners pack and label their rows, one grouped exchange — and the centre update,
+    the batch inertia and the reassignment then run replicated on identical data.  The init-subset k-means++ runs
+    replicated.  The final E-step labels this rank's rows with the one-GPU kernel choice; its fp64 inertia is summed over
+    the ranks.
+
+    Collective.  At entry one all-gather checks N, K, D, batch_size, max_iter, max_no_improvement, init_size, n_init,
+    the bits of tol and reassignment_ratio, compute_labels, the init kind, a digest of the RandomState and of an array
+    init; a mismatch raises ValueError on every rank.  A string init needs ``random_state``.
+
+    With tol = 0 the centres, every rank's labels (its slice of the one-GPU labels), n_steps_ and n_iter_ equal the
+    one-GPU fit's; inertia_ is equal at one rank and within fp64 rounding of the rank grouping otherwise.  With tol > 0
+    the tolerance comes from rank-grouped fp64 column sums.  Results: ``labels_`` int32 on the device (this rank's
+    rows); ``cluster_centers_`` [K, D] on the device, ``inertia_``, ``n_iter_``, ``n_steps_`` replicated."""
+
+    def __init__(self, n_clusters=8, *, init="k-means++", max_iter=100, batch_size=1024, verbose=0, compute_labels=True,
+                 random_state=None, tol=0.0, max_no_improvement=10, init_size=None, n_init="auto",
+                 reassignment_ratio=0.01, precision="auto", device=None, comm: Comm = None, ops=None):
+        super().__init__(n_clusters=n_clusters, init=init, max_iter=max_iter, batch_size=batch_size, verbose=verbose,
+                         compute_labels=compute_labels, random_state=random_state, tol=tol,
+                         max_no_improvement=max_no_improvement, init_size=init_size, n_init=n_init,
+                         reassignment_ratio=reassignment_ratio, precision=precision, device=device)
+        self.comm = comm or Comm()
+        self.ops = ops or CudaOps()
+
+    def _entry_values(self, D: int):
+        """(local error or None, the values every rank must pass alike)."""
+        from .kmeans import _check_random_state
+        err, kind, init_digest, rs_digest = None, 0, 0, 0
+        try:
+            self._mode(D)
+            if isinstance(self.init, str):
+                if self.init not in ("k-means++", "random"):
+                    raise ValueError(f"init should be 'k-means++', 'random' or an array, got {self.init!r}")
+                if self.random_state is None:
+                    raise ValueError("a string init needs the same random_state on every rank")
+                kind = 1 if self.init == "k-means++" else 2
+            else:
+                shape = tuple(self.init.shape) if isinstance(self.init, torch.Tensor) else np.shape(self.init)
+                if tuple(shape) != (int(self.n_clusters), D):
+                    raise ValueError(f"The shape of the initial centers {tuple(shape)} does not match "
+                                     f"the number of clusters {self.n_clusters} / features {D}.")
+                init_digest = _array_digest(self.init)
+            if self.n_init != "auto" and int(self.n_init) <= 0:
+                raise ValueError(f"n_init should be > 0, got {self.n_init} instead.")
+            rs_digest = random_state_digest(_check_random_state(self.random_state))
+            opt = lambda v: -1 if v is None else int(v)       # noqa: E731
+            vals = (int(self.n_clusters), D, int(self.batch_size), int(self.max_iter), opt(self.max_no_improvement),
+                    opt(self.init_size), -1 if self.n_init == "auto" else int(self.n_init), _f64_bits(self.tol),
+                    _f64_bits(self.reassignment_ratio), int(bool(self.compute_labels)), kind, init_digest, rs_digest)
+        except (ValueError, TypeError) as e:
+            err, vals = (e if isinstance(e, ValueError) else ValueError(str(e))), (0,) * 13
+        return err, vals
+
+    def fit(self, X_local: torch.Tensor, y=None, sample_weight=None):
+        from .kmeans import TcOperand, _check_random_state, minibatch_loop
+        from ._dev import new_padded, pad4
+        if sample_weight is not None:
+            raise NotImplementedError("sample_weight is not supported (the reference never passes it)")
+        ops, comm = self.ops, self.comm
+        if not hasattr(ops, "minibatch_batch"):
+            raise NotImplementedError(f"{type(ops).__name__} has no distributed mini-batch assembly")
+        if not isinstance(X_local, torch.Tensor) or not X_local.is_cuda or X_local.dim() != 2:
+            raise ValueError("X_local must be a 2-D CUDA tensor (this rank's rows)")
+        X = ops.prep_rows(X_local)
+        n_local, D = X.shape
+        dev = X.device
+        err, vals = self._entry_values(D)
+        row_off = _agree_on_entry(comm, dev, "DistMiniBatchKMeans.fit", err, n_local, *vals)
+        N = int(row_off[-1])
+        self._check_fit_args(N)          # depends on agreed values only: raises on every rank alike
+        rs = _check_random_state(self.random_state)
+        bufs = {}
+
+        def rows(idx):
+            idx = np.arange(N, dtype=np.int64) if idx is None else idx
+            out = new_padded(idx.shape[0], D, dev, zero=True)
+            return ops.minibatch_batch(comm, idx, row_off, X, None, out, None)
+
+        def assemble(idx, C, labels_b):
+            if "Xb" not in bufs:
+                bufs["Xb"] = new_padded(idx.shape[0], D, dev, zero=True)
+            return ops.minibatch_batch(comm, idx, row_off, X, C, bufs["Xb"], labels_b)
+
+        def var_mean():
+            sums = ops.column_sums(X)
+            comm.all_reduce(sums)
+            m64 = sums[:D] / N
+            return float(((sums[D:] / N - m64 * m64).clamp_min(0)).mean().item())
+
+        centers, ewa = minibatch_loop(self, N, D, dev, rs, rows, assemble, var_mean)
+        self._numpy_io = False
+        self._centers_dev = centers
+        self.n_features_in_ = D
+        self.cluster_centers_ = centers.contiguous() if pad4(D) == D else centers.clone().contiguous()
+        if self.compute_labels:
+            mode = self._mode(D)
+            labels = torch.empty(n_local, dtype=torch.int32, device=dev)
+            if n_local:
+                tc = TcOperand(X) if mode == 1 else None
+                inertia = self._labels_inertia(X, centers, labels, mode=mode, tc=tc)
+            else:
+                inertia = torch.zeros(1, dtype=torch.float64, device=dev)
+            comm.all_reduce(inertia)
+            self.inertia_ = float(inertia.item())
+            self._labels_dev = labels
+            self.labels_ = labels
+        else:
+            self.inertia_ = (ewa if ewa is not None else 0.0) * N
+        return self
+
+
 # ------------------------------------------------------------------------------------------
 # edge sparsification (between stages 3 and 4)
 # ------------------------------------------------------------------------------------------
@@ -1605,6 +1804,28 @@ def dist_standard_scale(comm: Comm, x_local: torch.Tensor, ops=None):
     bound = N * eps * var + (N * mean64 * eps) ** 2
     scale = torch.where(var <= bound, torch.ones_like(var), var.sqrt())
     return ops.standardize_apply(X, mean64.to(torch.float32).contiguous(), scale.to(torch.float32).contiguous())
+
+
+def dist_kmeans_cluster(comm: Comm, part: RowPartition, X_local: torch.Tensor, n_clusters: int, seed: int,
+                        minibatch: bool = True, batch_size: int = 2048, init="k-means++", ops=None):
+    """kmeans.kmeans_cluster (distill_recsys.py:158-181) on a row partition: z-scores the columns
+    (dist_standard_scale), then clusters with DistMiniBatchKMeans(n_clusters, random_state=seed, batch_size) when
+    ``minibatch`` and more than 20 000 rows, else DistKMeans(init, random_state=seed) — the reference's rule (:173-178).
+    K is capped to the global row count ``part.n``.  Collective.  Returns (this rank's labels int64, the centres
+    [K, D] f32, the same on every rank), both on the device."""
+    if n_clusters <= 0:
+        raise ValueError("n_clusters must be > 0")
+    N = int(part.n)
+    K = max(1, min(int(n_clusters), N))
+    ops = ops or CudaOps()
+    Xs = dist_standard_scale(comm, X_local, ops=ops)
+    if minibatch and N > 20000:
+        km = DistMiniBatchKMeans(n_clusters=K, random_state=seed, batch_size=batch_size, n_init="auto", init=init,
+                                 comm=comm, ops=ops)
+    else:
+        km = DistKMeans(K, init, random_state=seed, comm=comm, ops=ops)
+    km.fit(Xs)
+    return km.labels_.to(torch.int64), km.cluster_centers_
 
 
 def dist_build_condensed_bipartite(comm: Comm, part_u: RowPartition, part_i: RowPartition, u_slice: torch.Tensor,

@@ -526,6 +526,25 @@ int gdr_allreduce_f64(gdr_comm_t* comm, double* buf, int64_t n, int op_max, gdr_
 int gdr_alltoallv(gdr_comm_t* comm, const void* send, const int64_t* send_off_host, const int64_t* send_cnt_host,
                   void* recv, const int64_t* recv_off_host, const int64_t* recv_cnt_host, int64_t elem_bytes,
                   gdr_stream_t stream);
+/* One MiniBatchKMeans batch on a row partition (sklearn/_kmeans.py:2154-2166 behind distill_recsys.py:174-176): every
+ * rank ends with Xb[j][0..ldb) = the bytes of global row idx[j] (columns D..ldb zero) and, when C != NULL,
+ * labels_b[j] = that row's label against C with the bits of gdr_kmeans_assign(precision_mode = 0).  C == NULL
+ * assembles the rows only (labels_b is then ignored).  Device arrays: idx[m] (global row ids, the same on every rank,
+ * duplicates allowed), order[m] (the batch positions grouped by owning rank: rank order, ascending within a rank).
+ * counts_host[world] = positions each rank owns (sum m).  Every rank derives idx, order and counts from the same host
+ * draws and row offsets, so nothing about them is exchanged; X_local holds global rows [row_lo, row_lo + n_local).
+ * Steps: the owned rows are packed into a compact buffer in batch order, labelled there by k_row_sqnorm +
+ * k_assign_simt (each row tile scans all K, so a row's label does not depend on which rows share the launch), sent to
+ * every rank in ONE group of NCCL sends / receives (none at world 1) and placed at their positions.
+ * COLLECTIVE, but a per-step exchange like gdr_alltoallv: no collective entry check and no stream synchronisation.
+ * The caller agrees on every argument once (DistMiniBatchKMeans does so at fit entry); every check here is local and
+ * precedes the exchange, and the workspace size depends only on agreed values (m, K, D), so a workspace rejection is
+ * the same on every rank.  The world argument of the size query is unused. */
+int64_t gdr_minibatch_batch_dist_ws_bytes(int64_t m, int64_t K, int64_t D, int world);
+int     gdr_minibatch_batch_dist(gdr_comm_t* comm, int64_t m, const int64_t* idx, const int32_t* order,
+                                 const int64_t* counts_host, int64_t row_lo, int64_t n_local, int64_t K, int64_t D,
+                                 const float* X_local, int64_t ldx, const float* C, int64_t ldc, float* Xb, int64_t ldb,
+                                 int32_t* labels_b, void* ws, int64_t ws_bytes, gdr_stream_t stream);
 /* Symmetric buffers: the same device allocation on every rank, mapped into every peer over NVLink (CUDA IPC), so that a
  * kernel can store straight into the other GPUs' copies.  gdr_symm_create / _destroy are collective (and, with
  * gdr_comm_init's entry-check buffer, the only entry points of this library that allocate device memory).
