@@ -93,6 +93,8 @@ _SIGNATURES = {
     "gdr_segment_sum_ws_bytes": (i64, [i64, i64, i64]),
     "gdr_segment_sum": (i32, [i64, i64, i64, vp, i64, vp, vp, i64, vp, vp, i64, vp]),
     "gdr_label_histogram": (i32, [i64, i64, vp, vp, vp, vp]),
+    "gdr_segment_sum_dist_ws_bytes": (i64, [i64, i64, i64]),
+    "gdr_segment_sum_dist": (i32, [vp, i64, i64, i64, i64, vp, i64, vp, vp, i64, vp, vp, i64, vp]),
     "gdr_kmeans_finalize": (i32, [i64, i64, vp, i64, vp, vp, i64, vp, i64, vp, i32, vp]),
     "gdr_kmeans_relocate_ws_bytes": (i64, [i64, i64, i64]),
     "gdr_kmeans_relocate": (i32, [i64, i64, i64, vp, i64, vp, i64, vp, vp, i64, vp, vp, i64, vp]),

@@ -393,6 +393,9 @@ int launch_assign_simt_rows(int64_t max_rows, int64_t K, int64_t D, const float*
 // in flight), then thread c adds column c of the staged rows IN ASCENDING ROW ORDER — one fp32
 // chain per output element, exactly np.add.at / single-thread sklearn order — so the loads are
 // parallel while the summation order stays sequential (bit-identical to the oracle).
+// kCarry: each chain starts from sums[k][c] (the value at which the previous rank of a row partition ended it) instead
+// of +0.0 and the result is written back in place; a CTA reads and writes only its own cluster's row.
+template <bool kCarry>
 __global__ void __launch_bounds__(256) k_gather_sum(int64_t K, int Dp4, int R,
                                                     const int32_t* __restrict__ mptr,
                                                     const uint32_t* __restrict__ ids,
@@ -404,10 +407,13 @@ __global__ void __launch_bounds__(256) k_gather_sum(int64_t K, int Dp4, int R,
   const int F4 = Dp4 >> 2;
   constexpr int MAXC = 4;                            // columns per thread: Dp4 <= 1024 per pass
   for (int c0 = 0; c0 < Dp4; c0 += 256 * MAXC) {
+    const int w4 = min(F4 - (c0 >> 2), 64 * MAXC);   // float4 columns in this pass
     float acc[MAXC];
 #pragma unroll
-    for (int q = 0; q < MAXC; ++q) acc[q] = 0.f;
-    const int w4 = min(F4 - (c0 >> 2), 64 * MAXC);   // float4 columns in this pass
+    for (int q = 0; q < MAXC; ++q) {
+      const int c = threadIdx.x + 256 * q;
+      acc[q] = kCarry && c < 4 * w4 ? sums[k * lds + c0 + c] : 0.f;
+    }
     for (int i = b; i < e; i += R) {
       const int rc = min(R, e - i);
       for (int t = threadIdx.x; t < rc * w4; t += 256) {
@@ -974,6 +980,53 @@ int relocate_apply(int ne, const int32_t* order_dev, const int32_t* empties_dev,
   return GDR_OK;
 }
 
+// The membership lists of gdr_segment_sum: ids = the rows stably sorted by label, mptr[k] .. mptr[k + 1] = cluster k's
+// range of them (labels outside [0, K) fall outside every range).  Workspace layout: segment_members_carve.
+struct SegmentMembers {
+  uint64_t* keys;
+  uint32_t* ids;
+  int32_t* mptr;
+  void* sws;
+  int64_t sws_bytes, off;
+};
+
+SegmentMembers segment_members_carve(void* ws, int64_t N, int64_t K) {
+  Workspace W(ws, INT64_MAX);
+  SegmentMembers m;
+  m.keys = W.take<uint64_t>(N);
+  m.ids = W.take<uint32_t>(N);
+  m.mptr = W.take<int32_t>(K + 1);
+  m.sws_bytes = sort_pairs_ws_bytes(N);
+  m.sws = W.take<char>(m.sws_bytes);
+  m.off = W.off;
+  return m;
+}
+
+int segment_members(int64_t N, int64_t K, const int32_t* labels, const SegmentMembers& m, cudaStream_t s) {
+  unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(cdiv(N, 256), kSMs * 16));
+  if (N > 0) {
+    k_label_keys<<<grid, 256, 0, s>>>(N, labels, m.keys, m.ids);
+    GDR_LAUNCHED();
+    int bits = 1;
+    while ((1ll << bits) < K) ++bits;
+    int rc = sort_pairs(N, bits, m.keys, m.ids, m.sws, m.sws_bytes, s);
+    if (rc) return rc;
+  }
+  k_bounds_from_sorted<<<grid, 256, 0, s>>>(N, K, m.keys, m.mptr);
+  GDR_LAUNCHED();
+  return GDR_OK;
+}
+
+// k_gather_sum over the membership lists: R rows of Dp4 floats are staged per step (48 KB of shared memory)
+template <bool kCarry>
+void gather_sum(int64_t K, int64_t D, const SegmentMembers& m, const float* X, int64_t ldx, float* sums, int64_t lds,
+                cudaStream_t s) {
+  const int Dp4 = (int)align_up(D, 4);
+  const int R = (int)std::max<int64_t>(1, std::min<int64_t>(64, (48 * 1024) / ((int64_t)Dp4 * 4)));
+  ProfileScope prof(PROF_SPMM + 1, s);
+  k_gather_sum<kCarry><<<(unsigned)K, 256, (size_t)R * Dp4 * 4, s>>>(K, Dp4, R, m.mptr, m.ids, X, ldx, sums, lds);
+}
+
 }  // namespace gdr
 
 extern "C" {
@@ -1207,35 +1260,83 @@ int gdr_segment_sum(int64_t N, int64_t K, int64_t D, const float* X, int64_t ldx
     return GDR_EWORKSPACE;
   }
   cudaStream_t s = (cudaStream_t)stream;
-  Workspace W(ws, ws_bytes);
-  uint64_t* keys = W.take<uint64_t>(N);
-  uint32_t* ids = W.take<uint32_t>(N);
-  int32_t* mptr = W.take<int32_t>(K + 1);
-  int64_t sws_bytes = sort_pairs_ws_bytes(N);
-  void* sws = W.take<char>(sws_bytes);
-  unsigned grid = (unsigned)std::max<int64_t>(1, std::min<int64_t>(cdiv(N, 256), kSMs * 16));
-  if (N > 0) {
-    k_label_keys<<<grid, 256, 0, s>>>(N, labels, keys, ids);
-    GDR_LAUNCHED();
-    int bits = 1;
-    while ((1ll << bits) < K) ++bits;
-    int rc = sort_pairs(N, bits, keys, ids, sws, sws_bytes, s);
-    if (rc) return rc;
-  }
-  k_bounds_from_sorted<<<grid, 256, 0, s>>>(N, K, keys, mptr);
-  GDR_LAUNCHED();
+  const SegmentMembers m = segment_members_carve(ws, N, K);
+  if (int rc = segment_members(N, K, labels, m, s)) return rc;
   if (counts) {
-    k_counts_from_rowptr<<<(unsigned)cdiv(K, 256), 256, 0, s>>>(K, mptr, counts);
+    k_counts_from_rowptr<<<(unsigned)cdiv(K, 256), 256, 0, s>>>(K, m.mptr, counts);
     GDR_LAUNCHED();
   }
-  {
-    const int Dp4 = (int)align_up(D, 4);
-    const int R = (int)std::max<int64_t>(1, std::min<int64_t>(64, (48 * 1024) / ((int64_t)Dp4 * 4)));
-    ProfileScope prof(PROF_SPMM + 1, s);
-    k_gather_sum<<<(unsigned)K, 256, (size_t)R * Dp4 * 4, s>>>(K, Dp4, R, mptr, ids, X, ldx, sums, lds);
-  }
+  gather_sum<false>(K, D, m, X, ldx, sums, lds, s);
   GDR_LAUNCHED();
   return GDR_OK;
+}
+
+int64_t gdr_segment_sum_dist_ws_bytes(int64_t n_local, int64_t K, int64_t D) {
+  (void)D;
+  return ws_need(1, 4) + segment_members_carve(nullptr, n_local, K).off;   // [label status | members]
+}
+
+int gdr_segment_sum_dist(gdr_comm_t* comm, int64_t row_lo, int64_t n_local, int64_t K, int64_t D, const float* X,
+                         int64_t ldx, const int32_t* labels, float* sums, int64_t lds, int32_t* counts, void* ws,
+                         int64_t ws_bytes, gdr_stream_t stream) {
+  GDR_CHECK_ARG(comm, "segment_sum_dist: null communicator");
+  const int world = comm->world, rank = comm->rank;
+  cudaStream_t s = (cudaStream_t)stream;
+  // local checks are decided collectively in comm_entry_check: an early return would leave the others in a collective
+  int local_rc = GDR_OK;
+  if (!(row_lo >= 0 && n_local >= 0 && n_local < (1ll << 31) && K > 0 && K < (1ll << 31) && D > 0 && sums && counts &&
+        lds % 4 == 0 && lds >= align_up(D, 4) && ((uintptr_t)sums & 15) == 0 &&
+        (n_local == 0 || (X && labels && ldx % 4 == 0 && ldx >= align_up(D, 4) && ((uintptr_t)X & 15) == 0)))) {
+    set_error("segment_sum_dist: bad arguments (sizes, null pointer, or X/sums without 16B alignment and ld %% 4 == 0, "
+              "ld >= D rounded to 4)");
+    local_rc = GDR_EINVAL;
+  } else if (!ws || ws_bytes < gdr_segment_sum_dist_ws_bytes(n_local, K, D)) {
+    set_error("segment_sum_dist: workspace too small");
+    local_rc = GDR_EWORKSPACE;
+  }
+  if (local_rc == GDR_OK) {
+    // this rank's counts; a label outside [0, K) is this rank's GDR_ERANGE
+    int32_t* status = (int32_t*)ws;
+    int32_t bad = 0;
+    int rc = gdr_label_histogram(n_local, K, labels, counts, status, stream);
+    if (rc == GDR_OK && (cudaMemcpyAsync(&bad, status, 4, cudaMemcpyDeviceToHost, s) != cudaSuccess ||
+                         cudaStreamSynchronize(s) != cudaSuccess)) {
+      set_error("segment_sum_dist: read-back of the label check failed");
+      rc = GDR_ECUDA;
+    }
+    if (rc == GDR_OK && bad) {
+      set_error("segment_sum_dist: a label lies outside [0, %lld)", (long long)K);
+      rc = GDR_ERANGE;
+    }
+    local_rc = rc;
+  }
+  std::vector<int64_t> row_off((size_t)world + 1);
+  int rc = comm_entry_check(comm, s, "segment_sum_dist", local_rc, row_lo, n_local, -1, {K, D, lds}, "K, D or lds", 0,
+                            row_off.data());
+  if (rc != GDR_OK) return rc;
+  if (row_off[world] >= (1ll << 31)) {
+    set_error("segment_sum_dist: %lld rows in all, the counts need fewer than 2^31", (long long)row_off[world]);
+    return GDR_EINVAL;
+  }
+
+  // sort before the receive, so that the ranks sort concurrently
+  const SegmentMembers m = segment_members_carve((char*)ws + ws_need(1, 4), n_local, K);
+  if ((rc = segment_members(n_local, K, labels, m, s))) return rc;
+  // each chain of rank q continues where rank q - 1 ended it; rank 0 starts from +0.0, an empty rank hands on what it got
+  const int64_t bytes = K * lds * 4;
+  if (rank > 0) {
+    if ((rc = comm_recv(comm, sums, bytes, rank - 1, s))) return rc;
+  } else {
+    GDR_CUDA(cudaMemsetAsync(sums, 0, bytes, s));
+  }
+  if (n_local > 0) {
+    gather_sum<true>(K, D, m, X, ldx, sums, lds, s);
+    GDR_LAUNCHED();
+  }
+  if (rank + 1 < world && (rc = comm_send(comm, sums, bytes, rank + 1, s))) return rc;
+  // the last rank's sums are the result; the counts are exact int32 sums (fewer than 2^31 rows in all)
+  if ((rc = comm_broadcast(comm, sums, bytes, world - 1, s))) return rc;
+  return comm_allreduce_lloyd(comm, nullptr, 0, counts, K, s);
 }
 
 int gdr_kmeans_finalize(int64_t K, int64_t D, const float* sums, int64_t lds, const int32_t* counts,

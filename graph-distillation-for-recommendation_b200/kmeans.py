@@ -107,6 +107,20 @@ def segment_sum(X: torch.Tensor, labels: torch.Tensor, K: int, *, sums=None, cou
     return sums, counts
 
 
+def means_of_sums(sums: torch.Tensor, counts: torch.Tensor, empty_nan: bool) -> torch.Tensor:
+    """sums[c] / counts[c] from segment_sum's (sums, counts).  ``empty_nan``: gdr_kmeans_finalize in mean mode (fp32
+    division, an empty cluster gives a NaN row; a padded [K, D] view), else the division by counts.clamp_min(1) of
+    distill_recsys.py:635 (an empty segment gives a zero row)."""
+    if not empty_nan:
+        return sums / counts.clamp_min(1).unsqueeze(1).to(sums.dtype)
+    K, D = sums.shape
+    out = new_padded(K, D, sums.device)
+    stats = torch.zeros(2 + K, dtype=torch.float64, device=sums.device)
+    _lib.call("gdr_kmeans_finalize", K, D, ptr(sums), sums.stride(0), ptr(counts), 0, 0, ptr(out),
+              out.stride(0), ptr(stats), 1, stream())
+    return out
+
+
 def cluster_means(features: torch.Tensor, labels: torch.Tensor, n_clusters: int) -> torch.Tensor:
     """feat_syn[c] = mean(features[labels == c]); an empty cluster gives a NaN row.
 
@@ -114,13 +128,8 @@ def cluster_means(features: torch.Tensor, labels: torch.Tensor, n_clusters: int)
     (clustgdd_agent_induct.py:143-152)."""
     X = padded_rows(features.to(torch.float32))
     lab = labels.to(device=X.device, dtype=torch.int32).contiguous()
-    K, D = int(n_clusters), X.shape[1]
-    sums, counts = segment_sum(X, lab, K)
-    out = new_padded(K, D, X.device)
-    stats = torch.zeros(2 + K, dtype=torch.float64, device=X.device)
-    _lib.call("gdr_kmeans_finalize", K, D, ptr(sums), sums.stride(0), ptr(counts), 0, 0, ptr(out),
-              out.stride(0), ptr(stats), 1, stream())
-    return out
+    sums, counts = segment_sum(X, lab, int(n_clusters))
+    return means_of_sums(sums, counts, empty_nan=True)
 
 
 def segment_mean_pool(emb: torch.Tensor, assign: torch.Tensor, n_segments: int) -> torch.Tensor:
@@ -128,7 +137,7 @@ def segment_mean_pool(emb: torch.Tensor, assign: torch.Tensor, n_segments: int) 
     X = padded_rows(emb.to(torch.float32))
     lab = assign.to(device=X.device, dtype=torch.int32).contiguous()
     sums, counts = segment_sum(X, lab, int(n_segments))
-    return sums / counts.clamp_min(1).unsqueeze(1).to(sums.dtype)
+    return means_of_sums(sums, counts, empty_nan=False)
 
 
 class KMeans:

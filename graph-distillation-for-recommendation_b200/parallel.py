@@ -12,6 +12,8 @@ so nothing is ported here — the exchanges are the ones the algorithm needs:
   stage 3  per Lloyd iteration ONE all-reduce of the [K x D] partial sums and ONE of the
            packed int32 [counts | n_changed]; every rank finalises identically, so the
            replicated centres stay bit-identical across ranks;
+  means    the [K x D] per-cluster sums handed from rank to rank, each chain continued where the
+           previous rank ended it, then sent to all (dist_cluster_means: the one-GPU bytes);
   sparsify all-gather of the degree vector and the logits; per radix pass of the top-k one all-reduce
            of the per-rank histograms, then one all-gather of the tie counts (dist_graph_sparse);
   stage 4  all-gather of the labels, local segmented edge counting, dense n x n all-reduce of
@@ -657,6 +659,24 @@ class CudaOps:
                        self.ptr(A) if n_local else 0, A.stride(0) if n_local else p, self.ptr(B) if n_local else 0,
                        B.stride(0) if n_local else r, self.ptr(C), r, self.ptr(ws), ws.numel(), self.stream())
         return C
+
+    def segment_sum_dist(self, comm, row_lo, X, labels, K):
+        """segment_sum of the row-partitioned X (global rows row_lo .. row_lo + n_local) and int32 labels, replicated
+        with gdr_segment_sum's bits on the concatenated rows (gdr_segment_sum_dist; collective).  Returns (sums [K, D]
+        padded, counts int32 [K]).  A row count that differs between X and labels, or K <= 0, is this rank's rejection
+        inside the collective entry check, so every rank fails together."""
+        n_local, D = X.shape
+        dev = X.device
+        ok = labels.shape == (n_local,) and K > 0
+        Kb = max(int(K), 1)
+        sums = self.new_padded(Kb, D, dev, zero=True)
+        counts = torch.zeros(Kb, dtype=torch.int32, device=dev)
+        ws = self.workspace(self._lib.query("gdr_segment_sum_dist_ws_bytes", n_local, Kb, D), dev)
+        self._lib.call("gdr_segment_sum_dist", comm.lib_handle(), int(row_lo), n_local, int(K), D,
+                       self.ptr(X) if n_local else 0, X.stride(0) if n_local else sums.stride(0),
+                       self.ptr(labels) if n_local and ok else 0, self.ptr(sums), sums.stride(0), self.ptr(counts),
+                       self.ptr(ws), ws.numel(), self.stream())
+        return sums, counts
 
     def minibatch_batch(self, comm, idx, row_off, X, C, Xb, labels_b):
         """Rows ``idx`` (numpy int64, the same on every rank) of the row-partitioned X into Xb on every rank, with their
@@ -1826,6 +1846,52 @@ def dist_kmeans_cluster(comm: Comm, part: RowPartition, X_local: torch.Tensor, n
         km = DistKMeans(K, init, random_state=seed, comm=comm, ops=ops)
     km.fit(Xs)
     return km.labels_.to(torch.int64), km.cluster_centers_
+
+
+def dist_segment_sum(comm: Comm, part: RowPartition, X_local: torch.Tensor, labels_local: torch.Tensor, K: int, ops=None):
+    """kmeans.segment_sum on a row partition: X_local [part.n_local, F] and labels_local [part.n_local] (int32 or int64)
+    are this rank's rows of the features and labels, e.g. dist_propagate's padded blocks and DistKMeans.labels_ /
+    dist_kmeans_cluster's labels.  Nothing is gathered: each fp32 chain runs over rank 0's members of its cluster, then
+    continues on rank 1 from the value rank 0 ended it at, and so on (gdr_segment_sum_dist).  Collective.  Returns
+    (sums [K, F] padded, counts int32 [K]), the same on every rank and byte-equal to segment_sum of the rows
+    concatenated in rank order.  Raises ValueError on every rank when K <= 0, when the ranks pass different K or F, or
+    when a label lies outside [0, K); the communicator stays usable."""
+    from ._lib import GdrError
+    ops = ops or CudaOps()
+    if not hasattr(ops, "segment_sum_dist"):
+        raise NotImplementedError(f"{type(ops).__name__} has no distributed segment sum")
+    K = int(K)
+    X = ops.prep_rows(X_local)
+    lab = labels_local.to(X.device)
+    if lab.dtype != torch.int32:
+        lab = lab.clamp(-1, max(K, 0))      # out of int32 range stays out of [0, K) after the cast
+    lab = lab.to(torch.int32).contiguous()
+    try:
+        return ops.segment_sum_dist(comm, part.lo, X, lab, K)
+    except GdrError as e:
+        if e.code in (-1, -4):              # GDR_EINVAL, GDR_ERANGE: rejected on every rank by the entry check
+            raise ValueError(f"dist_segment_sum: {e}") from e
+        raise
+
+
+def dist_cluster_means(comm: Comm, part: RowPartition, features_local: torch.Tensor, labels_local: torch.Tensor,
+                       n_clusters: int, ops=None) -> torch.Tensor:
+    """kmeans.cluster_means (feat_syn, clustgdd_agent_transduct.py:116-127) of row-partitioned features and labels:
+    [K, F], the same on every rank and byte-equal to cluster_means of the rows concatenated in rank order, NaN rows of
+    empty clusters included.  Collective; the errors of dist_segment_sum."""
+    from .kmeans import means_of_sums
+    sums, counts = dist_segment_sum(comm, part, features_local, labels_local, n_clusters, ops=ops)
+    return means_of_sums(sums, counts, empty_nan=True)
+
+
+def dist_segment_mean_pool(comm: Comm, part: RowPartition, emb_local: torch.Tensor, assign_local: torch.Tensor,
+                           n_segments: int, ops=None) -> torch.Tensor:
+    """kmeans.segment_mean_pool (the teacher pooling of distill_recsys.py:623-636) of row-partitioned embeddings and
+    assignments (e.g. u2cu from dist_kmeans_cluster): [n_segments, F], the same on every rank and byte-equal to the
+    one-GPU pooling of the rows concatenated in rank order.  Collective; the errors of dist_segment_sum."""
+    from .kmeans import means_of_sums
+    sums, counts = dist_segment_sum(comm, part, emb_local, assign_local, n_segments, ops=ops)
+    return means_of_sums(sums, counts, empty_nan=False)
 
 
 def dist_build_condensed_bipartite(comm: Comm, part_u: RowPartition, part_i: RowPartition, u_slice: torch.Tensor,

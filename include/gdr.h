@@ -361,7 +361,8 @@ int     gdr_kmeans_plusplus(int64_t N, int64_t K, int64_t D, const float* X, int
  *             and the Python cluster-mean loop    clustgdd_agent_transduct.py:121-125
  *             and index_add_/bincount pooling     distill_recsys.py:628-636
  *   Deterministic: members of a cluster are summed in ascending row order, one
- *   fp32 chain per output element (== np.add.at order). */
+ *   fp32 chain per output element (== np.add.at order).  gdr_segment_sum_dist (with the
+ *   communicator calls below) gives the same bits on a row partition. */
 int64_t gdr_segment_sum_ws_bytes(int64_t N, int64_t K, int64_t D);
 int     gdr_segment_sum(int64_t N, int64_t K, int64_t D,
                         const float* X, int64_t ldx, const int32_t* labels,
@@ -498,7 +499,7 @@ int gdr_class_edge_weight(int64_t n, int64_t nnz, const int32_t* rowptr, const i
  * Protocol: rank 0 calls gdr_comm_unique_id, the host framework broadcasts the 128 bytes, every rank calls
  * gdr_comm_init (collective).  All exchange calls are collective and are enqueued on `stream`.
  * Collective entry check of the row-partitioned entry points (gdr_kmeans_plusplus_dist, gdr_dense_gram_dist,
- * gdr_sparsify_classes_dist): a rank does not return on its own argument checks.  Every rank all-gathers its verdict,
+ * gdr_sparsify_classes_dist, gdr_segment_sum_dist): a rank does not return on its own argument checks.  Every rank all-gathers its verdict,
  * its row block and the values every rank must pass alike (listed with each entry point) through a small buffer the
  * communicator owns (allocated by gdr_comm_init), reads them back and synchronises the stream once.  A rank whose own
  * arguments are rejected returns its own code (GDR_EINVAL, GDR_EWORKSPACE, GDR_EUNSUPPORTED, GDR_ERANGE), every other
@@ -545,6 +546,23 @@ int     gdr_minibatch_batch_dist(gdr_comm_t* comm, int64_t m, const int64_t* idx
                                  const int64_t* counts_host, int64_t row_lo, int64_t n_local, int64_t K, int64_t D,
                                  const float* X_local, int64_t ldx, const float* C, int64_t ldc, float* Xb, int64_t ldb,
                                  int32_t* labels_b, void* ws, int64_t ws_bytes, gdr_stream_t stream);
+/* gdr_segment_sum on a row partition (the cluster means of clustgdd_agent_transduct.py:116-127 and the pooling of
+ * distill_recsys.py:623-636 on row-partitioned features and labels).  COLLECTIVE over comm.  Each rank passes its rows
+ * X[n_local][ldx] and labels, global rows [row_lo, row_lo + n_local) (n_local = 0 allowed, X and labels may then be
+ * NULL).  sums[K][lds] and counts[K] come out on every rank with the bits gdr_segment_sum gives on the rows concatenated
+ * in rank order (columns [D, lds) zero).  gdr_segment_sum sums each element as one fp32 chain from +0.0 over the
+ * cluster's members in ascending row order, so cluster c's chain is rank 0's members, then rank 1's, and so on.
+ * Steps: this rank's counts (gdr_label_histogram; a label outside [0, K) is this rank's GDR_ERANGE, read back with a
+ * stream synchronisation); the collective entry check (see gdr_comm_init) on K, D and lds, with n_local < 2^31 per rank
+ * and fewer than 2^31 rows in all; this rank's stable sort by label (gdr_segment_sum's code and digit count), before it
+ * receives anything; then rank 0 zeroes sums and rank q > 0 receives K x lds floats from rank q - 1 into sums (NCCL
+ * point-to-point), continues every chain over its members from the received value, and sends sums to rank q + 1 (an
+ * empty rank hands on what it received).  The last rank's sums are sent to all, and the counts are all-reduced (exact
+ * int32 sums).  Synchronises the stream twice: the label read-back and the entry check. */
+int64_t gdr_segment_sum_dist_ws_bytes(int64_t n_local, int64_t K, int64_t D);
+int     gdr_segment_sum_dist(gdr_comm_t* comm, int64_t row_lo, int64_t n_local, int64_t K, int64_t D, const float* X,
+                             int64_t ldx, const int32_t* labels, float* sums, int64_t lds, int32_t* counts, void* ws,
+                             int64_t ws_bytes, gdr_stream_t stream);
 /* Symmetric buffers: the same device allocation on every rank, mapped into every peer over NVLink (CUDA IPC), so that a
  * kernel can store straight into the other GPUs' copies.  gdr_symm_create / _destroy are collective (and, with
  * gdr_comm_init's entry-check buffer, the only entry points of this library that allocate device memory).
